@@ -4,6 +4,7 @@ next to the reference's CPU path timed on the box's own host cores).
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one JSON line on rank 0)
   python bench.py --impl reference --gpus N ...             # the reference algorithm on the host cores (oracle port)
+  python bench.py ... --dump-outputs DIR                    # also write the last timed step's logits of every path as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of B=64 synthetic canonical windows per GPU
 (video (64,3,32,96,96) + log-mel (64,1,80,128); BASELINE.json configs[1]).  `value` is timed with the inputs already
@@ -255,9 +256,25 @@ def long_video_probe(pred, lb, ws, rank, dev, n_windows: int):
     ms = float(ms.item())
     lg = logits.cpu()
     del track
-    return {"windows": n_windows, "n_gpus": ws, "scaling": "strong", "ms": ms, "windows_per_s": n_windows / ms * 1e3,
-            "logits_sha256_16": hashlib.sha256(lg.numpy().tobytes()).hexdigest()[:16], "fake_votes": int((lg < 0).sum()),
-            "what": "uint8 track resident in HBM (rank-local span), windows built on the device, batches pipelined, one all-gather of fp32 logits"}
+    rec = {"windows": n_windows, "n_gpus": ws, "scaling": "strong", "ms": ms, "windows_per_s": n_windows / ms * 1e3,
+           "logits_sha256_16": hashlib.sha256(lg.numpy().tobytes()).hexdigest()[:16], "fake_votes": int((lg < 0).sum()),
+           "what": "uint8 track resident in HBM (rank-local span), windows built on the device, batches pipelined, one all-gather of fp32 logits"}
+    return rec, lg
+
+
+DUMP_MAX_ELEMS = 4 << 20     # 16 MB of float32 per array: the dump of a run stays below 64 MB in all
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each flattened array as `out_dir/<name>.npy` in float32.  An array longer than DUMP_MAX_ELEMS (only config5's
+    logits, at a large --config5-windows) is stored as every k-th element, the smallest k that fits: a fixed sample, so two
+    runs with the same arguments store the same windows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().to("cpu", torch.float32).reshape(-1)
+        a = a[::-(-a.numel() // DUMP_MAX_ELEMS)] if a.numel() > DUMP_MAX_ELEMS else a
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def _claim_stdout():
@@ -282,8 +299,13 @@ def main():
     ap.add_argument("--no-eager-gpu", action="store_true")
     ap.add_argument("--no-config5", action="store_true")
     ap.add_argument("--config5-windows", type=int, default=10000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the logits each timed path returned in its last step as DIR/<name>.npy "
+                         "(float32; rank 0) so that two builds can be compared output for output on the same seeded inputs")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
         return run_reference(args, out)
 
     import __graft_entry__ as ge
@@ -370,12 +392,13 @@ def main():
             model.profile_enable(2 if args.precision == 'bf16' else 1)
         n0 = model.launch_count()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        last = None
         e0.record()
         if whole:
-            fn(steps)
+            last = fn(steps)
         else:
             for _ in range(steps):
-                fn()
+                last = fn()
         if finalize is not None:
             finalize()
         e1.record()
@@ -394,7 +417,7 @@ def main():
             t = torch.tensor([ms], dtype=torch.float64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, launches, prof, sampler.result()
+        return ms, launches, prof, sampler.result(), last
 
     # uint8-track variant of the end-to-end path (SURVEY.md §8f-1): per step the host hands over the uint8 mouth-crop span of
     # the step's 64 windows (stride 8: 536 frames, 14.8 MB instead of 226 MB of fp32 windows) from pinned memory, the windows
@@ -431,16 +454,21 @@ def main():
         comp.synchronize()
         return host_out[-1]
 
-    ms, launches, prof, clocks = timed(step_resident, K, profile=True, finalize=gather_resident)
-    ms_e2e, _, _, _ = timed(run_e2e, K, whole=True)
-    ms_e2e_f32, _, _, _ = timed(lambda n: run_e2e(n, pred_f32), K, whole=True)
-    ms_trk, _, _, _ = timed(run_e2e_track, K, whole=True)
+    # outputs of the last timed step of every path (the `value`, `e2e*` and `config5` figures), for --dump-outputs
+    last_out = {}
+    ms, launches, prof, clocks, last_out["logits"] = timed(step_resident, K, profile=True, finalize=gather_resident)
+    if ws > 1:      # what every rank receives for the last step: the logits of all ranks
+        rows = local_logits.shape[0]
+        last_out["logits"] = gathered.view(ws, rows, B)[:, (step_no[0] - 1) % rows].clone()
+    ms_e2e, _, _, _, last_out["e2e_logits"] = timed(run_e2e, K, whole=True)
+    ms_e2e_f32, _, _, _, last_out["e2e_fp32_upload_logits"] = timed(lambda n: run_e2e(n, pred_f32), K, whole=True)
+    ms_trk, _, _, _, last_out["e2e_track_u8_logits"] = timed(run_e2e_track, K, whole=True)
     # sustained: the same resident step back to back for >= ~1.5 s (the K-step region above lasts ~60 ms: a burst figure, taken
     # before the 1000 W power cap pulls the SM clock down)
     k_sus = max(K, int(1500.0 / max(ms / K, 0.05)))
     if ws > 1:
         local_logits = torch.empty(1, B, dtype=torch.float32, device=dev)     # (the sustained run keeps only the last batch)
-    ms_sus, _, _, clocks_sus = timed(step_resident, k_sus)
+    ms_sus, _, _, clocks_sus, _ = timed(step_resident, k_sus)
     value = ws * B * K / (ms / 1e3)
     e2e = ws * B * K / (ms_e2e / 1e3)
     e2e_trk = ws * B * K / (ms_trk / 1e3)
@@ -452,7 +480,9 @@ def main():
     # BASELINE.json configs[4]: 10 000 sliding windows of one uint8 track, sharded over the ranks (strong scaling)
     c5 = None
     if not args.no_config5:
-        c5 = long_video_probe(pred, lb, ws, rank, dev, args.config5_windows)
+        c5, last_out["config5_logits"] = long_video_probe(pred, lb, ws, rank, dev, args.config5_windows)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_out)
 
     if rank == 0:
         peaks, peak_src = _peaks()

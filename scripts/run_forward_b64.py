@@ -1,5 +1,5 @@
 import sys, os, time
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import __graft_entry__ as ge; ge.build()
 import lipsync_b200 as lb
