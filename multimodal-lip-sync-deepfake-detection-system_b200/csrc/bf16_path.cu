@@ -12,9 +12,11 @@
 #include <cuda_fp16.h>
 
 #include <algorithm>
+#include <array>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 
 using namespace lsd;
 using namespace lsdfw;
@@ -193,6 +195,40 @@ struct Packer {
     while (w.size() % 64) w.push_back(0);
     h->blayers[name] = L;
   }
+  // The same 3x3x3 convolution (+ fused 1x1 downsample) for the folded small-map route (UcFoldSlice in umma_conv.cuh): the taps
+  // are packed in (kh, kw, kt) order, so the three temporal taps of one spatial tap — one band of a folded conv, A from the plane
+  // set of one input position — are one contiguous weight piece per K chunk.  Same bf16 values as the padded route's packing.
+  void add_fold(const std::string& name, const std::string& key, const std::string& ds_key, int ntile) {
+    const ConvP& c = h->convs.at(key);
+    if (c.kt != 3 || c.kh != 3 || c.kw != 3 || c.Cout % ntile) return;
+    BLayer L;
+    L.Cout = c.Cout;
+    L.ntile = ntile;
+    BGroup g;
+    g.Cin = c.Cin;
+    g.taps_total = 27;
+    g.k16 = c.Cin / 16;
+    for (int b = 0; b < 3; ++b)
+      for (int d = 0; d < 3; ++d) {
+        BBand band{b * 3 + d, {}};
+        for (int a = 0; a < 3; ++a) band.taps.push_back(BTap{(a * 3 + b) * 3 + d, a - 1, b - 1, d - 1});
+        g.bands.push_back(band);
+      }
+    pack_group(g, c, ntile);
+    L.groups.push_back(g);
+    L.bias_off = bias.size();
+    for (int i = 0; i < c.Cout; ++i) bias.push_back(f32[c.shift_off + i]);
+    if (!ds_key.empty()) {
+      const ConvP& d = h->convs.at(ds_key);
+      BGroup gd = make_group(d, 1, 1);
+      gd.src = 1;
+      pack_group(gd, d, ntile);
+      L.groups.push_back(gd);
+      for (int i = 0; i < c.Cout; ++i) bias[L.bias_off + i] += f32[d.shift_off + i];
+    }
+    while (w.size() % 64) w.push_back(0);
+    h->blayers[name] = L;
+  }
   // Split-bf16 ("bf16x3") layer for the token path: y = Ahi*Whi + Alo*Whi + Ahi*Wlo accumulated in one TMEM tile
   // (three K groups), which keeps ~16 mantissa bits of both operands; the dropped Alo*Wlo term is ~2^-16 relative.
   void add_split(const std::string& name, const std::string& key, int ntile) {
@@ -236,8 +272,17 @@ PBuf make_pbuf(int C, int sets, UcGeom g) {
   return b;
 }
 
+// Folded route (UcFoldSlice in umma_conv.cuh) for the residual stage whose output map is H x W: on small maps the padded layout
+// executes 49 positions per 36 (6x6) or 16 per 9 (3x3) and multiplies every tap, including those that only read padding.  Chosen
+// from the geometry alone (never from the batch); LSD_FOLD=0 keeps the padded route everywhere (reference for A/B runs).
+bool fold_route(int H, int W) {
+  static const bool off = LSD_ENV("LSD_FOLD") && atoi(LSD_ENV("LSD_FOLD")) == 0;
+  return !off && H * W <= 36;
+}
+
 struct BPlan {
   Shapes s;
+  bool fold3 = false, fold4 = false;      // layer3 / layer4 on the folded route
   Plan f32;                               // fp32 buffers (stage registry + bump allocator)
   std::map<std::string, PBuf> pb;
   size_t planar_begin = 0, planar_end = 0;
@@ -289,10 +334,14 @@ void build_plan(const Shapes& s, BPlan& P) {
   P.addp("l1a", 64, 1, g1);
   P.addp("y1", 64, 4, g2);       // parity-split: four half-resolution plane sets
   P.addp("l2a", 128, 1, g2);
-  P.addp("y2", 128, 4, g3);
-  P.addp("l3a", 256, 1, g3);
-  P.addp("y3", 256, 4, g4);
-  P.addp("l4a", 256, 1, g4);
+  // folded route (small maps): y2 / l3a / y3 / l4a hold one plane set per map position in the row geometry gr
+  P.fold3 = fold_route(s.H3, s.W3);
+  P.fold4 = fold_route(s.H4, s.W4);
+  const UcGeom gr = make_geom_ex(Bn, Tn, 1, 1, 1, 0, 0, 0, 0);
+  if (P.fold3) P.addp("y2", 128, s.H2 * s.W2, gr); else P.addp("y2", 128, 4, g3);
+  if (P.fold3) P.addp("l3a", 256, s.H3 * s.W3, gr); else P.addp("l3a", 256, 1, g3);
+  if (P.fold4) P.addp("y3", 256, s.H3 * s.W3, gr); else P.addp("y3", 256, 4, g4);
+  if (P.fold4) P.addp("l4a", 256, s.H4 * s.W4, gr); else P.addp("l4a", 256, 1, g4);
   P.addp("y4", 256, 1, g4);
   P.addp("art_a", 128, 1, g4);
   P.addp("art_b", 64, 1, g4);
@@ -367,6 +416,44 @@ struct UArgs {
   int res32_ld = 0;
 };
 
+// Stage program of a launch: expanded on the host by `build`, cached in device memory under a hash of the complete parameter block
+// (pointers, strides, geometry, tile shape, fold slices), so steady-state forwards only look it up.  Sets p.prog.
+// salt: what else the program depends on (folded convs: input map extents and set strides, which the parameter block does not hold)
+int stage_program(const BCtx& c, const std::string& name, UmmaConvP& p, const std::function<void(std::vector<UcStageDesc>&)>& build,
+                  std::initializer_list<uint64_t> salt = {}) {
+  uint64_t hkey = 1469598103934665603ull;
+  for (uint64_t v : salt) { hkey ^= v; hkey *= 1099511628211ull; hkey ^= hkey >> 29; }
+  static_assert(sizeof(UmmaConvP) % 8 == 0, "UmmaConvP is hashed in 8-byte words");
+  const uint64_t* pw = reinterpret_cast<const uint64_t*>(&p);   // (p was memset to 0 first: padding bytes are deterministic)
+  for (size_t i = 0; i < sizeof(p) / 8; ++i) { hkey ^= pw[i]; hkey *= 1099511628211ull; hkey ^= hkey >> 29; }
+  auto it = c.h->prog_cache.find(hkey);
+  if (it == c.h->prog_cache.end()) {
+    std::vector<UcStageDesc> host;
+    build(host);
+    const size_t bytes = host.size() * sizeof(UcStageDesc);
+    if (!c.h->prog_arena) {
+      c.h->prog_cap = 64u << 20;   // (a folded conv's slice programs are ~0.3 MB per shape and workspace)
+      if (cudaMalloc(&c.h->prog_arena, c.h->prog_cap) != cudaSuccess) return lsd_fail(c.h, LSD_ERR_CUDA, "stage-program arena allocation failed");
+      c.h->prog_cursor = 0;
+    }
+    if (c.h->prog_cursor + bytes > c.h->prog_cap) {   // arena full (many shapes / workspaces seen): start over once nothing is in flight
+      cudaDeviceSynchronize();
+      c.h->prog_cache.clear();
+      c.h->prog_cursor = 0;
+      ++c.h->generation;   // captured CUDA graphs hold addresses of the old programs
+    }
+    char* dst = c.h->prog_arena + c.h->prog_cursor;
+    // Cache miss only (first forward of a shape): a blocking copy, so the program is visible to every stream that later
+    // launches this layer (the cache is shared by the main, side, tail and helper streams).
+    cudaError_t e = cudaMemcpy(dst, host.data(), bytes, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) return lsd_fail(c.h, LSD_ERR_CUDA, "%s: stage program upload: %s", name.c_str(), cudaGetErrorString(e));
+    c.h->prog_cursor += (bytes + 255) & ~size_t(255);
+    it = c.h->prog_cache.emplace(hkey, dst).first;
+  }
+  p.prog = reinterpret_cast<const UcStageDesc*>(it->second);
+  return 0;
+}
+
 // One launch of the tcgen05 kernel for layer `name`.
 int run_umma(const BCtx& c, const std::string& name, const UArgs& a) {
   const BLayer& L = c.h->blayers.at(name);
@@ -387,6 +474,7 @@ int run_umma(const BCtx& c, const std::string& name, const UArgs& a) {
     p.y = c.org(*a.yp) + (int64_t)a.y_plane_off * a.yp->plane_stride;
     p.y_plane_stride = a.yp->plane_stride; p.y_set_stride = a.yp->set_stride;
     p.g2 = a.yp->g;
+    p.ymap_W = og.W;
     if (a.yp_lo) p.ylo = c.org(*a.yp_lo) + (int64_t)a.y_plane_off * a.yp_lo->plane_stride;
   }
   if (a.y32) {
@@ -518,39 +606,8 @@ int run_umma(const BCtx& c, const std::string& name, const UArgs& a) {
   if (L.groups[0].toeplitz) { const ConvP& cp = c.h->convs.at(name); kflop = (double)cp.kt * cp.kh * cp.kw * cp.Cin; }  // algorithmic K, not the padded one
   if (const char* e = getenv("LSD_UMMA_SKIP")) p.skip = atoi(e);
   if (const char* why = umma_conv_config_error(p)) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: %s", name.c_str(), why);
-  // stage program: expanded on the host, cached in device memory under a hash of the complete parameter block (pointers,
-  // strides, geometry, tile shape), so steady-state forwards only look it up
-  {
-    uint64_t hkey = 1469598103934665603ull;
-    static_assert(sizeof(UmmaConvP) % 8 == 0, "UmmaConvP is hashed in 8-byte words");
-    const uint64_t* pw = reinterpret_cast<const uint64_t*>(&p);   // (p was memset to 0 first: padding bytes are deterministic)
-    for (size_t i = 0; i < sizeof(p) / 8; ++i) { hkey ^= pw[i]; hkey *= 1099511628211ull; hkey ^= hkey >> 29; }
-    auto it = c.h->prog_cache.find(hkey);
-    if (it == c.h->prog_cache.end()) {
-      const size_t bytes = (size_t)p.nst_tile * sizeof(UcStageDesc);
-      if (!c.h->prog_arena) {
-        c.h->prog_cap = 16u << 20;
-        if (cudaMalloc(&c.h->prog_arena, c.h->prog_cap) != cudaSuccess) return lsd_fail(c.h, LSD_ERR_CUDA, "stage-program arena allocation failed");
-        c.h->prog_cursor = 0;
-      }
-      if (c.h->prog_cursor + bytes > c.h->prog_cap) {   // arena full (many shapes / workspaces seen): start over once nothing is in flight
-        cudaDeviceSynchronize();
-        c.h->prog_cache.clear();
-        c.h->prog_cursor = 0;
-        ++c.h->generation;   // captured CUDA graphs hold addresses of the old programs
-      }
-      std::vector<UcStageDesc> host((size_t)p.nst_tile);
-      umma_conv_build_program(p, host.data());
-      char* dst = c.h->prog_arena + c.h->prog_cursor;
-      // Cache miss only (first forward of a shape): a blocking copy, so the program is visible to every stream that later
-      // launches this layer (the cache is shared by the main, side, tail and helper streams).
-      cudaError_t e = cudaMemcpy(dst, host.data(), bytes, cudaMemcpyHostToDevice);
-      if (e != cudaSuccess) return lsd_fail(c.h, LSD_ERR_CUDA, "%s: stage program upload: %s", name.c_str(), cudaGetErrorString(e));
-      c.h->prog_cursor += (bytes + 255) & ~size_t(255);
-      it = c.h->prog_cache.emplace(hkey, dst).first;
-    }
-    p.prog = reinterpret_cast<const UcStageDesc*>(it->second);
-  }
+  if (int rc = stage_program(c, name, p, [&](std::vector<UcStageDesc>& v) { v.resize((size_t)p.nst_tile); umma_conv_build_program(p, v.data()); }))
+    return rc;
   // tile counters of this layer (dynamic tile scheduling, LSD_UMMA_DYNAMIC=1).  Off by default: measured at B=64 it shortens the
   // visual encoder by ~20 us per forward (CTAs delayed by the side stream's kernels take fewer tiles) but every one-tile
   // token-path launch pays the claim + counter re-arm (~1 us each), a net +2 % per step.
@@ -871,6 +928,144 @@ int res_stage_umma(const BCtx& b, const std::string& p, const PBuf& x, const PBu
   return 0;
 }
 
+// One folded small-map convolution (UcFoldSlice in umma_conv.cuh) of layer `name` (weights "<name>#fold"): x holds the input map
+// (Hi x Wi, one plane set per position, row geometry), read with stride `stride`; x_ds (optional) is the input of the fused 1x1
+// stride-2 downsample (map Hd x Wd).  Output map Ho x Wo, ReLU, to yp: folded (UC_Y_FOLD) or a plain padded map (UC_Y_MAP).
+int run_umma_fold(const BCtx& c, const std::string& name, const PBuf& x, int Hi, int Wi, int stride, const PBuf* x_ds, int Hd, int Wd,
+                  int Ho, int Wo, const PBuf& yp, int y_mode) {
+  const auto itL = c.h->blayers.find(name + "#fold");
+  if (itL == c.h->blayers.end()) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: no weights packed for the folded route (LSD_FOLD=0)", name.c_str());
+  const BLayer& L = itL->second;
+  const UcGeom& og = x.g;   // row geometry: the tile positions are frame rows
+  if (og.P_total >= ((int64_t)1 << 31) - 1024) return lsd_fail(c.h, LSD_ERR_SHAPE, "%s: more than 2^31 rows in one launch (reduce the batch)", name.c_str());
+  if ((L.groups.size() == 2) != (x_ds != nullptr) || x.sets != Hi * Wi || (x_ds && x_ds->sets != Hd * Wd))
+    return lsd_fail(c.h, LSD_ERR_ARG, "%s: folded inputs do not match the layer", name.c_str());
+  UmmaConvP p;
+  memset(&p, 0, sizeof(p));
+  p.w = reinterpret_cast<const __nv_bfloat16*>(c.h->barena);
+  p.bias = c.h->bbias + L.bias_off;
+  p.Cout = L.ntile;
+  p.act = ACT_RELU;
+  p.g = og;
+  p.fold = 1;
+  p.y_mode = y_mode;
+  p.y = c.org(yp);
+  p.y_plane_stride = yp.plane_stride; p.y_set_stride = yp.set_stride;
+  p.g2 = yp.g;
+  p.ymap_W = Wo;
+  // Tile shape: 2 M-tiles x 128 columns (LSD_FOLD_MT / LSD_FOLD_NT: tuning knobs), fewer M-tiles when the rows do not fill them.
+  // One tile per CTA: slices differ in K (4 / 6 / 9 input positions for corner / edge / centre), the heaviest come first and the
+  // block scheduler hands the rest to the SMs as they free up.
+  int mt = 2;
+  if (const char* e = LSD_ENV("LSD_FOLD_MT")) mt = std::max(1, std::min(4, atoi(e)));
+  p.MT = (int)std::max<int64_t>(1, std::min<int64_t>(mt, (og.P_total + 127) / 128));
+  p.nbuf = 1;
+  p.issuers = std::min(p.MT, 4);
+  uint32_t cols = 32;
+  while ((int)cols < p.MT * L.ntile) cols *= 2;
+  p.tmem_cols = cols;
+  const int S = p.MT * 128;
+  const PBuf* srcs[2] = {&x, x_ds};
+  p.ngroups = (int)L.groups.size();
+  p.nbands = p.ngroups;
+  int max_a = 0, max_w = 0, min_k16 = 1 << 30;
+  for (int gi = 0; gi < p.ngroups; ++gi) {
+    const BGroup& G = L.groups[gi];
+    UcGroup& ug = p.groups[gi];
+    ug.band_begin = gi; ug.band_end = gi + 1;
+    ug.k16 = G.k16; ug.taps_total = G.taps_total;
+    ug.w_off = (int64_t)G.w_off; ug.slice_stride = (int64_t)G.slice_stride;
+    // launch-wide band shapes the MMA issuer reads: main = 3 temporal taps (rows -1, 0, +1), downsample = 1 tap (row 0); each
+    // stage's A source (plane set of one input position) is baked into the slice programs below
+    UcBand& ub = p.bands[gi];
+    const PBuf& src = *srcs[gi];
+    ub.base = c.org(src);
+    ub.plane_stride = src.plane_stride;
+    ub.chunk_stride = 2 * src.plane_stride;
+    ub.ntaps = gi == 0 ? 3 : 1;
+    ub.start = gi == 0 ? -1 : 0;
+    ub.len_extra = gi == 0 ? 2 : 0;
+    for (int j = 0; j < ub.ntaps; ++j) ub.rel[j] = j;
+    if ((int64_t)8 > src.origin) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: guard zone too small", name.c_str());
+    max_a = std::max(max_a, 2 * (S + ub.len_extra) * 16);
+    max_w = std::max(max_w, ub.ntaps * L.ntile * 32);
+    min_k16 = std::min(min_k16, G.k16);
+  }
+  // K chunks per stage: the summation order (input position, K chunk, temporal tap) does not depend on kpack here, so the stages
+  // can be large enough to amortise the per-stage bookkeeping of the issuing warps
+  p.kpack = std::max(1, std::min(std::min(8, min_k16), (48 * 1024) / (max_a + max_w)));
+  p.a_stage_bytes = ((uint32_t)(max_a * p.kpack) + 127u) & ~127u;
+  p.w_stage_bytes = (uint32_t)(max_w * p.kpack);
+  // column slices: (output position, Cout slice), heaviest positions first
+  const int cslices = L.Cout / L.ntile;
+  std::vector<std::array<int, 3>> pos;   // (-in-bounds input positions, ho, wo)
+  auto inb = [&](int o, int k, int n) { const int i = stride * o + k - 1; return i >= 0 && i < n; };
+  for (int ho = 0; ho < Ho; ++ho)
+    for (int wo = 0; wo < Wo; ++wo) {
+      int nq = 0;
+      for (int kh = 0; kh < 3; ++kh)
+        for (int kw = 0; kw < 3; ++kw) nq += inb(ho, kh, Hi) && inb(wo, kw, Wi);
+      pos.push_back({-nq, ho, wo});
+    }
+  std::stable_sort(pos.begin(), pos.end(), [](const std::array<int, 3>& a, const std::array<int, 3>& b) { return a[0] < b[0]; });
+  const int nslices = (int)pos.size() * cslices;
+  if (nslices > UC_MAX_FSLICES || Ho > 255 || Wo > 255) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: map too large for the folded route", name.c_str());
+  auto chunks = [&](int k16) { return (k16 + p.kpack - 1) / p.kpack; };
+  int off = 0;
+  for (int i = 0; i < nslices; ++i) {
+    const auto& q = pos[(size_t)(i / cslices)];
+    const int nst = -q[0] * chunks(p.groups[0].k16) + (x_ds ? chunks(p.groups[1].k16) : 0);
+    p.fslice[i] = UcFoldSlice{(uint16_t)off, (uint16_t)nst, (uint8_t)q[1], (uint8_t)q[2], (uint8_t)(i % cslices), 0};
+    p.nst_tile = std::max(p.nst_tile, nst);
+    off += nst;
+  }
+  if (off > 65535) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: folded stage programs too long", name.c_str());
+  const uint32_t stage = p.a_stage_bytes + p.w_stage_bytes;
+  const uint32_t prog_bytes = (uint32_t)p.nst_tile * (uint32_t)umma_conv_stage_desc_bytes();
+  const uint32_t budget = 211u * 1024u - (uint32_t)umma_conv_extra_smem_bytes(p);
+  if (prog_bytes + 2 * stage > budget) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: stage program of %u bytes does not fit", name.c_str(), prog_bytes);
+  p.stages = std::max(2, std::min((int)((budget - prog_bytes) / stage), 8));
+  if (const char* e = getenv("LSD_UMMA_SKIP")) p.skip = atoi(e);
+  if (const char* why = umma_conv_config_error(p)) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: %s", name.c_str(), why);
+  // slice programs: per in-bounds input position q (ascending), per K-chunk block, one stage of 3 temporal taps with A from plane
+  // set q; then the downsample (input position (2 ho, 2 wo)).  Summation order (q, K chunk, dt): fixed by the geometry alone.
+  auto build = [&](std::vector<UcStageDesc>& v) {
+    for (int i = 0; i < nslices; ++i) {
+      const UcFoldSlice& f = p.fslice[i];
+      for (int kh = 0; kh < 3; ++kh)
+        for (int kw = 0; kw < 3; ++kw) {
+          if (!inb(f.h, kh, Hi) || !inb(f.w, kw, Wi)) continue;
+          UcBand bq = p.bands[0];
+          bq.base = c.org(x) + (int64_t)((stride * f.h + kh - 1) * Wi + stride * f.w + kw - 1) * x.set_stride;
+          bq.tap_begin = (kh * 3 + kw) * 3;   // (kh, kw, kt) packing order, see Packer::add_fold
+          for (int c0 = 0; c0 < p.groups[0].k16; c0 += p.kpack) v.push_back(umma_conv_stage(p, p.groups[0], bq, 0, c0, f.col));
+        }
+      if (x_ds) {
+        UcBand bd = p.bands[1];
+        bd.base = c.org(*x_ds) + (int64_t)(2 * f.h * Wd + 2 * f.w) * x_ds->set_stride;
+        for (int c0 = 0; c0 < p.groups[1].k16; c0 += p.kpack) v.push_back(umma_conv_stage(p, p.groups[1], bd, 1, c0, f.col));
+      }
+    }
+  };
+  if (int rc = stage_program(c, name + "#fold", p, build, {(uint64_t)Hi, (uint64_t)Wi, (uint64_t)stride, (uint64_t)Hd, (uint64_t)Wd,
+                                                          (uint64_t)x.set_stride, (uint64_t)(x_ds ? x_ds->set_stride : 0)})) return rc;
+  // profile FLOPs: the algorithmic count of the original convolution (the row geometry has H = W = 1)
+  double kflop = 0;
+  for (const BGroup& G : L.groups) kflop += (double)G.taps_total * G.Cin;
+  c.h->prof.begin(c.st, 2.0 * (double)og.N * og.T * Ho * Wo * L.Cout * kflop, 2);
+  launch_umma_conv(p, nslices, c.st, c.h->num_sms, c.max_ctas);
+  c.h->prof.end(c.st);
+  return 0;
+}
+
+// Residual stage with a stride-2 conv1 and a fused downsample on the folded route: x (folded, Hi x Wi) -> mid (folded, Ho x Wo)
+// -> y (folded, or the plain padded map when y_mode == UC_Y_MAP)
+int res_stage_fold(const BCtx& b, const std::string& p, const PBuf& x, int Hi, int Wi, const PBuf& mid, int Ho, int Wo, const PBuf& y, int y_mode) {
+  int rc = 0;
+  if ((rc = run_umma_fold(b, p + ".conv1", x, Hi, Wi, 2, nullptr, 0, 0, Ho, Wo, mid, UC_Y_FOLD))) return rc;
+  return run_umma_fold(b, p + ".conv2", mid, Ho, Wo, 1, &x, Hi, Wi, Ho, Wo, y, y_mode);
+}
+
 }  // namespace
 
 // Weight stream, stage table and small vectors of the fused temporal-transformer kernel (tok_fused.cu).
@@ -994,6 +1189,12 @@ int pack_bf16_weights(lsd_handle* h, const std::vector<float>& f32_arena) {
     P.add(p + ".conv1", p + ".conv1", s, s, "", nt, false, /*merge_kt=*/l >= 2, pairs);   // 12x12 / 6x6 / 3x3 maps: one band per parity set
     P.ds_sh = 2; P.ds_sw = 2;
     P.add(p + ".conv2", p + ".conv2", 1, 1, l == 1 ? "" : p + ".downsample", nt, false, false, pairs);
+    if (l >= 3) {   // folded small-map route (run_umma_fold)
+      int fnt = 128;
+      if (const char* e = LSD_ENV("LSD_FOLD_NT")) fnt = atoi(e) == 256 ? 256 : 128;   // tuning knob: columns per folded CTA
+      P.add_fold(p + ".conv1#fold", p + ".conv1", "", fnt);
+      P.add_fold(p + ".conv2#fold", p + ".conv2", p + ".downsample", fnt);
+    }
   }
   P.add_toeplitz("visual_encoder.stem", "visual_encoder.stem", 8, 0, false, cta2);  // 7 taps in w -> 8-pixel window starting at 2*wo-4
   for (int cv = 0; cv < 2; ++cv) {
@@ -1474,11 +1675,16 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
     } else if ((rc = res_stage_umma(b, "visual_encoder.layer1", x1, pb["l1a"], pb["y1"], false, UC_Y_PARITY))) return rc;
   }
   g_tl.mark(st, "M:layer1");
-  if ((rc = res_stage_umma(b, "visual_encoder.layer2", pb["y1"], pb["l2a"], pb["y2"], true, UC_Y_PARITY))) return rc;
+  // layer2 writes y2 folded when layer3 runs on the folded route (small maps, see fold_route); y4 is always the plain padded map
+  if ((rc = res_stage_umma(b, "visual_encoder.layer2", pb["y1"], pb["l2a"], pb["y2"], true, P.fold3 ? UC_Y_FOLD : UC_Y_PARITY))) return rc;
   g_tl.mark(st, "M:layer2");
-  if ((rc = res_stage_umma(b, "visual_encoder.layer3", pb["y2"], pb["l3a"], pb["y3"], true, UC_Y_PARITY))) return rc;
+  if (P.fold3) rc = res_stage_fold(b, "visual_encoder.layer3", pb["y2"], s.H2, s.W2, pb["l3a"], s.H3, s.W3, pb["y3"], UC_Y_FOLD);
+  else rc = res_stage_umma(b, "visual_encoder.layer3", pb["y2"], pb["l3a"], pb["y3"], true, P.fold4 ? UC_Y_FOLD : UC_Y_PARITY);
+  if (rc) return rc;
   g_tl.mark(st, "M:layer3");
-  if ((rc = res_stage_umma(b, "visual_encoder.layer4", pb["y3"], pb["l4a"], pb["y4"], true, UC_Y_PLAIN))) return rc;
+  if (P.fold4) rc = res_stage_fold(b, "visual_encoder.layer4", pb["y3"], s.H3, s.W3, pb["l4a"], s.H4, s.W4, pb["y4"], UC_Y_MAP);
+  else rc = res_stage_umma(b, "visual_encoder.layer4", pb["y3"], pb["l4a"], pb["y4"], true, UC_Y_PLAIN);
+  if (rc) return rc;
   g_tl.mark(st, "M:layer4");
   b.max_ctas = 0;
   const PBuf& y4 = pb["y4"];

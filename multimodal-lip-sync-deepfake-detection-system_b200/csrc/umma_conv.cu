@@ -130,7 +130,10 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
   const uint32_t stage_bytes = p.a_stage_bytes + p.w_stage_bytes;
   const int num_tiles = (int)((p.g.P_total + S - 1) / S);
   const uint32_t cta_rank = CTA2 ? cluster_ctarank() : 0u;
-  const int slice = blockIdx.y, ch0 = slice * p.Cout;
+  const int slice = blockIdx.y;
+  const bool fold = p.fold != 0;                                    // (folded conv: grid.y = (output position, Cout slice))
+  const int nst = fold ? (int)p.fslice[slice].nst : p.nst_tile;    // ring stages per tile of this CTA's column slice
+  const int ch0 = (fold ? (int)p.fslice[slice].col : slice) * p.Cout;
   const int bcols = CTA2 ? p.Cout >> 1 : p.Cout;         // weight columns in this CTA's shared memory
   const uint32_t buf_cols = (uint32_t)(p.MT * p.Cout);
   // tile walk: tile_first, tile_first + tile_step, ... < tile_end; tile i covers positions pbase + i*S .. + S
@@ -194,9 +197,9 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
   // stage program -> shared memory (one 16-byte piece per thread)
   UcStageDesc* prog = reinterpret_cast<UcStageDesc*>(smem + (size_t)p.stages * stage_bytes);
   {
-    const uint4* psrc = reinterpret_cast<const uint4*>(p.prog);
+    const uint4* psrc = reinterpret_cast<const uint4*>(p.prog + (fold ? (int)p.fslice[slice].prog_off : 0));
     uint4* pdst = reinterpret_cast<uint4*>(prog);
-    for (int i = tid; i < p.nst_tile * 4; i += UC_THREADS) pdst[i] = psrc[i];
+    for (int i = tid; i < nst * 4; i += UC_THREADS) pdst[i] = psrc[i];
   }
   tc_fence_before();
   if constexpr (CTA2) cluster_sync_all();   // (the peer's barriers are initialised before anything arrives on them remotely)
@@ -228,12 +231,12 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
     const uint64_t slice64 = CTA2 ? (uint64_t)cta_rank : (uint64_t)slice;   // (CTA2: the packed weights hold the two column halves as slices)
     int k = 0;                                              // global stage counter at the start of the tile
     int seq = 0;
-    for (int tile = tile_start; tile >= 0; k += p.nst_tile) {
+    for (int tile = tile_start; tile >= 0; k += nst) {
       unsigned claim = 0;
       if (dyn && warp == 0 && lane == 0) claim = atomicAdd(p.tile_ctr + slice, 1u);   // (consumed after this tile's stages are issued)
       const uint64_t p0_bytes = (uint64_t)tile_p0(tile) * 16u;
       // first stage of this tile owned by this warp: si = (warp - k) mod 4
-      for (int si = ((warp - k) % npw + npw) % npw; si < p.nst_tile; si += npw) {
+      for (int si = ((warp - k) % npw + npw) % npw; si < nst; si += npw) {
         const int kk = k + si;
         const int stage = kk % p.stages;
         const uint32_t ph = (uint32_t)(kk / p.stages) & 1u;
@@ -287,7 +290,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
         int stage = 0;
         uint32_t ph = 0;
         for (int tile = tile_first; tile < tile_end; tile += tile_step)
-          for (int si = 0; si < p.nst_tile; ++si) {
+          for (int si = 0; si < nst; ++si) {
             mbar_wait(&full_bar[stage], ph);
             if (lane == 0) mbar_arrive_cluster(mapa_shared(smem_u32(&full2_bar[stage]), 0u));
             __syncwarp();
@@ -333,59 +336,57 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
         }
         acc = 1u;
       }
-      // The loop nest reads the parameter block with warp-uniform indices (uniform constant loads) and runs on every lane;
-      // only the MMA / commit instructions are predicated on the elected lane, so the descriptor arithmetic stays in uniform
-      // registers instead of being moved there (R2UR) for every instruction.
-      for (int gi = 0; gi < p.ngroups; ++gi) {
-        const int k16 = p.groups[gi].k16, b0 = p.groups[gi].band_begin, b1 = p.groups[gi].band_end;
-        for (int c0 = 0; c0 < k16; c0 += p.kpack) {
-          const int nc = min(p.kpack, k16 - c0);
-          for (int b = b0; b < b1; ++b) {
-            const UcBand& bd = p.bands[b];
-            const int ntaps = bd.ntaps;
-            const uint32_t unitsA = (uint32_t)(S + bd.len_extra);
-            const uint32_t a_lbo = (bd.toeplitz ? 1u : unitsA) << 16;     // low descriptor word = LBO << 16 | start address >> 4
-            const uint32_t a_chunk = bd.toeplitz ? 2u : 2u * unitsA;
-            const uint32_t w_chunk = (uint32_t)ntaps * tap_w;
-            mbar_wait(&full_bar[stage], ph);
-            if constexpr (CTA2) mbar_wait_cluster(&full2_bar[stage], ph);   // the peer's A rows and weight half have landed too
-            tc_fence_after();
-            if (dbg && warp == UC_MMA_WARP0 && lane == 0 && acc == 0 && lt == 0) p.dbg[2] = clock64();   // first stage landed
-            if (dbg && warp == UC_MMA_WARP0 && lane == 0 && lt == 0 && dbg_it < 24) p.dbg[8 + dbg_it++] = clock64();
-            const uint32_t sa = ((smem_base + (uint32_t)stage * stage_bytes) >> 4) + (uint32_t)mt_lo * 128u;
-            const uint32_t sw = ((smem_base + (uint32_t)stage * stage_bytes + p.a_stage_bytes) >> 4) | b_lbo;
-            if (ntaps == 1) {
-              // Linear layers (one tap per band): one MMA per K chunk, descriptors advance by constant steps
-              uint32_t at = (sa | a_lbo) + (uint32_t)bd.rel[0], wj = sw;
+      // One iteration per ring stage of the tile's stage program (the program fixes the band and the K chunks of every stage, so
+      // a folded conv's slices run their own band lists).  The loop reads the parameter block with warp-uniform indices (the
+      // stage's counts word is broadcast from lane 0, which ptxas treats as uniform) and runs on every lane; only the MMA /
+      // commit instructions are predicated on the elected lane, so the descriptor arithmetic stays in uniform registers instead
+      // of being moved there (R2UR) for every instruction.
+      for (int si = 0; si < nst; ++si) {
+        const uint32_t counts = __shfl_sync(0xffffffffu, prog[si].counts, 0);
+        const int b = (int)((counts >> 16) & 0xffu), nc = (int)(counts >> 24);
+        const UcBand& bd = p.bands[b];
+        const int ntaps = bd.ntaps;
+        const uint32_t unitsA = (uint32_t)(S + bd.len_extra);
+        const uint32_t a_lbo = (bd.toeplitz ? 1u : unitsA) << 16;     // low descriptor word = LBO << 16 | start address >> 4
+        const uint32_t a_chunk = bd.toeplitz ? 2u : 2u * unitsA;
+        const uint32_t w_chunk = (uint32_t)ntaps * tap_w;
+        mbar_wait(&full_bar[stage], ph);
+        if constexpr (CTA2) mbar_wait_cluster(&full2_bar[stage], ph);   // the peer's A rows and weight half have landed too
+        tc_fence_after();
+        if (dbg && warp == UC_MMA_WARP0 && lane == 0 && acc == 0 && lt == 0) p.dbg[2] = clock64();   // first stage landed
+        if (dbg && warp == UC_MMA_WARP0 && lane == 0 && lt == 0 && dbg_it < 24) p.dbg[8 + dbg_it++] = clock64();
+        const uint32_t sa = ((smem_base + (uint32_t)stage * stage_bytes) >> 4) + (uint32_t)mt_lo * 128u;
+        const uint32_t sw = ((smem_base + (uint32_t)stage * stage_bytes + p.a_stage_bytes) >> 4) | b_lbo;
+        if (ntaps == 1) {
+          // Linear layers (one tap per band): one MMA per K chunk, descriptors advance by constant steps
+          uint32_t at = (sa | a_lbo) + (uint32_t)bd.rel[0], wj = sw;
 #pragma unroll 1
-              for (int j = 0; j < nc; ++j, at += a_chunk, wj += w_chunk) {
-                const uint64_t da = desc_hi64 | (uint64_t)at, db = desc_hi64 | (uint64_t)wj;
-                UC_MMA(tb, da, db, idesc, acc, leader);
-                if (mt_n > 1) UC_MMA(tb + (uint32_t)p.Cout, da + 128u, db, idesc, acc, leader);
-                acc = 1u;
-              }
-            } else
-            for (int j = 0; j < nc; ++j) {
-              const uint32_t aj = (sa + (uint32_t)j * a_chunk) | a_lbo;
-              uint32_t wj = sw + (uint32_t)j * w_chunk;
+          for (int j = 0; j < nc; ++j, at += a_chunk, wj += w_chunk) {
+            const uint64_t da = desc_hi64 | (uint64_t)at, db = desc_hi64 | (uint64_t)wj;
+            UC_MMA(tb, da, db, idesc, acc, leader);
+            if (mt_n > 1) UC_MMA(tb + (uint32_t)p.Cout, da + 128u, db, idesc, acc, leader);
+            acc = 1u;
+          }
+        } else
+        for (int j = 0; j < nc; ++j) {
+          const uint32_t aj = (sa + (uint32_t)j * a_chunk) | a_lbo;
+          uint32_t wj = sw + (uint32_t)j * w_chunk;
 #pragma unroll 1
-              for (int tp = 0; tp < ntaps; ++tp) {   // (not unrolled: the kernel must stay inside the instruction cache)
-                const uint32_t at = aj + (uint32_t)bd.rel[tp];
-                const uint64_t da = desc_hi64 | (uint64_t)at, db = desc_hi64 | (uint64_t)wj;
-                UC_MMA(tb, da, db, idesc, acc, leader);
-                if (mt_n > 1) UC_MMA(tb + (uint32_t)p.Cout, da + 128u, db, idesc, acc, leader);
-                if (mt_n > 2) {
-                  UC_MMA(tb + 2u * (uint32_t)p.Cout, da + 256u, db, idesc, acc, leader);
-                  UC_MMA(tb + 3u * (uint32_t)p.Cout, da + 384u, db, idesc, acc, leader);
-                }
-                acc = 1u;
-                wj += tap_w;
-              }
+          for (int tp = 0; tp < ntaps; ++tp) {   // (not unrolled: the kernel must stay inside the instruction cache)
+            const uint32_t at = aj + (uint32_t)bd.rel[tp];
+            const uint64_t da = desc_hi64 | (uint64_t)at, db = desc_hi64 | (uint64_t)wj;
+            UC_MMA(tb, da, db, idesc, acc, leader);
+            if (mt_n > 1) UC_MMA(tb + (uint32_t)p.Cout, da + 128u, db, idesc, acc, leader);
+            if (mt_n > 2) {
+              UC_MMA(tb + 2u * (uint32_t)p.Cout, da + 256u, db, idesc, acc, leader);
+              UC_MMA(tb + 3u * (uint32_t)p.Cout, da + 384u, db, idesc, acc, leader);
             }
-            UC_COMMIT(&empty_bar[stage], leader);  // frees the stage once the MMAs that read it have completed
-            if (++stage == p.stages) { stage = 0; ph ^= 1u; }
+            acc = 1u;
+            wj += tap_w;
           }
         }
+        UC_COMMIT(&empty_bar[stage], leader);  // frees the stage once the MMAs that read it have completed
+        if (++stage == p.stages) { stage = 0; ph ^= 1u; }
       }
       UC_COMMIT(&tfull_bar[buf], leader);   // accumulator of this tile complete -> epilogue
       if (dbg && warp == UC_MMA_WARP0 && lane == 0 && lt == 0) p.dbg[3] = clock64();   // all MMAs of the first tile issued
@@ -420,6 +421,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
         const int64_t P = P0 + (int64_t)m * 128 + rowt;
         int n = 0, t = 0, h = 0, w = 0;
         const bool valid = (p.skip & 8) ? true : uc_decode(p.g, P, n, t, h, w);   // (skip bit 3: timing experiment)
+        if (fold) { h = p.fslice[slice].h; w = p.fslice[slice].w; }               // (row geometry: P is the frame row)
         const bool inrange = P < p.g.P_total;
         const int64_t outer = valid ? ((int64_t)n * p.g.T + t) * p.g.H + h : 0;
         int64_t dst = P * 8;
@@ -427,6 +429,10 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
           dst = (int64_t)((h & 1) * 2 + (w & 1)) * p.y_set_stride + uc_flat(p.g2, n, t, h >> 1, w >> 1) * 8;
         else if (valid && p.y_mode == UC_Y_PARITY_H)
           dst = (int64_t)((h & 1) * 2) * p.y_set_stride + uc_flat(p.g2, n, t, h >> 1, w) * 8;
+        else if (valid && p.y_mode == UC_Y_FOLD)
+          dst = (int64_t)(h * p.ymap_W + w) * p.y_set_stride + uc_flat(p.g2, n, t, 0, 0) * 8;
+        else if (valid && p.y_mode == UC_Y_MAP)
+          dst = uc_flat(p.g2, n, t, h, w) * 8;
         const bool store_planar = ((p.y_mode == UC_Y_PLAIN && inrange) || (p.y_mode >= UC_Y_PARITY && valid)) && !(p.skip & 4);   // (skip bit 2: timing experiment)
         // this warp's columns: [half*Cout/2, (half+1)*Cout/2), or all of them when the warps split the M-tiles
         const int cbeg = split_c ? half * (p.Cout >> 1) : 0, cend = split_c ? cbeg + (p.Cout >> 1) : p.Cout;
@@ -633,40 +639,42 @@ done:
   if (dbg && tid == 0) { p.dbg[6] = clock64(); p.dbg[7] = num_tiles; }
 }
 
-void umma_conv_build_program(const UmmaConvP& p, UcStageDesc* out) {
+UcStageDesc umma_conv_stage(const UmmaConvP& p, const UcGroup& g, const UcBand& bd, int band, int c0, int col) {
   const int S = p.MT * 128;
   const int bcols = p.cta2 ? p.Cout / 2 : p.Cout;   // weight columns one CTA stages
+  const int nc = std::min(p.kpack, g.k16 - c0);
+  UcStageDesc d;
+  const uint32_t bytesW = (uint32_t)bd.ntaps * (uint32_t)bcols * 32u;
+  d.bytesA = bd.toeplitz ? (uint32_t)(S + bd.len_extra + 1 + 2 * (nc - 1)) * 16u : (uint32_t)(S + bd.len_extra) * 16u;
+  uint32_t n_a = bd.toeplitz ? 1u : 2u * (uint32_t)nc;   // Toeplitz: the K chunks are 32-byte shifts of one row region
+  // a band that holds all taps of its group (Linear layers, the fused 1x1 downsample): the weights of consecutive K chunks are
+  // contiguous -> one copy
+  const bool w_merged = bd.ntaps == g.taps_total;
+  uint32_t n_w = w_merged ? 1u : (uint32_t)nc;
+  d.w_copy_bytes = w_merged ? (uint32_t)nc * bytesW : bytesW;
+  d.w_dst_step = bytesW;
+  // (p.skip: timing experiments only — bit 0 drops the A copies, bit 1 the W copies; results are then garbage)
+  if (p.skip & 1) n_a = 0;
+  if (p.skip & 2) n_w = 0;
+  d.tx_bytes = n_a * d.bytesA + (n_w ? (uint32_t)nc * bytesW : 0u);
+  d.a_src = reinterpret_cast<uint64_t>(bd.base + (int64_t)c0 * bd.chunk_stride + (int64_t)bd.start * 8);
+  d.chunk_stride_b = (uint64_t)bd.chunk_stride * 2u;
+  d.plane_stride_b = (uint64_t)bd.plane_stride * 2u;
+  // weight piece j of the stage is the packed block [chunk c0 + j][taps of this band]: pieces are taps_total * Cout * 32 B apart
+  d.w_src = reinterpret_cast<uint64_t>(p.w + g.w_off + (col > 0 ? (int64_t)col * g.slice_stride : 0) +
+                                       ((int64_t)c0 * g.taps_total + bd.tap_begin) * (int64_t)bcols * 16);
+  d.w_slice_stride_b = col >= 0 ? 0u : (uint64_t)g.slice_stride * 2u;
+  d.w_src_step = (uint32_t)g.taps_total * (uint32_t)bcols * 32u;
+  d.counts = n_a | (n_w << 8) | ((uint32_t)band << 16) | ((uint32_t)nc << 24);
+  return d;
+}
+
+void umma_conv_build_program(const UmmaConvP& p, UcStageDesc* out) {
   int s = 0;
   for (int gi = 0; gi < p.ngroups; ++gi) {
     const UcGroup& g = p.groups[gi];
-    for (int c0 = 0; c0 < g.k16; c0 += p.kpack) {
-      const int nc = std::min(p.kpack, g.k16 - c0);
-      for (int b = g.band_begin; b < g.band_end; ++b, ++s) {
-        const UcBand& bd = p.bands[b];
-        UcStageDesc d;
-        const uint32_t bytesW = (uint32_t)bd.ntaps * (uint32_t)bcols * 32u;
-        d.bytesA = bd.toeplitz ? (uint32_t)(S + bd.len_extra + 1 + 2 * (nc - 1)) * 16u : (uint32_t)(S + bd.len_extra) * 16u;
-        uint32_t n_a = bd.toeplitz ? 1u : 2u * (uint32_t)nc;   // Toeplitz: the K chunks are 32-byte shifts of one row region
-        // single-band groups (Linear layers): the weights of consecutive K chunks are contiguous -> one copy
-        const bool w_merged = (g.band_end - g.band_begin) == 1;
-        uint32_t n_w = w_merged ? 1u : (uint32_t)nc;
-        d.w_copy_bytes = w_merged ? (uint32_t)nc * bytesW : bytesW;
-        d.w_dst_step = bytesW;
-        // (p.skip: timing experiments only — bit 0 drops the A copies, bit 1 the W copies; results are then garbage)
-        if (p.skip & 1) n_a = 0;
-        if (p.skip & 2) n_w = 0;
-        d.tx_bytes = n_a * d.bytesA + (n_w ? (uint32_t)nc * bytesW : 0u);
-        d.a_src = reinterpret_cast<uint64_t>(bd.base + (int64_t)c0 * bd.chunk_stride + (int64_t)bd.start * 8);
-        d.chunk_stride_b = (uint64_t)bd.chunk_stride * 2u;
-        d.plane_stride_b = (uint64_t)bd.plane_stride * 2u;
-        // weight piece j of the stage is the packed block [chunk c0 + j][taps of this band]: pieces are taps_total * Cout * 32 B apart
-        d.w_src = reinterpret_cast<uint64_t>(p.w + g.w_off + ((int64_t)c0 * g.taps_total + bd.tap_begin) * (int64_t)bcols * 16);
-        d.w_slice_stride_b = (uint64_t)g.slice_stride * 2u;
-        d.w_src_step = (uint32_t)g.taps_total * (uint32_t)bcols * 32u;
-        d.counts = n_a | (n_w << 8) | ((uint32_t)b << 16) | ((uint32_t)nc << 24);
-        out[s] = d;
-      }
-    }
+    for (int c0 = 0; c0 < g.k16; c0 += p.kpack)
+      for (int b = g.band_begin; b < g.band_end; ++b) out[s++] = umma_conv_stage(p, g, p.bands[b], b, c0);
   }
 }
 
@@ -694,6 +702,8 @@ const char* umma_conv_config_error(const UmmaConvP& p) {
   if (p.res && p.res32) return "bf16 and fp32 residuals are mutually exclusive";
   if (uc_is_generic(p) && (p.Cout & 63)) return "the generic epilogue needs a column slice that is a multiple of 64";
   if (p.MT / p.issuers > 4 || p.MT % p.issuers) return "unsupported M-tiles per issuing warp";
+  if (p.fold && (uc_is_generic(p) || p.cta2 || p.tile_ctr || p.y_mode == UC_Y_POOL || p.res || p.MT > 4))
+    return "folded convolutions need the lean epilogue, no residual, single CTAs, at most 4 M-tiles and the static tile walk";
   if (p.cta2 && (uc_is_generic(p) || p.y_mode == UC_Y_POOL || (p.Cout & 31) || p.tile_ctr)) return "CTA pairs need the lean epilogue, a multiple of 32 columns and the static tile walk";
   if (p.y_mode == UC_Y_POOL) {
     if (uc_is_generic(p) || p.res || p.act != ACT_RELU || p.Cout != 64 || p.tile_ctr) return "fused max-pool needs the lean epilogue, ReLU, 64 columns and the static tile walk";
@@ -742,6 +752,7 @@ void launch_umma_conv(const UmmaConvP& p, int n_slices, cudaStream_t s, int num_
     count_launch();
     return;
   }
+  if (p.fold) gx = tiles;   // folded convs: one tile per CTA; the heaviest slices come first and the block scheduler balances the rest
   if (generic) umma_conv_kernel<1><<<dim3(gx, n_slices), UC_THREADS, umma_conv_smem_bytes(p), s>>>(p);
   else if (p.y_mode == UC_Y_POOL) umma_conv_kernel<2><<<dim3(gx, n_slices), UC_THREADS, umma_conv_smem_bytes(p), s>>>(p);
   else umma_conv_kernel<0><<<dim3(gx, n_slices), UC_THREADS, umma_conv_smem_bytes(p), s>>>(p);
@@ -806,7 +817,8 @@ void launch_unpack_planar(const __nv_bfloat16* x, int64_t plane_stride, UcGeom g
   count_launch();
 }
 
-// Introspection: any planar buffer (plain, or parity-split with 4 plane sets) -> fp32 channels-last (N, T, Hf, Wf, C)
+// Introspection: any planar buffer (plain, parity-split with 4 plane sets, or folded: Hf*Wf sets in the row geometry) -> fp32
+// channels-last (N, T, Hf, Wf, C)
 __global__ void unpack_planar_any_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ xlo, int64_t plane_stride,
                                          int64_t set_stride, UcGeom g, int C, int sets, int Hf, int Wf, float* __restrict__ y, int64_t total) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -821,6 +833,7 @@ __global__ void unpack_planar_any_kernel(const __nv_bfloat16* __restrict__ x, co
   const int n = (int)(r / g.T);
   int64_t src;
   if (sets == 1) src = uc_flat(g, n, t, h, w) * 8;
+  else if (g.SL == 1 && sets == Hf * Wf) src = (int64_t)(h * Wf + w) * set_stride + uc_flat(g, n, t, 0, 0) * 8;   // folded (one set per position)
   else if (Wf == g.W) src = (int64_t)((h & 1) * 2) * set_stride + uc_flat(g, n, t, h >> 1, w) * 8;          // h-parity split
   else src = (int64_t)((h & 1) * 2 + (w & 1)) * set_stride + uc_flat(g, n, t, h >> 1, w >> 1) * 8;          // (h, w)-parity split
   src += (int64_t)chunk * plane_stride;

@@ -43,7 +43,22 @@ struct UcGroup {              // taps that share one K extent (main conv; option
 // UC_Y_POOL: the epilogue keeps the bf16 outputs of the last positions in a shared-memory ring and writes only the
 // 3x3 / stride-2 / pad-1 max-pool over (H, W) of them (plain layout, geometry g2 = (N, T, H/2, W/2)) — the stem + MaxPool3d of
 // visual_encoder.py:113-129 in one launch.  Needs ReLU (zero pads stand for the -inf padding), even H and W, 64 columns, one slice.
-enum UcOut { UC_Y_NONE = 0, UC_Y_PLAIN = 1, UC_Y_PARITY = 2, UC_Y_PARITY_H = 3, UC_Y_POOL = 4 };
+// UC_Y_FOLD: "folded" destination (small maps, see UcFoldSlice): plane set h*ymap_W + w, position = frame row uc_flat(g2, n, t, 0, 0).
+// UC_Y_MAP: plain padded planar destination in geometry g2 written at (n, t, h, w) — a folded conv's output back in the map layout.
+enum UcOut { UC_Y_NONE = 0, UC_Y_PLAIN = 1, UC_Y_PARITY = 2, UC_Y_PARITY_H = 3, UC_Y_POOL = 4, UC_Y_FOLD = 5, UC_Y_MAP = 6 };
+
+// Folded small-map convolution ("frames as rows").  A map of H x W x C per frame is stored as H*W plane sets (one per spatial
+// position) in the row geometry make_geom_ex(N, T, 1, 1, 1, 0, 0, 0, 0): position = frame row n*(T+1) + t + 1, with the shared
+// zero row of every window.  A 3x3x3 / pad-1 convolution is then, per output position p, a 3-tap temporal convolution (row
+// shifts -1 / 0 / +1) summed over the input positions q that p's 3x3 stencil reaches IN BOUNDS: no multiply reads padding,
+// and no position outside the map is computed.  Each column slice (grid.y) is one (output position, Cout slice) with its own
+// stage program: one band per in-bounds q (three temporal taps, A from plane set q), then the fused 1x1 downsample band.
+constexpr int UC_MAX_FSLICES = 96;
+struct UcFoldSlice {
+  uint16_t prog_off, nst;     // the slice's stage program: prog[prog_off .. prog_off + nst)
+  uint8_t h, w;               // output position in the map
+  uint8_t col, pad_;          // Cout slice (columns col*Cout ..)
+};
 
 // Padded flat geometry:  P = ((n*TS + t + ot)*HP + h + oh)*RW + w + ow,  SL = HP*RW.
 // Standard activation geometry: one shared zero slab / row / column (TS=T+1, ot=1, HP=H+1, oh=1, RW=W+1, ow=1).
@@ -119,9 +134,12 @@ struct UmmaConvP {
   int pool_sR;
   int cta2;                   // 1: CTA pairs (cluster of 2, tcgen05 cta_group::2): the packed weights hold two column halves as slices
   UcGeom g;                   // output geometry (== input geometry of every band)
-  UcGeom g2;                  // UC_Y_PARITY*: destination geometry of each parity plane set
+  UcGeom g2;                  // UC_Y_PARITY* / UC_Y_FOLD / UC_Y_MAP: destination geometry (of each plane set)
   UcGroup groups[UC_MAX_GROUPS];
   UcBand bands[UC_MAX_BANDS];
+  int ymap_W;                 // UC_Y_FOLD: width of the map whose positions are the destination's plane sets
+  int fold;                   // 1: folded conv — grid.y walks fslice[]; the stage program is per slice, one tile per CTA
+  UcFoldSlice fslice[UC_MAX_FSLICES];
 };
 
 size_t umma_conv_smem_bytes(const UmmaConvP& p);
@@ -130,6 +148,9 @@ size_t umma_conv_extra_smem_bytes(const UmmaConvP& p);   // behind the stage pro
 size_t umma_conv_pool_smem_bytes(int MT);   // UC_Y_POOL: shared memory behind the stage program (ring + per-position table)
 // host: expand the stage program of a launch (same arithmetic the kernel used to do per stage)
 void umma_conv_build_program(const UmmaConvP& p, UcStageDesc* out);
+// host: one stage (K chunks c0 .. c0 + nc of band bd, whose index in p.bands is `band`); col >= 0: the Cout slice is baked into
+// the weight address (folded convs, whose grid.y is not the Cout slice)
+UcStageDesc umma_conv_stage(const UmmaConvP& p, const UcGroup& g, const UcBand& bd, int band, int c0, int col = -1);
 // nullptr if the kernel supports this parameter block, else the reason (callers turn it into an error code instead of launching)
 const char* umma_conv_config_error(const UmmaConvP& p);
 void launch_umma_conv(const UmmaConvP& p, int n_slices, cudaStream_t s, int num_sms, int max_ctas = 0);
