@@ -145,6 +145,39 @@ int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, 
  * only its own span of a sharded track passes span-relative `starts` and the audio starts computed from the absolute frame
  * indices (SURVEY.md §8e); NULL = computed here from `starts` as predictor.py:540-547 does. */
 
+/* ---- audio-offset sweep: one visual-encoder pass, K audio windows per video ------------------------------------ */
+/* The reference trains with torch.roll-shifted audio as sync negatives (train.py:169-182), so its logit as a function of the
+ * audio offset is a sync profile: a real clip with a constant A/V delay peaks away from offset 0, a lip-sync fake has no clear
+ * peak.  Scoring K audio windows against one video this way repeats only the audio-dependent part of LipSyncModel.forward
+ * (lip_sync_model.py:86-136): the audio encoder, the cross-modal attention + temporal transformer and the classifier head.  The
+ * visual encoder and the artifact branch run once per video.
+ * The logit of (b, k) is bit for bit what lsd_forward gives video b with audio window k (same precision).  The tensor-core route
+ * with the fused token kernels shares the video side; every other configuration (fp32, the launch-by-launch token path) runs one
+ * lsd_forward per audio window, with the same results. */
+#define LSD_MAX_AUDIO_VARIANTS 64
+/* video as in lsd_forward; audio: device (B,K,1,F,Ta), window k of video b at row b*K + k; logits_out: device (B,K) fp32.
+ * LSD_ERR_SHAPE for K < 1 or K > LSD_MAX_AUDIO_VARIANTS. */
+size_t lsd_forward_audio_variants_workspace_bytes(lsd_handle* h, int B, int K, int T, int H, int W, int F, int Ta, int precision);
+int lsd_forward_audio_variants(lsd_handle* h, const void* video, int video_dtype, int video_layout,
+                               const void* audio, int audio_dtype,
+                               int B, int K, int T, int H, int W, int F, int Ta, int precision,
+                               float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
+/* lsd_score_windows with K audio offsets per window (Predictor._align_audio_chunk, predictor.py:525-552, moved by whole mel
+ * columns).  offsets_host: K int32 offsets d in mel columns (10 ms; d > 0 = the audio slice starts later).  Window i with base
+ * audio start a_i (computed, or audio_starts_host_or_null[i], exactly as lsd_score_windows does) reads its slice for offset d
+ * at clamp(a_i + d): past the end -> Ta_full - Ta, then never below 0 — the rule lsd_score_windows applies.  (i, k) is valid
+ * when no clamping was needed: 0 <= a_i + d_k <= Ta_full - Ta.
+ * logits_out: device (n_windows, K) fp32, entry (i, k) bit for bit lsd_score_windows for window i with the effective start
+ * as its explicit audio start.  eff_audio_starts_host_or_null: host (n_windows, K) int32 effective starts, written before any
+ * GPU work is enqueued.  LSD_ERR_ARG for offsets_host == NULL, LSD_ERR_SHAPE for K out of range or a window outside the track. */
+size_t lsd_score_offsets_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision);
+int lsd_score_offsets(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                      const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                      const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                      const int32_t* offsets_host, int K, int precision, int batch,
+                      float* logits_out, int32_t* eff_audio_starts_host_or_null,
+                      void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- speaking alignment / mouth motion: the per-window numpy loops of _predict_long_video ------------------ */
 /* Frame-difference energies of a track (Predictor._speaking_alignment_score, app/inference/predictor.py:339-345, and
  * _mouth_motion_energy_check, :395-402): for every frame pair f in [0, n_frames-1)

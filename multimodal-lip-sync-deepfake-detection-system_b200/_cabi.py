@@ -18,6 +18,7 @@ LSD_OK, LSD_ERR_SHAPE, LSD_ERR_ARG, LSD_ERR_WEIGHTS, LSD_ERR_CUDA, LSD_ERR_WORKS
 LSD_F32, LSD_F16, LSD_BF16, LSD_U8, LSD_I64 = 0, 1, 2, 3, 4
 LSD_NCDHW, LSD_NDHWC = 0, 1
 LSD_PREC_FP32, LSD_PREC_BF16 = 0, 1
+LSD_MAX_AUDIO_VARIANTS = 64
 
 # every symbol include/lsd_b200.h declares (checked by tests/test_cabi.py)
 EXPORTS = [
@@ -28,6 +29,7 @@ EXPORTS = [
     "lsd_audio_encoder_workspace_bytes", "lsd_audio_encoder", "lsd_token_path_workspace_bytes", "lsd_token_path",
     "lsd_track_motion", "lsd_speech_stats", "lsd_vad_frames", "lsd_frame_energy", "lsd_vad_mask",
     "lsd_workspace_invalidate", "lsd_planar_stage_read", "lsd_state_generation", "lsd_host_pack_u8_exact", "lsd_host_pack_u8_begin", "lsd_host_pack_u8_end", "lsd_host_pack_last_ms", "lsd_expand_u8",
+    "lsd_forward_audio_variants_workspace_bytes", "lsd_forward_audio_variants", "lsd_score_offsets_workspace_bytes", "lsd_score_offsets",
 ]
 
 
@@ -93,6 +95,13 @@ def lib() -> C.CDLL:
         L.lsd_host_pack_last_ms.argtypes = []; L.lsd_host_pack_last_ms.restype = C.c_double
         L.lsd_expand_u8.argtypes = [vp, vp, i64, vp]; L.lsd_expand_u8.restype = i
         L.lsd_planar_stage_read.argtypes = [vp, C.c_char_p, C.c_char_p, vp, vp, i64, i, i, vp]; L.lsd_planar_stage_read.restype = i
+        L.lsd_forward_audio_variants_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_forward_audio_variants_workspace_bytes.restype = sz
+        L.lsd_forward_audio_variants.argtypes = [vp, vp, i, i, vp, i, i, i, i, i, i, i, i, i, vp, vp, sz, vp]
+        L.lsd_forward_audio_variants.restype = i
+        L.lsd_score_offsets_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_offsets_workspace_bytes.restype = sz
+        L.lsd_score_offsets.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
+                                        C.POINTER(C.c_int32), i, i, i, vp, C.POINTER(C.c_int32), vp, sz, vp]
+        L.lsd_score_offsets.restype = i
         _lib = L
         return L
 

@@ -29,6 +29,29 @@ def _robust(conf: Sequence[float], smoothing: str, trim_ratio: float) -> float:
     return float(np.sort(arr)[k: n - k].mean())
 
 
+def av_offset_profile(confs, valid, offsets: Sequence[int], smoothing: str = "median", trim_ratio: float = 0.1) -> Dict[str, Any]:
+    """Sync profile of an audio-offset sweep.  `confs` / `valid`: (n_windows, K) calibrated confidences and the mask of entries
+    whose audio slice needed no clamping; `offsets`: the K offsets (mel columns).  Per offset, the robust aggregate of the valid
+    windows (`_robust`, the window aggregation of predictor.py:246-260) or None when no window is valid there.  `best_offset`:
+    the argmax; ties go to the smaller |d|, then the smaller d.  `confidence_at_zero` / `margin` are None when offset 0 is
+    not in the sweep or has no valid window."""
+    conf = np.asarray(confs, dtype=np.float32).reshape(-1, len(offsets))
+    ok = np.asarray(valid, dtype=bool).reshape(conf.shape)
+    profile: List[Optional[float]] = []
+    for k in range(len(offsets)):
+        sel = conf[ok[:, k], k]
+        profile.append(_robust(sel.tolist(), smoothing, trim_ratio) if sel.size else None)
+    scored = [(p, int(d)) for p, d in zip(profile, offsets) if p is not None]
+    best = max(scored, key=lambda pd: (pd[0], -abs(pd[1]), -pd[1])) if scored else None
+    at_zero = next((p for p, d in zip(profile, offsets) if int(d) == 0), None)
+    return {
+        "offsets": [int(d) for d in offsets], "profile": profile, "n_valid": [int(x) for x in ok.sum(axis=0)],
+        "best_offset": best[1] if best else None, "best_confidence": best[0] if best else None,
+        "confidence_at_zero": at_zero,
+        "margin": (best[0] - at_zero) if (best is not None and at_zero is not None) else None,
+    }
+
+
 def _speech_weighted(conf: Sequence[float], speaking: Sequence[float], vad: Optional[Sequence[float]], smoothing: str,
                      trim_ratio: float) -> float:
     # predictor.py:262-293

@@ -296,28 +296,34 @@ struct BPlan {
   }
 };
 
-void build_plan(const Shapes& s, BPlan& P) {
+// video = false: the audio side of the shared-visual forward (see VarTail), which runs the audio encoder and the fused token
+// kernels only: no video input, no visual-encoder, visual-token, aux or launch-by-launch token-path buffers
+void build_plan(const Shapes& s, BPlan& P, bool video = true) {
   P.s = s;
   Plan& p = P.f32;
   const int64_t B = s.B, T = s.T, TA = s.A4;
-  p.add("vid", B * T * s.H * s.W * 3);     // only used by the uint8-track window builder (lsd_score_windows)
+  if (video) p.add("vid", B * T * s.H * s.W * 3);     // only used by the uint8-track window builder (lsd_score_windows)
   p.add("aud", B * s.F * s.Ta);
-  p.add("v_feat", B * T * 256);
+  if (video) p.add("v_feat", B * T * 256);
   p.add("a_feat", B * TA * 256);
+  if (video) {
   p.add("v_emb", B * T * 256);
   p.add("a_emb", B * TA * 256);
   p.add("a_int", B * T * 256);
   p.add("proj_v", B * T * 768);
   p.add("proj_a", B * T * 768);
   p.add("vcomb", B * T * 1024);            // [v_emb | in-projection of the visual tokens] per token (fused token path)
+  }
   p.add("acomb", B * T * 1024);            // [interpolated a_emb | in-projection of the interpolated audio tokens]
   p.add("a_fint", B * T * 256);            // audio features interpolated to T tokens
   p.add("gate_in", B * T * 512);
-  p.add("gate_h", B * T * 256);
+  if (video) p.add("gate_h", B * T * 256);
   p.add("fused", B * T * 256);
   p.add("tok", B * (T + 1) * 256);
+  if (video) {
   p.add("tok_qkv", B * (T + 1) * 768);
   p.add("comb", B * 448);
+  }
   // planar bf16 buffers
   P.planar_begin = (p.cursor + 255) & ~size_t(255);
   const int Bn = s.B, Tn = s.T;
@@ -327,6 +333,7 @@ void build_plan(const Shapes& s, BPlan& P) {
   // (row = 2 zero units + W/2 data units: the 2 leading units of the NEXT row are this row's right padding — the 7-tap window of the
   //  last output reaches one unit past the data — so the row pitch is W/2 + 2, not W/2 + 4: 4 % fewer positions for the stem and hf0)
   const UcGeom gs = make_geom_ex(Bn, Tn, s.Hs, s.Ws, 1, 2, 0, 0, 2);
+  if (video) {
   P.addp("xs", 8, 2, gs);
   P.addp("xl", 8, 2, gs);
   P.addp("s_out", 64, 1, gs);    // stem conv output (stem geometry), before the max-pool
@@ -350,6 +357,7 @@ void build_plan(const Shapes& s, BPlan& P) {
   P.addp("artd_b", 64, 1, gd);
   P.addp("hf_f", 32, 4, gh);
   P.addp("hf_b", 64, 1, gh);
+  }
   // audio encoder: 2-D geometries (one slab per window, no temporal padding)
   const UcGeom as = make_geom_ex(Bn, 1, s.Fs, s.As, 0, 2, 0, 0, 4);
   auto g2d = [&](int H, int W) { return make_geom_ex(Bn, 1, H, W, 0, 1, 0, 1, 0); };
@@ -375,6 +383,7 @@ void build_plan(const Shapes& s, BPlan& P) {
   for (const char* sfx : {"", "_lo"}) {
     auto nm = [&](const char* n) { return std::string(n) + sfx; };
     P.addp(nm("afeat_p").c_str(), 256, 1, P.gta);
+    if (!video) { P.addp(nm("afint_p").c_str(), 256, 1, P.gt); continue; }
     for (const char* n : {"vfeat_p", "vemb_p", "aint_p", "afint_p", "att1_p", "att2_p", "blend_p", "fused_p"}) P.addp(nm(n).c_str(), 256, 1, P.gt);
     P.addp(nm("gatein_p").c_str(), 512, 1, P.gt);
     P.addp(nm("mscat_p").c_str(), 768, 1, P.gt);
@@ -1342,7 +1351,8 @@ static bool token_front_enabled(int T) {
   const char* e = getenv("LSD_TOK_FRONT");
   return !(e && atoi(e) == 0) && tok_front_supported(T);
 }
-static int token_path_bf16(const BCtx& b, const Shapes& s, bool combined = false) {
+// vcomb / K (shared-visual forward): the merged visual projection lives in another workspace, window w reads its row group w / K.
+static int token_path_bf16(const BCtx& b, const Shapes& s, bool combined = false, const float* vcomb = nullptr, int K = 1) {
   const BPlan& P = *b.P;
   auto pbf = [&](const char* n) -> const PBuf& { return P.pb.at(n); };
   cudaStream_t st = b.st;
@@ -1365,7 +1375,7 @@ static int token_path_bf16(const BCtx& b, const Shapes& s, bool combined = false
   auto fork = [&](int n) { if (par) { cudaEventRecord(h->ev_tok_fork, st); for (int i = 0; i < n; ++i) cudaStreamWaitEvent(h->tok_stream[i], h->ev_tok_fork, 0); } };
   auto join = [&](int n) { if (par) for (int i = 0; i < n; ++i) { cudaEventRecord(h->ev_tok_join[i], h->tok_stream[i]); cudaStreamWaitEvent(st, h->ev_tok_join[i], 0); } };
   // ---- cross-modal attention + gated fusion (fusion_module.py:54-87)
-  float *pv = b.f("proj_v"), *pa = b.f("proj_a"), *gi = b.f("gate_in");
+  float *pv = combined ? nullptr : b.f("proj_v"), *pa = combined ? nullptr : b.f("proj_a"), *gi = b.f("gate_in");   // (combined: tok_front reads vcomb / acomb)
   if (!combined) {
     fork(1);
     launch_lerp_tokens_p(b.f("a_emb"), b.f("a_int"), B, TA, T, 256, pout(b, pbf("aint_p"), &pbf("aint_p_lo")), b1.st);
@@ -1381,7 +1391,7 @@ static int token_path_bf16(const BCtx& b, const Shapes& s, bool combined = false
     TokFrontP fp;
     memset(&fp, 0, sizeof(fp));
     if (combined) {
-      fp.v_emb = b.f("vcomb"); fp.pv = fp.v_emb + 256; fp.a_int = b.f("acomb"); fp.pa = fp.a_int + 256;
+      fp.v_emb = vcomb ? vcomb : b.f("vcomb"); fp.pv = fp.v_emb + 256; fp.a_int = b.f("acomb"); fp.pa = fp.a_int + 256;
       fp.ld_e = 1024; fp.ld_p = 1024;
     } else {
       fp.pv = pv; fp.pa = pa; fp.v_emb = b.f("v_emb"); fp.a_int = b.f("a_int");
@@ -1390,7 +1400,7 @@ static int token_path_bf16(const BCtx& b, const Shapes& s, bool combined = false
     fp.gi = gi; fp.fused = b.f("fused"); fp.tok = tok;
     fp.w = reinterpret_cast<const __half*>(h->tokfr_w);
     fp.vec = h->tokfr_vec;
-    fp.B = B; fp.T = T;
+    fp.B = B; fp.T = T; fp.K = K;
     tok_front_geometry(T, fp.SL, fp.G, fp.KW);
     if (getenv("LSD_TOKF_TRACE")) {
       // debug: phase timestamps of CTA 0 (compute warp 0: start, then [hand-over, next accumulator arrival] per phase; MMA warp:
@@ -1491,16 +1501,17 @@ static int token_path_bf16(const BCtx& b, const Shapes& s, bool combined = false
 
 
 // Zero padding of the planar buffers lives in the workspace across calls: kernels only ever write valid positions (or zeros at
-// pad positions), so a workspace whose padding was initialised for these shapes is reused as is.  Two (pointer, bytes, shapes)
-// signatures are remembered — slot 1 belongs to the second half of a pipelined lsd_score_windows call, slot 0 to everything
-// else.  A call invalidates the OTHER slot whenever its byte range overlaps this call's workspace (a forward with other shapes
-// through the same memory overwrites that half's padding), and lsd_workspace_invalidate() drops both (the caller reused or
-// freed the memory between calls).
+// pad positions), so a workspace whose padding was initialised for these shapes is reused as is.  Three (pointer, bytes, shapes)
+// signatures are remembered — slot 1 belongs to the second half of a pipelined lsd_score_windows call or to the audio groups of a
+// shared-visual forward, slot 2 to the shorter last audio group of one (see VarTail), slot 0 to everything else.  A call
+// invalidates every OTHER slot whose byte range overlaps this call's workspace (a forward with other shapes through the same
+// memory overwrites that region's padding), and lsd_workspace_invalidate() drops all of them (the caller reused or freed the
+// memory between calls).
 static int ws_prepare(lsd_handle* h, const Shapes& s, const BPlan& P, char* ws, size_t ws_bytes, cudaStream_t st, int slot) {
   const int sig[6] = {s.B, s.T, s.H, s.W, s.F, s.Ta};
   WsSig& mine = h->ws_sig[slot];
-  WsSig& other = h->ws_sig[slot ^ 1];
-  if (other.ptr) {
+  for (WsSig& other : h->ws_sig) {
+    if (&other == &mine || !other.ptr) continue;
     const char* o0 = reinterpret_cast<const char*>(other.ptr);
     if (o0 < ws + ws_bytes && ws < o0 + other.bytes) other.ptr = nullptr;
   }
@@ -1511,11 +1522,32 @@ static int ws_prepare(lsd_handle* h, const Shapes& s, const BPlan& P, char* ws, 
   return 0;
 }
 
+// Audio side of the shared-visual forward (lsd_forward_audio_variants / lsd_score_offsets): K audio windows per video, window-major
+// rows (row = b*K + k).  The visual front runs once at B; audio encoder, token path and head run at B*K in groups of gB videos
+// (gB*K rows: bounded workspace, and each group's logits are one contiguous block of the (B, K) output) on a plan without video
+// buffers in a workspace of their own.  A call's groups all hold gB videos except possibly the last one, which has a region of
+// its own: each region keeps the zero padding of one plan shape, so repeated calls never re-zero either.
+struct VarTail {
+  int K = 1, gB = 1;
+  char* ws = nullptr;                 // workspace of the audio plan of a full group (gB*K rows; ws_prepare slot 1) ...
+  size_t ws_bytes = 0;
+  char* ws_last = nullptr;            // ... and of a shorter last group (< gB*K rows; slot 2)
+  size_t ws_last_bytes = 0;
+  const void* audio = nullptr;        // tensor entry: (B*K, 1, F, Ta) clips of dtype adt ...
+  int adt = LSD_F32;
+  const float* mel_full = nullptr;    // ... or track entry: B*K mel start columns into the clip log-mel (audio == nullptr)
+  int Ta_full = 0;
+  const int32_t* d_astarts = nullptr;
+};
+
+static size_t dtype_bytes(int dt) { return dt == LSD_F32 ? 4 : (dt == LSD_U8 ? 1 : 2); }
+
 // pipe_parity >= 0 (lsd_score_windows with a double workspace): everything after the visual encoder is enqueued on
 // h->tail_stream, ordered after the encoder by ev_front[parity]; ev_tail_done[parity] marks the batch's logits complete.
+// vt != nullptr: shared-visual forward (see VarTail); requires the fused token path (variants_shared_route) and no aux.
 static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, const lsd_aux* aux, char* ws, size_t ws_bytes,
                              cudaStream_t st, bool inputs_ready, const void* video, int vdt, int vlayout, const void* audio, int adt,
-                             const int32_t* vstarts = nullptr, int n_frames = 0, int pipe_parity = -1) {
+                             const int32_t* vstarts = nullptr, int n_frames = 0, int pipe_parity = -1, const VarTail* vt = nullptr) {
   BPlan P;
   build_plan(s, P);
   if (P.f32.cursor > ws_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", P.f32.cursor, ws_bytes);
@@ -1556,22 +1588,58 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   // [a_int | cross-attention in-projection] (see pack_comb_proj in lsd_api.cu), plus a_emb itself for the aux / stage output —
   // runs right behind the audio encoder, on its stream, long before the visual encoder is done.
   const bool tcomb = token_front_enabled(T);
-  auto audio_tokens = [&](const BCtx& c) -> int {
+  auto audio_tokens = [&](const BCtx& c, const Shapes& sc) -> int {
     int rc = 0;
-    launch_lerp_tokens_p(c.f("a_feat"), c.f("a_fint"), B, TA, T, 256, pout(c, pb["afint_p"], &pb["afint_p_lo"]), c.st);
-    RUNC(c, "cross.acomb", a_.in = &pb["afint_p"]; a_.in_lo = &pb["afint_p_lo"]; a_.og = P.gt; a_.y32 = c.f("acomb"); a_.y32_ld = 1024);
+    const auto& q = c.P->pb;
+    launch_lerp_tokens_p(c.f("a_feat"), c.f("a_fint"), sc.B, sc.A4, sc.T, 256, pout(c, q.at("afint_p"), &q.at("afint_p_lo")), c.st);
+    RUNC(c, "cross.acomb", a_.in = &q.at("afint_p"); a_.in_lo = &q.at("afint_p_lo"); a_.og = c.P->gt; a_.y32 = c.f("acomb"); a_.y32_ld = 1024);
     // a_emb itself (TA tokens per window) is an aux output only: the token path consumes the interpolated rows above
-    if (aux && aux->audio_tokens) RUNC(c, "projection.audio_proj", a_.in = &pb["afeat_p"]; a_.in_lo = &pb["afeat_p_lo"]; a_.og = P.gta; a_.y32 = c.f("a_emb"); a_.y32_ld = 256);
+    if (aux && aux->audio_tokens) RUNC(c, "projection.audio_proj", a_.in = &q.at("afeat_p"); a_.in_lo = &q.at("afeat_p_lo"); a_.og = c.P->gta; a_.y32 = c.f("a_emb"); a_.y32_ld = 256);
     return 0;
+  };
+  // shared-visual forward: plans of the audio groups (the last group may hold fewer videos) and the audio side of group g
+  const int n_groups = vt ? (B + vt->gB - 1) / vt->gB : 0;
+  const bool short_last = vt && B - (n_groups - 1) * vt->gB < vt->gB;   // the last group holds fewer than gB videos
+  auto plan_of = [&](int g) { return short_last && g == n_groups - 1 ? 1 : 0; };
+  Shapes sA[2];
+  BPlan PA[2];
+  char* aws[2] = {nullptr, nullptr};
+  if (vt) {
+    aws[0] = vt->ws; aws[1] = vt->ws_last;
+    for (int i = 0; i < 2; ++i) {
+      if (i != plan_of(0) && i != plan_of(n_groups - 1)) continue;
+      const int nb = i == 0 ? vt->gB : B - (n_groups - 1) * vt->gB;
+      const size_t cap = i == 0 ? vt->ws_bytes : vt->ws_last_bytes;
+      if ((rc = make_shapes(h, nb * vt->K, T, 16, 16, s.F, s.Ta, sA[i]))) return rc;
+      build_plan(sA[i], PA[i], false);
+      if (!aws[i] || PA[i].f32.cursor > cap) return lsd_fail(h, LSD_ERR_WORKSPACE, "audio-variant workspace too small: need %zu bytes, got %zu", PA[i].f32.cursor, cap);
+    }
+  }
+  auto var_audio = [&](int g, cudaStream_t stream, int max_ctas) -> int {
+    const int pi = plan_of(g);
+    int rc = ws_prepare(h, sA[pi], PA[pi], aws[pi], pi ? vt->ws_last_bytes : vt->ws_bytes, stream, 1 + pi);
+    if (rc) return rc;
+    BCtx c{h, aws[pi], &PA[pi], stream};
+    c.max_ctas = max_ctas;
+    const size_t r0 = (size_t)g * vt->gB * vt->K;
+    if (vt->d_astarts) launch_gather_audio(vt->mel_full, s.F, vt->Ta_full, vt->d_astarts + r0, c.f("aud"), sA[pi].B, s.Ta, stream);
+    const void* au = vt->audio ? reinterpret_cast<const char*>(vt->audio) + r0 * s.F * s.Ta * dtype_bytes(vt->adt) : nullptr;
+    if ((rc = audio_encoder_bf16(c, sA[pi], vt->d_astarts != nullptr, au, vt->adt))) return rc;
+    return audio_tokens(c, sA[pi]);
   };
   g_tl.on = LSD_ENV("LSD_TIMELINE") != nullptr;
   g_tl.mark(st, "start");
   const bool audio_after_rows = LSD_ENV("LSD_AUDIO_AFTER_ROWS") && atoi(LSD_ENV("LSD_AUDIO_AFTER_ROWS")) != 0;   // tuning knob, see below
-  if (audio_early && !audio_after_rows) {
+  if (vt) {                             // the first audio group takes the audio encoder's place next to the visual encoder
+    cudaEventRecord(h->ev_start, st);
+    cudaStreamWaitEvent(sst, h->ev_start, 0);
+    if ((rc = var_audio(0, sst, bs.max_ctas))) return rc;
+    cudaEventRecord(h->ev_audio, sst);
+  } else if (audio_early && !audio_after_rows) {
     cudaEventRecord(h->ev_start, st);
     cudaStreamWaitEvent(sst, h->ev_start, 0);
     if ((rc = audio_encoder_bf16(bs, s, inputs_ready, audio, adt))) return rc;
-    if (tcomb && (rc = audio_tokens(bs))) return rc;
+    if (tcomb && (rc = audio_tokens(bs, s))) return rc;
     g_tl.mark(sst, "S:audio_enc");
     cudaEventRecord(h->ev_audio, sst);
   }
@@ -1588,11 +1656,11 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   // (timeline at B=64: head at 2543 instead of 2665 us).  Back to back the early fork wins: scripts/exp_ab.py, 40 / 400 forwards:
   // 2.69 / 2.86 ms per forward against 2.73 / 2.89 — the audio encoder of forward k+1 then fills the SMs the tail of forward k
   // leaves idle.  Throughput is the metric, so the early fork stays the default.)
-  if (audio_early && audio_after_rows) {
+  if (!vt && audio_early && audio_after_rows) {
     cudaEventRecord(h->ev_start, st);
     cudaStreamWaitEvent(sst, h->ev_start, 0);
     if ((rc = audio_encoder_bf16(bs, s, inputs_ready, audio, adt))) return rc;
-    if (tcomb && (rc = audio_tokens(bs))) return rc;
+    if (tcomb && (rc = audio_tokens(bs, s))) return rc;
     g_tl.mark(sst, "S:audio_enc");
     cudaEventRecord(h->ev_audio, sst);
   }
@@ -1750,12 +1818,33 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   {
   BCtx b{h, ws, &P, tst};
   cudaStream_t st = tst;
+  HeadW hw;
+  auto cw = [&](const char* key) { return h->warena + h->convs.at(key).w_off; };
+  auto cb = [&](const char* key) { return h->warena + h->convs.at(key).shift_off; };
+  hw.w0 = cw("art.fuse0"); hw.b0 = cb("art.fuse0"); hw.w2 = cw("art.fuse2"); hw.b2 = cb("art.fuse2");
+  hw.wc = cw("head.fc0"); hw.bc = cb("head.fc0");
+  hw.lng = b.W("head.ln.w"); hw.lnb = b.W("head.ln.b"); hw.wo = b.W("head.out.w"); hw.bo = b.W("head.out.b");
+  if (vt) {
+    // token path + head per audio group: row b*K + k reads the visual projection and artifact features of video b
+    RUN("cross.vcomb", a_.in = &pb["vfeat_p"]; a_.in_lo = &pb["vfeat_p_lo"]; a_.og = P.gt; a_.y32 = b.f("vcomb"); a_.y32_ld = 1024);
+    for (int g = 0; g < n_groups; ++g) {
+      if (g == 0) cudaStreamWaitEvent(st, h->ev_audio, 0);
+      else if ((rc = var_audio(g, st, 0))) return rc;       // (the previous group's token path and head are done with this workspace)
+      const int pi = plan_of(g), b0 = g * vt->gB;
+      BCtx c{h, aws[pi], &PA[pi], st};
+      if ((rc = token_path_bf16(c, sA[pi], true, b.f("vcomb") + (size_t)b0 * T * 1024, vt->K))) return rc;
+      if (g == 0) cudaStreamWaitEvent(st, h->ev_join, 0);   // artifact features (comb[:, 256:448]) are complete
+      launch_head(c.f("tok"), (int64_t)NT * 256, comb + (size_t)b0 * 448, hw, logits + (size_t)b0 * vt->K, sA[pi].B, st, vt->K);
+    }
+    if (pipe_parity >= 0) cudaEventRecord(h->ev_tail_done[pipe_parity], st);
+    return 0;
+  }
   if (!audio_early) { if ((rc = audio_encoder_bf16(b, s, inputs_ready, audio, adt))) return rc; }
   // ---- projection (fusion_module.py:108-124)
   const UcGeom gt = P.gt;
   if (tcomb) {
     // fused token path: one GEMM gives [v_emb | cross-attention in-projection] per visual token (the audio half ran behind the audio encoder)
-    if (!audio_early) { if ((rc = audio_tokens(b))) return rc; }
+    if (!audio_early) { if ((rc = audio_tokens(b, s))) return rc; }
     RUN("cross.vcomb", a_.in = &pb["vfeat_p"]; a_.in_lo = &pb["vfeat_p_lo"]; a_.og = gt; a_.y32 = b.f("vcomb"); a_.y32_ld = 1024);
     if (audio_early) cudaStreamWaitEvent(st, h->ev_audio, 0);   // [a_int | in-projection] of the audio tokens is complete
   } else {
@@ -1770,12 +1859,6 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   // cls = tok[:,0]: no final norm (temporal.py:110-111); the head reads the CLS rows in place
   cudaStreamWaitEvent(st, h->ev_join, 0);   // artifact features (comb[:, 256:448]) are complete
   // ---- artifact fusion MLP + classification head, fused, fp32 (artifact_detector.py:142-147,180-181; classifier.py:14-34)
-  HeadW hw;
-  auto cw = [&](const char* key) { return h->warena + h->convs.at(key).w_off; };
-  auto cb = [&](const char* key) { return h->warena + h->convs.at(key).shift_off; };
-  hw.w0 = cw("art.fuse0"); hw.b0 = cb("art.fuse0"); hw.w2 = cw("art.fuse2"); hw.b2 = cb("art.fuse2");
-  hw.wc = cw("head.fc0"); hw.bc = cb("head.fc0");
-  hw.lng = b.W("head.ln.w"); hw.lnb = b.W("head.ln.b"); hw.wo = b.W("head.out.w"); hw.bo = b.W("head.out.b");
   launch_head(tok, (int64_t)NT * 256, comb, hw, logits, B, st);
   g_tl.mark(st, "T:head");
   g_tl.dump();
@@ -1908,4 +1991,90 @@ int score_batch_bf16(lsd_handle* h, const uint8_t* track, int n_frames, const in
     return forward_bf16_impl(h, s, logits, nullptr, ws, ws_bytes, st, true, track, LSD_U8, LSD_NDHWC, nullptr, 0, d_vstarts, n_frames, pipe_parity);
   launch_gather_windows_u8(track, n_frames, d_vstarts, b.f("vid"), nb, T, H * W * 3, st);
   return forward_bf16_impl(h, s, logits, nullptr, ws, ws_bytes, st, true, nullptr, 0, 0, nullptr, 0, nullptr, 0, pipe_parity);
+}
+
+// ---- shared-visual forward (lsd_forward_audio_variants / lsd_score_offsets)
+// The route needs the fused token kernels (tok_front reads the visual rows of its window group); every other configuration
+// scores one plain forward per audio variant instead (lsd_api.cu).
+bool variants_shared_route(int T) {
+  const char* fe = getenv("LSD_TOK_FUSED");
+  return token_front_enabled(T) && !(fe && atoi(fe) == 0) && tok_fused_supported(T + 1);
+}
+
+// Videos per audio group: at most LSD_VARIANT_ROWS (default 512) rows of B*K run through the audio side at once.  A group holds
+// whole videos, so its logits are a contiguous block of the (B, K) output; results do not depend on the grouping.
+static int variants_group(int B, int K) {
+  int cap = 512;
+  if (const char* e = getenv("LSD_VARIANT_ROWS")) cap = std::max(1, atoi(e));
+  const int per = std::max(1, cap / K);
+  const int n_groups = (B + per - 1) / per;
+  return std::max(1, (B + n_groups - 1) / n_groups);   // equal groups where B allows it: one audio plan for every group
+}
+
+static size_t variants_visual_bytes(const Shapes& s) {
+  BPlan P;
+  build_plan(s, P);
+  return (P.f32.cursor + 255) & ~size_t(255);
+}
+
+// audio plan of `rows` rows (see VarTail), 256-byte aligned; 0 for rows < 1
+static size_t variants_audio_bytes(int rows, int T, int F, int Ta) {
+  Shapes sa;
+  if (rows < 1 || make_shapes(nullptr, rows, T, 16, 16, F, Ta, sa) != 0) return 0;
+  BPlan PA;
+  build_plan(sa, PA, false);
+  return (PA.f32.cursor + 255) & ~size_t(255);
+}
+
+// Every call with at most `B` videos fits: the groups are sized from B (variants_group), a call with fewer videos keeps that
+// group size, and its shorter last group (at most gB - 1 videos) has its own region.
+size_t variants_bf16_bytes(lsd_handle* h, int B, int K, int T, int H, int W, int F, int Ta) {
+  Shapes s;
+  if (B < 1 || K < 1 || make_shapes(h, B, T, H, W, F, Ta, s) != 0) return 0;
+  const int gB = variants_group(B, K);
+  const size_t a0 = variants_audio_bytes(gB * K, T, F, Ta);
+  if (a0 == 0) return 0;
+  return variants_visual_bytes(s) + a0 + variants_audio_bytes((gB - 1) * K, T, F, Ta) + 256;
+}
+
+// ws: [visual plan at nb videos | audio plan of a full group | audio plan of a shorter last group].  plan_B: the largest call the
+// workspace was sized for (variants_bf16_bytes); the group size follows it, not nb, so a short last batch stays within the sizing.
+static int variants_run(lsd_handle* h, const Shapes& s, int plan_B, VarTail& vt, float* logits, char* ws, size_t ws_bytes, cudaStream_t st,
+                        bool inputs_ready, const void* video, int vdt, int vlayout, const int32_t* vstarts, int n_frames) {
+  const size_t vb = variants_visual_bytes(s);
+  vt.gB = variants_group(plan_B, vt.K);
+  const size_t a0 = variants_audio_bytes(vt.gB * vt.K, s.T, s.F, s.Ta);
+  if (vb + a0 > ws_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need more than %zu bytes, got %zu", vb + a0, ws_bytes);
+  vt.ws = ws + vb;
+  vt.ws_bytes = a0;
+  vt.ws_last = ws + vb + a0;
+  vt.ws_last_bytes = ws_bytes - vb - a0;
+  return forward_bf16_impl(h, s, logits, nullptr, ws, vb, st, inputs_ready, video, vdt, vlayout, nullptr, 0, vstarts, n_frames, -1, &vt);
+}
+
+int forward_variants_bf16(lsd_handle* h, int B, int K, int T, int H, int W, int F, int Ta, const void* video, int vdt, int vlayout,
+                          const void* audio, int adt, float* logits, char* ws, size_t ws_bytes, cudaStream_t st) {
+  Shapes s;
+  int rc = make_shapes(h, B, T, H, W, F, Ta, s);
+  if (rc) return rc;
+  VarTail vt;
+  vt.K = K; vt.audio = audio; vt.adt = adt;
+  return variants_run(h, s, B, vt, logits, ws, ws_bytes, st, false, video, vdt, vlayout, nullptr, 0);
+}
+
+int score_offsets_batch_bf16(lsd_handle* h, const uint8_t* track, int n_frames, const int32_t* d_vstarts, const int32_t* d_astarts,
+                             const float* mel_full, int Ta_full, int nb, int batch, int K, int T, int H, int W, int F, int Ta, float* logits,
+                             char* ws, size_t ws_bytes, cudaStream_t st) {
+  Shapes s;
+  int rc = make_shapes(h, nb, T, H, W, F, Ta, s);
+  if (rc) return rc;
+  VarTail vt;
+  vt.K = K; vt.mel_full = mel_full; vt.Ta_full = Ta_full; vt.d_astarts = d_astarts;
+  if (video_rows_bulk_ok(track, LSD_U8, LSD_NDHWC, W))
+    return variants_run(h, s, batch, vt, logits, ws, ws_bytes, st, true, track, LSD_U8, LSD_NDHWC, d_vstarts, n_frames);
+  BPlan P;
+  build_plan(s, P);
+  BCtx b{h, ws, &P, st};
+  launch_gather_windows_u8(track, n_frames, d_vstarts, b.f("vid"), nb, T, H * W * 3, st);
+  return variants_run(h, s, batch, vt, logits, ws, ws_bytes, st, true, nullptr, 0, 0, nullptr, 0);
 }

@@ -4,6 +4,7 @@
 #include "lsd_kernels.h"
 #include "lsd_internal.h"
 
+#include <algorithm>
 #include <cmath>
 #include <initializer_list>
 #include <cstdarg>
@@ -385,6 +386,38 @@ int check_dtype(lsd_handle* h, int dt, const char* what) {
   return 0;
 }
 
+// First mel column of an audio window of Ta columns that must end inside the clip (predictor.py:540-547): past the end -> the
+// last full window, then never before column 0.
+long clamp_audio_start(long a_start, int Ta, int Ta_full) {
+  if (a_start + Ta > Ta_full) a_start = Ta_full - Ta;
+  return a_start < 0 ? 0 : a_start;
+}
+
+// Base audio start of window i: explicit, or a_start = int(round(v_start * a_ratio)) (round-half-even), clamped
+long base_audio_start(const int32_t* starts_host, const int32_t* audio_starts_host, int i, int Ta, int Ta_full, int total_v_frames) {
+  const double a_ratio = (double)Ta_full / (double)(total_v_frames > 1 ? total_v_frames : 1);
+  const long a = audio_starts_host ? (long)audio_starts_host[i] : (long)nearbyint((double)starts_host[i] * a_ratio);
+  return clamp_audio_start(a, Ta, Ta_full);
+}
+
+// dst row r = src row r, `width` 2-byte units per row (the per-variant route of the audio-variant entry points)
+__global__ void copy_rows_u16_kernel(const uint16_t* __restrict__ src, int64_t src_ld, uint16_t* __restrict__ dst, int64_t dst_ld,
+                                     int rows, int64_t width) {
+  const int64_t n = (int64_t)rows * width;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / width, c = i - r * width;
+    dst[r * dst_ld + c] = src[r * src_ld + c];
+  }
+}
+void copy_rows_bytes(const void* src, int64_t src_ld, void* dst, int64_t dst_ld, int rows, int64_t width, cudaStream_t st) {
+  const int64_t n = (int64_t)rows * (width / 2);
+  const int grid = (int)std::min<int64_t>((n + 255) / 256, 4096);
+  copy_rows_u16_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<const uint16_t*>(src), src_ld / 2, reinterpret_cast<uint16_t*>(dst), dst_ld / 2,
+                                             rows, width / 2);
+  count_launch();
+}
+size_t align256(size_t n) { return (n + 255) & ~size_t(255); }
+
 }  // namespace
 
 extern "C" int lsd_audio_tokens(int Ta) {
@@ -426,7 +459,7 @@ extern "C" int lsd_forward(lsd_handle* h, const void* video, int video_dtype, in
     make_plan_f32(s, p);
     if (p.cursor > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", p.cursor, workspace_bytes);
     h->stages = p.stages;
-    h->ws_sig[0].ptr = nullptr; h->ws_sig[1].ptr = nullptr;  // the fp32 plan overwrites any bf16 zero padding kept in this workspace
+    for (WsSig& w : h->ws_sig) w.ptr = nullptr;  // the fp32 plan overwrites any bf16 zero padding kept in this workspace
     rc = forward_f32(h, s, p, reinterpret_cast<char*>(workspace), aux, logits_out, st, false, video, video_dtype, video_layout, audio, audio_dtype);
     if (rc) return rc;
   }
@@ -469,14 +502,9 @@ extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_fram
   char* fws = ws + 2 * idx_bytes;
   // all window/audio starts are staged once (pinned-free small copies are ordered on the stream)
   h->idx_host.resize((size_t)2 * n_windows);
-  const double a_ratio = (double)Ta_full / (double)(total_v_frames > 1 ? total_v_frames : 1);
   for (int i = 0; i < n_windows; ++i) {
-    // predictor.py:540-547: a_start = int(round(v_start * a_ratio)) (round-half-even), clamped so the chunk ends inside the clip
-    long a_start = audio_starts_host ? (long)audio_starts_host[i] : (long)nearbyint((double)starts_host[i] * a_ratio);
-    if (a_start + Ta > Ta_full) { a_start = Ta_full - Ta; if (a_start < 0) a_start = 0; }
-    if (a_start < 0) a_start = 0;
     h->idx_host[i] = starts_host[i];
-    h->idx_host[n_windows + i] = (int32_t)a_start;
+    h->idx_host[n_windows + i] = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
   }
   // Cross-batch pipelining (tensor-core route, more than one batch, workspace >= 2 x lsd_score_workspace_bytes): batches
   // alternate between the two halves of the workspace; the tail of batch k (audio encoder, token path, head, artifact branch)
@@ -504,7 +532,7 @@ extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_fram
       Plan pb;
       make_plan_f32(sb, pb);
       h->stages = pb.stages;
-      h->ws_sig[0].ptr = nullptr; h->ws_sig[1].ptr = nullptr;
+      for (WsSig& w : h->ws_sig) w.ptr = nullptr;
       Ctx c{h, fws, &pb, st};
       launch_gather_windows_u8(track, n_frames, d_vs, c.buf("vid"), nb, T, H * W * 3, st);
       launch_gather_audio(mel_full, F, Ta_full, d_as, c.buf("aud"), nb, Ta, st);
@@ -515,6 +543,139 @@ extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_fram
   if (pipelined) {   // the caller's stream sees every batch's logits
     CUDA_OK(h, cudaStreamWaitEvent(st, h->ev_tail_done[0], 0));
     if (k >= 2) CUDA_OK(h, cudaStreamWaitEvent(st, h->ev_tail_done[1], 0));
+  }
+  CUDA_OK(h, cudaGetLastError());
+  return LSD_OK;
+}
+
+// ================================================================================================
+// Audio variants / offset sweep: K audio windows per video, the video side computed once (bf16_path.cu, VarTail).  Configurations
+// the shared route does not cover (fp32, the launch-by-launch token path) run one plain forward / lsd_score_windows per variant.
+// ================================================================================================
+namespace {
+int check_variants(lsd_handle* h, int K) {
+  if (K < 1 || K > LSD_MAX_AUDIO_VARIANTS) return lsd_fail(h, LSD_ERR_SHAPE, "K = %d audio variants: expected 1 <= K <= %d", K, LSD_MAX_AUDIO_VARIANTS);
+  return 0;
+}
+bool shared_route(int precision, int T) { return precision == LSD_PREC_BF16 && variants_shared_route(T); }
+}  // namespace
+
+extern "C" size_t lsd_forward_audio_variants_workspace_bytes(lsd_handle* h, int B, int K, int T, int H, int W, int F, int Ta, int precision) {
+  if (!h || B < 1 || K < 1 || K > LSD_MAX_AUDIO_VARIANTS) return 0;
+  if (shared_route(precision, T)) return variants_bf16_bytes(h, B, K, T, H, W, F, Ta);
+  const size_t fw = lsd_workspace_bytes(h, B, T, H, W, F, Ta, precision);   // per variant: plain forward + its clips + B logits
+  if (fw == 0) return 0;
+  return align256(fw) + align256((size_t)B * F * Ta * sizeof(float)) + align256((size_t)B * sizeof(float)) + 256;
+}
+
+extern "C" int lsd_forward_audio_variants(lsd_handle* h, const void* video, int video_dtype, int video_layout, const void* audio, int audio_dtype,
+                                          int B, int K, int T, int H, int W, int F, int Ta, int precision, float* logits_out,
+                                          void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_forward_audio_variants: no weights loaded");
+  int rc = check_variants(h, K);
+  if (rc) return rc;
+  Shapes s;
+  if ((rc = make_shapes(h, B, T, H, W, F, Ta, s))) return rc;
+  if (B == 0) return LSD_OK;
+  if (!video || !audio || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_forward_audio_variants: null pointer argument");
+  if ((rc = check_dtype(h, video_dtype, "video")) || (rc = check_dtype(h, audio_dtype, "audio"))) return rc;
+  if (audio_dtype == LSD_U8) return lsd_fail(h, LSD_ERR_ARG, "audio: uint8 log-mel is not supported");
+  if (video_layout != LSD_NCDHW && video_layout != LSD_NDHWC) return lsd_fail(h, LSD_ERR_ARG, "bad video layout %d", video_layout);
+  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
+  const size_t need = lsd_forward_audio_variants_workspace_bytes(h, B, K, T, H, W, F, Ta, precision);
+  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  char* ws = reinterpret_cast<char*>(workspace);
+  if (shared_route(precision, T)) {
+    if ((rc = forward_variants_bf16(h, B, K, T, H, W, F, Ta, video, video_dtype, video_layout, audio, audio_dtype, logits_out, ws,
+                                    workspace_bytes, st))) return rc;
+  } else {
+    const size_t fw = align256(lsd_workspace_bytes(h, B, T, H, W, F, Ta, precision));
+    const size_t clip = (size_t)F * Ta * (audio_dtype == LSD_F32 ? 4 : 2);
+    char* aud = ws + fw;
+    float* lg = reinterpret_cast<float*>(aud + align256((size_t)B * F * Ta * sizeof(float)));
+    for (int k = 0; k < K; ++k) {
+      copy_rows_bytes(reinterpret_cast<const char*>(audio) + k * clip, (int64_t)(K * clip), aud, (int64_t)clip, B, (int64_t)clip, st);
+      if ((rc = lsd_forward(h, video, video_dtype, video_layout, aud, audio_dtype, B, T, H, W, F, Ta, precision, lg, nullptr, ws, fw, stream)))
+        return rc;
+      copy_rows_bytes(lg, 4, logits_out + k, (int64_t)K * 4, B, 4, st);
+    }
+  }
+  CUDA_OK(h, cudaGetLastError());
+  return LSD_OK;
+}
+
+extern "C" size_t lsd_score_offsets_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  if (!h || batch < 1 || K < 1 || K > LSD_MAX_AUDIO_VARIANTS) return 0;
+  if (shared_route(precision, T)) {
+    const size_t fw = variants_bf16_bytes(h, batch, K, T, H, W, F, Ta);
+    if (fw == 0) return 0;
+    return align256((size_t)batch * sizeof(int32_t)) + align256((size_t)batch * K * sizeof(int32_t)) + fw + 256;
+  }
+  const size_t sw = lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);   // per offset: lsd_score_windows + batch logits
+  if (sw == 0) return 0;
+  return align256(sw) + align256((size_t)batch * sizeof(float)) + 256;
+}
+
+extern "C" int lsd_score_offsets(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                 const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full,
+                                 int total_v_frames, int Ta, const int32_t* offsets_host, int K, int precision, int batch, float* logits_out,
+                                 int32_t* eff_audio_starts_host, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_offsets: no weights loaded");
+  if (!offsets_host) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_offsets: offsets is NULL");
+  int rc = check_variants(h, K);
+  if (rc) return rc;
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_offsets: null pointer argument");
+  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_offsets: bad extents");
+  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
+  Shapes s;
+  if ((rc = make_shapes(h, batch, T, H, W, F, Ta, s))) return rc;
+  for (int i = 0; i < n_windows; ++i)
+    if (starts_host[i] < 0 || starts_host[i] + T > n_frames)
+      return lsd_fail(h, LSD_ERR_SHAPE, "window %d [%d,%d) is outside the %d-frame track", i, starts_host[i], starts_host[i] + T, n_frames);
+  const size_t need = lsd_score_offsets_workspace_bytes(h, batch, K, T, H, W, F, Ta, precision);
+  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  // effective start of (i, k): the base start of window i (as lsd_score_windows computes it) moved by offsets[k], clamped the same way
+  std::vector<int32_t> eff((size_t)n_windows * K);
+  for (int i = 0; i < n_windows; ++i) {
+    const long a = base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
+    for (int k = 0; k < K; ++k) eff[(size_t)i * K + k] = (int32_t)clamp_audio_start(a + offsets_host[k], Ta, Ta_full);
+  }
+  if (eff_audio_starts_host) memcpy(eff_audio_starts_host, eff.data(), eff.size() * sizeof(int32_t));
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  char* ws = reinterpret_cast<char*>(workspace);
+  if (shared_route(precision, T)) {
+    const size_t vi = align256((size_t)batch * sizeof(int32_t)), ai = align256((size_t)batch * K * sizeof(int32_t));
+    int32_t* d_vs = reinterpret_cast<int32_t*>(ws);
+    int32_t* d_as = reinterpret_cast<int32_t*>(ws + vi);
+    h->idx_host.resize((size_t)n_windows * (K + 1));   // staged here: the copies below are ordered on the stream
+    memcpy(h->idx_host.data(), starts_host, (size_t)n_windows * sizeof(int32_t));
+    memcpy(h->idx_host.data() + n_windows, eff.data(), eff.size() * sizeof(int32_t));
+    for (int w0 = 0; w0 < n_windows; w0 += batch) {
+      const int nb = std::min(batch, n_windows - w0);
+      CUDA_OK(h, cudaMemcpyAsync(d_vs, &h->idx_host[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      CUDA_OK(h, cudaMemcpyAsync(d_as, &h->idx_host[n_windows + (size_t)w0 * K], (size_t)nb * K * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      if ((rc = score_offsets_batch_bf16(h, track, n_frames, d_vs, d_as, mel_full, Ta_full, nb, batch, K, T, H, W, F, Ta, logits_out + (size_t)w0 * K,
+                                         ws + vi + ai, workspace_bytes - vi - ai, st))) return rc;
+    }
+  } else {
+    const size_t sw = align256(lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision));
+    float* lg = reinterpret_cast<float*>(ws + sw);
+    std::vector<int32_t> col(batch);
+    for (int w0 = 0; w0 < n_windows; w0 += batch) {
+      const int nb = std::min(batch, n_windows - w0);
+      for (int k = 0; k < K; ++k) {
+        for (int i = 0; i < nb; ++i) col[i] = eff[(size_t)(w0 + i) * K + k];
+        if ((rc = lsd_score_windows(h, track, n_frames, H, W, starts_host + w0, col.data(), nb, T, mel_full, F, Ta_full, total_v_frames, Ta,
+                                    precision, batch, lg, ws, sw, stream))) return rc;
+        copy_rows_bytes(lg, 4, logits_out + (size_t)w0 * K + k, (int64_t)K * 4, nb, 4, st);
+      }
+    }
   }
   CUDA_OK(h, cudaGetLastError());
   return LSD_OK;
@@ -614,13 +775,9 @@ extern "C" int lsd_speech_stats(lsd_handle* h, const float* motion_full, const f
   ENTER_DEVICE(h);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   h->idx_host.resize((size_t)2 * n_windows);
-  const double a_ratio = (double)Ta_full / (double)(total_v_frames > 1 ? total_v_frames : 1);
   for (int i = 0; i < n_windows; ++i) {
-    long a_start = audio_starts_host ? (long)audio_starts_host[i] : (long)nearbyint((double)starts_host[i] * a_ratio);   // predictor.py:540-547
-    if (a_start + Ta > Ta_full) { a_start = Ta_full - Ta; }
-    if (a_start < 0) a_start = 0;
     h->idx_host[i] = starts_host[i];
-    h->idx_host[n_windows + i] = (int32_t)a_start;
+    h->idx_host[n_windows + i] = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);   // predictor.py:540-547
   }
   CUDA_OK(h, cudaMemcpyAsync(idx_scratch, h->idx_host.data(), (size_t)2 * n_windows * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   lsd::launch_speech_stats(motion_full, motion_low, idx_scratch, idx_scratch + n_windows, n_windows, T, mel_full, F, Ta_full, Ta, speaking_out,
@@ -672,7 +829,7 @@ extern "C" int64_t lsd_state_generation(lsd_handle* h) { return h ? h->generatio
 
 extern "C" int lsd_workspace_invalidate(lsd_handle* h) {
   if (!h) return LSD_ERR_ARG;
-  h->ws_sig[0].ptr = nullptr; h->ws_sig[1].ptr = nullptr;
+  for (WsSig& w : h->ws_sig) w.ptr = nullptr;
   return LSD_OK;
 }
 

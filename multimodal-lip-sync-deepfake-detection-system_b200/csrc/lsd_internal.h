@@ -76,7 +76,7 @@ struct lsd_handle {
   int tokf_n_stage = 0;
   uint32_t tokf_layer_bytes = 0;
   std::map<std::string, BLayer> blayers;
-  WsSig ws_sig[2];                         // bf16 workspaces whose zero padding is initialised (see ws_prepare in bf16_path.cu)
+  WsSig ws_sig[3];                         // bf16 workspaces whose zero padding is initialised (see ws_prepare in bf16_path.cu)
   // cross-batch pipelining of lsd_score_windows: the tail of batch k (audio encoder, token path, head; artifact branch on the
   // side stream) runs on tail_stream while the main stream already runs the visual encoder of batch k+1
   cudaStream_t tail_stream = nullptr;
@@ -141,5 +141,13 @@ int score_batch_bf16(lsd_handle* h, const uint8_t* track, int n_frames, const in
                      const float* mel_full, int Ta_full, int nb, int T, int H, int W, int F, int Ta, float* logits,
                      char* ws, size_t ws_bytes, cudaStream_t st, int pipe_parity = -1);
 int ensure_pipeline(lsd_handle* h);
+// shared-visual forward: K audio windows per video, visual front once (bf16_path.cu, VarTail)
+bool variants_shared_route(int T);
+size_t variants_bf16_bytes(lsd_handle* h, int B, int K, int T, int H, int W, int F, int Ta);
+int forward_variants_bf16(lsd_handle* h, int B, int K, int T, int H, int W, int F, int Ta, const void* video, int vdt, int vlayout,
+                          const void* audio, int adt, float* logits, char* ws, size_t ws_bytes, cudaStream_t st);
+int score_offsets_batch_bf16(lsd_handle* h, const uint8_t* track, int n_frames, const int32_t* d_vstarts, const int32_t* d_astarts,
+                             const float* mel_full, int Ta_full, int nb, int batch, int K, int T, int H, int W, int F, int Ta, float* logits,
+                             char* ws, size_t ws_bytes, cudaStream_t st);
 int planar_stage_read(lsd_handle* h, const char* name, const char* name_lo, const char* ws, float* out, int64_t out_elems, int Hf, int Wf,
                       cudaStream_t st);

@@ -197,6 +197,7 @@ __global__ void __launch_bounds__(FR_THREADS, 1) tok_front_kernel(const __grid_c
     int win = blockIdx.x * G + slot;
     bool valid = slot < G && win < p.B && lrow < T;
     size_t grow = valid ? (size_t)win * T + lrow : 0;                     // row of the (B*T, .) fp32 matrices
+    const size_t vgrow = valid ? (size_t)(win / p.K) * T + lrow : 0;      // row of the visual matrices (pv, v_emb)
     const uint32_t lane_base = tmem + ((uint32_t)(q * 32) << 16);
     const uint32_t O = lane_base + O_COL, ACC = lane_base + ACC_COL;
     const uint32_t row16 = (uint32_t)row * 16u;
@@ -240,8 +241,8 @@ __global__ void __launch_bounds__(FR_THREADS, 1) tok_front_kernel(const __grid_c
     // Q K V of head pair hp of direction dir -> fp16 planes.  dir 0 (v2a): Q from the visual tokens, K / V from the audio tokens;
     // dir 1 (a2v): the other way round.  cq 0: Q0 K0, cq 1: Q1 K1, cq 2: V0, cq 3: V1 (the transposing stores alone).
     auto load_qkv = [&](int dir, int hp) {
-      const float* qsrc = (dir == 0 ? p.pv : p.pa) + grow * p.ld_p;
-      const float* kvsrc = (dir == 0 ? p.pa : p.pv) + grow * p.ld_p;
+      const float* qsrc = dir == 0 ? p.pv + vgrow * p.ld_p : p.pa + grow * p.ld_p;
+      const float* kvsrc = dir == 0 ? p.pa + grow * p.ld_p : p.pv + vgrow * p.ld_p;
       float v[32];
       if (cq < 2) {
         const int head = 2 * hp + cq;
@@ -317,7 +318,7 @@ __global__ void __launch_bounds__(FR_THREADS, 1) tok_front_kernel(const __grid_c
       // ---- out = O + bias + residual -> scratch [v_out | a_out]; then the next direction's first Q K V, or the gate input planes
       wait_mma();
       {
-        const float* res = (dir == 0 ? p.v_emb : p.a_int) + grow * p.ld_e;
+        const float* res = dir == 0 ? p.v_emb + vgrow * p.ld_e : p.a_int + grow * p.ld_e;
         const float* bo = vec + (dir == 0 ? TFR_V_BO0 : TFR_V_BO1);
         float* dst = p.gi + grow * 512 + dir * D;
 #pragma unroll 1

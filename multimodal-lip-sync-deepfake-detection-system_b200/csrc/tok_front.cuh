@@ -35,6 +35,8 @@ struct TokFrontP {
   const float* vec;     // TFR_V_TOTAL floats
   void* dbg;            // optional (LSD_TOKF_TRACE): 256 x int64 phase timestamps of CTA 0 (MMA warp: [0,128), compute warp 0: [128,256))
   int B, T, SL, G, KW;  // windows, tokens per window, row slot per window (32 or 64; >= T + 3), windows per CTA, keys per window (16-multiple)
+  int K;                // visual row group: window w reads the visual rows (pv, v_emb) of window w / K (K audio variants share one
+                        // visual window, lsd_forward_audio_variants); 1 = every window has its own visual rows
 };
 
 cudaError_t tok_front_device_init();

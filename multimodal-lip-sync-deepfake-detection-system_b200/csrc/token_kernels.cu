@@ -245,12 +245,14 @@ void launch_audio_rows(const void* audio, int dtype, __nv_bfloat16* y, int64_t s
 // 512 threads: every layer splits its K range over 2 (448 -> 256) or 4 (256 -> 128, 384 -> 128) thread groups and keeps 16
 // independent weight loads in flight per thread — the kernel is L2-latency-bound (0.9 MB of fp32 weights per window, one
 // window per SM); partial sums are combined in a fixed order.
-// cls: row n of the CLS outputs at cls + n * cls_ld (read in place from the token buffer); comb[:, 256:448]: artifact features.
+// cls: row n of the CLS outputs at cls + n * cls_ld (read in place from the token buffer); comb[:, 256:448]: artifact features,
+// row n / K (K audio variants of one video share its artifact features; K = 1: one row per window).
 __global__ void __launch_bounds__(512) head_kernel(const float* __restrict__ cls, int64_t cls_ld, const float* __restrict__ comb, HeadW w,
-                                                   float* __restrict__ logits) {
+                                                   float* __restrict__ logits, int K) {
   __shared__ float x[448], h1[256], f[384], part[512], red[4];
   const int n = blockIdx.x, tid = threadIdx.x;
-  for (int i = tid; i < 448; i += 512) x[i] = i < 256 ? cls[(int64_t)n * cls_ld + i] : comb[(int64_t)n * 448 + i];
+  const int64_t crow = n / K;
+  for (int i = tid; i < 448; i += 512) x[i] = i < 256 ? cls[(int64_t)n * cls_ld + i] : comb[crow * 448 + i];
   __syncthreads();
   {
     const int o = tid & 255, half = tid >> 8;                 // K split: [0,224) and [224,448)
@@ -307,9 +309,9 @@ __global__ void __launch_bounds__(512) head_kernel(const float* __restrict__ cls
   __syncthreads();
   if (tid == 0) logits[n] = red[0] + red[1] + red[2] + red[3] + w.bo[0];
 }
-void launch_head(const float* cls, int64_t cls_ld, const float* comb, const HeadW& w, float* logits, int B, cudaStream_t s) {
+void launch_head(const float* cls, int64_t cls_ld, const float* comb, const HeadW& w, float* logits, int B, cudaStream_t s, int K) {
   if (B == 0) return;
-  head_kernel<<<B, 512, 0, s>>>(cls, cls_ld, comb, w, logits);
+  head_kernel<<<B, 512, 0, s>>>(cls, cls_ld, comb, w, logits, K);
   count_launch();
 }
 

@@ -25,7 +25,8 @@ void launch_gate_blend_p(const float* h, const float* w2, const float* b2, const
                          int D, PlanarOut o, cudaStream_t s);
 void launch_lerp_tokens_p(const float* x, float* y, int N, int Tin, int Tout, int D, PlanarOut o, cudaStream_t s);
 void launch_audio_rows(const void* audio, int dtype, __nv_bfloat16* y, int64_t set_stride, UcGeom g, int F, int Ta, cudaStream_t s);
-void launch_head(const float* cls, int64_t cls_ld, const float* comb, const HeadW& w, float* logits, int B, cudaStream_t s);
+// K: windows n = b*K + k read the artifact features comb[b] (audio variants of one video); 1 = one comb row per window
+void launch_head(const float* cls, int64_t cls_ld, const float* comb, const HeadW& w, float* logits, int B, cudaStream_t s, int K = 1);
 // mean of a planar tensor -> fp32 rows (y32, may be null) and/or planar bf16 rows (po.y, may be null)
 //   mode 0: one row per (n,t), mean over H*W;  mode 1: one row per window, mean over T*H*W;  mode 2: one row per (n,w), mean over H (T == 1)
 void launch_planar_mean2(const __nv_bfloat16* x, int64_t plane_stride, UcGeom g, int C, float* y32, int ld, int mode, PlanarOut po, cudaStream_t s,

@@ -17,7 +17,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import time
-from typing import Callable, List, Optional, Sequence, Tuple
+from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -25,6 +25,9 @@ import torch
 from . import _cabi
 from . import aggregate as _agg
 from .model import LipSyncModel
+
+#: one log-mel column: hop 160 at 16 kHz (app/preprocessing/audio.py:80-91)
+_MEL_HOP_SEC = 160.0 / 16000.0
 
 
 def partition_windows(n_windows: int, world_size: int, rank: int) -> Tuple[int, int]:
@@ -531,6 +534,86 @@ class Predictor:
                                      ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
             _cabi.check(h.ptr, rc)
         return logits
+
+    def score_track_offsets(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                            offsets: Sequence[int], chunk_a_size: int = 128, audio_starts_from: Optional[Sequence[int]] = None):
+        """`score_track_logits` with K audio offsets per window (`lsd_score_offsets`): offset d (mel columns, 10 ms, d > 0 =
+        audio later) moves the window's aligned audio start a_i to clamp(a_i + d), clamped like `_audio_start`.  The video side of
+        a window is computed once for all offsets.  Returns `(logits (n,K) fp32 on the device, effective audio starts (n,K)
+        np.int32, valid (n,K) bool)`; (i, k) is valid when 0 <= a_i + d_k <= T_full - chunk_a_size (no clamping)."""
+        m = self.model
+        dev = m._device()
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        if mel_full.dim() != 3 or mel_full.shape[0] != 1:
+            raise ValueError(f"mel_full must be (1, F, T_full), got {tuple(mel_full.shape)}")
+        offs = [int(d) for d in offsets]
+        K = len(offs)
+        if not 1 <= K <= _cabi.LSD_MAX_AUDIO_VARIANTS:
+            raise ValueError(f"{K} offsets: expected 1 to {_cabi.LSD_MAX_AUDIO_VARIANTS}")
+        n = len(starts)
+        if audio_starts_from is not None and len(audio_starts_from) != n:
+            raise ValueError("audio_starts_from must have one entry per window")
+        F_, Ta_full = int(mel_full.shape[1]), int(mel_full.shape[2])
+        base = np.array([self._audio_start(int(v), Ta_full, int(total_v_frames), chunk_a_size)
+                         for v in (audio_starts_from if audio_starts_from is not None else starts)], dtype=np.int64).reshape(n, 1)
+        moved = base + np.asarray(offs, dtype=np.int64).reshape(1, K)
+        valid = (moved >= 0) & (moved <= Ta_full - chunk_a_size)
+        logits = torch.empty(n, K, dtype=torch.float32, device=dev)
+        eff = np.zeros((n, K), dtype=np.int32)
+        if n == 0:
+            return logits, eff, valid
+        track_u8 = track_u8.contiguous()
+        mel_full = mel_full.to(torch.float32).contiguous()
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = m._precision()
+            batch = min(self.batch_size, n)
+            need = L.lsd_score_offsets_workspace_bytes(h.ptr, batch, K, self.chunk_size, H, W, F_, chunk_a_size, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            ws = m._workspace(need, dev)
+            st = (C.c_int32 * n)(*[int(s) for s in starts])
+            ast = None if audio_starts_from is None else (C.c_int32 * n)(*[int(a) for a in base[:, 0]])
+            offs_c = (C.c_int32 * K)(*offs)
+            eff_c = (C.c_int32 * (n * K))()
+            rc = L.lsd_score_offsets(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, self.chunk_size, mel_full.data_ptr(), F_, Ta_full,
+                                     int(total_v_frames), chunk_a_size, offs_c, K, prec, batch, logits.data_ptr(), eff_c,
+                                     ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        eff[:] = np.frombuffer(eff_c, dtype=np.int32).reshape(n, K)
+        return logits, eff, valid
+
+    @staticmethod
+    def default_av_offsets(Ta_full: int, total_v_frames: int, max_frames: int = 7) -> Tuple[List[int], List[int]]:
+        """Whole video frames -max_frames..+max_frames and their offsets in mel columns, converted with the ratio `_audio_start`
+        uses (round(f * T_full / total_v_frames), round-half-even)."""
+        frames = list(range(-int(max_frames), int(max_frames) + 1))
+        a_ratio = Ta_full / max(1, total_v_frames)
+        return frames, [int(round(f * a_ratio)) for f in frames]
+
+    def estimate_av_offset(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                           offsets: Optional[Sequence[int]] = None, chunk_a_size: int = 128,
+                           audio_starts_from: Optional[Sequence[int]] = None) -> Dict[str, Any]:
+        """Audio-visual offset of a track: `score_track_offsets` + `aggregate.av_offset_profile` on the calibrated confidences,
+        aggregated like the window confidences (`confidence_smoothing`, `trim_ratio`).  Default offsets: whole video frames
+        -7..+7 (`default_av_offsets`).  Offsets are also reported in seconds (one mel column = 10 ms).  Reporting only: the
+        offset changes no verdict."""
+        Ta_full = int(mel_full.shape[2])
+        frames = None
+        if offsets is None:
+            frames, offsets = self.default_av_offsets(Ta_full, total_v_frames)
+        offsets = [int(d) for d in offsets]
+        logits, _, valid = self.score_track_offsets(track_u8, starts, mel_full, total_v_frames, offsets, chunk_a_size, audio_starts_from)
+        confs = np.array([self._calibrate(float(x)) for x in logits.cpu().flatten().tolist()], dtype=np.float32).reshape(valid.shape)
+        res = _agg.av_offset_profile(confs, valid, offsets, self.confidence_smoothing, self.trim_ratio)
+        res["offsets_sec"] = [d * _MEL_HOP_SEC for d in offsets]
+        res["best_offset_sec"] = res["best_offset"] * _MEL_HOP_SEC if res["best_offset"] is not None else None
+        if frames is not None:
+            res["offset_frames"] = frames
+        return res
 
     def score_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int):
         logits = self.score_track_logits(track_u8, starts, mel_full, total_v_frames)

@@ -236,6 +236,49 @@ class LipSyncModel(nn.Module):
             return logits
         return logits, {k: v.to(out_dtype) for k, v in aux_t.items()}
 
+    def forward_audio_variants(self, visual: Tensor, audio: Tensor) -> Tensor:
+        """Score K audio windows against every video: visual `(B,3,T,H,W)`, audio `(B,K,1,F,T_a)` -> logits `(B,K)`.
+        `[:, k]` is bit for bit `forward(visual, audio[:, k])`; the visual encoder and the artifact branch run once per video
+        (`lsd_forward_audio_variants`).  1 <= K <= 64."""
+        if visual.dim() != 5:
+            raise ValueError(f"VisualEncoder expected input of shape (B, 3, T, H, W), got {tuple(visual.shape)}")
+        if audio.dim() != 5:
+            raise ValueError(f"expected audio variants of shape (B, K, 1, F, T), got {tuple(audio.shape)}")
+        B, Cv, T, H, W = visual.shape
+        K = int(audio.shape[1])
+        if Cv != 3:
+            raise ValueError(f"VisualEncoder expected 3 input channels, got {Cv}")
+        if audio.shape[0] != B or audio.shape[2] != 1:
+            raise ValueError(f"expected audio variants of shape ({B}, K, 1, F, T), got {tuple(audio.shape)}")
+        if not 1 <= K <= _cabi.LSD_MAX_AUDIO_VARIANTS:
+            raise ValueError(f"K = {K} audio variants: expected 1 <= K <= {_cabi.LSD_MAX_AUDIO_VARIANTS}")
+        if visual.dtype not in _DTYPES or audio.dtype not in _DTYPES or audio.dtype == torch.uint8:
+            raise RuntimeError(f"unsupported input dtypes {visual.dtype}/{audio.dtype}")
+        dev = self._device()
+        if visual.device != dev or audio.device != dev:
+            raise RuntimeError(f"inputs must live on the module's device {dev} (got {visual.device}, {audio.device})")
+        F_, Ta = int(audio.shape[3]), int(audio.shape[4])
+        out_dtype = visual.dtype if visual.dtype.is_floating_point else torch.float32
+        logits = torch.empty(int(B), K, dtype=torch.float32, device=dev)
+        if B == 0:
+            return logits.to(out_dtype)
+        with self._lsd_lock:
+            h = self._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = self._precision()
+            visual = visual.contiguous()
+            audio = audio.contiguous()
+            need = L.lsd_forward_audio_variants_workspace_bytes(h.ptr, int(B), K, int(T), int(H), int(W), F_, Ta, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            ws = self._workspace(need, dev)
+            rc = L.lsd_forward_audio_variants(h.ptr, visual.data_ptr(), _DTYPES[visual.dtype], _cabi.LSD_NCDHW, audio.data_ptr(),
+                                              _DTYPES[audio.dtype], int(B), K, int(T), int(H), int(W), F_, Ta, prec, logits.data_ptr(),
+                                              ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+            self._lsd_plan_dtype = prec
+        return logits.to(out_dtype)
+
     def forward_into(self, visual: Tensor, audio: Tensor, logits: Tensor, workspace: Tensor) -> None:
         """Allocation-free forward for CUDA-graph capture: device `visual (B,3,T,H,W)` / `audio (B,1,F,T_a)` (contiguous),
         fp32 device `logits (B,)`, caller-owned `workspace` (uint8, >= `workspace_bytes(...)`), current stream."""
