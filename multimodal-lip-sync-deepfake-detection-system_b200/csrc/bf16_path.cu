@@ -7,7 +7,6 @@
 #include "token_kernels.cuh"
 #include "umma_conv.cuh"
 #include "stem_ring.cuh"
-#include "conv_ring.cuh"
 
 #include <cuda_fp16.h>
 
@@ -477,7 +476,6 @@ int run_umma(const BCtx& c, const std::string& name, const UArgs& a) {
   p.act = a.act;
   p.g = og;
   p.cta2 = L.halves ? 1 : 0;
-  if (a.y_mode == UC_Y_POOL && p.cta2) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: the fused max-pool does not run on CTA pairs (LSD_UMMA_CTA2=0)", name.c_str());
   if (a.yp) {
     p.y_mode = a.y_mode >= 0 ? a.y_mode : (a.yp->sets == 4 ? UC_Y_PARITY : UC_Y_PLAIN);
     p.y = c.org(*a.yp) + (int64_t)a.y_plane_off * a.yp->plane_stride;
@@ -599,16 +597,12 @@ int run_umma(const BCtx& c, const std::string& name, const UArgs& a) {
     p.nst_tile += ((p.groups[gi].k16 + p.kpack - 1) / p.kpack) * (p.groups[gi].band_end - p.groups[gi].band_begin);
   const uint32_t prog_bytes = (uint32_t)p.nst_tile * (uint32_t)umma_conv_stage_desc_bytes();
   uint32_t budget = 211u * 1024u;   // one persistent CTA per SM owns the whole shared memory
-  if (p.y_mode == UC_Y_POOL) {     // fused max-pool: output ring + per-position table behind the stage program
-    p.pool_ring = (uint32_t)(p.MT * 128 + 128);
-    uc_magic(p.pool_ring, p.pool_mR, p.pool_sR);
-  }
-  const uint32_t pool_bytes = (uint32_t)umma_conv_extra_smem_bytes(p);   // bias operand tiles of the lean epilogue (+ the max-pool ring)
-  budget -= pool_bytes;
+  const uint32_t extra_bytes = (uint32_t)umma_conv_extra_smem_bytes(p);   // bias operand tiles of the lean epilogue
+  budget -= extra_bytes;
   if (prog_bytes + 2 * stage > budget) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: stage program of %u bytes does not fit", name.c_str(), prog_bytes);
   int stages = (int)((budget - prog_bytes) / stage);
   stages = std::max(2, std::min(stages, 8));
-  if ((size_t)stages * stage + prog_bytes + pool_bytes + 1024 > 223u * 1024u) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: stage of %u bytes does not fit", name.c_str(), stage);
+  if ((size_t)stages * stage + prog_bytes + extra_bytes + 1024 > 223u * 1024u) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: stage of %u bytes does not fit", name.c_str(), stage);
   p.stages = stages;
   double kflop = 0;
   for (const BGroup& G : L.groups) kflop += (double)G.taps_total * G.Cin;
@@ -617,24 +611,6 @@ int run_umma(const BCtx& c, const std::string& name, const UArgs& a) {
   if (const char* why = umma_conv_config_error(p)) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "%s: %s", name.c_str(), why);
   if (int rc = stage_program(c, name, p, [&](std::vector<UcStageDesc>& v) { v.resize((size_t)p.nst_tile); umma_conv_build_program(p, v.data()); }))
     return rc;
-  // tile counters of this layer (dynamic tile scheduling, LSD_UMMA_DYNAMIC=1).  Off by default: measured at B=64 it shortens the
-  // visual encoder by ~20 us per forward (CTAs delayed by the side stream's kernels take fewer tiles) but every one-tile
-  // token-path launch pays the claim + counter re-arm (~1 us each), a net +2 % per step.
-  static const bool dyn_tiles = LSD_ENV("LSD_UMMA_DYNAMIC") != nullptr;
-  if (dyn_tiles && p.y_mode != UC_Y_POOL && !p.cta2) {   // (the fused max-pool walks contiguous position ranges)
-    constexpr int kMaxLayers = 512;
-    if (!c.h->tile_ctr_arena) {
-      if (cudaMalloc(&c.h->tile_ctr_arena, kMaxLayers * 16 * sizeof(unsigned)) != cudaSuccess ||
-          cudaMemset(c.h->tile_ctr_arena, 0, kMaxLayers * 16 * sizeof(unsigned)) != cudaSuccess)
-        return lsd_fail(c.h, LSD_ERR_CUDA, "tile counter allocation failed");
-    }
-    auto it = c.h->tile_ctr_idx.find(name);
-    if (it == c.h->tile_ctr_idx.end()) {
-      if ((int)c.h->tile_ctr_idx.size() >= kMaxLayers) return lsd_fail(c.h, LSD_ERR_UNSUPPORTED, "too many tcgen05 layers");
-      it = c.h->tile_ctr_idx.emplace(name, (int)c.h->tile_ctr_idx.size()).first;
-    }
-    p.tile_ctr = c.h->tile_ctr_arena + (size_t)it->second * 16;
-  }
   if (const char* e = getenv("LSD_UMMA_TRACE")) {
     // debug: per-launch phase timestamps of CTA (0,0); prints after a sync (never enabled in timed runs)
     static long long* dbuf = nullptr;
@@ -667,17 +643,15 @@ int run_umma(const BCtx& c, const std::string& name, const UArgs& a) {
   return 0;
 }
 
-// Stem through the temporal-ring kernel (stem_ring.cu): xs (pixel rows, 2 parity sets) -> so (plain planar, 64 channels), same geometry.
-// Step table of the temporal-ring kernels (stem_ring.cu, conv_ring.cu) for geometry g: (column chunk, t) outputs numbered column-major,
-// cut into equal contiguous ranges, one per accumulator slot; cached per (batch, frames, geometry, CTA budget).
-int ring_table(const BCtx& c, const UcGeom& g, bool pool, const lsd_handle::RingTab** out) {
+// Step table of the temporal-ring stem (stem_ring.cu) for geometry g: (column chunk, t) outputs numbered column-major, cut into
+// equal contiguous ranges, one per accumulator slot; cached per (batch, frames, geometry, CTA budget).
+int ring_table(const BCtx& c, const UcGeom& g, const lsd_handle::RingTab** out) {
   lsd_handle* h = c.h;
-  const void* pool_to = pool ? (const void*)&g : nullptr;
   const int T = g.T, CH = (g.SL + 127) / 128;
   const int64_t G = (int64_t)g.N * CH * T;
   const int budget = (c.max_ctas > 0 && c.max_ctas < h->num_sms) ? c.max_ctas : h->num_sms;
   uint64_t key = 1469598103934665603ull;
-  for (uint64_t v : {(uint64_t)g.N, (uint64_t)T, (uint64_t)g.SL, (uint64_t)g.TS, (uint64_t)g.ot, (uint64_t)budget, (uint64_t)(pool_to != nullptr)}) { key ^= v; key *= 1099511628211ull; key ^= key >> 29; }
+  for (uint64_t v : {(uint64_t)g.N, (uint64_t)T, (uint64_t)g.SL, (uint64_t)g.TS, (uint64_t)g.ot, (uint64_t)budget}) { key ^= v; key *= 1099511628211ull; key ^= key >> 29; }
   auto it = h->ring_tabs.find(key);
   if (it == h->ring_tabs.end()) {
     int grid = budget;
@@ -686,7 +660,6 @@ int ring_table(const BCtx& c, const UcGeom& g, bool pool, const lsd_handle::Ring
     if (grid < 1) grid = 1;
     std::vector<std::vector<SrStep>> lists((size_t)2 * grid);
     size_t nsteps = 0;
-    const int nslots = 2 * grid;
     // steps of outputs [ta, tb) of column `col` (input slabs max(ta-1, 0) .. tb; the slab completed by a step is stored when it is in range)
     auto add_range = [&](int sg, int64_t col, int ta, int tb) {
       const int n = (int)(col / CH), sp = (int)(col % CH);
@@ -700,50 +673,22 @@ int ring_table(const BCtx& c, const UcGeom& g, bool pool, const lsd_handle::Ring
         lists[sg].push_back(st);
       }
     };
-    // Inline pooling wants the frames of a window to complete progressively: whole columns are dealt round-robin to the slots in
-    // window-major order (round r: columns r * nslots ..), and only the remaining columns are cut into equal output ranges.
-    const int64_t ncols = (int64_t)g.N * CH;
-    const int64_t rounds = pool_to ? ncols / nslots : 0;
-    std::vector<int> col_round((size_t)ncols, 0);       // step index at which a column's output t completes ~ round * (T + 1) + t
-    for (int64_t r = 0; r < rounds; ++r)
-      for (int sg = 0; sg < nslots; ++sg) { add_range(sg, r * nslots + sg, 0, T); col_round[(size_t)(r * nslots + sg)] = (int)r; }
-    {
-      const int64_t col0 = rounds * nslots, Grem = (ncols - col0) * T;
-      if (pool_to) Lr = (Grem + nslots - 1) / nslots;
-      for (int64_t cc = col0; cc < ncols; ++cc) col_round[(size_t)cc] = (int)rounds;
-      for (int sg = 0; sg < nslots && Lr > 0; ++sg) {
-        int64_t g0 = (int64_t)sg * Lr;
-        const int64_t g1 = std::min(Grem, g0 + Lr);
-        while (g0 < g1) {
-          const int64_t col = col0 + g0 / T;
-          const int ta = (int)(g0 % T), tb = (int)std::min<int64_t>(T, ta + (g1 - g0));
-          add_range(sg, col, ta, tb);
-          g0 += tb - ta;
-        }
+    for (int sg = 0; sg < 2 * grid; ++sg) {
+      int64_t g0 = (int64_t)sg * Lr;
+      const int64_t g1 = std::min(G, g0 + Lr);
+      while (g0 < g1) {
+        const int64_t col = g0 / T;
+        const int ta = (int)(g0 % T), tb = (int)std::min<int64_t>(T, ta + (g1 - g0));
+        add_range(sg, col, ta, tb);
+        g0 += tb - ta;
       }
     }
-    for (int sg = 0; sg < nslots; ++sg) nsteps = std::max(nsteps, lists[sg].size());
+    for (int sg = 0; sg < 2 * grid; ++sg) nsteps = std::max(nsteps, lists[sg].size());
     std::vector<SrStep> flat((size_t)2 * grid * nsteps);
     memset(flat.data(), 0, flat.size() * sizeof(SrStep));
     for (int sg = 0; sg < 2 * grid; ++sg) std::copy(lists[sg].begin(), lists[sg].end(), flat.begin() + (size_t)sg * nsteps);
     lsd_handle::RingTab tab;
     tab.nsteps = (int)nsteps; tab.grid = grid;
-    if (pool_to) {
-      // frames in expected order of completion (the latest of their columns), dealt round-robin to the CTAs
-      std::vector<std::pair<int64_t, int>> order;
-      for (int n = 0; n < g.N; ++n) {
-        int rmax = 0;
-        for (int sp = 0; sp < CH; ++sp) rmax = std::max(rmax, col_round[(size_t)n * CH + sp]);
-        for (int t = 0; t < T; ++t) order.push_back({(int64_t)rmax * (T + 1) + t, n * T + t});
-      }
-      std::stable_sort(order.begin(), order.end(), [](const std::pair<int64_t, int>& a, const std::pair<int64_t, int>& b) { return a.first < b.first; });
-      tab.nfr = (int)((order.size() + grid - 1) / grid) + 1;
-      std::vector<int> fl((size_t)grid * tab.nfr, -1);
-      for (size_t i = 0; i < order.size(); ++i) fl[(i % grid) * tab.nfr + i / grid] = order[i].second;
-      if (cudaMalloc(&tab.frames, fl.size() * sizeof(int)) != cudaSuccess ||
-          cudaMemcpy(tab.frames, fl.data(), fl.size() * sizeof(int), cudaMemcpyHostToDevice) != cudaSuccess)
-        return lsd_fail(h, LSD_ERR_CUDA, "stem: pool list upload failed");
-    }
     // cache miss only (first forward of a shape): blocking copy, visible to every stream afterwards
     if (cudaMalloc(&tab.dev, std::max<size_t>(flat.size(), 1) * sizeof(SrStep)) != cudaSuccess ||
         cudaMemcpy(tab.dev, flat.data(), flat.size() * sizeof(SrStep), cudaMemcpyHostToDevice) != cudaSuccess)
@@ -754,8 +699,8 @@ int ring_table(const BCtx& c, const UcGeom& g, bool pool, const lsd_handle::Ring
   return 0;
 }
 
-// pool_to != nullptr: the max-pool runs inside the kernel (four pool warps per CTA, see stem_ring.cu) and writes *pool_to.
-int run_stem_ring(const BCtx& c, const PBuf& xs, const PBuf& so, const PBuf* pool_to = nullptr) {
+// Stem through the temporal-ring kernel (stem_ring.cu): xs (pixel rows, 2 parity sets) -> so (plain planar, 64 channels), same geometry.
+int run_stem_ring(const BCtx& c, const PBuf& xs, const PBuf& so) {
   lsd_handle* h = c.h;
   const UcGeom& g = xs.g;
   if (g.P_total >= ((int64_t)1 << 31) - 4096) return lsd_fail(h, LSD_ERR_SHAPE, "stem: more than 2^31 padded positions in one launch (reduce the batch)");
@@ -775,29 +720,12 @@ int run_stem_ring(const BCtx& c, const PBuf& xs, const PBuf& so, const PBuf* poo
   p.start[0] = -g.RW; p.start[1] = -2 * g.RW;
   p.units[0] = 128 + 2 * g.RW + 3; p.units[1] = 128 + 3 * g.RW + 3;
   if ((int64_t)(2 * g.RW + 3) * 8 > xs.origin) return lsd_fail(h, LSD_ERR_UNSUPPORTED, "stem: guard zone too small");
-  const int T = g.T, CH = (g.SL + 127) / 128;
   const lsd_handle::RingTab* tab = nullptr;
-  if (int trc = ring_table(c, g, pool_to != nullptr, &tab)) return trc;
+  if (int trc = ring_table(c, g, &tab)) return trc;
   p.steps = reinterpret_cast<const SrStep*>(tab->dev);
   p.nsteps = tab->nsteps;
   p.nst = 6;
   if (const char* e = getenv("LSD_SR_SKIP")) p.skip = atoi(e);   // timing experiments only
-  if (pool_to) {
-    const size_t need = (size_t)g.N * T;
-    if (h->ring_cnt_cap < need) {
-      if (h->ring_cnt) { cudaStreamSynchronize(c.st); cudaFree(h->ring_cnt); h->ring_cnt = nullptr; ++h->generation; }
-      h->ring_cnt_cap = need * 2;
-      if (cudaMalloc(&h->ring_cnt, h->ring_cnt_cap * sizeof(unsigned)) != cudaSuccess) { h->ring_cnt_cap = 0; return lsd_fail(h, LSD_ERR_CUDA, "stem: frame counter allocation failed"); }
-    }
-    cudaMemsetAsync(h->ring_cnt, 0, need * sizeof(unsigned), c.st);
-    p.frame_cnt = h->ring_cnt;
-    p.pool_frames = tab->frames;
-    p.pool_nfr = tab->nfr;
-    p.pool_expected = 4 * CH;
-    p.yp = c.org(*pool_to);
-    p.yp_plane_stride = pool_to->plane_stride;
-    p.gp = pool_to->g;
-  }
   while (p.nst > 3 && stem_ring_smem_bytes(p) > 223u * 1024u) --p.nst;    // a long step table (large batches) takes ring stages
   if (stem_ring_smem_bytes(p) > 223u * 1024u) return lsd_fail(h, LSD_ERR_UNSUPPORTED, "stem: batch too large for the ring kernel (LSD_STEM_RING=0)");
   const ConvP& cp = h->convs.at("visual_encoder.stem");
@@ -836,60 +764,6 @@ int run_stem_ring(const BCtx& c, const PBuf& xs, const PBuf& so, const PBuf* poo
     return 0;
   }
   launch_stem_ring(p, tab->grid, c.st);
-  h->prof.end(c.st);
-  return 0;
-}
-
-// One 64 -> 64 channel 3x3x3 convolution of layer1 through the temporal-ring kernel (conv_ring.cu): x (plain planar) -> y (plain, or
-// parity-split when y.sets == 4), optional residual (plain), ReLU.  which: 0 = conv1, 1 = conv2.
-int run_conv_ring(const BCtx& c, const std::string& name, int which, const PBuf& x, const PBuf& y, const PBuf* res) {
-  lsd_handle* h = c.h;
-  const UcGeom& g = x.g;
-  if (g.P_total >= ((int64_t)1 << 31) - 4096) return lsd_fail(h, LSD_ERR_SHAPE, "%s: more than 2^31 padded positions in one launch (reduce the batch)", name.c_str());
-  const BLayer& L = h->blayers.at(name);
-  ConvRingP p;
-  memset(&p, 0, sizeof(p));
-  p.x = c.org(x);
-  p.x_plane_stride = x.plane_stride;
-  p.w = reinterpret_cast<const __nv_bfloat16*>(h->barena) + h->l1_ring_w_off[which];
-  p.bias = h->bbias + L.bias_off;
-  if (res) { p.res = c.org(*res); p.res_plane_stride = res->plane_stride; }
-  p.y = c.org(y);
-  p.y_plane_stride = y.plane_stride; p.y_set_stride = y.set_stride;
-  p.y_mode = y.sets == 4 ? UC_Y_PARITY : UC_Y_PLAIN;
-  p.g = g; p.g2 = y.g;
-  p.start = -(g.RW + 1);
-  p.units = 128 + 2 * g.RW + 2;
-  if ((int64_t)(g.RW + 1) * 8 > x.origin) return lsd_fail(h, LSD_ERR_UNSUPPORTED, "%s: guard zone too small", name.c_str());
-  const lsd_handle::RingTab* tab = nullptr;
-  if (int trc = ring_table(c, g, false, &tab)) return trc;
-  p.steps = reinterpret_cast<const SrStep*>(tab->dev);
-  p.nsteps = tab->nsteps;
-  p.nst = 4;
-  if (const char* e = getenv("LSD_SR_SKIP")) p.skip = atoi(e);   // timing experiments only
-  while (p.nst > 1 && conv_ring_smem_bytes(p) > 223u * 1024u) --p.nst;
-  if (conv_ring_smem_bytes(p) > 223u * 1024u) return lsd_fail(h, LSD_ERR_UNSUPPORTED, "%s: rows too wide / batch too large for the ring kernel (LSD_L1_RING=0)", name.c_str());
-  const ConvP& cp = h->convs.at(name);
-  h->prof.begin(c.st, 2.0 * (double)g.N * g.T * g.H * g.W * 64.0 * (double)cp.kt * cp.kh * cp.kw * cp.Cin, 2);
-  if (getenv("LSD_CR_TRACE")) {
-    static long long* dbuf = nullptr;
-    if (!dbuf) cudaMalloc(&dbuf, 4 * 160 * sizeof(long long));
-    cudaMemsetAsync(dbuf, 0, 4 * 160 * sizeof(long long), c.st);
-    p.dbg = dbuf;
-    launch_conv_ring(p, tab->grid, c.st);
-    long long hv[4 * 160];
-    cudaMemcpyAsync(hv, dbuf, sizeof(hv), cudaMemcpyDeviceToHost, c.st);
-    cudaStreamSynchronize(c.st);
-    long long g0 = INT64_MAX, g1 = 0, cmin = INT64_MAX, cmax = 0, csum = 0;
-    const int nc = std::min(tab->grid, 160);
-    for (int i = 0; i < nc; ++i) g0 = std::min(g0, hv[4 * i]);
-    for (int i = 0; i < nc; ++i) { g1 = std::max(g1, hv[4 * i + 1]); const long long cy = hv[4 * i + 3] - hv[4 * i + 2]; cmin = std::min(cmin, cy); cmax = std::max(cmax, cy); csum += cy; }
-    fprintf(stderr, "[cr] %s: %d CTAs x %d steps (nst %d): kernel span %.1f us, CTA cycles min %lld avg %lld max %lld\n", name.c_str(), nc, p.nsteps, p.nst,
-            (g1 - g0) / 1e3, cmin, csum / nc, cmax);
-    h->prof.end(c.st);
-    return 0;
-  }
-  launch_conv_ring(p, tab->grid, c.st);
   h->prof.end(c.st);
   return 0;
 }
@@ -1184,7 +1058,6 @@ int pack_bf16_weights(lsd_handle* h, const std::vector<float>& f32_arena) {
   memcpy(h->lapw_host, &f32_arena[h->convs.at("art.lap").w_off], sizeof(h->lapw_host));   // (video_rows takes them by value)
   h->blayers.clear();
   const int vstr[4] = {1, 2, 2, 2};
-  const bool cta2 = !(LSD_ENV("LSD_UMMA_CTA2") && atoi(LSD_ENV("LSD_UMMA_CTA2")) == 0);
   for (int l = 1; l <= 4; ++l) {
     const std::string p = "visual_encoder.layer" + std::to_string(l);
     const int s = vstr[l - 1];
@@ -1192,9 +1065,8 @@ int pack_bf16_weights(lsd_handle* h, const std::vector<float>& f32_arena) {
     // twice the MMA time per refill (4 M-tiles per weight stage instead of 2), measured 15-18 % faster than one 256-column slice.
     int nt = l >= 3 ? 128 : 0;
     if (const char* e = getenv(l == 3 ? "LSD_UMMA_NT3" : (l == 4 ? "LSD_UMMA_NT4" : "LSD_UMMA_NTX"))) nt = atoi(e);   // tuning knob
-    // CTA pairs (cta_group::2) for the Cout = 64 layers — stem and layer1, bound by the shared-memory read port — LSD_UMMA_CTA2=0 turns
-    // them off; the accumulation order is the same, so are the bits.
-    const bool pairs = cta2 && l == 1;
+    // CTA pairs (cta_group::2) for the Cout = 64 layers — stem and layer1, bound by the shared-memory read port
+    const bool pairs = l == 1;
     P.add(p + ".conv1", p + ".conv1", s, s, "", nt, false, /*merge_kt=*/l >= 2, pairs);   // 12x12 / 6x6 / 3x3 maps: one band per parity set
     P.ds_sh = 2; P.ds_sw = 2;
     P.add(p + ".conv2", p + ".conv2", 1, 1, l == 1 ? "" : p + ".downsample", nt, false, false, pairs);
@@ -1205,27 +1077,7 @@ int pack_bf16_weights(lsd_handle* h, const std::vector<float>& f32_arena) {
       P.add_fold(p + ".conv2#fold", p + ".conv2", p + ".downsample", fnt);
     }
   }
-  P.add_toeplitz("visual_encoder.stem", "visual_encoder.stem", 8, 0, false, cta2);  // 7 taps in w -> 8-pixel window starting at 2*wo-4
-  for (int cv = 0; cv < 2; ++cv) {
-    // layer1's 3x3x3 convolutions for the temporal-ring kernel (conv_ring.cu): per K16 chunk and spatial tap one block
-    // [2 K halves][192 = 3 temporal taps x 64 columns][8]; column block j holds the weights of temporal tap dt = j - 1
-    const ConvP& c = h->convs.at(cv == 0 ? "visual_encoder.layer1.conv1" : "visual_encoder.layer1.conv2");
-    h->l1_ring_w_off[cv] = 0;
-    if (c.kt != 3 || c.kh != 3 || c.kw != 3 || c.Cin != 64 || c.Cout != 64) continue;
-    h->l1_ring_w_off[cv] = P.w.size();
-    const float* W = &f32_arena[c.w_off];
-    const float* sc = c.has_scale ? &f32_arena[c.scale_off] : nullptr;
-    for (int ch = 0; ch < 4; ++ch)
-      for (int b = 0; b < 3; ++b)
-        for (int d = 0; d < 3; ++d)
-          for (int kc = 0; kc < 2; ++kc)
-            for (int n = 0; n < 192; ++n)
-              for (int e = 0; e < 8; ++e) {
-                const int ci = ch * 16 + kc * 8 + e, a = n / 64, co = n % 64;
-                P.w.push_back(f2bf(W[((size_t)((a * 3 + b) * 3 + d) * 64 + ci) * 64 + co] * (sc ? sc[co] : 1.0f)));
-              }
-    while (P.w.size() % 64) P.w.push_back(0);
-  }
+  P.add_toeplitz("visual_encoder.stem", "visual_encoder.stem", 8, 0, false, true);  // 7 taps in w -> 8-pixel window starting at 2*wo-4
   {
     // the same weights for the temporal-ring kernel (stem_ring.cu): per (parity set, kernel row) tap and K chunk one block
     // [2 K halves][192 = 3 temporal taps x 64 columns][8]; column block j holds the weights of temporal tap dt = j - 1
@@ -1359,11 +1211,10 @@ static int token_path_bf16(const BCtx& b, const Shapes& s, bool combined = false
   const int B = s.B, T = s.T, TA = s.A4, NT = T + 1;
   const UcGeom gt = P.gt;
   int rc = 0;
-  // Independent pieces run side by side on two helper streams (LSD_TOK_SERIAL=1 keeps everything on one stream): the token path is
-  // a chain of latency-bound launches, each far too small to fill the SMs it gets.
+  // Independent pieces run side by side on two helper streams: the token path is a chain of latency-bound launches, each far too
+  // small to fill the SMs it gets.
   lsd_handle* h = b.h;
-  const bool par = LSD_ENV("LSD_TOK_SERIAL") == nullptr;
-  if (par && !h->tok_stream[0]) {
+  if (!h->tok_stream[0]) {
     for (int i = 0; i < 2; ++i)
       if (cudaStreamCreateWithFlags(&h->tok_stream[i], cudaStreamNonBlocking) != cudaSuccess ||
           cudaEventCreateWithFlags(&h->ev_tok_join[i], cudaEventDisableTiming) != cudaSuccess)
@@ -1371,9 +1222,9 @@ static int token_path_bf16(const BCtx& b, const Shapes& s, bool combined = false
     if (cudaEventCreateWithFlags(&h->ev_tok_fork, cudaEventDisableTiming) != cudaSuccess) return lsd_fail(h, LSD_ERR_CUDA, "token helper event creation failed");
   }
   BCtx b1 = b, b2 = b;                      // helper-stream contexts (same workspace and plan)
-  if (par) { b1.st = h->tok_stream[0]; b2.st = h->tok_stream[1]; }
-  auto fork = [&](int n) { if (par) { cudaEventRecord(h->ev_tok_fork, st); for (int i = 0; i < n; ++i) cudaStreamWaitEvent(h->tok_stream[i], h->ev_tok_fork, 0); } };
-  auto join = [&](int n) { if (par) for (int i = 0; i < n; ++i) { cudaEventRecord(h->ev_tok_join[i], h->tok_stream[i]); cudaStreamWaitEvent(st, h->ev_tok_join[i], 0); } };
+  b1.st = h->tok_stream[0]; b2.st = h->tok_stream[1];
+  auto fork = [&](int n) { cudaEventRecord(h->ev_tok_fork, st); for (int i = 0; i < n; ++i) cudaStreamWaitEvent(h->tok_stream[i], h->ev_tok_fork, 0); };
+  auto join = [&](int n) { for (int i = 0; i < n; ++i) { cudaEventRecord(h->ev_tok_join[i], h->tok_stream[i]); cudaStreamWaitEvent(st, h->ev_tok_join[i], 0); } };
   // ---- cross-modal attention + gated fusion (fusion_module.py:54-87)
   float *pv = combined ? nullptr : b.f("proj_v"), *pa = combined ? nullptr : b.f("proj_a"), *gi = b.f("gate_in");   // (combined: tok_front reads vcomb / acomb)
   if (!combined) {
@@ -1629,13 +1480,12 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   };
   g_tl.on = LSD_ENV("LSD_TIMELINE") != nullptr;
   g_tl.mark(st, "start");
-  const bool audio_after_rows = LSD_ENV("LSD_AUDIO_AFTER_ROWS") && atoi(LSD_ENV("LSD_AUDIO_AFTER_ROWS")) != 0;   // tuning knob, see below
   if (vt) {                             // the first audio group takes the audio encoder's place next to the visual encoder
     cudaEventRecord(h->ev_start, st);
     cudaStreamWaitEvent(sst, h->ev_start, 0);
     if ((rc = var_audio(0, sst, bs.max_ctas))) return rc;
     cudaEventRecord(h->ev_audio, sst);
-  } else if (audio_early && !audio_after_rows) {
+  } else if (audio_early) {
     cudaEventRecord(h->ev_start, st);
     cudaStreamWaitEvent(sst, h->ev_start, 0);
     if ((rc = audio_encoder_bf16(bs, s, inputs_ready, audio, adt))) return rc;
@@ -1651,97 +1501,23 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   else if (inputs_ready) launch_video_rows(b.f("vid"), LSD_F32, LSD_NDHWC, lapw, h->lapw_host, b.org(xs), b.org(xl), xs.set_stride, xs.g, s.H, s.W, st, h->num_sms);
   else launch_video_rows(video, vdt, vlayout, lapw, h->lapw_host, b.org(xs), b.org(xl), xs.set_stride, xs.g, s.H, s.W, st, h->num_sms);
   g_tl.mark(st, "M:video_rows");
-  // (LSD_AUDIO_AFTER_ROWS=1 forks the audio encoder after video_rows instead.  video_rows walks its tiles with a static stride, so
-  // side-stream kernels holding SMs at its start delay it: 267 -> 123 us when it runs alone, and ONE forward is 110 us shorter
-  // (timeline at B=64: head at 2543 instead of 2665 us).  Back to back the early fork wins: scripts/exp_ab.py, 40 / 400 forwards:
-  // 2.69 / 2.86 ms per forward against 2.73 / 2.89 — the audio encoder of forward k+1 then fills the SMs the tail of forward k
-  // leaves idle.  Throughput is the metric, so the early fork stays the default.)
-  if (!vt && audio_early && audio_after_rows) {
-    cudaEventRecord(h->ev_start, st);
-    cudaStreamWaitEvent(sst, h->ev_start, 0);
-    if ((rc = audio_encoder_bf16(bs, s, inputs_ready, audio, adt))) return rc;
-    if (tcomb && (rc = audio_tokens(bs, s))) return rc;
-    g_tl.mark(sst, "S:audio_enc");
-    cudaEventRecord(h->ev_audio, sst);
-  }
-  // The high-frequency branch only needs the laplacian rows: LSD_HF_EARLY=1 (tuning knob) runs it on the side stream right after the
-  // audio encoder, next to the visual encoder, instead of in the tail.
-  const bool hf_early = LSD_ENV("LSD_HF_EARLY") != nullptr;
   float* comb = b.f("comb");
   PlanarOut none{nullptr, nullptr, 0, 0, 0, 0};
   const PBuf& hf = pb["hf_f"];
-  if (hf_early) {
-    cudaEventRecord(h->ev_fork, st);
-    cudaStreamWaitEvent(sst, h->ev_fork, 0);
-    RUNS("art.hf0", a_.in = &xl; a_.og = xl.g; a_.act = ACT_RELU; a_.yp = &hf);
-    RUNS("art.hf3", a_.in = &hf; a_.og = hf.g; a_.act = ACT_RELU; a_.yp = &pb["hf_b"]);
-    launch_planar_mean2(bs.org(pb["hf_b"]), pb["hf_b"].plane_stride, hf.g, 64, comb + 384, 448, 1, none, sst);
-    g_tl.mark(sst, "S:hf3");
+  // Stem + max-pool.  Default: the temporal-ring kernel (stem_ring.cu: the three temporal taps as one N = 192 MMA); LSD_STEM_RING=0,
+  // rows too wide for the ring or non-canonical stem weights take the flat shift-GEMM launch (CTA pairs).  The summation order
+  // differs between the two, the bits of a given route do not depend on the batch.
+  static const bool ring_env = !(LSD_ENV("LSD_STEM_RING") && atoi(LSD_ENV("LSD_STEM_RING")) == 0);
+  if (ring_env && h->stem_ring_w_off != 0 && 128 + 3 * xs.g.RW + 3 <= 640) {
+    if ((rc = run_stem_ring(b, xs, so))) return rc;
+  } else {
+    RUN("visual_encoder.stem", a_.in = &xs; a_.og = xs.g; a_.act = ACT_RELU; a_.yp = &so);
   }
-  // Stem + max-pool.  LSD_STEM_CHUNK=n (tuning knob, default 0 = one pass over the whole batch) runs them in sub-batches of n
-  // windows so that the stem output of a sub-batch (11 MB per window) is still in the 126 MB L2 when the max-pool reads it and the
-  // 640 MB stem output of a B=64 step never makes the round trip through HBM.  Measured at B=64: 20.7k windows/s in one pass,
-  // 19.1k with n=7, 19.7k with n=15 — the stem is tensor-bound, not HBM-bound, and the extra wave tails and launches of the
-  // sub-batches cost more than the saved DRAM traffic.  Sub-batch views share the buffers' plane strides; only the first position moves.
-  {
-    int chunk = 0;
-    if (const char* e = LSD_ENV("LSD_STEM_CHUNK")) chunk = atoi(e);
-    // LSD_STEM_POOL_FUSE=1 (with LSD_UMMA_CTA2=0: the fused epilogue is not built for CTA pairs): the max-pool rides in the stem's epilogue (UC_Y_POOL, umma_conv.cu): the 10 MB per window of stem
-    // output never leave the SM (DRAM traffic of stem + pool 1.6 GB -> 0.32 GB per 64 windows), same bits as the two-kernel path.
-    // Off by default: the stem is bound by the shared-memory read port (N = 64 MMAs), and the pooling pass reads its 3x3
-    // neighbourhoods through the same port — measured at B=64: stem 696 k -> 1 102 k cycles (708 k with the pooling reads skipped),
-    // which cancels the 0.21 ms of the separate max-pool kernel at burst clocks (2.880 vs 2.875 ms per step; +1.3 % under the
-    // power cap, where the saved DRAM traffic buys clock).
-    static const bool fuse_env = LSD_ENV("LSD_STEM_POOL_FUSE") && atoi(LSD_ENV("LSD_STEM_POOL_FUSE")) != 0;
-    const bool fuse_pool = fuse_env && !h->blayers.at("visual_encoder.stem").halves && !(xs.g.H & 1) && !(xs.g.W & 1) && x1.g.H * 2 == xs.g.H && x1.g.W * 2 == xs.g.W && 2 * xs.g.RW + 2 <= 128;
-    // Default: the temporal-ring kernel (stem_ring.cu: the three temporal taps as one N = 192 MMA); LSD_STEM_RING=0 keeps the flat
-    // shift-GEMM launch (CTA pairs).  The summation order differs between the two, the bits of a given route do not depend on the batch.
-    static const bool ring_env = !(LSD_ENV("LSD_STEM_RING") && atoi(LSD_ENV("LSD_STEM_RING")) == 0);
-    const bool ring = ring_env && h->stem_ring_w_off != 0 && !fuse_env && (chunk <= 0 || chunk >= B) && 128 + 3 * xs.g.RW + 3 <= 640;
-    // LSD_STEM_POOL_INLINE=1: the max-pool done inside the ring kernel by four extra warps per CTA (same bits; measured slower than the
-    // separate launch, see stem_ring.cu)
-    static const bool pool_inline = LSD_ENV("LSD_STEM_POOL_INLINE") && atoi(LSD_ENV("LSD_STEM_POOL_INLINE")) != 0;
-    if (ring && pool_inline && x1.g.H * 2 == xs.g.H && x1.g.W * 2 == xs.g.W) {
-      if ((rc = run_stem_ring(b, xs, so, &x1))) return rc;
-      g_tl.mark(st, "M:stem");
-    } else if (ring) {
-      if ((rc = run_stem_ring(b, xs, so))) return rc;
-      g_tl.mark(st, "M:stem");
-      launch_planar_maxpool(b.org(so), so.plane_stride, so.g, b.org(x1), x1.plane_stride, x1.g, 64, st);
-    } else if (fuse_pool && (chunk <= 0 || chunk >= B)) {
-      RUN("visual_encoder.stem", a_.in = &xs; a_.og = xs.g; a_.act = ACT_RELU; a_.yp = &x1; a_.y_mode = UC_Y_POOL);
-      g_tl.mark(st, "M:stem");
-    } else if (chunk <= 0 || chunk >= B) {
-      RUN("visual_encoder.stem", a_.in = &xs; a_.og = xs.g; a_.act = ACT_RELU; a_.yp = &so);
-      g_tl.mark(st, "M:stem");
-      launch_planar_maxpool(b.org(so), so.plane_stride, so.g, b.org(x1), x1.plane_stride, x1.g, 64, st);
-    } else {
-      auto view = [&](const PBuf& full, int n0, int nb) {
-        PBuf v = full;
-        v.g = make_geom_ex(nb, full.g.T, full.g.H, full.g.W, full.g.ot, full.g.oh, full.g.HP - full.g.H - full.g.oh, full.g.ow,
-                           full.g.RW - full.g.W - full.g.ow);
-        v.origin = full.origin + (int64_t)n0 * full.g.TS * full.g.SL * 8;
-        return v;
-      };
-      for (int n0 = 0; n0 < B; n0 += chunk) {
-        const int nb = std::min(chunk, B - n0);
-        const PBuf xs_v = view(xs, n0, nb), so_v = view(so, n0, nb), x1_v = view(x1, n0, nb);
-        RUN("visual_encoder.stem", a_.in = &xs_v; a_.og = xs_v.g; a_.act = ACT_RELU; a_.yp = &so_v);
-        launch_planar_maxpool(b.org(so_v), so_v.plane_stride, so_v.g, b.org(x1_v), x1_v.plane_stride, x1_v.g, 64, st);
-      }
-      g_tl.mark(st, "M:stem");
-    }
-  }
+  g_tl.mark(st, "M:stem");
+  launch_planar_maxpool(b.org(so), so.plane_stride, so.g, b.org(x1), x1.plane_stride, x1.g, 64, st);
   g_tl.mark(st, "M:maxpool");
   // ---- residual stages (visual_encoder.py:81-87, 133-152)
-  {
-    // layer1 (64 -> 64, 24x24 maps): LSD_L1_RING=1 runs its two convolutions through the temporal-ring kernel (conv_ring.cu)
-    static const bool l1_ring = LSD_ENV("LSD_L1_RING") && atoi(LSD_ENV("LSD_L1_RING")) != 0;
-    if (l1_ring && h->l1_ring_w_off[0] && h->l1_ring_w_off[1] && 128 + 2 * x1.g.RW + 2 <= 512) {
-      if ((rc = run_conv_ring(b, "visual_encoder.layer1.conv1", 0, x1, pb["l1a"], nullptr))) return rc;
-      if ((rc = run_conv_ring(b, "visual_encoder.layer1.conv2", 1, pb["l1a"], pb["y1"], &x1))) return rc;
-    } else if ((rc = res_stage_umma(b, "visual_encoder.layer1", x1, pb["l1a"], pb["y1"], false, UC_Y_PARITY))) return rc;
-  }
+  if ((rc = res_stage_umma(b, "visual_encoder.layer1", x1, pb["l1a"], pb["y1"], false, UC_Y_PARITY))) return rc;
   g_tl.mark(st, "M:layer1");
   // layer2 writes y2 folded when layer3 runs on the folded route (small maps, see fold_route); y4 is always the plain padded map
   if ((rc = res_stage_umma(b, "visual_encoder.layer2", pb["y1"], pb["l2a"], pb["y2"], true, P.fold3 ? UC_Y_FOLD : UC_Y_PARITY))) return rc;
@@ -1779,32 +1555,25 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   g_tl.mark(sst, "S:td_delta");
   // high-frequency branch: Conv3d 3->32 s(1,2,2) on the laplacian pixel rows (Toeplitz K), Conv3d 32->64 s(1,2,2) planar.
   // It depends on nothing but the laplacian rows, so in the tail it runs on a second side stream NEXT TO the
-  // temporal-inconsistency convolutions instead of behind them (LSD_HF_SERIAL=1 restores the single side stream): both
-  // chains are capped at half of the SMs, and the token path's small grids fit in between.
-  if (!hf_early) {
-    const bool hf_par = LSD_ENV("LSD_HF_SERIAL") == nullptr;   // (also when batches are pipelined: 10k-window run 19.6k -> 20.5k windows/s)
-    cudaStream_t hst = sst;
-    if (hf_par) {
-      if (!h->side2_stream) {
-        if (cudaStreamCreateWithFlags(&h->side2_stream, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&h->ev_join2, cudaEventDisableTiming) != cudaSuccess)
-          return lsd_fail(h, LSD_ERR_CUDA, "second side stream creation failed");
-      }
-      hst = h->side2_stream;
-      cudaStreamWaitEvent(hst, h->ev_fork, 0);
-    }
-    BCtx bh = bs;
-    bh.st = hst;
-    if (const char* e = LSD_ENV("LSD_HF_CTAS")) bh.max_ctas = atoi(e);
-    RUNC(bh, "art.hf0", a_.in = &xl; a_.og = xl.g; a_.act = ACT_RELU; a_.yp = &hf);
-    g_tl.mark(hst, "S:hf0");
-    RUNC(bh, "art.hf3", a_.in = &hf; a_.og = hf.g; a_.act = ACT_RELU; a_.yp = &pb["hf_b"]);
-    launch_planar_mean2(bh.org(pb["hf_b"]), pb["hf_b"].plane_stride, hf.g, 64, comb + 384, 448, 1, none, hst);
-    g_tl.mark(hst, "S:hf3");
-    if (hf_par) {                       // fold the second side stream back into the first: ev_join then covers both
-      cudaEventRecord(h->ev_join2, hst);
-      cudaStreamWaitEvent(sst, h->ev_join2, 0);
-    }
+  // temporal-inconsistency convolutions instead of behind them: both chains are capped at half of the SMs, and the token path's
+  // small grids fit in between (also when batches are pipelined: 10k-window run 19.6k -> 20.5k windows/s).
+  if (!h->side2_stream) {
+    if (cudaStreamCreateWithFlags(&h->side2_stream, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&h->ev_join2, cudaEventDisableTiming) != cudaSuccess)
+      return lsd_fail(h, LSD_ERR_CUDA, "second side stream creation failed");
   }
+  const cudaStream_t hst = h->side2_stream;
+  cudaStreamWaitEvent(hst, h->ev_fork, 0);
+  BCtx bh = bs;
+  bh.st = hst;
+  if (const char* e = LSD_ENV("LSD_HF_CTAS")) bh.max_ctas = atoi(e);
+  RUNC(bh, "art.hf0", a_.in = &xl; a_.og = xl.g; a_.act = ACT_RELU; a_.yp = &hf);
+  g_tl.mark(hst, "S:hf0");
+  RUNC(bh, "art.hf3", a_.in = &hf; a_.og = hf.g; a_.act = ACT_RELU; a_.yp = &pb["hf_b"]);
+  launch_planar_mean2(bh.org(pb["hf_b"]), pb["hf_b"].plane_stride, hf.g, 64, comb + 384, 448, 1, none, hst);
+  g_tl.mark(hst, "S:hf3");
+  // fold the second side stream back into the first: ev_join then covers both
+  cudaEventRecord(h->ev_join2, hst);
+  cudaStreamWaitEvent(sst, h->ev_join2, 0);
   }
   cudaEventRecord(h->ev_join, sst);
   // ---- everything below is the latency-bound tail (small grids): on the caller's stream, or on the tail stream when batches

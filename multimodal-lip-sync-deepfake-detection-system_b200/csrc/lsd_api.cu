@@ -15,7 +15,6 @@
 #include "tok_front.cuh"
 #include "tok_fused.cuh"
 #include "stem_ring.cuh"
-#include "conv_ring.cuh"
 #include "umma_conv.cuh"
 using namespace lsd;
 
@@ -86,7 +85,6 @@ extern "C" int lsd_create(lsd_handle** out, int device) {
     cudaError_t ce = lsd::umma_conv_device_init();
     if (ce == cudaSuccess) ce = lsd::tok_fused_device_init();
     if (ce == cudaSuccess) ce = lsd::stem_ring_device_init();
-    if (ce == cudaSuccess) ce = lsd::conv_ring_device_init();
     if (ce == cudaSuccess) ce = lsd::tok_front_device_init();
     if (ce != cudaSuccess) rc = lsd_fail(h, LSD_ERR_CUDA, "lsd_create: kernel attribute setup: %s", cudaGetErrorString(ce));
   }
@@ -108,9 +106,7 @@ extern "C" void lsd_destroy(lsd_handle* h) {
   if (h->tokf_vec) cudaFree(h->tokf_vec);
   if (h->mel_tables) cudaFree(h->mel_tables);
   if (h->prog_arena) cudaFree(h->prog_arena);
-  for (auto& kv : h->ring_tabs) { if (kv.second.dev) cudaFree(kv.second.dev); if (kv.second.frames) cudaFree(kv.second.frames); }
-  if (h->ring_cnt) cudaFree(h->ring_cnt);
-  if (h->tile_ctr_arena) cudaFree(h->tile_ctr_arena);
+  for (auto& kv : h->ring_tabs) if (kv.second.dev) cudaFree(kv.second.dev);
   if (h->lm_clips) cudaFree(h->lm_clips);
   if (h->ev_lm_clips) cudaEventDestroy(h->ev_lm_clips);
   for (cudaEvent_t e : h->prof.ev) cudaEventDestroy(e);

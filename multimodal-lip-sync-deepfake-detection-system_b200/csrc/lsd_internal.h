@@ -100,15 +100,8 @@ struct lsd_handle {
   std::unordered_map<uint64_t, const void*> prog_cache;
   // temporal-ring stem (stem_ring.cu): packed N = 192 weights inside barena, step tables per (batch, frames, geometry)
   size_t stem_ring_w_off = 0;              // bf16 elements into barena; 0 = not packed
-  size_t l1_ring_w_off[2] = {0, 0};        // temporal-ring weights of visual_encoder.layer1.conv1 / conv2 (conv_ring.cu); 0 = not packed
-  struct RingTab { void* dev = nullptr; int nsteps = 0, grid = 0; int* frames = nullptr; int nfr = 0; };   // frames: per-CTA pool lists (inline max-pool)
-  unsigned* ring_cnt = nullptr;            // per-frame completion counters of the inline max-pool (zeroed before every launch)
-  size_t ring_cnt_cap = 0;
+  struct RingTab { void* dev = nullptr; int nsteps = 0, grid = 0; };
   std::unordered_map<uint64_t, RingTab> ring_tabs;
-  // tile counters of the tcgen05 launches (dynamic tile scheduling): 16 words per layer name, zero whenever the layer is not
-  // running (the last CTA of a launch resets them); launches of one layer are always ordered on one stream
-  unsigned* tile_ctr_arena = nullptr;
-  std::map<std::string, int> tile_ctr_idx;
   // log-mel tables (device): hann[400], cos[400], sin[400], melw[80*32], lo[80], cnt[80]
   void* mel_tables = nullptr;
   const float *d_hann = nullptr, *d_cos = nullptr, *d_sin = nullptr, *d_melw = nullptr;

@@ -18,15 +18,8 @@
 // The summation order of an output (bias, then slabs t-1, t, t+1, each over parity sets, rows and K chunks) does not depend on how
 // the ranges are cut, so logits stay independent of the batch composition bit for bit.
 //
-// Warp roles (512 threads): warp 0 producer, warps 1-2 MMA issuers (one per slot), warp 3 TMEM allocation, warps 4-11 epilogue
-// (warps 4-7 slot 0, 8-11 slot 1; warp % 4 = TMEM lane quarter), warps 12-15 inline max-pool.
-//
-// Inline max-pool (opt-in, LSD_STEM_POOL_INLINE=1; measured slower: 128 pool threads per SM are latency-bound on their L2 reads —
-// stem + pool 587 us against 304 + 131 us with the separate launch): the host orders the columns so that the frames of a window complete progressively (full columns round-robin over
-// the slots, window-major; only the remainder is cut into ranges); every epilogue warp counts the chunk it has stored into a per-frame
-// counter (fence, then one atomic), and the pool warps of each CTA walk their share of the frames in completion order: wait for the
-// counter, read the 3x3 neighbourhoods from L2 (ld.global.cg), write the pooled plane.  The 0.6 GB of stem output are still written
-// (L2 write-back) but never read back from DRAM, and the separate max-pool launch (0.13 - 0.15 ms on the critical path) is gone.
+// Warp roles (384 threads): warp 0 producer, warps 1-2 MMA issuers (one per slot), warp 3 TMEM allocation, warps 4-11 epilogue
+// (warps 4-7 slot 0, 8-11 slot 1; warp % 4 = TMEM lane quarter).
 #include "stem_ring.cuh"
 
 #include <cstdio>
@@ -41,6 +34,7 @@ using namespace umma;
 namespace {
 
 constexpr int SR_NST = 6;   // SR_NST: most ring stages (barrier arrays); p.nst are in use
+constexpr int SR_THREADS = 384;
 
 __device__ __forceinline__ uint32_t sr_div(uint32_t n, uint32_t m, int s) { return (uint32_t)(((uint64_t)n * m) >> (31 + s)); }
 __device__ __forceinline__ bool sr_valid(const UcGeom& g, int64_t P) {
@@ -54,19 +48,6 @@ __device__ __forceinline__ bool sr_valid(const UcGeom& g, int64_t P) {
   const int h = row - g.oh, w = col - g.ow;
   return (unsigned)t < (unsigned)g.T && (unsigned)h < (unsigned)g.H && (unsigned)w < (unsigned)g.W && n < g.N;
 }
-__device__ __forceinline__ int64_t sr_flat(const UcGeom& g, int n, int t, int h, int w) {
-  return (((int64_t)n * g.TS + t + g.ot) * g.HP + h + g.oh) * g.RW + w + g.ow;
-}
-__device__ __forceinline__ unsigned sr_ld_acquire(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint4 sr_ld_cg(const uint4* p) {
-  uint4 v;
-  asm volatile("ld.global.cg.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  return v;
-}
 __device__ __forceinline__ uint4 sr_pack8_relu(const float* v) {
   uint4 o;
   uint32_t* ow = reinterpret_cast<uint32_t*>(&o);
@@ -75,16 +56,11 @@ __device__ __forceinline__ uint4 sr_pack8_relu(const float* v) {
   return o;
 }
 
-// POOLW: with the counting warp and the four pool warps of the inline max-pool (512 threads instead of 384)
-template <bool POOLW>
-__global__ void __launch_bounds__(POOLW ? 512 : 384, 1) stem_ring_kernel(const __grid_constant__ StemRingP p) {
-  constexpr int SR_THREADS = POOLW ? 512 : 384;
+__global__ void __launch_bounds__(SR_THREADS, 1) stem_ring_kernel(const __grid_constant__ StemRingP p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ uint64_t full_bar[SR_NST], empty_bar[SR_NST], tfull[2][4], tempty[2][4], wbar;
   __shared__ uint32_t tmem_base_s;
-  __shared__ unsigned done_cnt[2];   // per slot: epilogue warps that have finished a step (4 per step); read by the counting warp
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (tid < 2) done_cnt[tid] = 0u;
   const uint32_t r0 = ((uint32_t)p.units[0] * 16u + 127u) & ~127u, r1 = ((uint32_t)p.units[1] * 16u + 127u) & ~127u;
   const uint32_t slot_bytes = r0 + r1, stage_bytes = 2u * slot_bytes;
   uint8_t* const wsm = smem;                       // resident weights
@@ -233,86 +209,6 @@ __global__ void __launch_bounds__(POOLW ? 512 : 384, 1) stem_ring_kernel(const _
       }
       mma_commit_pred(&empty_bar[stage], leader);       // the stage is free once the MMAs that read it have completed
     }
-  } else if (warp == 3) {
-    // ------------------------------------------------ counting warp (inline max-pool): lane s follows slot s.  Steps whose four
-    // epilogue warps have all finished are published in batches: ONE device-scope fence (cumulative over the stores this CTA's
-    // epilogue warps made before their shared-memory counts), then one atomic per stored chunk on its frame's counter.
-    if (POOLW && lane < 2) {
-      const SrStep* const st = st0 + (size_t)lane * (size_t)p.nsteps;
-      int nact = 0;
-      for (int k = 0; k < p.nsteps; ++k) nact += (st[k].flags & SR_ACTIVE) ? 1 : 0;
-      int done = 0, k = 0;
-      unsigned spins = 0;
-      while (done < nact) {
-        const int m = (int)(*reinterpret_cast<volatile unsigned*>(&done_cnt[lane]) >> 2);
-        if (m <= done) {
-          __nanosleep(200);
-          if (++spins > (1u << 23)) __trap();
-          continue;
-        }
-        __threadfence_block();
-        __threadfence();
-        for (; done < m; ++k) {
-          const SrStep sd = st[k];
-          if (!(sd.flags & SR_ACTIVE)) continue;
-          if (sd.flags & SR_STORE) {
-            const uint32_t slab = sr_div((uint32_t)sd.in_pos, p.g.mSL, p.g.sSL) - 1u;       // the output slab: one before the input slab
-            const uint32_t n = sr_div(slab, p.g.mTS, p.g.sTS);
-            atomicAdd(p.frame_cnt + (size_t)n * p.g.T + (slab - n * (uint32_t)p.g.TS - (uint32_t)p.g.ot), 4u);
-          }
-          ++done;
-        }
-      }
-    }
-  } else if (warp >= 12) {
-    // ------------------------------------------------ inline max-pool of completed frames (4 warps; thread = pooled position)
-    if (POOLW) {
-      const int* fl = p.pool_frames + (size_t)blockIdx.x * (size_t)p.pool_nfr;
-      const int ptid = (warp - 12) * 32 + lane;
-      const uint32_t NINF2 = 0xFF80FF80u;                                   // (-inf, -inf) in bf16
-      const int total = p.gp.H * p.gp.W;
-      for (int fi = 0; fi < p.pool_nfr; ++fi) {
-        const int f = fl[fi];
-        if (f < 0) break;
-        if (lane == 0) {
-          unsigned spins = 0;
-          while (sr_ld_acquire(p.frame_cnt + f) < (unsigned)p.pool_expected) {
-            __nanosleep(256);
-            if (++spins > (1u << 22)) __trap();      // (~1 s: a counting bug must not hang the GPU)
-          }
-        }
-        __syncwarp();
-        const int n = f / p.g.T, t = f - n * p.g.T;
-        const int64_t xin = sr_flat(p.g, n, t, 0, 0) * 8, yout = sr_flat(p.gp, n, t, 0, 0) * 8;
-        for (int o = ptid; o < total; o += 128) {
-          const int h = o / p.gp.W, w = o - h * p.gp.W;
-#pragma unroll 2
-          for (int qp = 0; qp < 8; ++qp) {
-            const uint4* xc = reinterpret_cast<const uint4*>(p.y + (int64_t)qp * p.y_plane_stride + xin);
-            uint4 v[9];
-#pragma unroll
-            for (int dh = 0; dh < 3; ++dh)
-#pragma unroll
-              for (int dw = 0; dw < 3; ++dw) {
-                const int hi = 2 * h - 1 + dh, wi = 2 * w - 1 + dw;
-                v[dh * 3 + dw] = ((unsigned)hi < (unsigned)p.g.H && (unsigned)wi < (unsigned)p.g.W) ? sr_ld_cg(xc + hi * p.g.RW + wi)
-                                                                                                  : make_uint4(NINF2, NINF2, NINF2, NINF2);
-              }
-            uint32_t* m = reinterpret_cast<uint32_t*>(&v[0]);
-#pragma unroll
-            for (int kk = 1; kk < 9; ++kk) {
-              const uint32_t* r = reinterpret_cast<const uint32_t*>(&v[kk]);
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                const __nv_bfloat162 mx = __hmax2(*reinterpret_cast<const __nv_bfloat162*>(&m[e]), *reinterpret_cast<const __nv_bfloat162*>(&r[e]));
-                m[e] = *reinterpret_cast<const uint32_t*>(&mx);
-              }
-            }
-            *reinterpret_cast<uint4*>(p.yp + (int64_t)qp * p.yp_plane_stride + yout + (int64_t)(h * p.gp.RW + w) * 8) = v[0];
-          }
-        }
-      }
-    }
   } else if (warp >= 4) {
     // ------------------------------------------------ epilogue: drain the completed block (thread = position), ReLU, bf16, planar store
     const int slot = (warp - 4) >> 2, quarter = warp & 3;
@@ -351,9 +247,6 @@ __global__ void __launch_bounds__(POOLW ? 512 : 384, 1) stem_ring_kernel(const _
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tempty[slot][q & 3]);
-      // (inline max-pool: this warp's part of step q is stored; the counting warp publishes completed frames — a device-scope
-      //  fence per step HERE stalled the accumulator ring: 314 -> 719 us)
-      if (POOLW && lane == 0) { __threadfence_block(); atomicAdd(&done_cnt[slot], 1u); }
       if (warp == 4) stamp(3, k, 1);
       ++q;
     }
@@ -377,15 +270,12 @@ size_t stem_ring_smem_bytes(const StemRingP& p) {
 }
 
 cudaError_t stem_ring_device_init() {
-  cudaError_t e = cudaFuncSetAttribute(stem_ring_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 223 * 1024);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(stem_ring_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 223 * 1024);
-  return e;
+  return cudaFuncSetAttribute(stem_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 223 * 1024);
 }
 
 void launch_stem_ring(const StemRingP& p, int grid, cudaStream_t s) {
   if (grid <= 0 || p.nsteps <= 0) return;
-  if (p.frame_cnt) stem_ring_kernel<true><<<grid, 512, stem_ring_smem_bytes(p), s>>>(p);
-  else stem_ring_kernel<false><<<grid, 384, stem_ring_smem_bytes(p), s>>>(p);
+  stem_ring_kernel<<<grid, SR_THREADS, stem_ring_smem_bytes(p), s>>>(p);
   count_launch();
 }
 

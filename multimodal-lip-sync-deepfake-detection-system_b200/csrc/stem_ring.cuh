@@ -34,20 +34,11 @@ struct StemRingP {
   int skip;                     // timing experiments (LSD_SR_SKIP, garbage results): bit 0 epilogue without loads / stores, bit 1 no wrap MMAs
                                 // (D region pinned to block 0), bit 2 only two of the seven taps
   long long* dbg;               // optional (LSD_SR_TRACE): CTA 0 writes clock64 stamps of steps 16..47: [role 0..3][32 steps][2]
-  int nst;                      // ring stages of the pixel-row regions (6; fewer when a long step table needs the shared memory)
-  // Inline max-pool (optional): four extra warps per CTA pool the frames whose chunks have all been stored, while the data is in L2
-  // (MaxPool3d (1,3,3) / stride (1,2,2) / pad (0,1,1) of visual_encoder.py:122-126).  frame_cnt[n*T + t] counts the epilogue warps that
-  // have stored a chunk of frame (n, t); a frame is complete at pool_expected = 4 * chunks per slab.
-  unsigned* frame_cnt;          // device, N*T words, zero before the launch; nullptr: no inline pooling
-  const int* pool_frames;       // [gridDim.x][pool_nfr]: the frames this CTA pools, in expected order of completion (-1 = end)
-  int pool_nfr, pool_expected;
-  __nv_bfloat16* yp;            // pooled destination, plane 0 / position 0, geometry gp
-  int64_t yp_plane_stride;
-  UcGeom gp;
   int ntap[2];                  // taps per parity set
   int rel[2][4];                // tap offsets (positions) relative to the region start of their set
   int start[2];                 // region start relative to the chunk's first position
   int units[2];                 // region length in positions (16 B each)
+  int nst;                      // ring stages of the pixel-row regions (6; fewer when a long step table needs the shared memory)
 };
 
 cudaError_t stem_ring_device_init();

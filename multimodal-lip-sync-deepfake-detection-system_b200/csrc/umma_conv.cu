@@ -86,15 +86,11 @@ __device__ __forceinline__ void unpack8(const uint4& r, float* v) {
 //   warps 4-7  MMA issuers (1, 2 or 4 active; each owns an equal share of the tile's M-tiles); the loop nest runs
 //              warp-uniformly, only the tcgen05.mma / tcgen05.commit are predicated on one elected lane,
 //   warps 8-15 epilogue (two warps per TMEM lane quarter, each handling half of the columns).
-// Each CTA walks tiles blockIdx.x, blockIdx.x + gridDim.x, ...; the accumulators are double-buffered in TMEM when they fit so
-// that the epilogue of tile i overlaps the main loop of tile i+1, and the smem ring keeps streaming across tile boundaries.
-// Tiles are handed out dynamically: the first tile of a CTA is blockIdx.x, every further one is claimed from a per-slice global
-// counter (p.tile_ctr) by producer warp 0 — one tile ahead, so the atomic's latency hides behind the current tile — and published
-// to the other warps through a small shared-memory queue (tq_*).  A CTA that starts late because another stream's kernel still
-// held its SM then simply takes fewer tiles; with the static stride every concurrent side-stream kernel delayed the whole launch
-// by its own duration.  The last CTA to finish resets the counters for the layer's next launch.
-constexpr int UC_TQ = 8;
-constexpr int UC_CTR_DONE = 8;   // p.tile_ctr[0..7]: claims per Cout slice, [8]: finished CTAs
+// Tile walk (static stride): each CTA walks tiles blockIdx.x, blockIdx.x + gridDim.x, ... of its column slice (a folded conv
+// launches one CTA per tile).  On CTA pairs (MODE 3) the walk runs over tile pairs instead: pair blockIdx.x / 2 takes pairs
+// j, j + gridDim.x / 2, ..., and each CTA of a pair computes tile 2j + its rank in the cluster.  The accumulators are
+// double-buffered in TMEM when they fit so that the epilogue of tile i overlaps the main loop of tile i+1, and the smem ring keeps
+// streaming across tile boundaries.
 constexpr int UC_THREADS = 512;
 constexpr int UC_PROD_WARPS = 4, UC_MMA_WARP0 = 4, UC_MMA_WARPS = 4, UC_EPI_WARP0 = 8, UC_EPI_WARPS = 8;
 // (issuing one cp.async.bulk occupies the issuing thread for ~330 cycles; the cost overlaps across warps and partly across the
@@ -104,9 +100,6 @@ constexpr int UC_PROD_WARPS = 4, UC_MMA_WARP0 = 4, UC_MMA_WARPS = 4, UC_EPI_WARP
 // GENERIC = false: lean epilogue of the convolution layers (bias, ReLU/none, optional bf16 residual, planar / parity-split bf16
 // store).  GENERIC = true: everything (fp32 rows in/out, split-bf16 hi/lo outputs and residuals, GELU) for the audio encoder and
 // the token-path GEMMs.  Two instantiations keep each one small enough for the instruction cache.
-// MODE 2 (y_mode == UC_Y_POOL): the lean epilogue with the 3x3 / stride-2 max-pool of the stem fused in.  Every CTA then owns one
-// contiguous range of positions (tiles pbase, pbase + S, ... instead of the grid-strided walk), so that the rows a pooled output
-// needs from the previous tile are still in this CTA's shared-memory ring; ranges start 2 rows + 2 positions early (halo, 0.3 %).
 #define UC_MMA(...) do { if constexpr (CTA2) mma2_bf16_ss_pred(__VA_ARGS__); else mma_bf16_ss_pred(__VA_ARGS__); } while (0)
 #define UC_COMMIT(...) do { if constexpr (CTA2) mma2_commit_pred(__VA_ARGS__); else mma_commit_pred(__VA_ARGS__); } while (0)
 template <int MODE>
@@ -115,12 +108,10 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
   // 2j and 2j+1 (own A rows, own accumulator, own epilogue) but each stages only HALF of the weight columns; the leader's MMA
   // (M = 256) reads both halves.  A 64-column MMA then reads 4 KB of A + 1 KB of B from each SM's shared memory instead of 4 + 2:
   // 40 instead of 48 cycles of the 128 B/cycle read port that bounds the Cout = 64 layers (stem, layer1).
-  constexpr bool GENERIC = MODE == 1, POOL = MODE == 2, CTA2 = MODE == 3;
+  constexpr bool GENERIC = MODE == 1, CTA2 = MODE == 3;
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ uint64_t full_bar[8], empty_bar[8], tfull_bar[2], tempty_bar[2];
   __shared__ uint64_t full2_bar[8], tempty2_bar[2];      // CTA2, leader's copies used: peer's stage landed / peer's epilogue drained
-  __shared__ uint64_t tq_full[UC_TQ], tq_empty[UC_TQ];   // tile queue (dynamic tile scheduling, see below)
-  __shared__ int tq_tile[UC_TQ];
   __shared__ uint32_t tmem_base_s;
   __shared__ __align__(16) float bias_s[256];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -136,33 +127,21 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
   const int ch0 = (fold ? (int)p.fslice[slice].col : slice) * p.Cout;
   const int bcols = CTA2 ? p.Cout >> 1 : p.Cout;         // weight columns in this CTA's shared memory
   const uint32_t buf_cols = (uint32_t)(p.MT * p.Cout);
-  // tile walk: tile_first, tile_first + tile_step, ... < tile_end; tile i covers positions pbase + i*S .. + S
+  // tile walk: tile_first, tile_first + tile_step, ... < tile_end; tile i covers positions i*S .. + S
   int tile_first = blockIdx.x, tile_step = gridDim.x, tile_end = num_tiles;
-  int64_t pbase = 0, emit_lo = 0, emit_hi = 0;      // POOL: this CTA writes the pooled outputs whose last input position is in [emit_lo, emit_hi)
-  if constexpr (POOL) {
-    const int64_t per = (p.g.P_total + gridDim.x - 1) / gridDim.x;
-    emit_lo = min((int64_t)blockIdx.x * per, p.g.P_total);
-    emit_hi = min(emit_lo + per, p.g.P_total);
-    pbase = max((int64_t)0, emit_lo - (2 * p.g.RW + 2));
-    tile_first = 0; tile_step = 1;
-    tile_end = emit_hi > emit_lo ? (int)((emit_hi - pbase + S - 1) / S) : 0;
-  }
   if constexpr (CTA2) {   // the walk runs over tile PAIRS; this CTA's tile of pair j is 2j + rank (the last pair may repeat the last tile)
     tile_first = blockIdx.x >> 1; tile_step = gridDim.x >> 1; tile_end = (num_tiles + 1) >> 1;
   }
   auto tile_p0 = [&](int tile) -> int64_t {
     if constexpr (CTA2) return (int64_t)min(2 * tile + (int)cta_rank, num_tiles - 1) * S;
-    return pbase + (int64_t)tile * S;
+    return (int64_t)tile * S;
   };
-  const int tile_start = tile_first < tile_end ? tile_first : -1;   // (-1: nothing to do for this CTA)
 
   const int n_issuers = p.issuers;          // MMA-issuing warps (M-tiles are independent accumulators), chosen on the host
   if (tid == 0) {
     for (int i = 0; i < p.stages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], n_issuers); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], n_issuers); mbar_init(&tempty_bar[i], UC_EPI_WARPS); mbar_init(&tempty2_bar[i], UC_EPI_WARPS); }
     for (int i = 0; i < p.stages; ++i) mbar_init(&full2_bar[i], 1);
-    // queue readers: the producer warps other than warp 0, the MMA issuers, the epilogue warps
-    for (int i = 0; i < UC_TQ; ++i) { mbar_init(&tq_full[i], 1); mbar_init(&tq_empty[i], (uint32_t)(min(UC_PROD_WARPS, p.stages) - 1 + n_issuers + UC_EPI_WARPS)); }
     fence_barrier_init();
   }
   if (warp == UC_EPI_WARP0) {
@@ -176,7 +155,6 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
   // B = per column (hi, mid, lo, 0, ...) with b = hi + mid + lo in bf16 parts (24 mantissa bits: exact), second K half zero.
   uint8_t* const bias_a = smem + (size_t)p.stages * stage_bytes + (((size_t)p.nst_tile * sizeof(UcStageDesc) + 127) & ~(size_t)127);
   uint8_t* const bias_b = bias_a + 2048;
-  uint8_t* const lean_end = bias_b + (size_t)bcols * 32u;
   if constexpr (!GENERIC) {
     for (int i = tid; i < 128; i += UC_THREADS) reinterpret_cast<uint4*>(bias_a)[i] = make_uint4(0x3F803F80u, 0x00003F80u, 0u, 0u);
     for (int i = tid; i < 2 * bcols; i += UC_THREADS) {
@@ -207,16 +185,6 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
   tc_fence_after();
   const uint32_t tmem_base = tmem_base_s;
   if (dbg && tid == 0) p.dbg[1] = clock64();   // prologue done
-  const bool dyn = p.tile_ctr != nullptr;
-  // tile number seq (>= 1) of this CTA, as published by producer warp 0 (whole warp calls this); -1 = no more tiles
-  auto tq_read = [&](int seq) -> int {
-    const int slot = (seq - 1) % UC_TQ;
-    mbar_wait(&tq_full[slot], (uint32_t)((seq - 1) / UC_TQ) & 1u);
-    const int t = *reinterpret_cast<volatile int*>(&tq_tile[slot]);
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&tq_empty[slot]);
-    return t;
-  };
 
   if (warp < UC_PROD_WARPS) {
     // ------------------------------------------------ producers (every warp runs the loop; lane 0 of each issues its share)
@@ -230,10 +198,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
     const uint32_t smem_base = smem_u32(smem);
     const uint64_t slice64 = CTA2 ? (uint64_t)cta_rank : (uint64_t)slice;   // (CTA2: the packed weights hold the two column halves as slices)
     int k = 0;                                              // global stage counter at the start of the tile
-    int seq = 0;
-    for (int tile = tile_start; tile >= 0; k += nst) {
-      unsigned claim = 0;
-      if (dyn && warp == 0 && lane == 0) claim = atomicAdd(p.tile_ctr + slice, 1u);   // (consumed after this tile's stages are issued)
+    for (int tile = tile_first; tile < tile_end; tile += tile_step, k += nst) {
       const uint64_t p0_bytes = (uint64_t)tile_p0(tile) * 16u;
       // first stage of this tile owned by this warp: si = (warp - k) mod 4
       for (int si = ((warp - k) % npw + npw) % npw; si < nst; si += npw) {
@@ -259,25 +224,6 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
         if (mine) bulk_s2(dst, reinterpret_cast<const void*>(gsrc), nbytes, &full_bar[stage]);
         __syncwarp();
         if (dbg && lane == 0 && tile == (int)blockIdx.x && si < 8) p.dbg[56 + si] = clock64();   // copies issued
-      }
-      // next tile
-      ++seq;
-      if (!dyn) {
-        tile += tile_step;
-        if (tile >= tile_end) tile = -1;
-      } else if (warp == 0) {
-        int nt = 0;
-        if (lane == 0) {
-          nt = (int)gridDim.x + (int)claim;
-          if (nt >= num_tiles) nt = -1;
-          const int slot = (seq - 1) % UC_TQ;
-          mbar_wait(&tq_empty[slot], ((uint32_t)((seq - 1) / UC_TQ) & 1u) ^ 1u);
-          *reinterpret_cast<volatile int*>(&tq_tile[slot]) = nt;
-          mbar_arrive(&tq_full[slot]);
-        }
-        tile = __shfl_sync(0xffffffffu, nt, 0);
-      } else {
-        tile = tq_read(seq);
       }
     }
   } else if (warp < UC_MMA_WARP0 + UC_MMA_WARPS) {
@@ -314,9 +260,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
     const uint32_t leader = elect_one() ? 1u : 0u;                                 // the lane that issues (fixed for the whole kernel)
     int stage = 0, lt = 0, dbg_it = 0;
     uint32_t ph = 0;
-    // (the loop must stay provably warp-uniform for the descriptor arithmetic to live in uniform registers: "another tile?" is
-    // taken from a warp vote, which ptxas treats as uniform, not from the per-thread value read from the queue)
-    for (int tile = tile_first; tile < tile_end; ++lt, tile = dyn ? (__any_sync(0xffffffffu, tq_read(lt) >= 0) ? 0 : tile_end) : tile + tile_step) {
+    for (int tile = tile_first; tile < tile_end; ++lt, tile += tile_step) {
       const int buf = p.nbuf == 2 ? (lt & 1) : 0;
       const uint32_t use = p.nbuf == 2 ? ((uint32_t)lt >> 1) : (uint32_t)lt;   // how many times this buffer was used before
       const uint32_t tb = tmem_base + (uint32_t)buf * buf_cols + (uint32_t)(mt_lo * p.Cout);
@@ -398,11 +342,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
     const float act_lo = p.act == ACT_RELU ? 0.0f : -INFINITY;   // ReLU as one FMNMX; GELU (token GEMMs only) branches once per chunk
     const int rowt = quarter * 32 + lane;
     int lt = 0;
-    // POOL: ring of the last pool_ring positions ([slot][8 chunks of 8 channels], chunk index XOR-swizzled with the slot) and, per
-    // tile position, (pooled destination position or -1, ring slot)
-    uint8_t* const ring = lean_end;
-    int2* const pool_dst = reinterpret_cast<int2*>(ring + (size_t)p.pool_ring * 128u);
-    for (int tile = tile_start; tile >= 0; ++lt, tile = dyn ? tq_read(lt) : (tile + tile_step < tile_end ? tile + tile_step : -1)) {
+    for (int tile = tile_first; tile < tile_end; ++lt, tile += tile_step) {
       const int buf = p.nbuf == 2 ? (lt & 1) : 0;
       const uint32_t use = p.nbuf == 2 ? ((uint32_t)lt >> 1) : (uint32_t)lt;
       const uint32_t tb = tmem_base + (uint32_t)buf * buf_cols + ((uint32_t)(quarter * 32) << 16);
@@ -416,7 +356,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
       // (the lean epilogue works in 32-column steps: with a single M-tile the columns are split only if both halves are whole
       // steps, otherwise the first warp of the quarter takes all of them)
       const bool split_c = !split_m && (GENERIC || (p.Cout & 63) == 0);
-      const int m_end = (!split_m && (!split_c || POOL) && half == 1) ? 0 : p.MT;   // (POOL: a thread takes all 64 columns of its position)
+      const int m_end = (!split_m && !split_c && half == 1) ? 0 : p.MT;
       for (int m = split_m ? half : 0; m < m_end; m += split_m ? 2 : 1) {
         const int64_t P = P0 + (int64_t)m * 128 + rowt;
         int n = 0, t = 0, h = 0, w = 0;
@@ -436,30 +376,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
         const bool store_planar = ((p.y_mode == UC_Y_PLAIN && inrange) || (p.y_mode >= UC_Y_PARITY && valid)) && !(p.skip & 4);   // (skip bit 2: timing experiment)
         // this warp's columns: [half*Cout/2, (half+1)*Cout/2), or all of them when the warps split the M-tiles
         const int cbeg = split_c ? half * (p.Cout >> 1) : 0, cend = split_c ? cbeg + (p.Cout >> 1) : p.Cout;
-        if constexpr (POOL) {
-          // bias + ReLU + pad mask as in the lean path, but the packed words go to the ring; the thread also records whether its
-          // position is the last input (odd h, odd w) of a pooled output this CTA owns, and where that output lives
-          const uint32_t rel = (uint32_t)(P - pbase);
-          const uint32_t slot = rel - uc_div(rel, p.pool_mR, p.pool_sR) * p.pool_ring;
-          const bool emit = valid && (h & 1) && (w & 1) && P >= emit_lo && P < emit_hi;
-          pool_dst[m * 128 + rowt] = make_int2(emit ? (int)uc_flat(p.g2, n, t, h >> 1, w >> 1) : -1, (int)slot);
-          uint8_t* const rrow = ring + (size_t)slot * 128u;
-          const uint32_t sw = slot & 7u;
-          const uint32_t vmask = valid ? 0xffffffffu : 0u;
-          uint32_t ta = tb + (uint32_t)(m * p.Cout);
-#pragma unroll 1
-          for (int c = 0; c < 64; c += 32, ta += 32) {
-            float v[32];
-            tmem_ld32(ta, v);
-            tmem_ld_wait();          // (the bias is already in the accumulator)
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              uint4 o = pack8_relu(v + 8 * q);
-              o.x &= vmask; o.y &= vmask; o.z &= vmask; o.w &= vmask;
-              if (!(p.skip & 32)) *reinterpret_cast<uint4*>(rrow + ((((uint32_t)(c >> 3) + q) ^ sw) << 4)) = o;   // (skip bits 4-6: timing experiments)
-            }
-          }
-        } else if constexpr (!GENERIC) {
+        if constexpr (!GENERIC) {
           // lean path (Cout % 32 == 0, checked on the host): 32 columns per step.  One 32-column TMEM load, the bias (shared
           // memory) and the residual (global) are fetched before the single wait, the activation rides on the bf16 conversion
           // (cvt.rn.relu), pads are zeroed by a mask on the packed words.  ~110 instructions per step instead of ~450: the stem and
@@ -587,34 +504,6 @@ __global__ void __launch_bounds__(UC_THREADS, 1) umma_conv_kernel(const __grid_c
         if (CTA2 && cta_rank != 0) mbar_arrive_cluster(mapa_shared(smem_u32(&tempty2_bar[buf]), 0u));
         else mbar_arrive(&tempty_bar[buf]);
       }
-      if constexpr (POOL) {
-        // the tile's outputs are in the ring: pooled outputs whose last input lies in this tile are complete.  One thread per
-        // (position, 8-channel chunk), positions fastest (coalesced 16-byte stores into the destination plane).
-        asm volatile("bar.sync 1, 256;" ::: "memory");
-        const int etid = tid - UC_EPI_WARP0 * 32;
-        const int RW = p.g.RW, R = (int)p.pool_ring, sS = 31 - __clz(S);
-        for (int idx = etid; idx < ((p.skip & 16) ? 0 : S * 8); idx += UC_EPI_WARPS * 32) {
-          const int pos = idx & (S - 1), q = idx >> sS;
-          const int2 d = pool_dst[pos];
-          if (d.x < 0) continue;
-          __nv_bfloat162 mx[4];
-#pragma unroll
-          for (int e = 0; e < 4; ++e) mx[e] = __floats2bfloat162_rn(0.0f, 0.0f);
-#pragma unroll
-          for (int a = 0; a < 3; ++a)
-#pragma unroll
-            for (int bb = 0; bb < 3; ++bb) {
-              int sn = d.y - a * RW - bb;
-              sn += sn < 0 ? R : 0;
-              const uint4 r = *reinterpret_cast<const uint4*>(ring + (size_t)sn * 128u + (((uint32_t)q ^ ((uint32_t)sn & 7u)) << 4));
-              const __nv_bfloat162* rb = reinterpret_cast<const __nv_bfloat162*>(&r);
-#pragma unroll
-              for (int e = 0; e < 4; ++e) mx[e] = __hmax2(mx[e], rb[e]);
-            }
-          *reinterpret_cast<uint4*>(p.y + (int64_t)((ch0 >> 3) + q) * p.y_plane_stride + (int64_t)d.x * 8) = *reinterpret_cast<const uint4*>(mx);
-        }
-        asm volatile("bar.sync 1, 256;" ::: "memory");   // the next tile's outputs overwrite the oldest ring slots
-      }
       if (dbg && warp == UC_EPI_WARP0 && lane == 0 && lt == 0) p.dbg[5] = clock64();   // first epilogue done
     }
   }
@@ -625,16 +514,6 @@ done:
   if (warp == UC_EPI_WARP0) {
     if constexpr (CTA2) tmem_dealloc2(tmem_base, p.tmem_cols);
     else tmem_dealloc(tmem_base, p.tmem_cols);
-  }
-  if (dyn && tid == 0) {
-    // every claim of this CTA has completed (its queue saw the end marker): the last CTA of the launch re-arms the counters
-    __threadfence();
-    const unsigned n_ctas = gridDim.x * gridDim.y;
-    if (atomicAdd(p.tile_ctr + UC_CTR_DONE, 1u) == n_ctas - 1) {
-      for (unsigned y = 0; y < gridDim.y; ++y) p.tile_ctr[y] = 0;
-      p.tile_ctr[UC_CTR_DONE] = 0;
-      __threadfence();
-    }
   }
   if (dbg && tid == 0) { p.dbg[6] = clock64(); p.dbg[7] = num_tiles; }
 }
@@ -683,15 +562,11 @@ size_t umma_conv_smem_bytes(const UmmaConvP& p) {
   return b + umma_conv_extra_smem_bytes(p);
 }
 int umma_conv_stage_desc_bytes() { return (int)sizeof(UcStageDesc); }
-// UC_Y_POOL: ring of (tile + 128) positions x 64 channels bf16 + one int2 per tile position
-size_t umma_conv_pool_smem_bytes(int MT) { return (size_t)(MT * 128 + 128) * 128u + (size_t)MT * 128 * sizeof(int2); }
 static bool uc_is_generic(const UmmaConvP& p);
-// shared memory behind the stage program: the bias operand tiles of the lean instantiations (+ the max-pool ring)
+// shared memory behind the stage program: the bias operand tiles of the lean instantiations
 size_t umma_conv_extra_smem_bytes(const UmmaConvP& p) {
   if (uc_is_generic(p)) return 0;
-  size_t b = 128 + 2048 + (size_t)(p.cta2 ? p.Cout / 2 : p.Cout) * 32u;
-  if (p.y_mode == UC_Y_POOL) b += 128 + umma_conv_pool_smem_bytes(p.MT);
-  return b;
+  return 128 + 2048 + (size_t)(p.cta2 ? p.Cout / 2 : p.Cout) * 32u;
 }
 
 static bool uc_is_generic(const UmmaConvP& p) {
@@ -702,14 +577,9 @@ const char* umma_conv_config_error(const UmmaConvP& p) {
   if (p.res && p.res32) return "bf16 and fp32 residuals are mutually exclusive";
   if (uc_is_generic(p) && (p.Cout & 63)) return "the generic epilogue needs a column slice that is a multiple of 64";
   if (p.MT / p.issuers > 4 || p.MT % p.issuers) return "unsupported M-tiles per issuing warp";
-  if (p.fold && (uc_is_generic(p) || p.cta2 || p.tile_ctr || p.y_mode == UC_Y_POOL || p.res || p.MT > 4))
-    return "folded convolutions need the lean epilogue, no residual, single CTAs, at most 4 M-tiles and the static tile walk";
-  if (p.cta2 && (uc_is_generic(p) || p.y_mode == UC_Y_POOL || (p.Cout & 31) || p.tile_ctr)) return "CTA pairs need the lean epilogue, a multiple of 32 columns and the static tile walk";
-  if (p.y_mode == UC_Y_POOL) {
-    if (uc_is_generic(p) || p.res || p.act != ACT_RELU || p.Cout != 64 || p.tile_ctr) return "fused max-pool needs the lean epilogue, ReLU, 64 columns and the static tile walk";
-    if ((p.g.H & 1) || (p.g.W & 1) || p.g2.H * 2 != p.g.H || p.g2.W * 2 != p.g.W || 2 * p.g.RW + 2 > 128) return "fused max-pool: unsupported geometry";
-    if (p.pool_ring != (uint32_t)(p.MT * 128 + 128) || (p.MT & (p.MT - 1))) return "fused max-pool: ring size mismatch";
-  }
+  if (p.fold && (uc_is_generic(p) || p.cta2 || p.res || p.MT > 4))
+    return "folded convolutions need the lean epilogue, no residual, single CTAs and at most 4 M-tiles";
+  if (p.cta2 && (uc_is_generic(p) || (p.Cout & 31))) return "CTA pairs need the lean epilogue and a multiple of 32 columns";
   return nullptr;
 }
 
@@ -718,7 +588,6 @@ cudaError_t umma_conv_device_init() {
   // the opt-in limit (227 KB) covers static + dynamic shared memory; ~3.7 KB is static (barriers, bias, band / group tables)
   cudaError_t e = cudaFuncSetAttribute(umma_conv_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 223 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(umma_conv_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 223 * 1024);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(umma_conv_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 223 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(umma_conv_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 223 * 1024);
   if (e == cudaSuccess) e = video_rows_device_init();
   return e;
@@ -754,7 +623,6 @@ void launch_umma_conv(const UmmaConvP& p, int n_slices, cudaStream_t s, int num_
   }
   if (p.fold) gx = tiles;   // folded convs: one tile per CTA; the heaviest slices come first and the block scheduler balances the rest
   if (generic) umma_conv_kernel<1><<<dim3(gx, n_slices), UC_THREADS, umma_conv_smem_bytes(p), s>>>(p);
-  else if (p.y_mode == UC_Y_POOL) umma_conv_kernel<2><<<dim3(gx, n_slices), UC_THREADS, umma_conv_smem_bytes(p), s>>>(p);
   else umma_conv_kernel<0><<<dim3(gx, n_slices), UC_THREADS, umma_conv_smem_bytes(p), s>>>(p);
   count_launch();
 }
@@ -1000,56 +868,9 @@ __global__ void __launch_bounds__(256) planar_maxpool_kernel(const __nv_bfloat16
     }
   }
 }
-// Same mapping, plain bf16 tensors (no hi/lo split): the maximum is taken on packed bf16 pairs (HMNMX2) — the maximum of bf16
-// values is exact in bf16, so no unpack / repack and half the shuffles; the float version above was instruction-issue-bound.
-__global__ void __launch_bounds__(256) planar_maxpool_bf16_kernel(const __nv_bfloat16* __restrict__ x, int64_t xs, UcGeom gi,
-                                                                  __nv_bfloat16* __restrict__ y, int64_t ys, UcGeom go) {
-  const int frame = blockIdx.x, chunk = blockIdx.y;
-  const int n = frame / go.T, t = frame - n * go.T;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-  const uint4* xc = reinterpret_cast<const uint4*>(x + (int64_t)chunk * xs + uc_flat(gi, n, t, 0, 0) * 8);
-  uint4* yc = reinterpret_cast<uint4*>(y + (int64_t)chunk * ys + uc_flat(go, n, t, 0, 0) * 8);
-  const uint32_t NINF2 = 0xFF80FF80u;                                   // (-inf, -inf) in bf16
-  auto mx4 = [](uint4 a, uint4 b) {
-    uint4 r;
-    __nv_bfloat162 t0 = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a.x), *reinterpret_cast<__nv_bfloat162*>(&b.x));
-    __nv_bfloat162 t1 = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a.y), *reinterpret_cast<__nv_bfloat162*>(&b.y));
-    __nv_bfloat162 t2 = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a.z), *reinterpret_cast<__nv_bfloat162*>(&b.z));
-    __nv_bfloat162 t3 = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a.w), *reinterpret_cast<__nv_bfloat162*>(&b.w));
-    r.x = *reinterpret_cast<uint32_t*>(&t0); r.y = *reinterpret_cast<uint32_t*>(&t1);
-    r.z = *reinterpret_cast<uint32_t*>(&t2); r.w = *reinterpret_cast<uint32_t*>(&t3);
-    return r;
-  };
-  const int nseg = (gi.W + 31) >> 5;
-  const int npairs = go.H * nseg;
-  for (int pair = warp; pair < npairs; pair += nwarps) {
-    const int h = pair / nseg, seg = pair - h * nseg;
-    const int c = seg * 32 + lane;                         // this lane's input column
-    uint4 mv = make_uint4(NINF2, NINF2, NINF2, NINF2), ml = mv;
-    const bool extra_left = lane == 0 && seg > 0;
-#pragma unroll
-    for (int dh = 0; dh < 3; ++dh) {
-      const int hi = 2 * h - 1 + dh;
-      if ((unsigned)hi >= (unsigned)gi.H) continue;
-      if (c < gi.W) mv = mx4(mv, xc[hi * gi.RW + c]);
-      if (extra_left) ml = mx4(ml, xc[hi * gi.RW + c - 1]);
-    }
-    const int sa = (2 * lane) & 31, sb = (2 * lane + 1) & 31, sc = (2 * lane - 1) & 31;
-    uint4 a, b, cl;
-    a.x = __shfl_sync(0xffffffffu, mv.x, sa); a.y = __shfl_sync(0xffffffffu, mv.y, sa);
-    a.z = __shfl_sync(0xffffffffu, mv.z, sa); a.w = __shfl_sync(0xffffffffu, mv.w, sa);
-    b.x = __shfl_sync(0xffffffffu, mv.x, sb); b.y = __shfl_sync(0xffffffffu, mv.y, sb);
-    b.z = __shfl_sync(0xffffffffu, mv.z, sb); b.w = __shfl_sync(0xffffffffu, mv.w, sb);
-    cl.x = __shfl_sync(0xffffffffu, mv.x, sc); cl.y = __shfl_sync(0xffffffffu, mv.y, sc);
-    cl.z = __shfl_sync(0xffffffffu, mv.z, sc); cl.w = __shfl_sync(0xffffffffu, mv.w, sc);
-    if (lane == 0) cl = ml;                                // (seg == 0: ml stays -inf = the reference's padding)
-    const int w = seg * 16 + lane;
-    if (lane < 16 && w < go.W) yc[h * go.RW + w] = mx4(mx4(a, b), cl);
-  }
-}
-
-// Same result, one thread per pooled position: nine independent predicated 16-byte loads (the 3x3 window; neighbours' re-reads hit
-// L1), no shuffles, no idle lanes at the store.  The warp-per-row version above was bound by its dependent load -> shuffle chain
+// Same result for plain bf16 tensors (no hi/lo split), one thread per pooled position: nine independent predicated 16-byte loads (the
+// 3x3 window; neighbours' re-reads hit L1), no shuffles, no idle lanes at the store; the maximum is taken on packed bf16 pairs
+// (HMNMX2, exact in bf16).  The warp-per-row mapping above, on packed bf16 pairs, was bound by its dependent load -> shuffle chain
 // (209 us for the 811 MB of the stem's max-pool at B=64: 3.9 TB/s).
 __global__ void __launch_bounds__(192) planar_maxpool_direct_kernel(const __nv_bfloat16* __restrict__ x, int64_t xs, UcGeom gi,
                                                                     __nv_bfloat16* __restrict__ y, int64_t ys, UcGeom go) {
@@ -1087,9 +908,7 @@ void launch_planar_maxpool(const __nv_bfloat16* x, int64_t x_plane_stride, UcGeo
                            int C, cudaStream_t s, const __nv_bfloat16* xlo, __nv_bfloat16* ylo) {
   const int frames = go.N * go.T;
   if (frames == 0 || go.H * go.W == 0) return;
-  static const bool warp_rows = getenv("LSD_POOL_WARP_ROWS") != nullptr;   // (the previous kernel, for comparison)
-  if (!xlo && !ylo && !warp_rows) planar_maxpool_direct_kernel<<<dim3((unsigned)frames, (unsigned)(C / 8)), 192, 0, s>>>(x, x_plane_stride, gi, y, y_plane_stride, go);
-  else if (!xlo && !ylo) planar_maxpool_bf16_kernel<<<dim3((unsigned)frames, (unsigned)(C / 8)), 256, 0, s>>>(x, x_plane_stride, gi, y, y_plane_stride, go);
+  if (!xlo && !ylo) planar_maxpool_direct_kernel<<<dim3((unsigned)frames, (unsigned)(C / 8)), 192, 0, s>>>(x, x_plane_stride, gi, y, y_plane_stride, go);
   else planar_maxpool_kernel<<<dim3((unsigned)frames, (unsigned)(C / 8)), 256, 0, s>>>(x, x_plane_stride, gi, y, y_plane_stride, go, xlo, ylo);
   count_launch();
 }

@@ -40,12 +40,9 @@ struct UcGroup {              // taps that share one K extent (main conv; option
 };
 
 // bf16 planar output modes (an fp32 row output can be produced in addition to, or instead of, the planar one)
-// UC_Y_POOL: the epilogue keeps the bf16 outputs of the last positions in a shared-memory ring and writes only the
-// 3x3 / stride-2 / pad-1 max-pool over (H, W) of them (plain layout, geometry g2 = (N, T, H/2, W/2)) — the stem + MaxPool3d of
-// visual_encoder.py:113-129 in one launch.  Needs ReLU (zero pads stand for the -inf padding), even H and W, 64 columns, one slice.
 // UC_Y_FOLD: "folded" destination (small maps, see UcFoldSlice): plane set h*ymap_W + w, position = frame row uc_flat(g2, n, t, 0, 0).
 // UC_Y_MAP: plain padded planar destination in geometry g2 written at (n, t, h, w) — a folded conv's output back in the map layout.
-enum UcOut { UC_Y_NONE = 0, UC_Y_PLAIN = 1, UC_Y_PARITY = 2, UC_Y_PARITY_H = 3, UC_Y_POOL = 4, UC_Y_FOLD = 5, UC_Y_MAP = 6 };
+enum UcOut { UC_Y_NONE = 0, UC_Y_PLAIN = 1, UC_Y_PARITY = 2, UC_Y_PARITY_H = 3, UC_Y_FOLD = 5, UC_Y_MAP = 6 };
 
 // Folded small-map convolution ("frames as rows").  A map of H x W x C per frame is stored as H*W plane sets (one per spatial
 // position) in the row geometry make_geom_ex(N, T, 1, 1, 1, 0, 0, 0, 0): position = frame row n*(T+1) + t + 1, with the shared
@@ -122,16 +119,11 @@ struct UmmaConvP {
   int issuers;                // MMA-issuing warps (1, 2 or 4; divides MT): each issues MT / issuers M-tiles per tap
   int nbuf;                   // TMEM accumulator buffers: 2 = epilogue overlaps the next tile, 1 = all 512 columns for one tile
   long long* dbg;             // optional: CTA (0,0) writes clock64 phase timestamps (debug builds of the bench only)
-  unsigned* tile_ctr;         // device memory, 16 words, zero between launches: dynamic tile scheduling (nullptr: static stride)
   const UcStageDesc* prog;    // device memory: the stage program (nst_tile entries)
   int nst_tile;               // ring stages per tile (sum over groups of ceil(k16 / kpack) * bands): length of the stage program
   int skip;                   // debug (LSD_UMMA_SKIP): bit 0 = no A copies, bit 1 = no W copies — timing experiments only
   int kpack;                  // k16 chunks per pipeline stage (small-K-step layers amortise the mbarrier round trip)
   uint32_t a_stage_bytes, w_stage_bytes, tmem_cols;
-  // UC_Y_POOL: ring of pool_ring positions (tile positions + 128 >= tile + 2 rows + 2) behind the stage program; division by
-  // pool_ring as multiply + shift (uc_magic)
-  uint32_t pool_ring, pool_mR;
-  int pool_sR;
   int cta2;                   // 1: CTA pairs (cluster of 2, tcgen05 cta_group::2): the packed weights hold two column halves as slices
   UcGeom g;                   // output geometry (== input geometry of every band)
   UcGeom g2;                  // UC_Y_PARITY* / UC_Y_FOLD / UC_Y_MAP: destination geometry (of each plane set)
@@ -144,8 +136,7 @@ struct UmmaConvP {
 
 size_t umma_conv_smem_bytes(const UmmaConvP& p);
 int umma_conv_stage_desc_bytes();
-size_t umma_conv_extra_smem_bytes(const UmmaConvP& p);   // behind the stage program: bias operand tiles (lean epilogue) + max-pool ring
-size_t umma_conv_pool_smem_bytes(int MT);   // UC_Y_POOL: shared memory behind the stage program (ring + per-position table)
+size_t umma_conv_extra_smem_bytes(const UmmaConvP& p);   // behind the stage program: bias operand tiles (lean epilogue)
 // host: expand the stage program of a launch (same arithmetic the kernel used to do per stage)
 void umma_conv_build_program(const UmmaConvP& p, UcStageDesc* out);
 // host: one stage (K chunks c0 .. c0 + nc of band bd, whose index in p.bands is `band`); col >= 0: the Cout slice is baked into

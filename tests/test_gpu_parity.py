@@ -401,10 +401,9 @@ def test_bf16_odd_shapes_against_oracle(model, seed0_sd, shape):
 
 
 def test_scheduling_knobs_do_not_change_logits(model):
-    """The scheduling variants of the tcgen05 kernel (dynamic tile claims, side-stream SM share, artifact branch placement, audio
-    fork point) only move work between CTAs and streams, and the stem's fused max-pool epilogue (LSD_STEM_POOL_FUSE=1) computes the same maxima
-    as the separate max-pool kernel: logits must be bit-identical to the default schedule.  The knobs are read
-    from the environment inside the library (the first one once per process), so each variant runs in a fresh interpreter."""
+    """The side stream's SM share (LSD_SIDE_CTAS) only moves work between CTAs and streams: logits must be bit-identical to the
+    default schedule.  The knob is read from the environment inside the library once per process, so each variant runs in a
+    fresh interpreter."""
     import os, subprocess, sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     code = ("import sys; sys.path.insert(0, %r)\n"
@@ -414,10 +413,7 @@ def test_scheduling_knobs_do_not_change_logits(model):
             "out = m(v.cuda(), a.cuda()).float().cpu()\n"
             "print('DIGEST', hashlib.sha256(out.numpy().tobytes()).hexdigest())\n") % root
     digests = {}
-    for name, env in {"default": {}, "dynamic_tiles": {"LSD_UMMA_DYNAMIC": "1"}, "side_all_sms": {"LSD_SIDE_CTAS": "148"},
-                      "hf_early": {"LSD_HF_EARLY": "1"}, "audio_after_rows": {"LSD_AUDIO_AFTER_ROWS": "1"},
-                      "stem_pool_fused": {"LSD_STEM_POOL_FUSE": "1", "LSD_UMMA_CTA2": "0"}, "no_cta_pairs": {"LSD_UMMA_CTA2": "0"},
-                      "pool_warp_rows": {"LSD_POOL_WARP_ROWS": "1"}}.items():
+    for name, env in {"default": {}, "side_all_sms": {"LSD_SIDE_CTAS": "148"}}.items():
         # (LSD_STEM_RING=0: all variants run the flat shift-GEMM stem — the temporal-ring stem sums in a different order, it is
         #  compared with a tolerance in test_stem_ring_matches_flat_stem)
         r = subprocess.run([sys.executable, "-c", code], env={**os.environ, "LSD_STEM_RING": "0", **env}, capture_output=True, text=True, timeout=300)
@@ -443,18 +439,13 @@ def test_stem_ring_matches_flat_stem(model):
             "out['one'] = m(v[:3, :, :1].contiguous().cuda(), a[:3].cuda()).float().cpu().tolist()\n"
             "print('OUT', json.dumps(out))\n") % root
     res = {}
-    for name, env in {"ring": {}, "ring_pool_inline": {"LSD_STEM_POOL_INLINE": "1"}, "flat": {"LSD_STEM_RING": "0"},
-                      "l1_ring": {"LSD_L1_RING": "1"}}.items():
+    for name, env in {"ring": {}, "flat": {"LSD_STEM_RING": "0"}}.items():
         r = subprocess.run([sys.executable, "-c", code], env={**os.environ, **env}, capture_output=True, text=True, timeout=300)
         assert r.returncode == 0, (name, r.stderr[-2000:])
         res[name] = json.loads([l for l in r.stdout.splitlines() if l.startswith("OUT")][-1][4:])
-    # the max-pool done by the ring kernel's own pool warps (LSD_STEM_POOL_INLINE=1) and by the separate launch give the same bits
-    assert res["ring"] == res["ring_pool_inline"], (res["ring"], res["ring_pool_inline"])
-    # "l1_ring": layer1's two convolutions through the same scheme (conv_ring.cu, opt-in: measured no faster — the step is power-bound)
-    for other in ("flat", "l1_ring"):
-        for k in res["ring"]:
-            d = np.abs(np.asarray(res["ring"][k]) - np.asarray(res[other][k])).max()
-            assert d <= 5e-3, (other, k, d, res["ring"][k], res[other][k])
+    for k in res["ring"]:
+        d = np.abs(np.asarray(res["ring"][k]) - np.asarray(res["flat"][k])).max()
+        assert d <= 5e-3, (k, d, res["ring"][k], res["flat"][k])
 
 
 def test_temporal_smoothed_confidence_values_match_oracle(model, seed0_sd):
