@@ -178,6 +178,32 @@ int lsd_score_offsets(lsd_handle* h, const uint8_t* track, int n_frames, int H, 
                       float* logits_out, int32_t* eff_audio_starts_host_or_null,
                       void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- occlusion evidence: window scores with a region of the window hidden ---------------------------------- */
+/* This entry has no reference counterpart.  It builds on the scoring loop of Predictor._run_chunked_inference
+ * (predictor.py:554-580, lsd_score_windows): every window is scored K times, once per occlusion box, and the change of the
+ * logit is that region's evidence.  A box is seven int32 values in window coordinates.  With win the un-occluded uint8 window
+ * (frames starts_host[i] .. starts_host[i]+T-1 of the track), the occluded window is
+ *   out[t,y,x,:] = (t0<=t<t1 && y0<=y<y1 && x0<=x<x1) ? (src < 0 ? fill : win[src,y,x,:]) : win[t,y,x,:]
+ * src >= 0 copies frame src of the UN-occluded window, also when src lies inside the box.  A box with t0==t1, y0==y1 or x0==x1
+ * is empty: the row is the plain window.  Typical boxes: a freeze of frames [t0,t1) (full frame, src = t0-1, or t1 when t0 == 0)
+ * and a fill of a spatial cell over all frames (src = -1). */
+typedef struct { int32_t t0, t1, y0, y1, x0, x1, src; } lsd_occlusion;
+#define LSD_MAX_OCCLUSIONS 1024
+/* Rows are (window, box) pairs in window-major order, row r = i*K + k; `batch` counts rows.  A row's audio slice is its window's
+ * slice, with the base-start rule of lsd_score_windows (computed, or audio_starts_host_or_null[i], clamped).  The occluded windows
+ * of a batch are built on the device (16-byte loads and stores, reading only the window's frames) and scored by the plain batch
+ * path of lsd_score_windows, so logits_out (device, (n_windows, K) fp32) entry (i, k) is bit for bit lsd_score_windows on window
+ * i occluded on the host, with the same audio start.  A workspace of at least twice lsd_score_occlusions_workspace_bytes enables
+ * the cross-batch pipelining of lsd_score_windows; a short last batch runs in exactly the queried size.  Everything is checked
+ * before any GPU work: LSD_ERR_SHAPE for K outside 1..LSD_MAX_OCCLUSIONS, a box outside [0,T]x[0,H]x[0,W] or with t0>t1
+ * (likewise y, x), src outside -1..T-1, or a window outside the track; LSD_ERR_ARG for boxes == NULL or fill outside 0..255. */
+size_t lsd_score_occlusions_workspace_bytes(lsd_handle* h, int batch, int T, int H, int W, int F, int Ta, int precision);
+int lsd_score_occlusions(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                         const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                         const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                         const lsd_occlusion* boxes, int K, int fill, int precision, int batch,
+                         float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- speaking alignment / mouth motion: the per-window numpy loops of _predict_long_video ------------------ */
 /* Frame-difference energies of a track (Predictor._speaking_alignment_score, app/inference/predictor.py:339-345, and
  * _mouth_motion_energy_check, :395-402): for every frame pair f in [0, n_frames-1)

@@ -19,6 +19,7 @@ LSD_F32, LSD_F16, LSD_BF16, LSD_U8, LSD_I64 = 0, 1, 2, 3, 4
 LSD_NCDHW, LSD_NDHWC = 0, 1
 LSD_PREC_FP32, LSD_PREC_BF16 = 0, 1
 LSD_MAX_AUDIO_VARIANTS = 64
+LSD_MAX_OCCLUSIONS = 1024
 
 # every symbol include/lsd_b200.h declares (checked by tests/test_cabi.py)
 EXPORTS = [
@@ -30,11 +31,18 @@ EXPORTS = [
     "lsd_track_motion", "lsd_speech_stats", "lsd_vad_frames", "lsd_frame_energy", "lsd_vad_mask",
     "lsd_workspace_invalidate", "lsd_planar_stage_read", "lsd_state_generation", "lsd_host_pack_u8_exact", "lsd_host_pack_u8_begin", "lsd_host_pack_u8_end", "lsd_host_pack_last_ms", "lsd_expand_u8",
     "lsd_forward_audio_variants_workspace_bytes", "lsd_forward_audio_variants", "lsd_score_offsets_workspace_bytes", "lsd_score_offsets",
+    "lsd_score_occlusions_workspace_bytes", "lsd_score_occlusions",
 ]
 
 
 class LsdTensor(C.Structure):
     _fields_ = [("name", C.c_char_p), ("dtype", C.c_int), ("ndim", C.c_int), ("shape", C.c_int64 * 8), ("data", C.c_void_p)]
+
+
+class LsdOcclusion(C.Structure):
+    """One occlusion box in window coordinates: frames [t0,t1) x rows [y0,y1) x columns [x0,x1), filled from frame `src` of the
+    un-occluded window (src >= 0) or with the call's fill value (src = -1)."""
+    _fields_ = [(f, C.c_int32) for f in ("t0", "t1", "y0", "y1", "x0", "x1", "src")]
 
 
 class LsdAux(C.Structure):
@@ -102,6 +110,10 @@ def lib() -> C.CDLL:
         L.lsd_score_offsets.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
                                         C.POINTER(C.c_int32), i, i, i, vp, C.POINTER(C.c_int32), vp, sz, vp]
         L.lsd_score_offsets.restype = i
+        L.lsd_score_occlusions_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i]; L.lsd_score_occlusions_workspace_bytes.restype = sz
+        L.lsd_score_occlusions.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
+                                           C.POINTER(LsdOcclusion), i, i, i, i, vp, vp, sz, vp]
+        L.lsd_score_occlusions.restype = i
         _lib = L
         return L
 

@@ -52,6 +52,28 @@ def av_offset_profile(confs, valid, offsets: Sequence[int], smoothing: str = "me
     }
 
 
+def frame_evidence_timeline(starts: Sequence[int], temporal, segment_frames: int, T: int):
+    """Per-frame timeline of occlusion evidence.  `starts`: first frame of every window; `temporal`: (n_windows, S) evidence of
+    the window's frame segments [j*s, min((j+1)*s, T)), s = `segment_frames` (`Predictor.explain_track`).  Returns
+    `(first_frame, values)`: values[f] belongs to frame first_frame + f, from the first window's start to the last window's end.
+    A frame's value is the mean over every (window, segment) pair that covers it, None where no window covers it."""
+    s, T = int(segment_frames), int(T)
+    if not len(starts):
+        return 0, []
+    ev = np.asarray(temporal, dtype=np.float64).reshape(len(starts), -1)
+    if ev.shape[1] != -(-T // s):
+        raise ValueError(f"temporal has {ev.shape[1]} segments, {T} frames in segments of {s} make {-(-T // s)}")
+    st = np.asarray(starts, dtype=np.int64)
+    first = int(st.min())
+    total = np.zeros(int(st.max()) + T - first, dtype=np.float64)
+    count = np.zeros_like(total)
+    seg_of = np.arange(T) // s                                       # segment of every frame of a window
+    for i, a in enumerate(st - first):
+        total[a:a + T] += ev[i, seg_of]
+        count[a:a + T] += 1
+    return first, [float(t / c) if c else None for t, c in zip(total, count)]
+
+
 def _speech_weighted(conf: Sequence[float], speaking: Sequence[float], vad: Optional[Sequence[float]], smoothing: str,
                      trim_ratio: float) -> float:
     # predictor.py:262-293

@@ -10,6 +10,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 
 #include "forward_common.h"
 #include "tok_front.cuh"
@@ -472,50 +473,37 @@ extern "C" size_t lsd_score_workspace_bytes(lsd_handle* h, int batch, int T, int
   return fw + 2 * (((size_t)batch * sizeof(int32_t) + 255) & ~size_t(255)) + 256;
 }
 
-extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
-                                 const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
-                                 int precision, int batch, float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!h) return LSD_ERR_ARG;
-  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_windows: no weights loaded");
-  if (n_windows == 0) return LSD_OK;
-  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_windows: null pointer argument");
-  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_windows: bad extents");
-  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
-  Shapes s;
-  int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
-  if (rc) return rc;
-  for (int i = 0; i < n_windows; ++i)
-    if (starts_host[i] < 0 || starts_host[i] + T > n_frames)
-      return lsd_fail(h, LSD_ERR_SHAPE, "window %d [%d,%d) is outside the %d-frame track", i, starts_host[i], starts_host[i] + T, n_frames);
-  ENTER_DEVICE(h);
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const size_t need = lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
-  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+namespace {
+// Returns the track a batch of rows [r0, r0+nb) reads, after enqueueing on `st` whatever builds it (lsd_score_occlusions: its
+// occluded pseudo-track).  Empty: every batch reads the caller's track.
+using BatchTrack = std::function<int(int r0, int nb, const uint8_t*& track, int& n_frames)>;
+
+// The batch loop of lsd_score_windows, shared with lsd_score_occlusions.  h->idx_host holds the first track frame of row r at [r]
+// and its first mel column at [n_rows + r]; the caller has checked every argument and the workspace size.
+int score_rows(lsd_handle* h, const uint8_t* track, int n_frames, int n_rows, int T, int H, int W, const float* mel_full, int F,
+               int Ta_full, int Ta, int precision, int batch, float* logits_out, void* workspace, size_t workspace_bytes,
+               cudaStream_t st, const BatchTrack& batch_track) {
+  int rc = 0;
   const size_t idx_bytes = ((size_t)batch * sizeof(int32_t) + 255) & ~size_t(255);
   char* ws = reinterpret_cast<char*>(workspace);
   int32_t* d_vs = reinterpret_cast<int32_t*>(ws);
   int32_t* d_as = reinterpret_cast<int32_t*>(ws + idx_bytes);
   char* fws = ws + 2 * idx_bytes;
-  // all window/audio starts are staged once (pinned-free small copies are ordered on the stream)
-  h->idx_host.resize((size_t)2 * n_windows);
-  for (int i = 0; i < n_windows; ++i) {
-    h->idx_host[i] = starts_host[i];
-    h->idx_host[n_windows + i] = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
-  }
   // Cross-batch pipelining (tensor-core route, more than one batch, workspace >= 2 x lsd_score_workspace_bytes): batches
   // alternate between the two halves of the workspace; the tail of batch k (audio encoder, token path, head, artifact branch)
   // runs on side streams while this stream continues with the visual encoder of batch k+1.
   const size_t fw_bytes = ((lsd_workspace_bytes(h, batch, T, H, W, F, Ta, precision) + 255) & ~size_t(255));
-  const bool pipelined = precision == LSD_PREC_BF16 && n_windows > batch && workspace_bytes >= 2 * idx_bytes + 2 * fw_bytes &&
+  const bool pipelined = precision == LSD_PREC_BF16 && n_rows > batch && workspace_bytes >= 2 * idx_bytes + 2 * fw_bytes &&
                          getenv("LSD_NO_PIPELINE") == nullptr;
   if (pipelined && (rc = ensure_pipeline(h))) return rc;
   int k = 0;
-  for (int w0 = 0; w0 < n_windows; w0 += batch, ++k) {
-    const int nb = (n_windows - w0) < batch ? (n_windows - w0) : batch;
+  for (int w0 = 0; w0 < n_rows; w0 += batch, ++k) {
+    const int nb = (n_rows - w0) < batch ? (n_rows - w0) : batch;
     const int parity = k & 1;
     if (pipelined && k >= 2) CUDA_OK(h, cudaStreamWaitEvent(st, h->ev_tail_done[parity], 0));   // this half of the workspace is free again
     CUDA_OK(h, cudaMemcpyAsync(d_vs, &h->idx_host[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    CUDA_OK(h, cudaMemcpyAsync(d_as, &h->idx_host[n_windows + w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CUDA_OK(h, cudaMemcpyAsync(d_as, &h->idx_host[n_rows + w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    if (batch_track && (rc = batch_track(w0, nb, track, n_frames))) return rc;
     if (precision == LSD_PREC_BF16) {
       if (pipelined) rc = score_batch_bf16(h, track, n_frames, d_vs, d_as, mel_full, Ta_full, nb, T, H, W, F, Ta, logits_out + w0,
                                            fws + (size_t)parity * fw_bytes, fw_bytes, st, parity);
@@ -542,6 +530,119 @@ extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_fram
   }
   CUDA_OK(h, cudaGetLastError());
   return LSD_OK;
+}
+
+int check_windows(lsd_handle* h, const int32_t* starts_host, int n_windows, int T, int n_frames) {
+  for (int i = 0; i < n_windows; ++i)
+    if (starts_host[i] < 0 || starts_host[i] + T > n_frames)
+      return lsd_fail(h, LSD_ERR_SHAPE, "window %d [%d,%d) is outside the %d-frame track", i, starts_host[i], starts_host[i] + T, n_frames);
+  return 0;
+}
+}  // namespace
+
+extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                 const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                                 int precision, int batch, float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_windows: no weights loaded");
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_windows: null pointer argument");
+  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_windows: bad extents");
+  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
+  Shapes s;
+  int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
+  if (rc) return rc;
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  ENTER_DEVICE(h);
+  const size_t need = lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
+  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  // all window/audio starts are staged once (pinned-free small copies are ordered on the stream)
+  h->idx_host.resize((size_t)2 * n_windows);
+  for (int i = 0; i < n_windows; ++i) {
+    h->idx_host[i] = starts_host[i];
+    h->idx_host[n_windows + i] = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
+  }
+  return score_rows(h, track, n_frames, n_windows, T, H, W, mel_full, F, Ta_full, Ta, precision, batch, logits_out, workspace,
+                    workspace_bytes, reinterpret_cast<cudaStream_t>(stream), BatchTrack());
+}
+
+// ================================================================================================
+// Occlusion evidence: K occluded copies of every window (occlusion.cu), scored by the batch loop of lsd_score_windows
+// ================================================================================================
+// Workspace: [boxes (LSD_MAX_OCCLUSIONS x 7 int32) | track starts of one batch's windows | pseudo-track of `batch` occluded
+// windows | lsd_score_windows workspace].  The pseudo-track is read only by the batch's first kernel on the caller's stream
+// (the tensor-core pixel rows or the fp32 gather), so one copy serves pipelined batches too.
+namespace {
+size_t occlusion_extra_bytes(int batch, int T, int H, int W) {
+  return align256((size_t)LSD_MAX_OCCLUSIONS * 7 * sizeof(int32_t)) + align256(((size_t)batch + 1) * sizeof(int32_t)) +
+         align256((size_t)batch * T * H * W * 3);
+}
+}  // namespace
+
+extern "C" size_t lsd_score_occlusions_workspace_bytes(lsd_handle* h, int batch, int T, int H, int W, int F, int Ta, int precision) {
+  if (batch < 1) return 0;
+  const size_t sw = lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
+  if (sw == 0) return 0;
+  return occlusion_extra_bytes(batch, T, H, W) + align256(sw);
+}
+
+extern "C" int lsd_score_occlusions(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                    const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full,
+                                    int total_v_frames, int Ta, const lsd_occlusion* boxes, int K, int fill, int precision, int batch,
+                                    float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_occlusions: no weights loaded");
+  if (!boxes) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_occlusions: boxes is NULL");
+  if (K < 1 || K > LSD_MAX_OCCLUSIONS) return lsd_fail(h, LSD_ERR_SHAPE, "K = %d occlusion boxes: expected 1 <= K <= %d", K, LSD_MAX_OCCLUSIONS);
+  if (fill < 0 || fill > 255) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_occlusions: fill %d is not a uint8 value", fill);
+  for (int k = 0; k < K; ++k) {
+    const lsd_occlusion& b = boxes[k];
+    if (b.t0 < 0 || b.t0 > b.t1 || b.t1 > T || b.y0 < 0 || b.y0 > b.y1 || b.y1 > H || b.x0 < 0 || b.x0 > b.x1 || b.x1 > W)
+      return lsd_fail(h, LSD_ERR_SHAPE, "box %d [%d,%d)x[%d,%d)x[%d,%d) is not inside the %dx%dx%d window", k, b.t0, b.t1, b.y0, b.y1,
+                      b.x0, b.x1, T, H, W);
+    if (b.src < -1 || b.src >= T) return lsd_fail(h, LSD_ERR_SHAPE, "box %d: src %d is outside -1..%d", k, b.src, T - 1);
+  }
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_occlusions: null pointer argument");
+  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_occlusions: bad extents");
+  if ((int64_t)n_windows * K > INT32_MAX) return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d boxes: too many rows for one call", n_windows, K);
+  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
+  Shapes s;
+  int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
+  if (rc) return rc;
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = lsd_score_occlusions_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
+  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const int n_rows = n_windows * K;
+  // row r reads frames (r % batch) * T .. of the batch's pseudo-track, and the audio slice of window r / K
+  h->idx_host.resize((size_t)2 * n_rows);
+  for (int i = 0; i < n_windows; ++i) {
+    const int32_t a = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
+    for (int k = 0; k < K; ++k) {
+      const int r = i * K + k;
+      h->idx_host[r] = (r % batch) * T;
+      h->idx_host[n_rows + r] = a;
+    }
+  }
+  char* ws = reinterpret_cast<char*>(workspace);
+  int32_t* d_boxes = reinterpret_cast<int32_t*>(ws);
+  int32_t* d_wins = reinterpret_cast<int32_t*>(ws + align256((size_t)LSD_MAX_OCCLUSIONS * 7 * sizeof(int32_t)));
+  uint8_t* pseudo = reinterpret_cast<uint8_t*>(d_wins) + align256(((size_t)batch + 1) * sizeof(int32_t));
+  const size_t extra = occlusion_extra_bytes(batch, T, H, W);
+  static_assert(sizeof(lsd_occlusion) == 7 * sizeof(int32_t), "lsd_occlusion is seven packed int32");
+  CUDA_OK(h, cudaMemcpyAsync(d_boxes, boxes, (size_t)K * sizeof(lsd_occlusion), cudaMemcpyHostToDevice, st));
+  const BatchTrack occluded = [&](int r0, int nb, const uint8_t*& trk, int& nf) -> int {
+    const int wa = r0 / K, wb = (r0 + nb - 1) / K;
+    CUDA_OK(h, cudaMemcpyAsync(d_wins, starts_host + wa, (size_t)(wb - wa + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    launch_occlude_windows(track, d_wins, d_boxes, K, r0, nb, T, H, W, fill, pseudo, st);
+    trk = pseudo;
+    nf = nb * T;
+    return 0;
+  };
+  return score_rows(h, pseudo, batch * T, n_rows, T, H, W, mel_full, F, Ta_full, Ta, precision, batch, logits_out, ws + extra,
+                    workspace_bytes - extra, st, occluded);
 }
 
 // ================================================================================================

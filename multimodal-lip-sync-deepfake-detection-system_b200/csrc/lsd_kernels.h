@@ -33,6 +33,10 @@ void launch_cast_to_f32(const void* src, int dtype, float* dst, int64_t n, float
 // uint8 track (frames,H,W,3) + window starts -> (n,T,H,W,3) fp32 = u8/255 (video.py:552-556)
 void launch_gather_windows_u8(const uint8_t* track, int n_frames, const int32_t* starts, float* dst,
                               int n, int T, int frame_elems, cudaStream_t s);
+// occluded windows (occlusion.cu): rows r0 .. r0+nb-1 = (window r / K, box r % K) -> uint8 pseudo-track out (nb*T, H, W, 3);
+// win_starts: track start of windows r0 / K, r0 / K + 1, ...; boxes: K x 7 int32 (t0, t1, y0, y1, x0, x1, src)
+void launch_occlude_windows(const uint8_t* track, const int32_t* win_starts, const int32_t* boxes, int K, int r0, int nb, int T,
+                            int H, int W, int fill, uint8_t* out, cudaStream_t s);
 // mel_full (F, Ta_full) + per-window a_start -> (n, F, Ta) with repeat-last-column padding (predictor.py:525-552)
 void launch_gather_audio(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, float* dst,
                          int n, int Ta, cudaStream_t s);

@@ -615,6 +615,128 @@ class Predictor:
             res["offset_frames"] = frames
         return res
 
+    # ------------------------------------------------------------------ occlusion evidence (lsd_score_occlusions)
+    def score_track_occlusions(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                               boxes, fill: int = 128, chunk_a_size: int = 128,
+                               audio_starts_from: Optional[Sequence[int]] = None) -> torch.Tensor:
+        """`score_track_logits` with K occlusion boxes per window (`lsd_score_occlusions`).  `boxes`: a `(K, 7)` int array or a
+        sequence of 7-tuples `(t0, t1, y0, y1, x0, x1, src)` in window coordinates; pixels of frames [t0,t1) x rows [y0,y1) x columns
+        [x0,x1) are replaced by frame `src` of the un-occluded window (src >= 0) or by `fill` (src = -1).  An empty box leaves the
+        window as it is.  The occluded windows are built on the device.  Returns fp32 logits `(n, K)` on the device; entry (i, k)
+        is bit for bit the logit of window i occluded by box k, with window i's audio slice."""
+        m = self.model
+        dev = m._device()
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        if mel_full.dim() != 3 or mel_full.shape[0] != 1:
+            raise ValueError(f"mel_full must be (1, F, T_full), got {tuple(mel_full.shape)}")
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T = self.chunk_size
+        bx = np.asarray(boxes, dtype=np.int64)
+        if bx.ndim != 2 or bx.shape[1] != 7:
+            raise ValueError(f"boxes must be (K, 7) (t0, t1, y0, y1, x0, x1, src), got shape {bx.shape}")
+        K = int(bx.shape[0])
+        if not 1 <= K <= _cabi.LSD_MAX_OCCLUSIONS:
+            raise ValueError(f"{K} occlusion boxes: expected 1 to {_cabi.LSD_MAX_OCCLUSIONS}")
+        for k, (t0, t1, y0, y1, x0, x1, src) in enumerate(bx.tolist()):
+            if not (0 <= t0 <= t1 <= T and 0 <= y0 <= y1 <= H and 0 <= x0 <= x1 <= W):
+                raise ValueError(f"box {k} {bx[k].tolist()} is not inside the {T}x{H}x{W} window")
+            if not -1 <= src < T:
+                raise ValueError(f"box {k}: src {src} is outside -1..{T - 1}")
+        if not 0 <= int(fill) <= 255:
+            raise ValueError(f"fill must be a uint8 value, got {fill}")
+        n = len(starts)
+        if audio_starts_from is not None and len(audio_starts_from) != n:
+            raise ValueError("audio_starts_from must have one entry per window")
+        for i, s in enumerate(starts):
+            if not 0 <= int(s) <= n_frames - T:
+                raise ValueError(f"window {i} [{int(s)},{int(s) + T}) is outside the {n_frames}-frame track")
+        logits = torch.empty(n, K, dtype=torch.float32, device=dev)
+        if n == 0:
+            return logits
+        track_u8 = track_u8.contiguous()
+        mel_full = mel_full.to(torch.float32).contiguous()
+        F_, Ta_full = int(mel_full.shape[1]), int(mel_full.shape[2])
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = m._precision()
+            batch = min(self.batch_size, n * K)
+            need = L.lsd_score_occlusions_workspace_bytes(h.ptr, batch, T, H, W, F_, chunk_a_size, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            if n * K > batch and prec == _cabi.LSD_PREC_BF16:
+                need = 2 * need      # a double workspace lets the batches overlap as in score_track_logits
+            ws = m._workspace(need, dev)
+            st = (C.c_int32 * n)(*[int(s) for s in starts])
+            ast = None
+            if audio_starts_from is not None:
+                ast = (C.c_int32 * n)(*[self._audio_start(int(v), Ta_full, int(total_v_frames), chunk_a_size) for v in audio_starts_from])
+            boxes_c = (_cabi.LsdOcclusion * K)(*[_cabi.LsdOcclusion(*row) for row in bx.tolist()])
+            rc = L.lsd_score_occlusions(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, T, mel_full.data_ptr(), F_, Ta_full,
+                                        int(total_v_frames), chunk_a_size, boxes_c, K, int(fill), prec, batch, logits.data_ptr(),
+                                        ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return logits
+
+    @staticmethod
+    def freeze_segment_boxes(T: int, segment_frames: int, H: int = 96, W: int = 96) -> List[Tuple[int, ...]]:
+        """Freeze boxes: segment j = frames [j*s, min((j+1)*s, T)) replaced, over the whole H x W frame, by the frame just before
+        it (the frame just after it for the first segment).  It asks: what if the mouth stopped moving here?"""
+        T, s = int(T), int(segment_frames)
+        if s < 1:
+            raise ValueError(f"segment_frames must be >= 1, got {segment_frames}")
+        if s >= T:
+            raise ValueError(f"a segment of {s} frames covers the whole {T}-frame window: there is no frame to freeze to")
+        out = []
+        for t0 in range(0, T, s):
+            t1 = min(t0 + s, T)
+            out.append((t0, t1, 0, int(H), 0, int(W), t0 - 1 if t0 > 0 else t1))
+        return out
+
+    @staticmethod
+    def fill_cell_boxes(T: int, H: int, W: int, grid: int) -> List[Tuple[int, ...]]:
+        """Fill boxes: the crop cut into grid x grid cells (edges round(j*H/grid), round(j*W/grid)), row-major, each cell filled
+        over all T frames with the call's fill value."""
+        g = int(grid)
+        if not 1 <= g <= min(int(H), int(W)):
+            raise ValueError(f"grid must be in 1..{min(int(H), int(W))}, got {grid}")
+        ye = [int(round(j * H / g)) for j in range(g + 1)]
+        xe = [int(round(j * W / g)) for j in range(g + 1)]
+        return [(0, int(T), ye[a], ye[a + 1], xe[b], xe[b + 1], -1) for a in range(g) for b in range(g)]
+
+    def explain_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                      segment_frames: int = 4, grid: int = 4, fill: int = 128,
+                      audio_starts_from: Optional[Sequence[int]] = None) -> Dict[str, Any]:
+        """Occlusion evidence of every window of a track: one `score_track_occlusions` call with an empty box, the freeze segments
+        (`freeze_segment_boxes`) and the fill cells (`fill_cell_boxes`), K = 1 + 8 + 16 = 25 at the defaults.
+        Returns calibrated values:
+          `confidence` (n,): P(real) of the plain window;
+          `temporal` (n, S), `spatial` (n, grid, grid): P(real) with the region hidden MINUS `confidence`.  A value > 0 means
+            hiding the region made the window look more real: the region carried evidence of a fake.  A value < 0: it carried
+            evidence of a real video;
+          `spatial_mean` (grid, grid): `spatial` averaged over the windows;
+          `frame_first`, `frame_evidence`: the per-frame timeline of `temporal` (`aggregate.frame_evidence_timeline`), in the
+            frame numbers of `audio_starts_from` when given (absolute video frames), otherwise of `starts`;
+          `segment_frames`, `grid`, `fill`."""
+        T = self.chunk_size
+        H, W = int(track_u8.shape[1]), int(track_u8.shape[2])
+        freeze = self.freeze_segment_boxes(T, segment_frames, H, W)
+        cells = self.fill_cell_boxes(T, H, W, grid)
+        boxes = [(0, 0, 0, 0, 0, 0, -1)] + freeze + cells
+        logits = self.score_track_occlusions(track_u8, starts, mel_full, total_v_frames, boxes, fill=fill, audio_starts_from=audio_starts_from)
+        n, S, g = len(starts), len(freeze), int(grid)
+        probs = np.array([self._calibrate(float(x)) for x in logits.cpu().flatten().tolist()], dtype=np.float64).reshape(n, len(boxes))
+        conf = probs[:, 0]
+        temporal = probs[:, 1:1 + S] - conf[:, None]
+        spatial = (probs[:, 1 + S:] - conf[:, None]).reshape(n, g, g)
+        pos = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
+        first, timeline = _agg.frame_evidence_timeline(pos, temporal, int(segment_frames), T)
+        return {"confidence": conf, "temporal": temporal, "spatial": spatial,
+                "spatial_mean": spatial.mean(axis=0) if n else np.zeros((g, g)),
+                "frame_first": first, "frame_evidence": timeline,
+                "segment_frames": int(segment_frames), "grid": g, "fill": int(fill)}
+
     def score_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int):
         logits = self.score_track_logits(track_u8, starts, mel_full, total_v_frames)
         confs = [self._calibrate(float(x)) for x in logits.cpu().tolist()]
