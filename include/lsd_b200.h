@@ -204,6 +204,33 @@ int lsd_score_occlusions(lsd_handle* h, const uint8_t* track, int n_frames, int 
                          const lsd_occlusion* boxes, int K, int fill, int precision, int batch,
                          float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- audio occlusion evidence: window scores with a region of the window's log-mel masked ------------------ */
+/* This entry has no reference counterpart.  Window i's audio slice is the (F, Ta) log-mel window of Predictor._align_audio_chunk
+ * (predictor.py:525-552) that lsd_score_windows gives it: first column the base start a_i (computed, or
+ * audio_starts_host_or_null[i], clamped as there), the last column of the clip repeated past its end.  A box is four int32
+ * values in window coordinates, columns [c0,c1) x mel bins [f0,f1); the masked slice is
+ *   out[f,c] = (c0<=c<c1 && f0<=f<f1) ? fill : win[f,c]
+ * applied after the padding, so a box may cover repeated columns.  A box with c0==c1 or f0==f1 is empty: the row is the plain
+ * window.  fill -80 is the floor of the library's log-mel (power_to_db(ref=max, top_db=80), logmel.cu), i.e. silence relative to
+ * the clip's maximum.  Typical boxes: a time segment over all bins and a mel band over all columns. */
+typedef struct { int32_t c0, c1, f0, f1; } lsd_audio_occlusion;
+#define LSD_MAX_AUDIO_OCCLUSIONS LSD_MAX_AUDIO_VARIANTS
+/* Rows are (window, box) pairs in window-major order, row r = i*K + k; `batch` counts windows, as in lsd_score_offsets.  The masked
+ * slices of a batch are written on the device, end to end, into a pseudo clip (F, nb*K*Ta) in the workspace, and row j of the
+ * batch reads columns [j*Ta, (j+1)*Ta) of it as its explicit audio start.  The tensor-core route with the fused token kernels
+ * scores them with the shared-visual forward of lsd_score_offsets (visual encoder and artifact branch once per window); every
+ * other configuration scores them with lsd_score_windows, each window repeated K times.  logits_out: device (n_windows, K) fp32,
+ * entry (i, k) bit for bit lsd_score_windows on window i with slice k masked on the host (any such clip, explicit audio start).
+ * Everything is checked before any GPU work: LSD_ERR_SHAPE for K outside 1..LSD_MAX_AUDIO_OCCLUSIONS, a box outside
+ * [0,Ta]x[0,F] or with c0>c1 or f0>f1, or a window outside the track; LSD_ERR_ARG for boxes == NULL, a non-finite fill or a
+ * null pointer. */
+size_t lsd_score_audio_occlusions_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision);
+int lsd_score_audio_occlusions(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                               const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                               const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                               const lsd_audio_occlusion* boxes, int K, float fill, int precision, int batch,
+                               float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- speaking alignment / mouth motion: the per-window numpy loops of _predict_long_video ------------------ */
 /* Frame-difference energies of a track (Predictor._speaking_alignment_score, app/inference/predictor.py:339-345, and
  * _mouth_motion_energy_check, :395-402): for every frame pair f in [0, n_frames-1)

@@ -20,6 +20,7 @@ LSD_NCDHW, LSD_NDHWC = 0, 1
 LSD_PREC_FP32, LSD_PREC_BF16 = 0, 1
 LSD_MAX_AUDIO_VARIANTS = 64
 LSD_MAX_OCCLUSIONS = 1024
+LSD_MAX_AUDIO_OCCLUSIONS = LSD_MAX_AUDIO_VARIANTS
 
 # every symbol include/lsd_b200.h declares (checked by tests/test_cabi.py)
 EXPORTS = [
@@ -32,6 +33,7 @@ EXPORTS = [
     "lsd_workspace_invalidate", "lsd_planar_stage_read", "lsd_state_generation", "lsd_host_pack_u8_exact", "lsd_host_pack_u8_begin", "lsd_host_pack_u8_end", "lsd_host_pack_last_ms", "lsd_expand_u8",
     "lsd_forward_audio_variants_workspace_bytes", "lsd_forward_audio_variants", "lsd_score_offsets_workspace_bytes", "lsd_score_offsets",
     "lsd_score_occlusions_workspace_bytes", "lsd_score_occlusions",
+    "lsd_score_audio_occlusions_workspace_bytes", "lsd_score_audio_occlusions",
 ]
 
 
@@ -43,6 +45,12 @@ class LsdOcclusion(C.Structure):
     """One occlusion box in window coordinates: frames [t0,t1) x rows [y0,y1) x columns [x0,x1), filled from frame `src` of the
     un-occluded window (src >= 0) or with the call's fill value (src = -1)."""
     _fields_ = [(f, C.c_int32) for f in ("t0", "t1", "y0", "y1", "x0", "x1", "src")]
+
+
+class LsdAudioOcclusion(C.Structure):
+    """One audio occlusion box in window coordinates: mel columns [c0,c1) x mel bins [f0,f1) of the window's (F, Ta) log-mel
+    slice, set to the call's fill value."""
+    _fields_ = [(f, C.c_int32) for f in ("c0", "c1", "f0", "f1")]
 
 
 class LsdAux(C.Structure):
@@ -114,6 +122,11 @@ def lib() -> C.CDLL:
         L.lsd_score_occlusions.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
                                            C.POINTER(LsdOcclusion), i, i, i, i, vp, vp, sz, vp]
         L.lsd_score_occlusions.restype = i
+        L.lsd_score_audio_occlusions_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]
+        L.lsd_score_audio_occlusions_workspace_bytes.restype = sz
+        L.lsd_score_audio_occlusions.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
+                                                 C.POINTER(LsdAudioOcclusion), i, C.c_float, i, i, vp, vp, sz, vp]
+        L.lsd_score_audio_occlusions.restype = i
         _lib = L
         return L
 

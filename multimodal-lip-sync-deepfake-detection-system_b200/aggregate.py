@@ -74,6 +74,28 @@ def frame_evidence_timeline(starts: Sequence[int], temporal, segment_frames: int
     return first, [float(t / c) if c else None for t, c in zip(total, count)]
 
 
+def columns_to_frames(first_col: int, values: Sequence[Optional[float]], Ta_full: int, total_v_frames: int):
+    """A per-mel-column timeline (`values[c]` belongs to column first_col + c, None where nothing covers it) as a per-video-frame
+    timeline.  Column c belongs to frame c * total_v_frames // Ta_full, in integers, the ratio `_audio_start` uses to place a
+    window's audio.  Returns `(first_frame, frame_values)`, from the frame of the first column to the frame of the last one; a
+    frame's value is the mean of its columns that are not None, None when it has none (also a frame no column maps to)."""
+    Ta_full, nv = int(Ta_full), int(total_v_frames)
+    if Ta_full < 1 or nv < 1:
+        raise ValueError(f"Ta_full and total_v_frames must be >= 1, got {Ta_full} and {nv}")
+    if not len(values):
+        return 0, []
+    cols = np.arange(int(first_col), int(first_col) + len(values), dtype=np.int64)
+    frames = cols * nv // Ta_full
+    first = int(frames[0])
+    total = np.zeros(int(frames[-1]) - first + 1, dtype=np.float64)
+    count = np.zeros_like(total)
+    for f, v in zip(frames - first, values):
+        if v is not None:
+            total[f] += float(v)
+            count[f] += 1
+    return first, [float(t / c) if c else None for t, c in zip(total, count)]
+
+
 def _speech_weighted(conf: Sequence[float], speaking: Sequence[float], vad: Optional[Sequence[float]], smoothing: str,
                      trim_ratio: float) -> float:
     # predictor.py:262-293

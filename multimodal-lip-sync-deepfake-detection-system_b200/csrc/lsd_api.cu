@@ -779,6 +779,103 @@ extern "C" int lsd_score_offsets(lsd_handle* h, const uint8_t* track, int n_fram
 }
 
 // ================================================================================================
+// Audio occlusion evidence: K masked log-mel slices per window (occlusion.cu), laid end to end in a pseudo clip and scored as an
+// audio-variant sweep with explicit audio starts j*Ta; the clip is never clamped or padded, so the gather copies the slices as built
+// ================================================================================================
+// Workspace: [boxes (LSD_MAX_AUDIO_OCCLUSIONS x 4 int32) | base audio starts of one batch's windows | pseudo clip (F, batch*K*Ta)
+// fp32 | scoring workspace: lsd_score_offsets' on the shared route, otherwise lsd_score_windows' at `batch` rows].
+namespace {
+size_t audio_occlusion_extra_bytes(int batch, int K, int F, int Ta) {
+  return align256((size_t)LSD_MAX_AUDIO_OCCLUSIONS * 4 * sizeof(int32_t)) + align256((size_t)batch * sizeof(int32_t)) +
+         align256((size_t)F * batch * K * Ta * sizeof(float));
+}
+}  // namespace
+
+extern "C" size_t lsd_score_audio_occlusions_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  if (!h || batch < 1 || K < 1 || K > LSD_MAX_AUDIO_OCCLUSIONS) return 0;
+  const size_t sw = shared_route(precision, T) ? lsd_score_offsets_workspace_bytes(h, batch, K, T, H, W, F, Ta, precision)
+                                               : lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
+  if (sw == 0) return 0;
+  return audio_occlusion_extra_bytes(batch, K, F, Ta) + align256(sw);
+}
+
+extern "C" int lsd_score_audio_occlusions(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                          const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full,
+                                          int total_v_frames, int Ta, const lsd_audio_occlusion* boxes, int K, float fill, int precision,
+                                          int batch, float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_audio_occlusions: no weights loaded");
+  if (!boxes) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_audio_occlusions: boxes is NULL");
+  if (K < 1 || K > LSD_MAX_AUDIO_OCCLUSIONS)
+    return lsd_fail(h, LSD_ERR_SHAPE, "K = %d audio occlusion boxes: expected 1 <= K <= %d", K, LSD_MAX_AUDIO_OCCLUSIONS);
+  if (!std::isfinite(fill)) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_audio_occlusions: fill %f is not finite", (double)fill);
+  for (int k = 0; k < K; ++k) {
+    const lsd_audio_occlusion& b = boxes[k];
+    if (b.c0 < 0 || b.c0 > b.c1 || b.c1 > Ta || b.f0 < 0 || b.f0 > b.f1 || b.f1 > F)
+      return lsd_fail(h, LSD_ERR_SHAPE, "audio box %d [%d,%d)x[%d,%d) is not inside the %d-column x %d-bin window", k, b.c0, b.c1, b.f0,
+                      b.f1, Ta, F);
+  }
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !mel_full || !logits_out || !workspace)
+    return lsd_fail(h, LSD_ERR_ARG, "lsd_score_audio_occlusions: null pointer argument");
+  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_audio_occlusions: bad extents");
+  if ((int64_t)n_windows * K > INT32_MAX || (int64_t)batch * K * Ta > INT32_MAX)
+    return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d boxes in batches of %d: too many rows for one call", n_windows, K, batch);
+  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
+  Shapes s;
+  int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
+  if (rc) return rc;
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = lsd_score_audio_occlusions_workspace_bytes(h, batch, K, T, H, W, F, Ta, precision);
+  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  char* ws = reinterpret_cast<char*>(workspace);
+  int32_t* d_boxes = reinterpret_cast<int32_t*>(ws);
+  int32_t* d_abase = reinterpret_cast<int32_t*>(ws + align256((size_t)LSD_MAX_AUDIO_OCCLUSIONS * 4 * sizeof(int32_t)));
+  float* clip = reinterpret_cast<float*>(reinterpret_cast<char*>(d_abase) + align256((size_t)batch * sizeof(int32_t)));
+  const size_t extra = audio_occlusion_extra_bytes(batch, K, F, Ta);
+  char* sws = ws + extra;
+  const size_t sws_bytes = workspace_bytes - extra;
+  std::vector<int32_t> abase(n_windows), rows((size_t)batch * K);
+  for (int i = 0; i < n_windows; ++i) abase[i] = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
+  for (size_t j = 0; j < rows.size(); ++j) rows[j] = (int32_t)j * Ta;   // row j of a batch: columns [j*Ta, (j+1)*Ta) of the clip
+  static_assert(sizeof(lsd_audio_occlusion) == 4 * sizeof(int32_t), "lsd_audio_occlusion is four packed int32");
+  CUDA_OK(h, cudaMemcpyAsync(d_boxes, boxes, (size_t)K * sizeof(lsd_audio_occlusion), cudaMemcpyHostToDevice, st));
+  // One clip serves every batch: batch k+1's builder is enqueued on `st` after every reader of batch k's clip.  On the shared
+  // route the only readers are the mel gathers of the audio groups (forward_bf16_impl with a VarTail, not pipelined): group 0 runs
+  // on the side stream after ev_start, recorded on `st` behind this batch's builder, and `st` waits for its ev_audio before
+  // groups 1.. run on `st` itself, so `st` is past every gather when score_offsets_batch_bf16 returns.  lsd_score_windows
+  // gathers the audio of each of its batches on `st`, ahead of the encoders, pipelined or not.
+  if (shared_route(precision, T)) {
+    const size_t vi = align256((size_t)batch * sizeof(int32_t)), ai = align256((size_t)batch * K * sizeof(int32_t));
+    int32_t* d_vs = reinterpret_cast<int32_t*>(sws);
+    int32_t* d_as = reinterpret_cast<int32_t*>(sws + vi);
+    CUDA_OK(h, cudaMemcpyAsync(d_as, rows.data(), rows.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    for (int w0 = 0; w0 < n_windows; w0 += batch) {
+      const int nb = std::min(batch, n_windows - w0);
+      CUDA_OK(h, cudaMemcpyAsync(d_vs, starts_host + w0, nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      CUDA_OK(h, cudaMemcpyAsync(d_abase, &abase[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      launch_mask_audio_windows(mel_full, F, Ta_full, d_abase, d_boxes, K, w0 * K, nb * K, Ta, fill, clip, st);
+      if ((rc = score_offsets_batch_bf16(h, track, n_frames, d_vs, d_as, clip, nb * K * Ta, nb, batch, K, T, H, W, F, Ta,
+                                         logits_out + (size_t)w0 * K, sws + vi + ai, sws_bytes - vi - ai, st))) return rc;
+    }
+  } else {
+    std::vector<int32_t> vrep((size_t)batch * K);   // window i's track start, once per box
+    for (int w0 = 0; w0 < n_windows; w0 += batch) {
+      const int nb = std::min(batch, n_windows - w0);
+      for (int j = 0; j < nb * K; ++j) vrep[j] = starts_host[w0 + j / K];
+      CUDA_OK(h, cudaMemcpyAsync(d_abase, &abase[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      launch_mask_audio_windows(mel_full, F, Ta_full, d_abase, d_boxes, K, w0 * K, nb * K, Ta, fill, clip, st);
+      if ((rc = lsd_score_windows(h, track, n_frames, H, W, vrep.data(), rows.data(), nb * K, T, clip, F, nb * K * Ta, total_v_frames, Ta,
+                                  precision, batch, logits_out + (size_t)w0 * K, sws, sws_bytes, stream))) return rc;
+    }
+  }
+  CUDA_OK(h, cudaGetLastError());
+  return LSD_OK;
+}
+
+// ================================================================================================
 // Sub-paths (tensor-core route): AudioEncoder.forward and CrossModalAttention + TemporalTransformer
 // ================================================================================================
 extern "C" size_t lsd_audio_encoder_workspace_bytes(lsd_handle* h, int B, int F, int Ta) {

@@ -37,6 +37,10 @@ void launch_gather_windows_u8(const uint8_t* track, int n_frames, const int32_t*
 // win_starts: track start of windows r0 / K, r0 / K + 1, ...; boxes: K x 7 int32 (t0, t1, y0, y1, x0, x1, src)
 void launch_occlude_windows(const uint8_t* track, const int32_t* win_starts, const int32_t* boxes, int K, int r0, int nb, int T,
                             int H, int W, int fill, uint8_t* out, cudaStream_t s);
+// masked audio windows (occlusion.cu): rows r0 .. r0+nb-1 = (window r / K, box r % K) -> fp32 pseudo clip out (F, nb*Ta), row j in
+// columns [j*Ta, (j+1)*Ta); a_starts: base mel column of windows r0 / K, r0 / K + 1, ...; boxes: K x 4 int32 (c0, c1, f0, f1)
+void launch_mask_audio_windows(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, const int32_t* boxes, int K,
+                               int r0, int nb, int Ta, float fill, float* out, cudaStream_t s);
 // mel_full (F, Ta_full) + per-window a_start -> (n, F, Ta) with repeat-last-column padding (predictor.py:525-552)
 void launch_gather_audio(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, float* dst,
                          int n, int Ta, cudaStream_t s);

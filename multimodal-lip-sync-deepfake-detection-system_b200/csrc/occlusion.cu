@@ -2,6 +2,7 @@
 // another into a pseudo-track of nb*T frames, which the plain scoring path then reads with window starts 0, T, 2T, ...
 //   out[t,y,x,:] = (t0<=t<t1 && y0<=y<y1 && x0<=x<x1) ? (src < 0 ? fill : win[src,y,x,:]) : win[t,y,x,:]
 // win = frames s_i .. s_i+T-1 of the track (the un-occluded window); only those frames are read.
+// The masked log-mel windows of lsd_score_audio_occlusions are built the same way, as a pseudo clip (mask_audio_windows_kernel).
 #include "lsd_kernels.h"
 
 namespace lsd {
@@ -91,6 +92,46 @@ void launch_occlude_windows(const uint8_t* track, const int32_t* win_starts, con
   const unsigned grid = (unsigned)nb * (unsigned)T;
   if (vec) occlude_windows_kernel<true><<<grid, 256, 0, s>>>(track, win_starts, boxes, K, r0, T, H, W, (uint32_t)fill, out);
   else occlude_windows_kernel<false><<<grid, 256, 0, s>>>(track, win_starts, boxes, K, r0, T, H, W, (uint32_t)fill, out);
+  count_launch();
+}
+
+namespace {
+// Masked audio windows for lsd_score_audio_occlusions: one block per row j (window r / K, box r % K, r = r0 + j) writes the row's
+// (F, Ta) slice into columns [j*Ta, (j+1)*Ta) of the pseudo clip (F, cols):
+//   out[f, j*Ta + c] = (c0<=c<c1 && f0<=f<f1) ? fill : mel[f, clamp(a_i + c, 0, Ta_full-1)]
+// The unmasked values are gather_audio_kernel's (kernels_f32.cu) copy of the same column.  Consecutive threads take consecutive
+// columns of one bin, so every warp stores 128 contiguous bytes.
+__global__ void __launch_bounds__(256) mask_audio_windows_kernel(const float* __restrict__ mel, int F, int Ta_full,
+                                                                 const int32_t* __restrict__ a_starts, const int4* __restrict__ boxes,
+                                                                 int K, int r0, int Ta, float fill, int64_t cols, float* __restrict__ out) {
+  const int j = blockIdx.x, r = r0 + j;
+  const int wi = r / K;
+  const int4 b = boxes[r - wi * K];   // (c0, c1, f0, f1)
+  const int a = a_starts[wi - r0 / K];
+  float* dst = out + (int64_t)j * Ta;
+  const int n = F * Ta;
+  for (int e = threadIdx.x; e < n; e += blockDim.x) {
+    const int f = e / Ta, c = e - f * Ta;
+    float v;
+    if (c >= b.x && c < b.y && f >= b.z && f < b.w) {
+      v = fill;
+    } else {
+      int col = a + c;
+      col = col >= Ta_full ? Ta_full - 1 : col;
+      col = col < 0 ? 0 : col;
+      v = mel[(int64_t)f * Ta_full + col];
+    }
+    dst[(int64_t)f * cols + c] = v;
+  }
+}
+
+}  // namespace
+
+void launch_mask_audio_windows(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, const int32_t* boxes, int K,
+                               int r0, int nb, int Ta, float fill, float* out, cudaStream_t s) {
+  if (nb < 1) return;
+  mask_audio_windows_kernel<<<(unsigned)nb, 256, 0, s>>>(mel_full, F, Ta_full, a_starts, reinterpret_cast<const int4*>(boxes), K, r0,
+                                                         Ta, fill, (int64_t)nb * Ta, out);
   count_launch();
 }
 

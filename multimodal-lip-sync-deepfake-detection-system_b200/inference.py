@@ -737,6 +737,124 @@ class Predictor:
                 "frame_first": first, "frame_evidence": timeline,
                 "segment_frames": int(segment_frames), "grid": g, "fill": int(fill)}
 
+    # ------------------------------------------------------------------ audio occlusion evidence (lsd_score_audio_occlusions)
+    def score_track_audio_occlusions(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                                     boxes, fill: float = -80.0, chunk_a_size: int = 128,
+                                     audio_starts_from: Optional[Sequence[int]] = None) -> torch.Tensor:
+        """`score_track_logits` with K audio occlusion boxes per window (`lsd_score_audio_occlusions`).  `boxes`: a `(K, 4)` int
+        array or a sequence of 4-tuples `(c0, c1, f0, f1)` in window coordinates; mel columns [c0,c1) x bins [f0,f1) of the window's
+        `(F, chunk_a_size)` log-mel slice (`_align_audio_chunk`, after its padding) are set to `fill`.  The default -80 is the floor
+        of the library's log-mel (`power_to_db(ref=max, top_db=80)`): silence relative to the clip's maximum.  An empty box leaves
+        the slice as it is.  The video side of a window runs once for all its boxes.  Returns fp32 logits `(n, K)` on the device;
+        entry (i, k) is bit for bit the logit of window i with its audio slice masked by box k."""
+        m = self.model
+        dev = m._device()
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        if mel_full.dim() != 3 or mel_full.shape[0] != 1:
+            raise ValueError(f"mel_full must be (1, F, T_full), got {tuple(mel_full.shape)}")
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        F_, Ta_full = int(mel_full.shape[1]), int(mel_full.shape[2])
+        T, Ta = self.chunk_size, int(chunk_a_size)
+        bx = np.asarray(boxes, dtype=np.int64)
+        if bx.ndim != 2 or bx.shape[1] != 4:
+            raise ValueError(f"boxes must be (K, 4) (c0, c1, f0, f1), got shape {bx.shape}")
+        K = int(bx.shape[0])
+        if not 1 <= K <= _cabi.LSD_MAX_AUDIO_OCCLUSIONS:
+            raise ValueError(f"{K} audio occlusion boxes: expected 1 to {_cabi.LSD_MAX_AUDIO_OCCLUSIONS}")
+        for k, (c0, c1, f0, f1) in enumerate(bx.tolist()):
+            if not (0 <= c0 <= c1 <= Ta and 0 <= f0 <= f1 <= F_):
+                raise ValueError(f"audio box {k} {bx[k].tolist()} is not inside the {Ta}-column x {F_}-bin window")
+        if not np.isfinite(float(fill)):
+            raise ValueError(f"fill must be finite, got {fill}")
+        n = len(starts)
+        if audio_starts_from is not None and len(audio_starts_from) != n:
+            raise ValueError("audio_starts_from must have one entry per window")
+        for i, s in enumerate(starts):
+            if not 0 <= int(s) <= n_frames - T:
+                raise ValueError(f"window {i} [{int(s)},{int(s) + T}) is outside the {n_frames}-frame track")
+        logits = torch.empty(n, K, dtype=torch.float32, device=dev)
+        if n == 0:
+            return logits
+        track_u8 = track_u8.contiguous()
+        mel_full = mel_full.to(torch.float32).contiguous()
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = m._precision()
+            batch = min(self.batch_size, n)
+            need = L.lsd_score_audio_occlusions_workspace_bytes(h.ptr, batch, K, T, H, W, F_, Ta, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            ws = m._workspace(need, dev)
+            st = (C.c_int32 * n)(*[int(s) for s in starts])
+            ast = None
+            if audio_starts_from is not None:
+                ast = (C.c_int32 * n)(*[self._audio_start(int(v), Ta_full, int(total_v_frames), Ta) for v in audio_starts_from])
+            boxes_c = (_cabi.LsdAudioOcclusion * K)(*[_cabi.LsdAudioOcclusion(*row) for row in bx.tolist()])
+            rc = L.lsd_score_audio_occlusions(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, T, mel_full.data_ptr(), F_, Ta_full,
+                                              int(total_v_frames), Ta, boxes_c, K, float(fill), prec, batch, logits.data_ptr(),
+                                              ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return logits
+
+    @staticmethod
+    def mute_segment_boxes(Ta: int, segment_cols: int, F: int = 80) -> List[Tuple[int, ...]]:
+        """Mute boxes: segment j = mel columns [j*s, min((j+1)*s, Ta)) of the window's slice, over all F bins.  It asks: what if
+        the speech stopped here?  (16 columns = 160 ms.)"""
+        Ta, s, F = int(Ta), int(segment_cols), int(F)
+        if s < 1 or Ta < 1 or F < 1:
+            raise ValueError(f"Ta, segment_cols and F must be >= 1, got {Ta}, {segment_cols} and {F}")
+        return [(c0, min(c0 + s, Ta), 0, F) for c0 in range(0, Ta, s)]
+
+    @staticmethod
+    def mel_band_boxes(Ta: int, F: int, bands: int) -> List[Tuple[int, ...]]:
+        """Band boxes: the F mel bins cut into `bands` bands (edges round(j*F/bands)), low to high, each over all Ta columns."""
+        Ta, F, b = int(Ta), int(F), int(bands)
+        if Ta < 1:
+            raise ValueError(f"Ta must be >= 1, got {Ta}")
+        if not 1 <= b <= F:
+            raise ValueError(f"bands must be in 1..{F}, got {bands}")
+        e = [int(round(j * F / b)) for j in range(b + 1)]
+        return [(0, Ta, e[j], e[j + 1]) for j in range(b)]
+
+    def explain_track_audio(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                            segment_cols: int = 16, bands: int = 8, fill: float = -80.0,
+                            audio_starts_from: Optional[Sequence[int]] = None) -> Dict[str, Any]:
+        """Audio occlusion evidence of every window of a track: one `score_track_audio_occlusions` call with an empty box, the mute
+        segments (`mute_segment_boxes`) and the mel bands (`mel_band_boxes`), K = 1 + 8 + 8 = 17 at the defaults (128-column slices).
+        Returns calibrated values with the sign convention of `explain_track`:
+          `confidence` (n,): P(real) of the plain window (equal to `explain_track`'s);
+          `audio_temporal` (n, S), `audio_spectral` (n, bands): P(real) with the box masked MINUS `confidence`.  A value > 0 means
+            masking the region made the window look more real: that stretch of speech or band carried evidence of a fake;
+          `audio_spectral_mean` (bands,): `audio_spectral` averaged over the windows;
+          `column_first`, `column_evidence`: the per-mel-column timeline of `audio_temporal` (`aggregate.frame_evidence_timeline`
+            on the windows' audio starts), in absolute clip columns when `audio_starts_from` is given, cut to the clip's columns;
+          `frame_first`, `frame_evidence`: that timeline in video frames (`aggregate.columns_to_frames`), to line up with
+            `explain_track`'s `frame_evidence`;
+          `segment_cols`, `bands`, `band_edges` (bands + 1 mel-bin edges), `fill`."""
+        Ta = 128
+        F_, Ta_full = int(mel_full.shape[1]), int(mel_full.shape[2])
+        mute = self.mute_segment_boxes(Ta, segment_cols, F_)
+        band = self.mel_band_boxes(Ta, F_, bands)
+        boxes = [(0, 0, 0, 0)] + mute + band
+        logits = self.score_track_audio_occlusions(track_u8, starts, mel_full, total_v_frames, boxes, fill=fill, chunk_a_size=Ta,
+                                                   audio_starts_from=audio_starts_from)
+        n, S, nb = len(starts), len(mute), int(bands)
+        probs = np.array([self._calibrate(float(x)) for x in logits.cpu().flatten().tolist()], dtype=np.float64).reshape(n, len(boxes))
+        conf = probs[:, 0]
+        temporal = probs[:, 1:1 + S] - conf[:, None]
+        spectral = probs[:, 1 + S:] - conf[:, None]
+        pos = [self._audio_start(int(s), Ta_full, int(total_v_frames), Ta)
+               for s in (audio_starts_from if audio_starts_from is not None else starts)]
+        first, cols = _agg.frame_evidence_timeline(pos, temporal, int(segment_cols), Ta)
+        cols = cols[:max(0, Ta_full - first)]                             # a slice past the clip's end repeats its last column
+        f_first, frames = _agg.columns_to_frames(first, cols, Ta_full, int(total_v_frames))
+        return {"confidence": conf, "audio_temporal": temporal, "audio_spectral": spectral,
+                "audio_spectral_mean": spectral.mean(axis=0) if n else np.zeros(nb),
+                "column_first": first, "column_evidence": cols, "frame_first": f_first, "frame_evidence": frames,
+                "segment_cols": int(segment_cols), "bands": nb, "band_edges": [b[2] for b in band] + [band[-1][3]], "fill": float(fill)}
+
     def score_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int):
         logits = self.score_track_logits(track_u8, starts, mel_full, total_v_frames)
         confs = [self._calibrate(float(x)) for x in logits.cpu().tolist()]
