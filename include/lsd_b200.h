@@ -204,6 +204,40 @@ int lsd_score_occlusions(lsd_handle* h, const uint8_t* track, int n_frames, int 
                          const lsd_occlusion* boxes, int K, int fill, int precision, int batch,
                          float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- crop-jitter robustness: window scores of re-cropped windows ------------------------------------------ */
+/* This entry has no reference counterpart.  The reference's mouth crops come from a CPU face tracker whose boxes move with the
+ * detector that fired and jitter from frame to frame (app/preprocessing/face_detection.py, video.py:455-590); it asks whether a window's score would hold
+ * had the crop been placed differently.  Every window is scored K times, once per variant.  Variant k re-crops frame t of the
+ * window with its own forward 2x3 matrix (a different matrix per frame models tracker jitter):
+ *   out[t] = cv2.warpAffine(win[t], M[k,t], (W, H), flags=cv2.INTER_LINEAR, borderMode=cv2.BORDER_REPLICATE)
+ * bit for bit (8-bit integer arithmetic on tables built on the host exactly as cv::warpAffine builds them, including its
+ * inversion of M in double).  lsd_warp is cv2's forward matrix, row-major, src -> dst: the convention of cv2.warpAffine and
+ * cv2.getRotationMatrix2D. */
+typedef struct { double m[6]; } lsd_warp;
+#define LSD_MAX_WARPS 64
+/* warps: host, K*T matrices, variant-major (warps[k*T + t]).  Rows are (window, variant) pairs in window-major order, row
+ * r = i*K + k; `batch` counts rows.  A row's audio slice is its window's slice, with the base-start rule of lsd_score_windows
+ * (computed, or audio_starts_host_or_null[i], clamped).  The warped windows of a batch are built on the device and scored by the
+ * plain batch path of lsd_score_windows, so logits_out (device, (n_windows, K) fp32) entry (i, k) is bit for bit lsd_score_windows
+ * on window i warped on the host, with the same audio start.  A workspace of at least twice lsd_score_warps_workspace_bytes enables
+ * the cross-batch pipelining of lsd_score_windows; a short last batch runs in exactly the queried size.  Everything is checked
+ * before any GPU work: LSD_ERR_SHAPE for K outside 1..LSD_MAX_WARPS, a window outside the track, or a matrix whose inverse maps a
+ * pixel of the frame to a coordinate beyond +-32767 (cv2's int16 tap coordinates would saturate); LSD_ERR_ARG for warps == NULL,
+ * a non-finite entry or a singular matrix. */
+size_t lsd_score_warps_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision);
+int lsd_score_warps(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                    const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                    const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                    const lsd_warp* warps, int K, int precision, int batch,
+                    float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
+/* The re-cropped windows themselves, built by the same kernel lsd_score_warps scores: out (device uint8, (n_windows, K, T, H, W, 3))
+ * holds window i under variant k at [i][k], each frame bit for bit the cv2.warpAffine above.  Same checks as lsd_score_warps;
+ * workspace: lsd_warp_windows_workspace_bytes (the tables and the window starts). */
+size_t lsd_warp_windows_workspace_bytes(int n_windows, int K, int T, int H, int W);
+int lsd_warp_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                     const int32_t* starts_host, int n_windows, int T, const lsd_warp* warps, int K,
+                     uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- audio occlusion evidence: window scores with a region of the window's log-mel masked ------------------ */
 /* This entry has no reference counterpart.  Window i's audio slice is the (F, Ta) log-mel window of Predictor._align_audio_chunk
  * (predictor.py:525-552) that lsd_score_windows gives it: first column the base start a_i (computed, or

@@ -21,6 +21,7 @@ LSD_PREC_FP32, LSD_PREC_BF16 = 0, 1
 LSD_MAX_AUDIO_VARIANTS = 64
 LSD_MAX_OCCLUSIONS = 1024
 LSD_MAX_AUDIO_OCCLUSIONS = LSD_MAX_AUDIO_VARIANTS
+LSD_MAX_WARPS = 64
 
 # every symbol include/lsd_b200.h declares (checked by tests/test_cabi.py)
 EXPORTS = [
@@ -34,6 +35,7 @@ EXPORTS = [
     "lsd_forward_audio_variants_workspace_bytes", "lsd_forward_audio_variants", "lsd_score_offsets_workspace_bytes", "lsd_score_offsets",
     "lsd_score_occlusions_workspace_bytes", "lsd_score_occlusions",
     "lsd_score_audio_occlusions_workspace_bytes", "lsd_score_audio_occlusions",
+    "lsd_score_warps_workspace_bytes", "lsd_score_warps", "lsd_warp_windows_workspace_bytes", "lsd_warp_windows",
 ]
 
 
@@ -51,6 +53,12 @@ class LsdAudioOcclusion(C.Structure):
     """One audio occlusion box in window coordinates: mel columns [c0,c1) x mel bins [f0,f1) of the window's (F, Ta) log-mel
     slice, set to the call's fill value."""
     _fields_ = [(f, C.c_int32) for f in ("c0", "c1", "f0", "f1")]
+
+
+class LsdWarp(C.Structure):
+    """One re-crop: cv2's forward 2x3 affine matrix (src -> dst), row-major, as `cv2.warpAffine` and `cv2.getRotationMatrix2D`
+    use it."""
+    _fields_ = [("m", C.c_double * 6)]
 
 
 class LsdAux(C.Structure):
@@ -127,6 +135,13 @@ def lib() -> C.CDLL:
         L.lsd_score_audio_occlusions.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
                                                  C.POINTER(LsdAudioOcclusion), i, C.c_float, i, i, vp, vp, sz, vp]
         L.lsd_score_audio_occlusions.restype = i
+        L.lsd_score_warps_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_warps_workspace_bytes.restype = sz
+        L.lsd_score_warps.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
+                                      C.POINTER(LsdWarp), i, i, i, vp, vp, sz, vp]
+        L.lsd_score_warps.restype = i
+        L.lsd_warp_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_warp_windows_workspace_bytes.restype = sz
+        L.lsd_warp_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdWarp), i, vp, vp, sz, vp]
+        L.lsd_warp_windows.restype = i
         _lib = L
         return L
 

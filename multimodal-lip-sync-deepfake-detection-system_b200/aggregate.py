@@ -96,6 +96,33 @@ def columns_to_frames(first_col: int, values: Sequence[Optional[float]], Ta_full
     return first, [float(t / c) if c else None for t, c in zip(total, count)]
 
 
+def augmentation_stability(probs, confidence_threshold: float = 0.5, smoothing: str = "median", trim_ratio: float = 0.1,
+                           identity: int = 0) -> Dict[str, Any]:
+    """Stability of a verdict under K variants of every window (`Predictor.robustness_track`).  `probs`: (n_windows, K) P(real);
+    column `identity` is the unmodified window.  A window's decision is real when P(real) >= `confidence_threshold`.
+      `confidence`: the robust aggregate (`_robust`, predictor.py:246-260) of the identity column;
+      `variant_confidence` (K,): the same aggregate per variant;
+      `tta_confidence`: the aggregate over windows of each window's mean P(real) over the variants;
+      `window_spread` (n,): per window, the largest minus the smallest P(real) over the variants;
+      `decision_flip_rate`: the fraction of (window, variant) entries whose decision differs from the identity's in that window;
+      `verdict_stable`: every variant confidence lies on the same side of the threshold as `confidence`."""
+    p = np.asarray(probs, dtype=np.float64)
+    if p.ndim != 2 or not 0 <= int(identity) < p.shape[1]:
+        raise ValueError(f"probs must be (n_windows, K) with column {identity} present, got shape {p.shape}")
+    thr = float(confidence_threshold)
+    conf = _robust(p[:, identity].tolist(), smoothing, trim_ratio)
+    per_variant = [_robust(p[:, k].tolist(), smoothing, trim_ratio) for k in range(p.shape[1])]
+    real = p >= thr
+    return {
+        "confidence": conf,
+        "variant_confidence": per_variant,
+        "tta_confidence": _robust(p.mean(axis=1).tolist(), smoothing, trim_ratio),
+        "window_spread": p.max(axis=1) - p.min(axis=1),
+        "decision_flip_rate": float((real != real[:, identity:identity + 1]).mean()) if p.size else 0.0,
+        "verdict_stable": all((c >= thr) == (conf >= thr) for c in per_variant),
+    }
+
+
 def _speech_weighted(conf: Sequence[float], speaking: Sequence[float], vad: Optional[Sequence[float]], smoothing: str,
                      trim_ratio: float) -> float:
     # predictor.py:262-293

@@ -87,6 +87,7 @@ extern "C" int lsd_create(lsd_handle** out, int device) {
     if (ce == cudaSuccess) ce = lsd::tok_fused_device_init();
     if (ce == cudaSuccess) ce = lsd::stem_ring_device_init();
     if (ce == cudaSuccess) ce = lsd::tok_front_device_init();
+    if (ce == cudaSuccess) ce = lsd::warp_windows_device_init();
     if (ce != cudaSuccess) rc = lsd_fail(h, LSD_ERR_CUDA, "lsd_create: kernel attribute setup: %s", cudaGetErrorString(ce));
   }
   if (rc != 0) { g_create_error = h->err; delete h; return rc; }
@@ -643,6 +644,121 @@ extern "C" int lsd_score_occlusions(lsd_handle* h, const uint8_t* track, int n_f
   };
   return score_rows(h, pseudo, batch * T, n_rows, T, H, W, mel_full, F, Ta_full, Ta, precision, batch, logits_out, ws + extra,
                     workspace_bytes - extra, st, occluded);
+}
+
+// ================================================================================================
+// Crop-jitter robustness: K re-cropped copies of every window (warp.cu), scored by the batch loop of lsd_score_windows
+// ================================================================================================
+// Workspace: [warp tables (K*T*2(H+W) int32) | track starts of one batch's windows | pseudo-track of `batch` warped windows |
+// lsd_score_windows workspace].  As in lsd_score_occlusions, the pseudo-track is read only by the batch's first kernel on the
+// caller's stream (the tensor-core pixel rows or the fp32 gather), so one copy serves pipelined batches too.
+namespace {
+size_t warps_extra_bytes(int batch, int K, int T, int H, int W) {
+  return align256(warp_tables_ints(K, T, H, W) * sizeof(int32_t)) + align256(((size_t)batch + 1) * sizeof(int32_t)) +
+         align256((size_t)batch * T * H * W * 3);
+}
+
+// The checks every warp entry makes before any GPU work; on success h->warp_tab_host holds the tables of the K*T matrices.
+int warp_tables_checked(lsd_handle* h, const char* fn, const lsd_warp* warps, int K, int T, int H, int W) {
+  if (!warps) return lsd_fail(h, LSD_ERR_ARG, "%s: warps is NULL", fn);
+  if (K < 1 || K > LSD_MAX_WARPS) return lsd_fail(h, LSD_ERR_SHAPE, "K = %d warp variants: expected 1 <= K <= %d", K, LSD_MAX_WARPS);
+  if (T < 1 || H < 1 || W < 1 || (int64_t)H * W * 3 > INT32_MAX || !warp_extents_ok(H, W))
+    return lsd_fail(h, LSD_ERR_SHAPE, "%s: bad window extents T=%d H=%d W=%d", fn, T, H, W);
+  static_assert(sizeof(lsd_warp) == 6 * sizeof(double), "lsd_warp is six packed doubles");
+  h->warp_tab_host.resize(warp_tables_ints(K, T, H, W));
+  int bad = 0;
+  const int rc = warp_tables(reinterpret_cast<const double*>(warps), K * T, H, W, h->warp_tab_host.data(), &bad);
+  if (rc == -1)
+    return lsd_fail(h, LSD_ERR_ARG, "warp %d (variant %d, frame %d) has a non-finite entry or is singular", bad, bad / T, bad % T);
+  if (rc == -2)
+    return lsd_fail(h, LSD_ERR_SHAPE, "warp %d (variant %d, frame %d) maps the %dx%d frame beyond +-32767 px", bad, bad / T, bad % T, H, W);
+  return 0;
+}
+}  // namespace
+
+extern "C" size_t lsd_score_warps_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  if (batch < 1 || K < 1 || K > LSD_MAX_WARPS) return 0;
+  const size_t sw = lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
+  if (sw == 0) return 0;
+  return warps_extra_bytes(batch, K, T, H, W) + align256(sw);
+}
+
+extern "C" int lsd_score_warps(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                               const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full,
+                               int total_v_frames, int Ta, const lsd_warp* warps, int K, int precision, int batch, float* logits_out,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_warps: no weights loaded");
+  int rc = warp_tables_checked(h, "lsd_score_warps", warps, K, T, H, W);
+  if (rc) return rc;
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_warps: null pointer argument");
+  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_warps: bad extents");
+  if ((int64_t)n_windows * K > INT32_MAX) return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d warps: too many rows for one call", n_windows, K);
+  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
+  Shapes s;
+  if ((rc = make_shapes(h, batch, T, H, W, F, Ta, s))) return rc;
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = lsd_score_warps_workspace_bytes(h, batch, K, T, H, W, F, Ta, precision);
+  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const int n_rows = n_windows * K;
+  // row r reads frames (r % batch) * T .. of the batch's pseudo-track, and the audio slice of window r / K
+  h->idx_host.resize((size_t)2 * n_rows);
+  for (int i = 0; i < n_windows; ++i) {
+    const int32_t a = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
+    for (int k = 0; k < K; ++k) {
+      const int r = i * K + k;
+      h->idx_host[r] = (r % batch) * T;
+      h->idx_host[n_rows + r] = a;
+    }
+  }
+  char* ws = reinterpret_cast<char*>(workspace);
+  int32_t* d_tabs = reinterpret_cast<int32_t*>(ws);
+  int32_t* d_wins = reinterpret_cast<int32_t*>(ws + align256(h->warp_tab_host.size() * sizeof(int32_t)));
+  uint8_t* pseudo = reinterpret_cast<uint8_t*>(d_wins) + align256(((size_t)batch + 1) * sizeof(int32_t));
+  const size_t extra = warps_extra_bytes(batch, K, T, H, W);
+  CUDA_OK(h, cudaMemcpyAsync(d_tabs, h->warp_tab_host.data(), h->warp_tab_host.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  const BatchTrack warped = [&](int r0, int nb, const uint8_t*& trk, int& nf) -> int {
+    const int wa = r0 / K, wb = (r0 + nb - 1) / K;
+    CUDA_OK(h, cudaMemcpyAsync(d_wins, starts_host + wa, (size_t)(wb - wa + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    launch_warp_windows(track, d_wins, d_tabs, K, r0, nb, T, H, W, pseudo, st);
+    trk = pseudo;
+    nf = nb * T;
+    return 0;
+  };
+  return score_rows(h, pseudo, batch * T, n_rows, T, H, W, mel_full, F, Ta_full, Ta, precision, batch, logits_out, ws + extra,
+                    workspace_bytes - extra, st, warped);
+}
+
+// The warped windows themselves, written to a caller buffer by the builder lsd_score_warps uses: what the K variants look like.
+extern "C" size_t lsd_warp_windows_workspace_bytes(int n_windows, int K, int T, int H, int W) {
+  if (n_windows < 1 || K < 1 || K > LSD_MAX_WARPS || T < 1 || H < 1 || W < 1) return 0;
+  return align256(warp_tables_ints(K, T, H, W) * sizeof(int32_t)) + align256((size_t)n_windows * sizeof(int32_t));
+}
+
+extern "C" int lsd_warp_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host, int n_windows,
+                                int T, const lsd_warp* warps, int K, uint8_t* out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  int rc = warp_tables_checked(h, "lsd_warp_windows", warps, K, T, H, W);
+  if (rc) return rc;
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_warp_windows: null pointer argument");
+  if (n_windows < 0 || n_frames < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_warp_windows: bad extents");
+  if ((int64_t)n_windows * K * T > INT32_MAX) return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d warps: too many frames for one call", n_windows, K);
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = lsd_warp_windows_workspace_bytes(n_windows, K, T, H, W);
+  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  int32_t* d_tabs = reinterpret_cast<int32_t*>(workspace);
+  int32_t* d_wins = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(workspace) + align256(h->warp_tab_host.size() * sizeof(int32_t)));
+  CUDA_OK(h, cudaMemcpyAsync(d_tabs, h->warp_tab_host.data(), h->warp_tab_host.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  CUDA_OK(h, cudaMemcpyAsync(d_wins, starts_host, (size_t)n_windows * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  launch_warp_windows(track, d_wins, d_tabs, K, 0, n_windows * K, T, H, W, out, st);
+  CUDA_OK(h, cudaGetLastError());
+  return LSD_OK;
 }
 
 // ================================================================================================

@@ -84,6 +84,7 @@ struct lsd_handle {
   std::vector<Stage> stages;
   std::map<std::string, PlanarStage> planar_stages;
   std::vector<int32_t> idx_host;
+  std::vector<int32_t> warp_tab_host;      // lsd_score_warps: host copy of the warp tables, kept until the next call (async copy)
   Prof prof;
   cudaStream_t side_stream = nullptr;      // artifact branch runs here, concurrently with the token path
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_start = nullptr, ev_audio = nullptr;

@@ -41,6 +41,15 @@ void launch_occlude_windows(const uint8_t* track, const int32_t* win_starts, con
 // columns [j*Ta, (j+1)*Ta); a_starts: base mel column of windows r0 / K, r0 / K + 1, ...; boxes: K x 4 int32 (c0, c1, f0, f1)
 void launch_mask_audio_windows(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, const int32_t* boxes, int K,
                                int r0, int nb, int Ta, float fill, float* out, cudaStream_t s);
+// re-cropped windows (warp.cu): rows r0 .. r0+nb-1 = (window r / K, variant r % K) -> uint8 pseudo-track out (nb*T, H, W, 3), frame t
+// warped like cv2.warpAffine(INTER_LINEAR, BORDER_REPLICATE) with the tables of (variant k, frame t); win_starts: track start of
+// windows r0 / K, r0 / K + 1, ...; tabs: warp_tables of the K*T matrices, variant-major
+void launch_warp_windows(const uint8_t* track, const int32_t* win_starts, const int32_t* tabs, int K, int r0, int nb, int T, int H, int W,
+                         uint8_t* out, cudaStream_t s);
+size_t warp_tables_ints(int K, int T, int H, int W);
+int warp_tables(const double* m, int n, int H, int W, int32_t* out, int* bad);
+cudaError_t warp_windows_device_init();
+bool warp_extents_ok(int H, int W);
 // mel_full (F, Ta_full) + per-window a_start -> (n, F, Ta) with repeat-last-column padding (predictor.py:525-552)
 void launch_gather_audio(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, float* dst,
                          int n, int Ta, cudaStream_t s);

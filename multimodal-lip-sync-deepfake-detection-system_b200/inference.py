@@ -855,6 +855,161 @@ class Predictor:
                 "column_first": first, "column_evidence": cols, "frame_first": f_first, "frame_evidence": frames,
                 "segment_cols": int(segment_cols), "bands": nb, "band_edges": [b[2] for b in band] + [band[-1][3]], "fill": float(fill)}
 
+    # ------------------------------------------------------------------ crop-jitter robustness (lsd_score_warps)
+    def score_track_warps(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                          warps, chunk_a_size: int = 128, audio_starts_from: Optional[Sequence[int]] = None) -> torch.Tensor:
+        """`score_track_logits` with K re-cropped variants per window (`lsd_score_warps`).  `warps`: `(K, 2, 3)` forward affine
+        matrices in cv2's convention (src -> dst, as `cv2.warpAffine` takes them), the same for every frame, or `(K, T, 2, 3)`, one
+        per frame of the window.  Frame t of variant k is `cv2.warpAffine(frame, M[k, t], (W, H), INTER_LINEAR, BORDER_REPLICATE)`,
+        bit for bit, built on the device.  Returns fp32 logits `(n, K)` on the device; entry (i, k) is bit for bit the logit of
+        window i re-cropped by variant k, with window i's audio slice."""
+        m = self.model
+        dev = m._device()
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        if mel_full.dim() != 3 or mel_full.shape[0] != 1:
+            raise ValueError(f"mel_full must be (1, F, T_full), got {tuple(mel_full.shape)}")
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T = self.chunk_size
+        w = self._warp_matrices(warps, T)
+        K = int(w.shape[0])
+        n = len(starts)
+        if audio_starts_from is not None and len(audio_starts_from) != n:
+            raise ValueError("audio_starts_from must have one entry per window")
+        for i, s in enumerate(starts):
+            if not 0 <= int(s) <= n_frames - T:
+                raise ValueError(f"window {i} [{int(s)},{int(s) + T}) is outside the {n_frames}-frame track")
+        logits = torch.empty(n, K, dtype=torch.float32, device=dev)
+        if n == 0:
+            return logits
+        track_u8 = track_u8.contiguous()
+        mel_full = mel_full.to(torch.float32).contiguous()
+        F_, Ta_full = int(mel_full.shape[1]), int(mel_full.shape[2])
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = m._precision()
+            batch = min(self.batch_size, n * K)
+            need = L.lsd_score_warps_workspace_bytes(h.ptr, batch, K, T, H, W, F_, chunk_a_size, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            if n * K > batch and prec == _cabi.LSD_PREC_BF16:
+                need = 2 * need      # a double workspace lets the batches overlap as in score_track_logits
+            ws = m._workspace(need, dev)
+            st = (C.c_int32 * n)(*[int(s) for s in starts])
+            ast = None
+            if audio_starts_from is not None:
+                ast = (C.c_int32 * n)(*[self._audio_start(int(v), Ta_full, int(total_v_frames), chunk_a_size) for v in audio_starts_from])
+            warps_c = (_cabi.LsdWarp * (K * T)).from_buffer_copy(w.tobytes())
+            rc = L.lsd_score_warps(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, T, mel_full.data_ptr(), F_, Ta_full,
+                                   int(total_v_frames), chunk_a_size, warps_c, K, prec, batch, logits.data_ptr(), ws.data_ptr(),
+                                   ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return logits
+
+    @staticmethod
+    def _warp_matrices(warps, T: int) -> np.ndarray:
+        """`(K, 2, 3)` or `(K, T, 2, 3)` matrices as a contiguous float64 `(K, T, 2, 3)` array, K checked."""
+        w = np.asarray(warps, dtype=np.float64)
+        if w.ndim == 3 and w.shape[1:] == (2, 3):
+            w = np.broadcast_to(w[:, None], (w.shape[0], T, 2, 3))
+        elif not (w.ndim == 4 and w.shape[1:] == (T, 2, 3)):
+            raise ValueError(f"warps must be (K, 2, 3) or (K, {T}, 2, 3), got shape {w.shape}")
+        if not 1 <= w.shape[0] <= _cabi.LSD_MAX_WARPS:
+            raise ValueError(f"{w.shape[0]} warp variants: expected 1 to {_cabi.LSD_MAX_WARPS}")
+        return np.ascontiguousarray(w)
+
+    def warp_track_windows(self, track_u8: torch.Tensor, starts: Sequence[int], warps) -> torch.Tensor:
+        """The re-cropped windows `score_track_warps` scores, built by the same kernel (`lsd_warp_windows`): uint8
+        `(n, K, T, H, W, 3)` on the device, window i under variant k at [i, k].  To look at what a variant does to the crop."""
+        m = self.model
+        dev = m._device()
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T = self.chunk_size
+        w = self._warp_matrices(warps, T)
+        K, n = int(w.shape[0]), len(starts)
+        for i, s in enumerate(starts):
+            if not 0 <= int(s) <= n_frames - T:
+                raise ValueError(f"window {i} [{int(s)},{int(s) + T}) is outside the {n_frames}-frame track")
+        out = torch.empty((n, K, T, H, W, 3), dtype=torch.uint8, device=dev)
+        if n == 0:
+            return out
+        track_u8 = track_u8.contiguous()
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            need = L.lsd_warp_windows_workspace_bytes(n, K, T, H, W)
+            ws = torch.empty(max(int(need), 1), dtype=torch.uint8, device=dev)
+            warps_c = (_cabi.LsdWarp * (K * T)).from_buffer_copy(w.tobytes())
+            rc = L.lsd_warp_windows(h.ptr, track_u8.data_ptr(), n_frames, H, W, (C.c_int32 * n)(*[int(s) for s in starts]), n, T, warps_c,
+                                    K, out.data_ptr(), ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return out
+
+    @staticmethod
+    def flip_warp(W: int) -> np.ndarray:
+        """Horizontal mirror of a W-pixel-wide crop: x -> W-1-x (cv2.flip(frame, 1) as a warp)."""
+        return np.array([[-1.0, 0.0, float(W) - 1.0], [0.0, 1.0, 0.0]])
+
+    @staticmethod
+    def shift_scale_rotate_warp(H: int, W: int, dx: float = 0.0, dy: float = 0.0, scale: float = 1.0, angle_deg: float = 0.0) -> np.ndarray:
+        """`cv2.getRotationMatrix2D(((W-1)/2, (H-1)/2), angle_deg, scale)` followed by a shift of (dx, dy) pixels: the crop scaled
+        by `scale` and turned by `angle_deg` (counter-clockwise, as cv2) about its centre, then moved."""
+        a = float(angle_deg) * (np.pi / 180.0)
+        alpha, beta = np.cos(a) * float(scale), np.sin(a) * float(scale)
+        cx, cy = (float(W) - 1.0) / 2.0, (float(H) - 1.0) / 2.0
+        return np.array([[alpha, beta, (1.0 - alpha) * cx - beta * cy + float(dx)],
+                         [-beta, alpha, beta * cx + (1.0 - alpha) * cy + float(dy)]])
+
+    @staticmethod
+    def jitter_warps(T: int, H: int, W: int, sigma_px: float = 1.5, sigma_scale: float = 0.02, seed: int = 0) -> np.ndarray:
+        """(T, 2, 3) per-frame re-crops that model a face tracker's jitter: frame t shifted by (dx_t, dy_t) ~ N(0, sigma_px) and
+        scaled about the centre by 1 + s_t, s_t ~ N(0, sigma_scale), all independent (numpy generator seeded with `seed`)."""
+        g = np.random.default_rng(int(seed))
+        d = g.normal(0.0, float(sigma_px), size=(int(T), 2))
+        s = 1.0 + g.normal(0.0, float(sigma_scale), size=int(T))
+        return np.stack([Predictor.shift_scale_rotate_warp(H, W, d[t, 0], d[t, 1], s[t]) for t in range(int(T))])
+
+    @staticmethod
+    def robustness_variants(T: int, H: int, W: int) -> Tuple[List[str], np.ndarray]:
+        """The K = 12 re-crops of `robustness_track`: names and `(K, T, 2, 3)` matrices.  The identity; a horizontal flip; shifts of
+        +-4 px in x and in y; scales 0.92 and 1.08; rotations of +-6 degrees; two per-frame tracker jitters (`jitter_warps`,
+        sigma 1.5 px and 2 % scale, seeds 0 and 1)."""
+        ssr = Predictor.shift_scale_rotate_warp
+        fixed = [("identity", ssr(H, W)), ("flip", Predictor.flip_warp(W)),
+                 ("shift_x+4", ssr(H, W, dx=4)), ("shift_x-4", ssr(H, W, dx=-4)),
+                 ("shift_y+4", ssr(H, W, dy=4)), ("shift_y-4", ssr(H, W, dy=-4)),
+                 ("scale_0.92", ssr(H, W, scale=0.92)), ("scale_1.08", ssr(H, W, scale=1.08)),
+                 ("rotate+6", ssr(H, W, angle_deg=6)), ("rotate-6", ssr(H, W, angle_deg=-6))]
+        mats = [np.broadcast_to(M, (int(T), 2, 3)) for _, M in fixed]
+        mats += [Predictor.jitter_warps(T, H, W, 1.5, 0.02, seed) for seed in (0, 1)]
+        return [name for name, _ in fixed] + ["jitter_0", "jitter_1"], np.stack(mats)
+
+    def robustness_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                         confidence_threshold: float = 0.5, audio_starts_from: Optional[Sequence[int]] = None) -> Dict[str, Any]:
+        """Crop-jitter robustness of a track's verdict: one `score_track_warps` call with the K = 12 `robustness_variants`, the
+        calibrated P(real) summarised by `aggregate.augmentation_stability`:
+          `variants`: the variant names (column order);
+          `confidence`: the robust aggregate of the identity column (the plain windows' score);
+          `variant_confidence` (K,): the same aggregate per variant;
+          `tta_confidence`: the aggregate over windows of the mean P(real) over the variants (flip / shift test-time augmentation);
+          `window_spread` (n,): per window, the largest minus the smallest P(real) over the variants;
+          `decision_flip_rate`: the fraction of (window, variant) entries whose decision differs from the identity's;
+          `verdict_stable`: every variant confidence lies on the identity's side of `confidence_threshold`;
+          `window_starts`: the windows' first frames (those of `audio_starts_from` when given: absolute video frames).
+        It reports only: nothing here enters a verdict."""
+        T = self.chunk_size
+        H, W = int(track_u8.shape[1]), int(track_u8.shape[2])
+        names, mats = self.robustness_variants(T, H, W)
+        logits = self.score_track_warps(track_u8, starts, mel_full, total_v_frames, mats, audio_starts_from=audio_starts_from)
+        probs = np.array([self._calibrate(float(x)) for x in logits.cpu().flatten().tolist()], dtype=np.float64).reshape(len(starts), len(names))
+        res = _agg.augmentation_stability(probs, confidence_threshold, self.confidence_smoothing, self.trim_ratio)
+        res["variants"] = names
+        res["window_starts"] = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
+        return res
+
     def score_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int):
         logits = self.score_track_logits(track_u8, starts, mel_full, total_v_frames)
         confs = [self._calibrate(float(x)) for x in logits.cpu().tolist()]
