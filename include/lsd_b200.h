@@ -238,6 +238,48 @@ int lsd_warp_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, i
                      const int32_t* starts_host, int n_windows, int T, const lsd_warp* warps, int K,
                      uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- compression robustness: window scores of JPEG round-tripped windows ----------------------------------- */
+/* This entry has no reference counterpart.  A clip that passes through a messaging app or a platform upload is recompressed, and
+ * artifact-based detectors are known to lose their signal under compression; it asks whether a window's score would hold had
+ * every frame been recompressed.  Every window is scored K times, once per variant.  Variant k passes every frame of the window
+ * through one baseline JPEG encode and decode at its quality and chroma sampling (4:2:0 is cv2's default):
+ *   BGR track: out[t] = cv2.imdecode(cv2.imencode('.jpg', win[t], [IMWRITE_JPEG_QUALITY, quality (, IMWRITE_JPEG_SAMPLING_FACTOR,
+ *              IMWRITE_JPEG_SAMPLING_FACTOR_444)]), IMREAD_COLOR)
+ *   RGB track: the same between cv2.cvtColor(.., RGB2BGR) and cv2.cvtColor(.., BGR2RGB)
+ * bit for bit (OpenCV's libjpeg-turbo, JDCT_ISLOW: integer colour conversion, downsampling, DCT, quantisation with the IJG
+ * tables scaled by quality, inverse DCT, fancy upsampling).  The colour transform is not symmetric in R and B, so the result
+ * depends on the track's channel order, given as channel_order.  LSD_JPEG_NONE copies the frame: the uncompressed column. */
+typedef struct { int32_t quality, sampling; } lsd_jpeg;
+#define LSD_JPEG_NONE 0
+#define LSD_JPEG_444 1
+#define LSD_JPEG_420 2
+#define LSD_MAX_JPEG_VARIANTS 64
+#define LSD_RGB 0
+#define LSD_BGR 1
+/* variants: host, K entries.  Rows are (window, variant) pairs in window-major order, row r = i*K + k; `batch` counts rows.  A
+ * row's audio slice is its window's slice, with the base-start rule of lsd_score_windows (computed, or audio_starts_host_or_null[i],
+ * clamped).  The round-tripped windows of a batch are built on the device and scored by the plain batch path of lsd_score_windows,
+ * so logits_out (device, (n_windows, K) fp32) entry (i, k) is bit for bit lsd_score_windows on window i round-tripped on the host,
+ * with the same audio start.  A workspace of at least twice lsd_score_jpeg_workspace_bytes enables the cross-batch pipelining of
+ * lsd_score_windows; a short last batch runs in exactly the queried size.  Everything is checked before any GPU work:
+ * LSD_ERR_SHAPE for K outside 1..LSD_MAX_JPEG_VARIANTS, a window outside the track, H or W not a multiple of 16 when a variant
+ * samples 4:2:0 or of 8 when one samples 4:4:4 (partial MCUs are not covered), or a frame whose planes do not fit in shared memory
+ * (H*W above 34 304 with 4:2:0 only, 17 216 with 4:4:4); LSD_ERR_ARG for variants == NULL, a sampling other than the three
+ * above, a quality outside 1..100 (not checked, and not used, for LSD_JPEG_NONE) or a channel_order other than LSD_RGB / LSD_BGR. */
+size_t lsd_score_jpeg_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision);
+int lsd_score_jpeg(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                   const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                   const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                   const lsd_jpeg* variants, int K, int channel_order, int precision, int batch,
+                   float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
+/* The round-tripped windows themselves, built by the same kernel lsd_score_jpeg scores: out (device uint8, (n_windows, K, T, H, W, 3))
+ * holds window i under variant k at [i][k].  Same checks as lsd_score_jpeg; workspace: lsd_jpeg_windows_workspace_bytes (the
+ * quantisation tables and the window starts). */
+size_t lsd_jpeg_windows_workspace_bytes(int n_windows, int K, int T, int H, int W);
+int lsd_jpeg_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                     const int32_t* starts_host, int n_windows, int T, const lsd_jpeg* variants, int K, int channel_order,
+                     uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- audio occlusion evidence: window scores with a region of the window's log-mel masked ------------------ */
 /* This entry has no reference counterpart.  Window i's audio slice is the (F, Ta) log-mel window of Predictor._align_audio_chunk
  * (predictor.py:525-552) that lsd_score_windows gives it: first column the base start a_i (computed, or

@@ -22,6 +22,9 @@ LSD_MAX_AUDIO_VARIANTS = 64
 LSD_MAX_OCCLUSIONS = 1024
 LSD_MAX_AUDIO_OCCLUSIONS = LSD_MAX_AUDIO_VARIANTS
 LSD_MAX_WARPS = 64
+LSD_JPEG_NONE, LSD_JPEG_444, LSD_JPEG_420 = 0, 1, 2
+LSD_MAX_JPEG_VARIANTS = 64
+LSD_RGB, LSD_BGR = 0, 1
 
 # every symbol include/lsd_b200.h declares (checked by tests/test_cabi.py)
 EXPORTS = [
@@ -36,6 +39,7 @@ EXPORTS = [
     "lsd_score_occlusions_workspace_bytes", "lsd_score_occlusions",
     "lsd_score_audio_occlusions_workspace_bytes", "lsd_score_audio_occlusions",
     "lsd_score_warps_workspace_bytes", "lsd_score_warps", "lsd_warp_windows_workspace_bytes", "lsd_warp_windows",
+    "lsd_score_jpeg_workspace_bytes", "lsd_score_jpeg", "lsd_jpeg_windows_workspace_bytes", "lsd_jpeg_windows",
 ]
 
 
@@ -59,6 +63,11 @@ class LsdWarp(C.Structure):
     """One re-crop: cv2's forward 2x3 affine matrix (src -> dst), row-major, as `cv2.warpAffine` and `cv2.getRotationMatrix2D`
     use it."""
     _fields_ = [("m", C.c_double * 6)]
+
+
+class LsdJpeg(C.Structure):
+    """One recompression: baseline JPEG quality 1..100 and chroma sampling (LSD_JPEG_420 / LSD_JPEG_444; LSD_JPEG_NONE copies)."""
+    _fields_ = [("quality", C.c_int32), ("sampling", C.c_int32)]
 
 
 class LsdAux(C.Structure):
@@ -142,6 +151,13 @@ def lib() -> C.CDLL:
         L.lsd_warp_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_warp_windows_workspace_bytes.restype = sz
         L.lsd_warp_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdWarp), i, vp, vp, sz, vp]
         L.lsd_warp_windows.restype = i
+        L.lsd_score_jpeg_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_jpeg_workspace_bytes.restype = sz
+        L.lsd_score_jpeg.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
+                                     C.POINTER(LsdJpeg), i, i, i, i, vp, vp, sz, vp]
+        L.lsd_score_jpeg.restype = i
+        L.lsd_jpeg_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_jpeg_windows_workspace_bytes.restype = sz
+        L.lsd_jpeg_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdJpeg), i, i, vp, vp, sz, vp]
+        L.lsd_jpeg_windows.restype = i
         _lib = L
         return L
 

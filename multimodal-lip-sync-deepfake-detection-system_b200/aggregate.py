@@ -123,6 +123,27 @@ def augmentation_stability(probs, confidence_threshold: float = 0.5, smoothing: 
     }
 
 
+def lowest_stable_quality(qualities: Sequence[Optional[int]], variant_confidence: Sequence[float], confidence: float,
+                          threshold: float = 0.5) -> Optional[int]:
+    """The lowest JPEG quality q such that every variant of quality >= q has its confidence on the same side of `threshold` as
+    `confidence` (the plain window's; real when >= threshold).  Variants whose quality is None (uncompressed) are ignored.  None
+    when the highest quality already lands on the other side, or when no variant has a quality.  A flip at some quality hides
+    every lower quality, also those that land on the plain side again."""
+    if len(qualities) != len(variant_confidence):
+        raise ValueError(f"{len(qualities)} qualities for {len(variant_confidence)} variant confidences")
+    side = float(confidence) >= float(threshold)
+    by_q: Dict[int, bool] = {}
+    for q, c in zip(qualities, variant_confidence):
+        if q is not None:
+            by_q[int(q)] = by_q.get(int(q), True) and ((float(c) >= float(threshold)) == side)
+    lowest = None
+    for q in sorted(by_q, reverse=True):
+        if not by_q[q]:
+            break
+        lowest = q
+    return lowest
+
+
 def _speech_weighted(conf: Sequence[float], speaking: Sequence[float], vad: Optional[Sequence[float]], smoothing: str,
                      trim_ratio: float) -> float:
     # predictor.py:262-293

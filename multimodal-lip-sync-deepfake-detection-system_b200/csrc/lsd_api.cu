@@ -88,6 +88,7 @@ extern "C" int lsd_create(lsd_handle** out, int device) {
     if (ce == cudaSuccess) ce = lsd::stem_ring_device_init();
     if (ce == cudaSuccess) ce = lsd::tok_front_device_init();
     if (ce == cudaSuccess) ce = lsd::warp_windows_device_init();
+    if (ce == cudaSuccess) ce = lsd::jpeg_windows_device_init();
     if (ce != cudaSuccess) rc = lsd_fail(h, LSD_ERR_CUDA, "lsd_create: kernel attribute setup: %s", cudaGetErrorString(ce));
   }
   if (rc != 0) { g_create_error = h->err; delete h; return rc; }
@@ -475,11 +476,11 @@ extern "C" size_t lsd_score_workspace_bytes(lsd_handle* h, int batch, int T, int
 }
 
 namespace {
-// Returns the track a batch of rows [r0, r0+nb) reads, after enqueueing on `st` whatever builds it (lsd_score_occlusions: its
-// occluded pseudo-track).  Empty: every batch reads the caller's track.
+// Returns the track a batch of rows [r0, r0+nb) reads, after enqueueing on `st` whatever builds it (score_window_variants: the
+// batch's pseudo-track).  Empty: every batch reads the caller's track.
 using BatchTrack = std::function<int(int r0, int nb, const uint8_t*& track, int& n_frames)>;
 
-// The batch loop of lsd_score_windows, shared with lsd_score_occlusions.  h->idx_host holds the first track frame of row r at [r]
+// The batch loop of lsd_score_windows, shared with score_window_variants.  h->idx_host holds the first track frame of row r at [r]
 // and its first mel column at [n_rows + r]; the caller has checked every argument and the workspace size.
 int score_rows(lsd_handle* h, const uint8_t* track, int n_frames, int n_rows, int T, int H, int W, const float* mel_full, int F,
                int Ta_full, int Ta, int precision, int batch, float* logits_out, void* workspace, size_t workspace_bytes,
@@ -568,23 +569,105 @@ extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_fram
 }
 
 // ================================================================================================
-// Occlusion evidence: K occluded copies of every window (occlusion.cu), scored by the batch loop of lsd_score_windows
+// Window variants: K device-built copies of every window (occlusion.cu, warp.cu, jpeg.cu), scored by the batch loop of
+// lsd_score_windows
 // ================================================================================================
-// Workspace: [boxes (LSD_MAX_OCCLUSIONS x 7 int32) | track starts of one batch's windows | pseudo-track of `batch` occluded
-// windows | lsd_score_windows workspace].  The pseudo-track is read only by the batch's first kernel on the caller's stream
-// (the tensor-core pixel rows or the fp32 gather), so one copy serves pipelined batches too.
+// Workspace: [variant tables | track starts of one batch's windows | pseudo-track of `batch` built windows | lsd_score_windows
+// workspace].  The pseudo-track is read only by the batch's first kernel on the caller's stream (the tensor-core pixel rows or the
+// fp32 gather), so one copy serves pipelined batches too.
 namespace {
-size_t occlusion_extra_bytes(int batch, int T, int H, int W) {
-  return align256((size_t)LSD_MAX_OCCLUSIONS * 7 * sizeof(int32_t)) + align256(((size_t)batch + 1) * sizeof(int32_t)) +
-         align256((size_t)batch * T * H * W * 3);
+size_t variant_extra_bytes(size_t table_bytes, int batch, int T, int H, int W) {
+  return align256(table_bytes) + align256(((size_t)batch + 1) * sizeof(int32_t)) + align256((size_t)batch * T * H * W * 3);
 }
-}  // namespace
 
-extern "C" size_t lsd_score_occlusions_workspace_bytes(lsd_handle* h, int batch, int T, int H, int W, int F, int Ta, int precision) {
-  if (batch < 1) return 0;
+size_t variant_workspace_bytes(lsd_handle* h, size_t table_bytes, int batch, int T, int H, int W, int F, int Ta, int precision) {
   const size_t sw = lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
   if (sw == 0) return 0;
-  return occlusion_extra_bytes(batch, T, H, W) + align256(sw);
+  return variant_extra_bytes(table_bytes, batch, T, H, W) + align256(sw);
+}
+
+// Enqueues on `st` the kernel that writes rows r0 .. r0+nb-1 (window r / K, variant r % K) into `pseudo`; d_tabs: the variant
+// tables, d_wins: the track starts of windows r0 / K, r0 / K + 1, ...
+using VariantBuilder = std::function<void(const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* pseudo, cudaStream_t st)>;
+
+// The common part of lsd_score_occlusions / lsd_score_warps / lsd_score_jpeg, after each has checked its variants: the remaining
+// argument checks, the row table (row r reads frames (r % batch) * T .. of the batch's pseudo-track and the audio slice of window
+// r / K), one copy of the K variants' tables (`table_bytes` of them, from tables_host; their region is table_region bytes) and the
+// per-batch hook that copies the batch's window starts and runs `build`.  `what` names the variants in messages.
+int score_window_variants(lsd_handle* h, const char* fn, const char* what, const uint8_t* track, int n_frames, int H, int W,
+                          const int32_t* starts_host, const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F,
+                          int Ta_full, int total_v_frames, int Ta, int K, int precision, int batch, float* logits_out, void* workspace,
+                          size_t workspace_bytes, void* stream, const void* tables_host, size_t table_bytes, size_t table_region,
+                          const VariantBuilder& build) {
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "%s: null pointer argument", fn);
+  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "%s: bad extents", fn);
+  if ((int64_t)n_windows * K > INT32_MAX) return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d %s: too many rows for one call", n_windows, K, what);
+  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
+  Shapes s;
+  int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
+  if (rc) return rc;
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = variant_workspace_bytes(h, table_region, batch, T, H, W, F, Ta, precision);
+  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const int n_rows = n_windows * K;
+  h->idx_host.resize((size_t)2 * n_rows);
+  for (int i = 0; i < n_windows; ++i) {
+    const int32_t a = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
+    for (int k = 0; k < K; ++k) {
+      const int r = i * K + k;
+      h->idx_host[r] = (r % batch) * T;
+      h->idx_host[n_rows + r] = a;
+    }
+  }
+  char* ws = reinterpret_cast<char*>(workspace);
+  int32_t* d_tabs = reinterpret_cast<int32_t*>(ws);
+  int32_t* d_wins = reinterpret_cast<int32_t*>(ws + align256(table_region));
+  uint8_t* pseudo = reinterpret_cast<uint8_t*>(d_wins) + align256(((size_t)batch + 1) * sizeof(int32_t));
+  const size_t extra = variant_extra_bytes(table_region, batch, T, H, W);
+  CUDA_OK(h, cudaMemcpyAsync(d_tabs, tables_host, table_bytes, cudaMemcpyHostToDevice, st));
+  const BatchTrack built = [&](int r0, int nb, const uint8_t*& trk, int& nf) -> int {
+    const int wa = r0 / K, wb = (r0 + nb - 1) / K;
+    CUDA_OK(h, cudaMemcpyAsync(d_wins, starts_host + wa, (size_t)(wb - wa + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    build(d_tabs, d_wins, r0, nb, pseudo, st);
+    trk = pseudo;
+    nf = nb * T;
+    return 0;
+  };
+  return score_rows(h, pseudo, batch * T, n_rows, T, H, W, mel_full, F, Ta_full, Ta, precision, batch, logits_out, ws + extra,
+                    workspace_bytes - extra, st, built);
+}
+
+// The variant tables and the window starts of the entries that return the built windows themselves (lsd_warp_windows,
+// lsd_jpeg_windows): one launch over all n_windows x K rows into the caller's buffer.
+int build_window_variants(lsd_handle* h, const int32_t* starts_host, int n_windows, int K, void* workspace, void* stream,
+                          const void* tables_host, size_t table_bytes, uint8_t* out, const VariantBuilder& build) {
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  int32_t* d_tabs = reinterpret_cast<int32_t*>(workspace);
+  int32_t* d_wins = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(workspace) + align256(table_bytes));
+  CUDA_OK(h, cudaMemcpyAsync(d_tabs, tables_host, table_bytes, cudaMemcpyHostToDevice, st));
+  CUDA_OK(h, cudaMemcpyAsync(d_wins, starts_host, (size_t)n_windows * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  build(d_tabs, d_wins, 0, n_windows * K, out, st);
+  CUDA_OK(h, cudaGetLastError());
+  return LSD_OK;
+}
+
+size_t built_windows_workspace_bytes(size_t table_bytes, int n_windows) {
+  return align256(table_bytes) + align256((size_t)n_windows * sizeof(int32_t));
+}
+
+constexpr size_t OCCLUSION_TABLE_BYTES = (size_t)LSD_MAX_OCCLUSIONS * 7 * sizeof(int32_t);
+}  // namespace
+
+// ------------------------------------------------------------------------------------------------
+// Occlusion evidence: K occluded copies of every window (occlusion.cu)
+// ------------------------------------------------------------------------------------------------
+extern "C" size_t lsd_score_occlusions_workspace_bytes(lsd_handle* h, int batch, int T, int H, int W, int F, int Ta, int precision) {
+  if (batch < 1) return 0;
+  return variant_workspace_bytes(h, OCCLUSION_TABLE_BYTES, batch, T, H, W, F, Ta, precision);
 }
 
 extern "C" int lsd_score_occlusions(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
@@ -603,71 +686,29 @@ extern "C" int lsd_score_occlusions(lsd_handle* h, const uint8_t* track, int n_f
                       b.x0, b.x1, T, H, W);
     if (b.src < -1 || b.src >= T) return lsd_fail(h, LSD_ERR_SHAPE, "box %d: src %d is outside -1..%d", k, b.src, T - 1);
   }
-  if (n_windows == 0) return LSD_OK;
-  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_occlusions: null pointer argument");
-  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_occlusions: bad extents");
-  if ((int64_t)n_windows * K > INT32_MAX) return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d boxes: too many rows for one call", n_windows, K);
-  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
-  Shapes s;
-  int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
-  if (rc) return rc;
-  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
-  const size_t need = lsd_score_occlusions_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
-  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-  ENTER_DEVICE(h);
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int n_rows = n_windows * K;
-  // row r reads frames (r % batch) * T .. of the batch's pseudo-track, and the audio slice of window r / K
-  h->idx_host.resize((size_t)2 * n_rows);
-  for (int i = 0; i < n_windows; ++i) {
-    const int32_t a = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
-    for (int k = 0; k < K; ++k) {
-      const int r = i * K + k;
-      h->idx_host[r] = (r % batch) * T;
-      h->idx_host[n_rows + r] = a;
-    }
-  }
-  char* ws = reinterpret_cast<char*>(workspace);
-  int32_t* d_boxes = reinterpret_cast<int32_t*>(ws);
-  int32_t* d_wins = reinterpret_cast<int32_t*>(ws + align256((size_t)LSD_MAX_OCCLUSIONS * 7 * sizeof(int32_t)));
-  uint8_t* pseudo = reinterpret_cast<uint8_t*>(d_wins) + align256(((size_t)batch + 1) * sizeof(int32_t));
-  const size_t extra = occlusion_extra_bytes(batch, T, H, W);
   static_assert(sizeof(lsd_occlusion) == 7 * sizeof(int32_t), "lsd_occlusion is seven packed int32");
-  CUDA_OK(h, cudaMemcpyAsync(d_boxes, boxes, (size_t)K * sizeof(lsd_occlusion), cudaMemcpyHostToDevice, st));
-  const BatchTrack occluded = [&](int r0, int nb, const uint8_t*& trk, int& nf) -> int {
-    const int wa = r0 / K, wb = (r0 + nb - 1) / K;
-    CUDA_OK(h, cudaMemcpyAsync(d_wins, starts_host + wa, (size_t)(wb - wa + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  const VariantBuilder occlude = [&](const int32_t* d_boxes, const int32_t* d_wins, int r0, int nb, uint8_t* pseudo, cudaStream_t st) {
     launch_occlude_windows(track, d_wins, d_boxes, K, r0, nb, T, H, W, fill, pseudo, st);
-    trk = pseudo;
-    nf = nb * T;
-    return 0;
   };
-  return score_rows(h, pseudo, batch * T, n_rows, T, H, W, mel_full, F, Ta_full, Ta, precision, batch, logits_out, ws + extra,
-                    workspace_bytes - extra, st, occluded);
+  return score_window_variants(h, "lsd_score_occlusions", "boxes", track, n_frames, H, W, starts_host, audio_starts_host, n_windows, T,
+                               mel_full, F, Ta_full, total_v_frames, Ta, K, precision, batch, logits_out, workspace, workspace_bytes,
+                               stream, boxes, (size_t)K * sizeof(lsd_occlusion), OCCLUSION_TABLE_BYTES, occlude);
 }
 
-// ================================================================================================
-// Crop-jitter robustness: K re-cropped copies of every window (warp.cu), scored by the batch loop of lsd_score_windows
-// ================================================================================================
-// Workspace: [warp tables (K*T*2(H+W) int32) | track starts of one batch's windows | pseudo-track of `batch` warped windows |
-// lsd_score_windows workspace].  As in lsd_score_occlusions, the pseudo-track is read only by the batch's first kernel on the
-// caller's stream (the tensor-core pixel rows or the fp32 gather), so one copy serves pipelined batches too.
+// ------------------------------------------------------------------------------------------------
+// Crop-jitter robustness: K re-cropped copies of every window (warp.cu); tables K*T*2(H+W) int32
+// ------------------------------------------------------------------------------------------------
 namespace {
-size_t warps_extra_bytes(int batch, int K, int T, int H, int W) {
-  return align256(warp_tables_ints(K, T, H, W) * sizeof(int32_t)) + align256(((size_t)batch + 1) * sizeof(int32_t)) +
-         align256((size_t)batch * T * H * W * 3);
-}
-
-// The checks every warp entry makes before any GPU work; on success h->warp_tab_host holds the tables of the K*T matrices.
+// The checks every warp entry makes before any GPU work; on success h->variant_tab_host holds the tables of the K*T matrices.
 int warp_tables_checked(lsd_handle* h, const char* fn, const lsd_warp* warps, int K, int T, int H, int W) {
   if (!warps) return lsd_fail(h, LSD_ERR_ARG, "%s: warps is NULL", fn);
   if (K < 1 || K > LSD_MAX_WARPS) return lsd_fail(h, LSD_ERR_SHAPE, "K = %d warp variants: expected 1 <= K <= %d", K, LSD_MAX_WARPS);
   if (T < 1 || H < 1 || W < 1 || (int64_t)H * W * 3 > INT32_MAX || !warp_extents_ok(H, W))
     return lsd_fail(h, LSD_ERR_SHAPE, "%s: bad window extents T=%d H=%d W=%d", fn, T, H, W);
   static_assert(sizeof(lsd_warp) == 6 * sizeof(double), "lsd_warp is six packed doubles");
-  h->warp_tab_host.resize(warp_tables_ints(K, T, H, W));
+  h->variant_tab_host.resize(warp_tables_ints(K, T, H, W));
   int bad = 0;
-  const int rc = warp_tables(reinterpret_cast<const double*>(warps), K * T, H, W, h->warp_tab_host.data(), &bad);
+  const int rc = warp_tables(reinterpret_cast<const double*>(warps), K * T, H, W, h->variant_tab_host.data(), &bad);
   if (rc == -1)
     return lsd_fail(h, LSD_ERR_ARG, "warp %d (variant %d, frame %d) has a non-finite entry or is singular", bad, bad / T, bad % T);
   if (rc == -2)
@@ -678,9 +719,7 @@ int warp_tables_checked(lsd_handle* h, const char* fn, const lsd_warp* warps, in
 
 extern "C" size_t lsd_score_warps_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
   if (batch < 1 || K < 1 || K > LSD_MAX_WARPS) return 0;
-  const size_t sw = lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
-  if (sw == 0) return 0;
-  return warps_extra_bytes(batch, K, T, H, W) + align256(sw);
+  return variant_workspace_bytes(h, warp_tables_ints(K, T, H, W) * sizeof(int32_t), batch, T, H, W, F, Ta, precision);
 }
 
 extern "C" int lsd_score_warps(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
@@ -689,53 +728,21 @@ extern "C" int lsd_score_warps(lsd_handle* h, const uint8_t* track, int n_frames
                                void* workspace, size_t workspace_bytes, void* stream) {
   if (!h) return LSD_ERR_ARG;
   if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_warps: no weights loaded");
-  int rc = warp_tables_checked(h, "lsd_score_warps", warps, K, T, H, W);
+  const int rc = warp_tables_checked(h, "lsd_score_warps", warps, K, T, H, W);
   if (rc) return rc;
-  if (n_windows == 0) return LSD_OK;
-  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_warps: null pointer argument");
-  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_warps: bad extents");
-  if ((int64_t)n_windows * K > INT32_MAX) return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d warps: too many rows for one call", n_windows, K);
-  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
-  Shapes s;
-  if ((rc = make_shapes(h, batch, T, H, W, F, Ta, s))) return rc;
-  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
-  const size_t need = lsd_score_warps_workspace_bytes(h, batch, K, T, H, W, F, Ta, precision);
-  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-  ENTER_DEVICE(h);
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int n_rows = n_windows * K;
-  // row r reads frames (r % batch) * T .. of the batch's pseudo-track, and the audio slice of window r / K
-  h->idx_host.resize((size_t)2 * n_rows);
-  for (int i = 0; i < n_windows; ++i) {
-    const int32_t a = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
-    for (int k = 0; k < K; ++k) {
-      const int r = i * K + k;
-      h->idx_host[r] = (r % batch) * T;
-      h->idx_host[n_rows + r] = a;
-    }
-  }
-  char* ws = reinterpret_cast<char*>(workspace);
-  int32_t* d_tabs = reinterpret_cast<int32_t*>(ws);
-  int32_t* d_wins = reinterpret_cast<int32_t*>(ws + align256(h->warp_tab_host.size() * sizeof(int32_t)));
-  uint8_t* pseudo = reinterpret_cast<uint8_t*>(d_wins) + align256(((size_t)batch + 1) * sizeof(int32_t));
-  const size_t extra = warps_extra_bytes(batch, K, T, H, W);
-  CUDA_OK(h, cudaMemcpyAsync(d_tabs, h->warp_tab_host.data(), h->warp_tab_host.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  const BatchTrack warped = [&](int r0, int nb, const uint8_t*& trk, int& nf) -> int {
-    const int wa = r0 / K, wb = (r0 + nb - 1) / K;
-    CUDA_OK(h, cudaMemcpyAsync(d_wins, starts_host + wa, (size_t)(wb - wa + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  const size_t tab_bytes = h->variant_tab_host.size() * sizeof(int32_t);
+  const VariantBuilder warp = [&](const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* pseudo, cudaStream_t st) {
     launch_warp_windows(track, d_wins, d_tabs, K, r0, nb, T, H, W, pseudo, st);
-    trk = pseudo;
-    nf = nb * T;
-    return 0;
   };
-  return score_rows(h, pseudo, batch * T, n_rows, T, H, W, mel_full, F, Ta_full, Ta, precision, batch, logits_out, ws + extra,
-                    workspace_bytes - extra, st, warped);
+  return score_window_variants(h, "lsd_score_warps", "warps", track, n_frames, H, W, starts_host, audio_starts_host, n_windows, T,
+                               mel_full, F, Ta_full, total_v_frames, Ta, K, precision, batch, logits_out, workspace, workspace_bytes,
+                               stream, h->variant_tab_host.data(), tab_bytes, tab_bytes, warp);
 }
 
 // The warped windows themselves, written to a caller buffer by the builder lsd_score_warps uses: what the K variants look like.
 extern "C" size_t lsd_warp_windows_workspace_bytes(int n_windows, int K, int T, int H, int W) {
   if (n_windows < 1 || K < 1 || K > LSD_MAX_WARPS || T < 1 || H < 1 || W < 1) return 0;
-  return align256(warp_tables_ints(K, T, H, W) * sizeof(int32_t)) + align256((size_t)n_windows * sizeof(int32_t));
+  return built_windows_workspace_bytes(warp_tables_ints(K, T, H, W) * sizeof(int32_t), n_windows);
 }
 
 extern "C" int lsd_warp_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host, int n_windows,
@@ -750,15 +757,93 @@ extern "C" int lsd_warp_windows(lsd_handle* h, const uint8_t* track, int n_frame
   if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
   const size_t need = lsd_warp_windows_workspace_bytes(n_windows, K, T, H, W);
   if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-  ENTER_DEVICE(h);
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  int32_t* d_tabs = reinterpret_cast<int32_t*>(workspace);
-  int32_t* d_wins = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(workspace) + align256(h->warp_tab_host.size() * sizeof(int32_t)));
-  CUDA_OK(h, cudaMemcpyAsync(d_tabs, h->warp_tab_host.data(), h->warp_tab_host.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  CUDA_OK(h, cudaMemcpyAsync(d_wins, starts_host, (size_t)n_windows * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  launch_warp_windows(track, d_wins, d_tabs, K, 0, n_windows * K, T, H, W, out, st);
-  CUDA_OK(h, cudaGetLastError());
-  return LSD_OK;
+  const VariantBuilder warp = [&](const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* o, cudaStream_t st) {
+    launch_warp_windows(track, d_wins, d_tabs, K, r0, nb, T, H, W, o, st);
+  };
+  return build_window_variants(h, starts_host, n_windows, K, workspace, stream, h->variant_tab_host.data(),
+                               h->variant_tab_host.size() * sizeof(int32_t), out, warp);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Compression robustness: K JPEG round-tripped copies of every window (jpeg.cu); tables JPEG_TAB_INTS int32 per variant
+// ------------------------------------------------------------------------------------------------
+namespace {
+// The checks every JPEG entry makes before any GPU work; on success h->variant_tab_host holds the K variants' tables and *any444
+// tells whether one samples 4:4:4.
+int jpeg_tables_checked(lsd_handle* h, const char* fn, const lsd_jpeg* v, int K, int channel_order, int T, int H, int W, bool* any444) {
+  if (!v) return lsd_fail(h, LSD_ERR_ARG, "%s: variants is NULL", fn);
+  if (K < 1 || K > LSD_MAX_JPEG_VARIANTS)
+    return lsd_fail(h, LSD_ERR_SHAPE, "K = %d JPEG variants: expected 1 <= K <= %d", K, LSD_MAX_JPEG_VARIANTS);
+  if (channel_order != LSD_RGB && channel_order != LSD_BGR) return lsd_fail(h, LSD_ERR_ARG, "%s: bad channel order %d", fn, channel_order);
+  bool any420 = false;
+  *any444 = false;
+  for (int k = 0; k < K; ++k) {
+    if (v[k].sampling != LSD_JPEG_NONE && v[k].sampling != LSD_JPEG_444 && v[k].sampling != LSD_JPEG_420)
+      return lsd_fail(h, LSD_ERR_ARG, "JPEG variant %d: bad sampling %d", k, v[k].sampling);
+    if (v[k].sampling != LSD_JPEG_NONE && (v[k].quality < 1 || v[k].quality > 100))
+      return lsd_fail(h, LSD_ERR_ARG, "JPEG variant %d: quality %d is outside 1..100", k, v[k].quality);
+    any420 |= v[k].sampling == LSD_JPEG_420;
+    *any444 |= v[k].sampling == LSD_JPEG_444;
+  }
+  const int mcu = any420 ? 16 : 8;
+  if (T < 1 || H < 1 || W < 1 || H % mcu || W % mcu || !jpeg_extents_ok(H, W, *any444))
+    return lsd_fail(h, LSD_ERR_SHAPE, "%s: bad window extents T=%d H=%d W=%d (sides multiples of %d, planes within shared memory)", fn, T,
+                    H, W, mcu);
+  static_assert(sizeof(lsd_jpeg) == 2 * sizeof(int32_t), "lsd_jpeg is two packed int32");
+  h->variant_tab_host.resize((size_t)K * JPEG_TAB_INTS);
+  jpeg_tables(reinterpret_cast<const int32_t*>(v), K, h->variant_tab_host.data());
+  return 0;
+}
+}  // namespace
+
+extern "C" size_t lsd_score_jpeg_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  if (batch < 1 || K < 1 || K > LSD_MAX_JPEG_VARIANTS) return 0;
+  return variant_workspace_bytes(h, (size_t)K * JPEG_TAB_INTS * sizeof(int32_t), batch, T, H, W, F, Ta, precision);
+}
+
+extern "C" int lsd_score_jpeg(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                              const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full,
+                              int total_v_frames, int Ta, const lsd_jpeg* variants, int K, int channel_order, int precision, int batch,
+                              float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_jpeg: no weights loaded");
+  bool any444 = false;
+  const int rc = jpeg_tables_checked(h, "lsd_score_jpeg", variants, K, channel_order, T, H, W, &any444);
+  if (rc) return rc;
+  const size_t tab_bytes = h->variant_tab_host.size() * sizeof(int32_t);
+  const VariantBuilder jpeg = [&](const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* pseudo, cudaStream_t st) {
+    launch_jpeg_windows(track, d_wins, d_tabs, K, r0, nb, T, H, W, any444, channel_order == LSD_BGR, pseudo, st);
+  };
+  return score_window_variants(h, "lsd_score_jpeg", "JPEG variants", track, n_frames, H, W, starts_host, audio_starts_host, n_windows, T,
+                               mel_full, F, Ta_full, total_v_frames, Ta, K, precision, batch, logits_out, workspace, workspace_bytes,
+                               stream, h->variant_tab_host.data(), tab_bytes, tab_bytes, jpeg);
+}
+
+// The round-tripped windows themselves, written to a caller buffer by the builder lsd_score_jpeg uses.
+extern "C" size_t lsd_jpeg_windows_workspace_bytes(int n_windows, int K, int T, int H, int W) {
+  if (n_windows < 1 || K < 1 || K > LSD_MAX_JPEG_VARIANTS || T < 1 || H < 1 || W < 1) return 0;
+  return built_windows_workspace_bytes((size_t)K * JPEG_TAB_INTS * sizeof(int32_t), n_windows);
+}
+
+extern "C" int lsd_jpeg_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host, int n_windows,
+                                int T, const lsd_jpeg* variants, int K, int channel_order, uint8_t* out, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  bool any444 = false;
+  int rc = jpeg_tables_checked(h, "lsd_jpeg_windows", variants, K, channel_order, T, H, W, &any444);
+  if (rc) return rc;
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_jpeg_windows: null pointer argument");
+  if (n_windows < 0 || n_frames < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_jpeg_windows: bad extents");
+  if ((int64_t)n_windows * K * T > INT32_MAX) return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d JPEG variants: too many frames for one call", n_windows, K);
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = lsd_jpeg_windows_workspace_bytes(n_windows, K, T, H, W);
+  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  const VariantBuilder jpeg = [&](const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* o, cudaStream_t st) {
+    launch_jpeg_windows(track, d_wins, d_tabs, K, r0, nb, T, H, W, any444, channel_order == LSD_BGR, o, st);
+  };
+  return build_window_variants(h, starts_host, n_windows, K, workspace, stream, h->variant_tab_host.data(),
+                               h->variant_tab_host.size() * sizeof(int32_t), out, jpeg);
 }
 
 // ================================================================================================

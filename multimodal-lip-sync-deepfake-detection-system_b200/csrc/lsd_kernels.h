@@ -50,6 +50,16 @@ size_t warp_tables_ints(int K, int T, int H, int W);
 int warp_tables(const double* m, int n, int H, int W, int32_t* out, int* bad);
 cudaError_t warp_windows_device_init();
 bool warp_extents_ok(int H, int W);
+// JPEG round-tripped windows (jpeg.cu): rows r0 .. r0+nb-1 = (window r / K, variant r % K) -> uint8 pseudo-track out (nb*T, H, W, 3),
+// every frame of row r as cv2.imdecode(cv2.imencode('.jpg', ...)) of variant k with its tables; win_starts: track start of windows
+// r0 / K, r0 / K + 1, ...; tabs: jpeg_tables of the K variants; any444: some variant samples 4:4:4 (shared-memory size); bgr:
+// byte 0 of a pixel is blue
+constexpr int JPEG_TAB_INTS = 264, JPEG_TAB_LUMA = 8, JPEG_TAB_CHROMA = 136;
+void launch_jpeg_windows(const uint8_t* track, const int32_t* win_starts, const int32_t* tabs, int K, int r0, int nb, int T, int H, int W,
+                         bool any444, int bgr, uint8_t* out, cudaStream_t s);
+void jpeg_tables(const int32_t* qs, int K, int32_t* out);
+cudaError_t jpeg_windows_device_init();
+bool jpeg_extents_ok(int H, int W, bool any444);
 // mel_full (F, Ta_full) + per-window a_start -> (n, F, Ta) with repeat-last-column padding (predictor.py:525-552)
 void launch_gather_audio(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, float* dst,
                          int n, int Ta, cudaStream_t s);

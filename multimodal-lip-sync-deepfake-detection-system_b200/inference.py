@@ -1010,6 +1010,134 @@ class Predictor:
         res["window_starts"] = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
         return res
 
+    # ------------------------------------------------------------------ compression robustness (lsd_score_jpeg)
+    _SAMPLING = {None: _cabi.LSD_JPEG_NONE, "444": _cabi.LSD_JPEG_444, "420": _cabi.LSD_JPEG_420}
+    _CHANNEL_ORDER = {"rgb": _cabi.LSD_RGB, "bgr": _cabi.LSD_BGR}
+
+    def _jpeg_args(self, track_u8: torch.Tensor, starts: Sequence[int], variants, channel_order: str):
+        """Checks what `lsd_score_jpeg` / `lsd_jpeg_windows` would reject, as ValueError; returns (K, variants as lsd_jpeg, order)."""
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        if channel_order not in self._CHANNEL_ORDER:
+            raise ValueError(f"channel_order must be 'rgb' or 'bgr', got {channel_order!r}")
+        vs = [tuple(v) for v in variants]
+        if not 1 <= len(vs) <= _cabi.LSD_MAX_JPEG_VARIANTS:
+            raise ValueError(f"{len(vs)} JPEG variants: expected 1 to {_cabi.LSD_MAX_JPEG_VARIANTS}")
+        for k, (q, sampling) in enumerate(vs):
+            if sampling not in self._SAMPLING:
+                raise ValueError(f"JPEG variant {k}: sampling must be '420', '444' or None, got {sampling!r}")
+            if sampling is not None and not (isinstance(q, (int, np.integer)) and 1 <= int(q) <= 100):
+                raise ValueError(f"JPEG variant {k}: quality must be an integer in 1..100, got {q!r}")
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        mcu = 16 if any(v[1] == "420" for v in vs) else 8
+        if H % mcu or W % mcu:
+            raise ValueError(f"{H}x{W} crops: JPEG sides must be multiples of {mcu} (partial MCUs are not supported)")
+        T = self.chunk_size
+        for i, s in enumerate(starts):
+            if not 0 <= int(s) <= n_frames - T:
+                raise ValueError(f"window {i} [{int(s)},{int(s) + T}) is outside the {n_frames}-frame track")
+        arr = (_cabi.LsdJpeg * len(vs))(*[_cabi.LsdJpeg(int(q) if s is not None else 0, self._SAMPLING[s]) for q, s in vs])
+        return len(vs), arr, self._CHANNEL_ORDER[channel_order]
+
+    def score_track_jpeg(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int, variants,
+                         chunk_a_size: int = 128, audio_starts_from: Optional[Sequence[int]] = None,
+                         channel_order: str = "rgb") -> torch.Tensor:
+        """`score_track_logits` with K recompressed variants per window (`lsd_score_jpeg`).  `variants`: a sequence of
+        `(quality, sampling)`, sampling `"420"` (cv2's default), `"444"` or `None` (the plain window; its quality is ignored).  Every
+        frame of variant k is one baseline JPEG encode + decode, bit for bit `cv2.imdecode(cv2.imencode('.jpg', frame,
+        [IMWRITE_JPEG_QUALITY, quality, ...]))` on the frame in `channel_order` (`"rgb"`: converted to BGR and back around the
+        round trip), built on the device.  Returns fp32 logits `(n, K)` on the device; entry (i, k) is bit for bit the logit of window
+        i recompressed by variant k, with window i's audio slice."""
+        if mel_full.dim() != 3 or mel_full.shape[0] != 1:
+            raise ValueError(f"mel_full must be (1, F, T_full), got {tuple(mel_full.shape)}")
+        K, vc, order = self._jpeg_args(track_u8, starts, variants, channel_order)
+        m = self.model
+        dev = m._device()
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T = self.chunk_size
+        n = len(starts)
+        if audio_starts_from is not None and len(audio_starts_from) != n:
+            raise ValueError("audio_starts_from must have one entry per window")
+        logits = torch.empty(n, K, dtype=torch.float32, device=dev)
+        if n == 0:
+            return logits
+        track_u8 = track_u8.contiguous()
+        mel_full = mel_full.to(torch.float32).contiguous()
+        F_, Ta_full = int(mel_full.shape[1]), int(mel_full.shape[2])
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = m._precision()
+            batch = min(self.batch_size, n * K)
+            need = L.lsd_score_jpeg_workspace_bytes(h.ptr, batch, K, T, H, W, F_, chunk_a_size, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            if n * K > batch and prec == _cabi.LSD_PREC_BF16:
+                need = 2 * need      # a double workspace lets the batches overlap as in score_track_logits
+            ws = m._workspace(need, dev)
+            st = (C.c_int32 * n)(*[int(s) for s in starts])
+            ast = None
+            if audio_starts_from is not None:
+                ast = (C.c_int32 * n)(*[self._audio_start(int(v), Ta_full, int(total_v_frames), chunk_a_size) for v in audio_starts_from])
+            rc = L.lsd_score_jpeg(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, T, mel_full.data_ptr(), F_, Ta_full,
+                                  int(total_v_frames), chunk_a_size, vc, K, order, prec, batch, logits.data_ptr(), ws.data_ptr(),
+                                  ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return logits
+
+    def jpeg_track_windows(self, track_u8: torch.Tensor, starts: Sequence[int], variants, channel_order: str = "rgb") -> torch.Tensor:
+        """The recompressed windows `score_track_jpeg` scores, built by the same kernel (`lsd_jpeg_windows`): uint8
+        `(n, K, T, H, W, 3)` on the device, window i under variant k at [i, k].  To look at what a quality does to the crop."""
+        K, vc, order = self._jpeg_args(track_u8, starts, variants, channel_order)
+        m = self.model
+        dev = m._device()
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T, n = self.chunk_size, len(starts)
+        out = torch.empty((n, K, T, H, W, 3), dtype=torch.uint8, device=dev)
+        if n == 0:
+            return out
+        track_u8 = track_u8.contiguous()
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            need = L.lsd_jpeg_windows_workspace_bytes(n, K, T, H, W)
+            ws = torch.empty(max(int(need), 1), dtype=torch.uint8, device=dev)
+            rc = L.lsd_jpeg_windows(h.ptr, track_u8.data_ptr(), n_frames, H, W, (C.c_int32 * n)(*[int(s) for s in starts]), n, T, vc, K,
+                                    order, out.data_ptr(), ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return out
+
+    @staticmethod
+    def compression_variants() -> Tuple[List[str], List[Tuple[Optional[int], Optional[str]]]]:
+        """The K = 8 recompressions of `compression_track`: names and `(quality, sampling)`.  The plain window, then 4:2:0 (cv2's
+        default sampling) at qualities 95, 85, 75, 60, 45, 30 and 15."""
+        qualities = (95, 85, 75, 60, 45, 30, 15)
+        return ["none"] + [f"q{q}" for q in qualities], [(None, None)] + [(q, "420") for q in qualities]
+
+    def compression_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                          confidence_threshold: float = 0.5, audio_starts_from: Optional[Sequence[int]] = None,
+                          channel_order: str = "rgb") -> Dict[str, Any]:
+        """Compression robustness of a track's verdict: one `score_track_jpeg` call with the K = 8 `compression_variants`, the
+        calibrated P(real) summarised by `aggregate.augmentation_stability` (column 0, the plain window, is the identity):
+          `variants`: the variant names (column order); `qualities`: their JPEG qualities (None for the plain window);
+          `confidence`, `variant_confidence`, `tta_confidence`, `window_spread`, `decision_flip_rate`, `verdict_stable`: as in
+          `robustness_track`;
+          `lowest_stable_quality`: the lowest quality q such that every variant of quality >= q keeps the plain confidence's side
+          of `confidence_threshold` (`aggregate.lowest_stable_quality`), None when the highest quality already flips it;
+          `window_starts`: the windows' first frames (those of `audio_starts_from` when given: absolute video frames).
+        It reports only: nothing here enters a verdict."""
+        names, variants = self.compression_variants()
+        logits = self.score_track_jpeg(track_u8, starts, mel_full, total_v_frames, variants, audio_starts_from=audio_starts_from,
+                                       channel_order=channel_order)
+        probs = np.array([self._calibrate(float(x)) for x in logits.cpu().flatten().tolist()], dtype=np.float64).reshape(len(starts), len(names))
+        res = _agg.augmentation_stability(probs, confidence_threshold, self.confidence_smoothing, self.trim_ratio)
+        qualities = [q for q, _ in variants]
+        res["variants"] = names
+        res["qualities"] = qualities
+        res["lowest_stable_quality"] = _agg.lowest_stable_quality(qualities, res["variant_confidence"], res["confidence"], confidence_threshold)
+        res["window_starts"] = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
+        return res
+
     def score_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int):
         logits = self.score_track_logits(track_u8, starts, mel_full, total_v_frames)
         confs = [self._calibrate(float(x)) for x in logits.cpu().tolist()]
