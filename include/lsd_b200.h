@@ -307,6 +307,55 @@ int lsd_score_audio_occlusions(lsd_handle* h, const uint8_t* track, int n_frames
                                const lsd_audio_occlusion* boxes, int K, float fill, int precision, int batch,
                                float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- audio robustness: degraded copies of the speech, and window scores against K clip log-mels ------------ */
+/* These entries have no reference counterpart.  Ordinary speech audio is noisy, reverberant, phone-band or clipped, and such audio
+ * weakens the audio-visual correspondence the model relies on; they ask whether a window's score would hold had the speech been
+ * recorded that way.  lsd_degrade_audio writes K degraded copies of one 16 kHz mono clip; the caller takes their log-mel with
+ * lsd_logmel (the front end of preprocess_audio, audio.py:80-91, which runs after the degradation) and scores every window against
+ * each with lsd_score_audio_clips.
+ * A variant is a chain of optional stages, each enabled by one bit of `stages`, always run in this order:
+ *   LSD_AD_REVERB  rt60 in [0.05, 2] s: x convolved with h, cut to n samples.  h has L = round(rt60 * 16000) taps, h[0] = 1 and
+ *                  h[j] = g_j 10^(-3 j / L) for j >= 1, the tail scaled to the direct path's energy (direct-to-reverberant 0 dB)
+ *   LSD_AD_NOISE   snr_db in [-20, 60]: x + sqrt(P_x / (P_g 10^(snr/10))) g, P = mean square over the clip (fp64); a silent clip
+ *                  passes unchanged
+ *   LSD_AD_CLIP    gain_db in [0, 40]: clamp(x * fl32(10^(gain/20)), -1, 1), a microphone or converter driven into overdrive
+ *   LSD_AD_BAND    band_rate 8000 or 4000: scipy.signal.resample_poly(x, 1, f) then resample_poly(., f, 1), cut to n, f = 16000 /
+ *                  band_rate (scipy's defaults: firwin taps, Kaiser beta 5, half length 10 f)
+ *   LSD_AD_MULAW   G.711 8-bit: int16 = clamp(rint(x * 32768), -32768, 32767), audioop.lin2ulaw then audioop.ulaw2lin, / 32768
+ * g and g_j are white Gaussian draws of a counter-based generator: draw i of stream s (0 noise, 1 impulse response) takes
+ * r = splitmix64(splitmix64(seed << 32 | s) + i), u1 = ((r >> 40) + 1) 2^-24, u2 = ((r >> 16) & 0xFFFFFF) 2^-24 and gives
+ * sqrt(-2 ln u1) cos(2 pi u2) in double (oracle/audio_degrade_oracle.py restates every stage).  A variant with stages == 0 copies
+ * the clip.  Parameters of stages a variant does not enable are ignored. */
+typedef struct { int32_t stages; float rt60, snr_db, gain_db; int32_t band_rate; uint32_t seed; } lsd_audio_degradation;
+#define LSD_AD_REVERB 1
+#define LSD_AD_NOISE 2
+#define LSD_AD_CLIP 4
+#define LSD_AD_BAND 8
+#define LSD_AD_MULAW 16
+#define LSD_MAX_AUDIO_DEGRADATIONS LSD_MAX_AUDIO_VARIANTS
+/* pcm: device fp32 (n); variants: host, K entries; out: device fp32 (K, n), variant k at row k.  Workspace:
+ * lsd_degrade_audio_workspace_bytes(n, K) (the variant table, the impulse responses, the noise sums and the band stage's
+ * intermediate).  Everything is checked before any GPU work: LSD_ERR_SHAPE for K outside 1..LSD_MAX_AUDIO_DEGRADATIONS or n < 1;
+ * LSD_ERR_ARG for a null pointer, unknown stage bits, a non-finite or out-of-range parameter of an enabled stage or a band_rate
+ * other than 8000 / 4000; LSD_ERR_WORKSPACE for a workspace below the queried size. */
+size_t lsd_degrade_audio_workspace_bytes(int64_t n, int K);
+int lsd_degrade_audio(lsd_handle* h, const float* pcm, int64_t n, const lsd_audio_degradation* variants, int K,
+                      float* out, void* workspace, size_t workspace_bytes, void* stream);
+/* Window i scored against K clip log-mels: row (i, k) is window i's video with the (F, Ta) slice of mels[k] (device fp32,
+ * (K, F, Ta_full)) that lsd_score_windows gives window i on mels[k] alone: first column the base start a_i (computed, or
+ * audio_starts_host_or_null[i], clamped as there), the clip's last column repeated past its end.  Rows are (window, clip) pairs in
+ * window-major order; `batch` counts windows, as in lsd_score_audio_occlusions.  The slices of a batch are written on the device,
+ * end to end, into a pseudo clip in the workspace and scored as there: the tensor-core route with the fused token kernels runs the
+ * visual encoder and the artifact branch once per window, every other configuration runs lsd_score_windows with each window
+ * repeated K times.  logits_out: device (n_windows, K) fp32, entry (i, k) bit for bit lsd_score_windows on mels[k].  The mels may
+ * come from anywhere, e.g. lsd_degrade_audio + lsd_logmel, or a lossy codec run on the host.  Everything is checked before any GPU
+ * work: LSD_ERR_SHAPE for K outside 1..LSD_MAX_AUDIO_DEGRADATIONS or a window outside the track; LSD_ERR_ARG for a null pointer. */
+size_t lsd_score_audio_clips_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision);
+int lsd_score_audio_clips(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                          const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                          const float* mels, int F, int Ta_full, int total_v_frames, int Ta, int K, int precision, int batch,
+                          float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- speaking alignment / mouth motion: the per-window numpy loops of _predict_long_video ------------------ */
 /* Frame-difference energies of a track (Predictor._speaking_alignment_score, app/inference/predictor.py:339-345, and
  * _mouth_motion_energy_check, :395-402): for every frame pair f in [0, n_frames-1)

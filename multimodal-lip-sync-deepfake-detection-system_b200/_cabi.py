@@ -25,6 +25,8 @@ LSD_MAX_WARPS = 64
 LSD_JPEG_NONE, LSD_JPEG_444, LSD_JPEG_420 = 0, 1, 2
 LSD_MAX_JPEG_VARIANTS = 64
 LSD_RGB, LSD_BGR = 0, 1
+LSD_AD_REVERB, LSD_AD_NOISE, LSD_AD_CLIP, LSD_AD_BAND, LSD_AD_MULAW = 1, 2, 4, 8, 16
+LSD_MAX_AUDIO_DEGRADATIONS = LSD_MAX_AUDIO_VARIANTS
 
 # every symbol include/lsd_b200.h declares (checked by tests/test_cabi.py)
 EXPORTS = [
@@ -40,6 +42,7 @@ EXPORTS = [
     "lsd_score_audio_occlusions_workspace_bytes", "lsd_score_audio_occlusions",
     "lsd_score_warps_workspace_bytes", "lsd_score_warps", "lsd_warp_windows_workspace_bytes", "lsd_warp_windows",
     "lsd_score_jpeg_workspace_bytes", "lsd_score_jpeg", "lsd_jpeg_windows_workspace_bytes", "lsd_jpeg_windows",
+    "lsd_degrade_audio_workspace_bytes", "lsd_degrade_audio", "lsd_score_audio_clips_workspace_bytes", "lsd_score_audio_clips",
 ]
 
 
@@ -68,6 +71,13 @@ class LsdWarp(C.Structure):
 class LsdJpeg(C.Structure):
     """One recompression: baseline JPEG quality 1..100 and chroma sampling (LSD_JPEG_420 / LSD_JPEG_444; LSD_JPEG_NONE copies)."""
     _fields_ = [("quality", C.c_int32), ("sampling", C.c_int32)]
+
+
+class LsdAudioDegradation(C.Structure):
+    """One audio degradation: the `stages` bits (LSD_AD_*) and the parameters of the stages they enable: reverb time rt60 (s), noise
+    SNR (dB), overdrive gain (dB), band rate (8000 or 4000 Hz) and the generator's seed."""
+    _fields_ = [("stages", C.c_int32), ("rt60", C.c_float), ("snr_db", C.c_float), ("gain_db", C.c_float), ("band_rate", C.c_int32),
+                ("seed", C.c_uint32)]
 
 
 class LsdAux(C.Structure):
@@ -158,6 +168,12 @@ def lib() -> C.CDLL:
         L.lsd_jpeg_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_jpeg_windows_workspace_bytes.restype = sz
         L.lsd_jpeg_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdJpeg), i, i, vp, vp, sz, vp]
         L.lsd_jpeg_windows.restype = i
+        L.lsd_degrade_audio_workspace_bytes.argtypes = [i64, i]; L.lsd_degrade_audio_workspace_bytes.restype = sz
+        L.lsd_degrade_audio.argtypes = [vp, vp, i64, C.POINTER(LsdAudioDegradation), i, vp, vp, sz, vp]; L.lsd_degrade_audio.restype = i
+        L.lsd_score_audio_clips_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_audio_clips_workspace_bytes.restype = sz
+        L.lsd_score_audio_clips.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i, i, i, i,
+                                            vp, vp, sz, vp]
+        L.lsd_score_audio_clips.restype = i
         _lib = L
         return L
 

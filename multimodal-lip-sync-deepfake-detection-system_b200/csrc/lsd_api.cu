@@ -980,24 +980,102 @@ extern "C" int lsd_score_offsets(lsd_handle* h, const uint8_t* track, int n_fram
 }
 
 // ================================================================================================
-// Audio occlusion evidence: K masked log-mel slices per window (occlusion.cu), laid end to end in a pseudo clip and scored as an
+// Audio rows: K device-built (F, Ta) slices per window (occlusion.cu), laid end to end in a pseudo clip and scored as an
 // audio-variant sweep with explicit audio starts j*Ta; the clip is never clamped or padded, so the gather copies the slices as built
 // ================================================================================================
-// Workspace: [boxes (LSD_MAX_AUDIO_OCCLUSIONS x 4 int32) | base audio starts of one batch's windows | pseudo clip (F, batch*K*Ta)
-// fp32 | scoring workspace: lsd_score_offsets' on the shared route, otherwise lsd_score_windows' at `batch` rows].
+// Workspace: [variant table | base audio starts of one batch's windows | pseudo clip (F, batch*K*Ta) fp32 | scoring workspace:
+// lsd_score_offsets' on the shared route, otherwise lsd_score_windows' at `batch` rows].
 namespace {
-size_t audio_occlusion_extra_bytes(int batch, int K, int F, int Ta) {
-  return align256((size_t)LSD_MAX_AUDIO_OCCLUSIONS * 4 * sizeof(int32_t)) + align256((size_t)batch * sizeof(int32_t)) +
-         align256((size_t)F * batch * K * Ta * sizeof(float));
+size_t audio_rows_extra_bytes(size_t table_region, int batch, int K, int F, int Ta) {
+  return align256(table_region) + align256((size_t)batch * sizeof(int32_t)) + align256((size_t)F * batch * K * Ta * sizeof(float));
 }
-}  // namespace
 
-extern "C" size_t lsd_score_audio_occlusions_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
-  if (!h || batch < 1 || K < 1 || K > LSD_MAX_AUDIO_OCCLUSIONS) return 0;
+size_t audio_rows_workspace_bytes(lsd_handle* h, size_t table_region, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  if (!h || batch < 1 || K < 1 || K > LSD_MAX_AUDIO_VARIANTS) return 0;
   const size_t sw = shared_route(precision, T) ? lsd_score_offsets_workspace_bytes(h, batch, K, T, H, W, F, Ta, precision)
                                                : lsd_score_workspace_bytes(h, batch, T, H, W, F, Ta, precision);
   if (sw == 0) return 0;
-  return audio_occlusion_extra_bytes(batch, K, F, Ta) + align256(sw);
+  return audio_rows_extra_bytes(table_region, batch, K, F, Ta) + align256(sw);
+}
+
+// Enqueues on `st` the kernel that writes rows r0 .. r0+nb-1 (window r / K, variant r % K) into columns [j*Ta, (j+1)*Ta) of `clip`,
+// j = r - r0; d_tabs: the variant table, d_abase: the base audio starts of windows r0 / K, r0 / K + 1, ...
+using AudioRowBuilder = std::function<void(const int32_t* d_tabs, const int32_t* d_abase, int r0, int nb, float* clip, cudaStream_t st)>;
+
+// The common part of lsd_score_audio_occlusions / lsd_score_audio_clips, after each has checked its variants: the remaining argument
+// checks, one copy of the variant table (`table_bytes` from tables_host; its region is table_region bytes) and the batch loop.
+// `src` is the log-mel the builder reads (checked for NULL), `what` names the variants in messages.
+int score_audio_rows(lsd_handle* h, const char* fn, const char* what, const uint8_t* track, int n_frames, int H, int W,
+                     const int32_t* starts_host, const int32_t* audio_starts_host, int n_windows, int T, const float* src, int F,
+                     int Ta_full, int total_v_frames, int Ta, int K, int precision, int batch, float* logits_out, void* workspace,
+                     size_t workspace_bytes, void* stream, const void* tables_host, size_t table_bytes, size_t table_region,
+                     const AudioRowBuilder& build) {
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !src || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "%s: null pointer argument", fn);
+  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "%s: bad extents", fn);
+  if ((int64_t)n_windows * K > INT32_MAX || (int64_t)batch * K * Ta > INT32_MAX)
+    return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d %s in batches of %d: too many rows for one call", n_windows, K, what, batch);
+  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
+  Shapes s;
+  int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
+  if (rc) return rc;
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = audio_rows_workspace_bytes(h, table_region, batch, K, T, H, W, F, Ta, precision);
+  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  char* ws = reinterpret_cast<char*>(workspace);
+  int32_t* d_tabs = reinterpret_cast<int32_t*>(ws);
+  int32_t* d_abase = reinterpret_cast<int32_t*>(ws + align256(table_region));
+  float* clip = reinterpret_cast<float*>(reinterpret_cast<char*>(d_abase) + align256((size_t)batch * sizeof(int32_t)));
+  const size_t extra = audio_rows_extra_bytes(table_region, batch, K, F, Ta);
+  char* sws = ws + extra;
+  const size_t sws_bytes = workspace_bytes - extra;
+  std::vector<int32_t> abase(n_windows), rows((size_t)batch * K);
+  for (int i = 0; i < n_windows; ++i) abase[i] = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
+  for (size_t j = 0; j < rows.size(); ++j) rows[j] = (int32_t)j * Ta;   // row j of a batch: columns [j*Ta, (j+1)*Ta) of the clip
+  if (table_bytes) CUDA_OK(h, cudaMemcpyAsync(d_tabs, tables_host, table_bytes, cudaMemcpyHostToDevice, st));
+  // One clip serves every batch: batch k+1's builder is enqueued on `st` after every reader of batch k's clip.  On the shared
+  // route the only readers are the mel gathers of the audio groups (forward_bf16_impl with a VarTail, not pipelined): group 0 runs
+  // on the side stream after ev_start, recorded on `st` behind this batch's builder, and `st` waits for its ev_audio before
+  // groups 1.. run on `st` itself, so `st` is past every gather when score_offsets_batch_bf16 returns.  lsd_score_windows
+  // gathers the audio of each of its batches on `st`, ahead of the encoders, pipelined or not.
+  if (shared_route(precision, T)) {
+    const size_t vi = align256((size_t)batch * sizeof(int32_t)), ai = align256((size_t)batch * K * sizeof(int32_t));
+    int32_t* d_vs = reinterpret_cast<int32_t*>(sws);
+    int32_t* d_as = reinterpret_cast<int32_t*>(sws + vi);
+    CUDA_OK(h, cudaMemcpyAsync(d_as, rows.data(), rows.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    for (int w0 = 0; w0 < n_windows; w0 += batch) {
+      const int nb = std::min(batch, n_windows - w0);
+      CUDA_OK(h, cudaMemcpyAsync(d_vs, starts_host + w0, nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      CUDA_OK(h, cudaMemcpyAsync(d_abase, &abase[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      build(d_tabs, d_abase, w0 * K, nb * K, clip, st);
+      if ((rc = score_offsets_batch_bf16(h, track, n_frames, d_vs, d_as, clip, nb * K * Ta, nb, batch, K, T, H, W, F, Ta,
+                                         logits_out + (size_t)w0 * K, sws + vi + ai, sws_bytes - vi - ai, st))) return rc;
+    }
+  } else {
+    std::vector<int32_t> vrep((size_t)batch * K);   // window i's track start, once per variant
+    for (int w0 = 0; w0 < n_windows; w0 += batch) {
+      const int nb = std::min(batch, n_windows - w0);
+      for (int j = 0; j < nb * K; ++j) vrep[j] = starts_host[w0 + j / K];
+      CUDA_OK(h, cudaMemcpyAsync(d_abase, &abase[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      build(d_tabs, d_abase, w0 * K, nb * K, clip, st);
+      if ((rc = lsd_score_windows(h, track, n_frames, H, W, vrep.data(), rows.data(), nb * K, T, clip, F, nb * K * Ta, total_v_frames, Ta,
+                                  precision, batch, logits_out + (size_t)w0 * K, sws, sws_bytes, stream))) return rc;
+    }
+  }
+  CUDA_OK(h, cudaGetLastError());
+  return LSD_OK;
+}
+
+constexpr size_t AUDIO_OCCLUSION_TABLE_BYTES = (size_t)LSD_MAX_AUDIO_OCCLUSIONS * 4 * sizeof(int32_t);
+}  // namespace
+
+// ------------------------------------------------------------------------------------------------
+// Audio occlusion evidence: K masked log-mel slices per window (mask_audio_windows_kernel)
+// ------------------------------------------------------------------------------------------------
+extern "C" size_t lsd_score_audio_occlusions_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  return audio_rows_workspace_bytes(h, AUDIO_OCCLUSION_TABLE_BYTES, batch, K, T, H, W, F, Ta, precision);
 }
 
 extern "C" int lsd_score_audio_occlusions(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
@@ -1016,64 +1094,83 @@ extern "C" int lsd_score_audio_occlusions(lsd_handle* h, const uint8_t* track, i
       return lsd_fail(h, LSD_ERR_SHAPE, "audio box %d [%d,%d)x[%d,%d) is not inside the %d-column x %d-bin window", k, b.c0, b.c1, b.f0,
                       b.f1, Ta, F);
   }
-  if (n_windows == 0) return LSD_OK;
-  if (!track || !starts_host || !mel_full || !logits_out || !workspace)
-    return lsd_fail(h, LSD_ERR_ARG, "lsd_score_audio_occlusions: null pointer argument");
-  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_audio_occlusions: bad extents");
-  if ((int64_t)n_windows * K > INT32_MAX || (int64_t)batch * K * Ta > INT32_MAX)
-    return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d boxes in batches of %d: too many rows for one call", n_windows, K, batch);
-  if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
-  Shapes s;
-  int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
-  if (rc) return rc;
-  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
-  const size_t need = lsd_score_audio_occlusions_workspace_bytes(h, batch, K, T, H, W, F, Ta, precision);
-  if (need == 0 || need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  static_assert(sizeof(lsd_audio_occlusion) == 4 * sizeof(int32_t), "lsd_audio_occlusion is four packed int32");
+  const AudioRowBuilder mask = [&](const int32_t* d_boxes, const int32_t* d_abase, int r0, int nb, float* clip, cudaStream_t st) {
+    launch_mask_audio_windows(mel_full, F, Ta_full, d_abase, d_boxes, K, r0, nb, Ta, fill, clip, st);
+  };
+  return score_audio_rows(h, "lsd_score_audio_occlusions", "boxes", track, n_frames, H, W, starts_host, audio_starts_host, n_windows, T,
+                          mel_full, F, Ta_full, total_v_frames, Ta, K, precision, batch, logits_out, workspace, workspace_bytes, stream,
+                          boxes, (size_t)K * sizeof(lsd_audio_occlusion), AUDIO_OCCLUSION_TABLE_BYTES, mask);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Audio robustness: K degraded copies of one clip (audio_degrade.cu), and every window scored against K clip log-mels
+// ------------------------------------------------------------------------------------------------
+// Degrade workspace: [variant table, band taps, impulse responses (at most K * DEGRADE_MAX_RIR floats) | noise partial sums |
+// band intermediate K * ceil(n / 2) floats]
+namespace {
+size_t degrade_table_region(int K) { return ((size_t)K * DEGRADE_TAB_INTS + 2 * (41 + 81) + (size_t)K * DEGRADE_MAX_RIR) * sizeof(int32_t); }
+}  // namespace
+
+extern "C" size_t lsd_degrade_audio_workspace_bytes(int64_t n, int K) {
+  if (n < 1 || K < 1 || K > LSD_MAX_AUDIO_DEGRADATIONS) return 0;
+  return align256(degrade_table_region(K)) + align256(degrade_partials_bytes(K)) + align256((size_t)K * ((n + 1) / 2) * sizeof(float));
+}
+
+extern "C" int lsd_degrade_audio(lsd_handle* h, const float* pcm, int64_t n, const lsd_audio_degradation* variants, int K, float* out,
+                                 void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (K < 1 || K > LSD_MAX_AUDIO_DEGRADATIONS)
+    return lsd_fail(h, LSD_ERR_SHAPE, "K = %d audio degradations: expected 1 <= K <= %d", K, LSD_MAX_AUDIO_DEGRADATIONS);
+  if (n < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_degrade_audio: %lld samples, expected at least 1", (long long)n);
+  if ((int64_t)K * n > INT64_MAX / 8) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_degrade_audio: %d x %lld samples is too large", K, (long long)n);
+  if (!pcm || !variants || !out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_degrade_audio: null pointer argument");
+  const int all = LSD_AD_REVERB | LSD_AD_NOISE | LSD_AD_CLIP | LSD_AD_BAND | LSD_AD_MULAW;
+  for (int k = 0; k < K; ++k) {
+    const lsd_audio_degradation& v = variants[k];
+    if (v.stages & ~all) return lsd_fail(h, LSD_ERR_ARG, "audio degradation %d: unknown stage bits 0x%x", k, v.stages & ~all);
+    if ((v.stages & LSD_AD_REVERB) && !(std::isfinite(v.rt60) && v.rt60 >= 0.05f && v.rt60 <= 2.0f))
+      return lsd_fail(h, LSD_ERR_ARG, "audio degradation %d: rt60 %g s is outside [0.05, 2]", k, (double)v.rt60);
+    if ((v.stages & LSD_AD_NOISE) && !(std::isfinite(v.snr_db) && v.snr_db >= -20.f && v.snr_db <= 60.f))
+      return lsd_fail(h, LSD_ERR_ARG, "audio degradation %d: snr %g dB is outside [-20, 60]", k, (double)v.snr_db);
+    if ((v.stages & LSD_AD_CLIP) && !(std::isfinite(v.gain_db) && v.gain_db >= 0.f && v.gain_db <= 40.f))
+      return lsd_fail(h, LSD_ERR_ARG, "audio degradation %d: gain %g dB is outside [0, 40]", k, (double)v.gain_db);
+    if ((v.stages & LSD_AD_BAND) && v.band_rate != 8000 && v.band_rate != 4000)
+      return lsd_fail(h, LSD_ERR_ARG, "audio degradation %d: band_rate %d is not 8000 or 4000", k, v.band_rate);
+  }
+  const size_t need = lsd_degrade_audio_workspace_bytes(n, K);
+  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
   ENTER_DEVICE(h);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  degrade_tables(variants, K, h->variant_tab_host);   // kept until the next call: the copy below is asynchronous
   char* ws = reinterpret_cast<char*>(workspace);
-  int32_t* d_boxes = reinterpret_cast<int32_t*>(ws);
-  int32_t* d_abase = reinterpret_cast<int32_t*>(ws + align256((size_t)LSD_MAX_AUDIO_OCCLUSIONS * 4 * sizeof(int32_t)));
-  float* clip = reinterpret_cast<float*>(reinterpret_cast<char*>(d_abase) + align256((size_t)batch * sizeof(int32_t)));
-  const size_t extra = audio_occlusion_extra_bytes(batch, K, F, Ta);
-  char* sws = ws + extra;
-  const size_t sws_bytes = workspace_bytes - extra;
-  std::vector<int32_t> abase(n_windows), rows((size_t)batch * K);
-  for (int i = 0; i < n_windows; ++i) abase[i] = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
-  for (size_t j = 0; j < rows.size(); ++j) rows[j] = (int32_t)j * Ta;   // row j of a batch: columns [j*Ta, (j+1)*Ta) of the clip
-  static_assert(sizeof(lsd_audio_occlusion) == 4 * sizeof(int32_t), "lsd_audio_occlusion is four packed int32");
-  CUDA_OK(h, cudaMemcpyAsync(d_boxes, boxes, (size_t)K * sizeof(lsd_audio_occlusion), cudaMemcpyHostToDevice, st));
-  // One clip serves every batch: batch k+1's builder is enqueued on `st` after every reader of batch k's clip.  On the shared
-  // route the only readers are the mel gathers of the audio groups (forward_bf16_impl with a VarTail, not pipelined): group 0 runs
-  // on the side stream after ev_start, recorded on `st` behind this batch's builder, and `st` waits for its ev_audio before
-  // groups 1.. run on `st` itself, so `st` is past every gather when score_offsets_batch_bf16 returns.  lsd_score_windows
-  // gathers the audio of each of its batches on `st`, ahead of the encoders, pipelined or not.
-  if (shared_route(precision, T)) {
-    const size_t vi = align256((size_t)batch * sizeof(int32_t)), ai = align256((size_t)batch * K * sizeof(int32_t));
-    int32_t* d_vs = reinterpret_cast<int32_t*>(sws);
-    int32_t* d_as = reinterpret_cast<int32_t*>(sws + vi);
-    CUDA_OK(h, cudaMemcpyAsync(d_as, rows.data(), rows.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    for (int w0 = 0; w0 < n_windows; w0 += batch) {
-      const int nb = std::min(batch, n_windows - w0);
-      CUDA_OK(h, cudaMemcpyAsync(d_vs, starts_host + w0, nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-      CUDA_OK(h, cudaMemcpyAsync(d_abase, &abase[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-      launch_mask_audio_windows(mel_full, F, Ta_full, d_abase, d_boxes, K, w0 * K, nb * K, Ta, fill, clip, st);
-      if ((rc = score_offsets_batch_bf16(h, track, n_frames, d_vs, d_as, clip, nb * K * Ta, nb, batch, K, T, H, W, F, Ta,
-                                         logits_out + (size_t)w0 * K, sws + vi + ai, sws_bytes - vi - ai, st))) return rc;
-    }
-  } else {
-    std::vector<int32_t> vrep((size_t)batch * K);   // window i's track start, once per box
-    for (int w0 = 0; w0 < n_windows; w0 += batch) {
-      const int nb = std::min(batch, n_windows - w0);
-      for (int j = 0; j < nb * K; ++j) vrep[j] = starts_host[w0 + j / K];
-      CUDA_OK(h, cudaMemcpyAsync(d_abase, &abase[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-      launch_mask_audio_windows(mel_full, F, Ta_full, d_abase, d_boxes, K, w0 * K, nb * K, Ta, fill, clip, st);
-      if ((rc = lsd_score_windows(h, track, n_frames, H, W, vrep.data(), rows.data(), nb * K, T, clip, F, nb * K * Ta, total_v_frames, Ta,
-                                  precision, batch, logits_out + (size_t)w0 * K, sws, sws_bytes, stream))) return rc;
-    }
-  }
+  int32_t* d_tab = reinterpret_cast<int32_t*>(ws);
+  double* part = reinterpret_cast<double*>(ws + align256(degrade_table_region(K)));
+  float* mid = reinterpret_cast<float*>(reinterpret_cast<char*>(part) + align256(degrade_partials_bytes(K)));
+  CUDA_OK(h, cudaMemcpyAsync(d_tab, h->variant_tab_host.data(), h->variant_tab_host.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  launch_degrade_audio(pcm, n, variants, K, d_tab, part, mid, out, st);
   CUDA_OK(h, cudaGetLastError());
   return LSD_OK;
+}
+
+extern "C" size_t lsd_score_audio_clips_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  return audio_rows_workspace_bytes(h, 0, batch, K, T, H, W, F, Ta, precision);
+}
+
+extern "C" int lsd_score_audio_clips(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                     const int32_t* audio_starts_host, int n_windows, int T, const float* mels, int F, int Ta_full,
+                                     int total_v_frames, int Ta, int K, int precision, int batch, float* logits_out, void* workspace,
+                                     size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_audio_clips: no weights loaded");
+  if (K < 1 || K > LSD_MAX_AUDIO_DEGRADATIONS)
+    return lsd_fail(h, LSD_ERR_SHAPE, "K = %d clips: expected 1 <= K <= %d", K, LSD_MAX_AUDIO_DEGRADATIONS);
+  const AudioRowBuilder gather = [&](const int32_t*, const int32_t* d_abase, int r0, int nb, float* clip, cudaStream_t st) {
+    launch_gather_audio_variants(mels, F, Ta_full, d_abase, K, r0, nb, Ta, clip, st);
+  };
+  return score_audio_rows(h, "lsd_score_audio_clips", "clips", track, n_frames, H, W, starts_host, audio_starts_host, n_windows, T, mels, F,
+                          Ta_full, total_v_frames, Ta, K, precision, batch, logits_out, workspace, workspace_bytes, stream, nullptr, 0, 0,
+                          gather);
 }
 
 // ================================================================================================

@@ -4,6 +4,9 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <stdint.h>
+#include <vector>
+
+#include "../../include/lsd_b200.h"
 
 namespace lsd {
 
@@ -41,6 +44,19 @@ void launch_occlude_windows(const uint8_t* track, const int32_t* win_starts, con
 // columns [j*Ta, (j+1)*Ta); a_starts: base mel column of windows r0 / K, r0 / K + 1, ...; boxes: K x 4 int32 (c0, c1, f0, f1)
 void launch_mask_audio_windows(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, const int32_t* boxes, int K,
                                int r0, int nb, int Ta, float fill, float* out, cudaStream_t s);
+// audio slices of K clips (occlusion.cu): rows r0 .. r0+nb-1 = (window r / K, clip r % K) -> fp32 pseudo clip out (F, nb*Ta) as
+// launch_mask_audio_windows writes it, slice k read from mels[k] of (K, F, Ta_full)
+void launch_gather_audio_variants(const float* mels, int F, int Ta_full, const int32_t* a_starts, int K, int r0, int nb, int Ta,
+                                  float* out, cudaStream_t s);
+// degraded PCM (audio_degrade.cu): degrade_tables builds the device table of K variants on the host (DEGRADE_TAB_INTS int32 per
+// variant, then the band taps and the impulse responses); launch_degrade_audio writes out (K, n) from pcm (n), with part
+// (degrade_partials_bytes) and mid (K * ceil(n / 2) floats) as scratch
+constexpr int DEGRADE_TAB_INTS = 8, DEGRADE_MAX_RIR = 32000;
+int degrade_rir_length(float rt60);
+void degrade_tables(const lsd_audio_degradation* v, int K, std::vector<int32_t>& out);
+size_t degrade_partials_bytes(int K);
+void launch_degrade_audio(const float* pcm, int64_t n, const lsd_audio_degradation* v, int K, const int32_t* tab, double* part,
+                          float* mid, float* out, cudaStream_t s);
 // re-cropped windows (warp.cu): rows r0 .. r0+nb-1 = (window r / K, variant r % K) -> uint8 pseudo-track out (nb*T, H, W, 3), frame t
 // warped like cv2.warpAffine(INTER_LINEAR, BORDER_REPLICATE) with the tables of (variant k, frame t); win_starts: track start of
 // windows r0 / K, r0 / K + 1, ...; tabs: warp_tables of the K*T matrices, variant-major

@@ -125,7 +125,36 @@ __global__ void __launch_bounds__(256) mask_audio_windows_kernel(const float* __
   }
 }
 
+// Audio slices of lsd_score_audio_clips, built like mask_audio_windows_kernel with a clip per variant instead of a box: row j
+// (window r / K, variant r % K, r = r0 + j) gets
+//   out[f, j*Ta + c] = mels[k][f, clamp(a_i + c, 0, Ta_full-1)]
+// mels: (K, F, Ta_full), the copy gather_audio_kernel makes of mels[k].
+__global__ void __launch_bounds__(256) gather_audio_variants_kernel(const float* __restrict__ mels, int F, int Ta_full,
+                                                                    const int32_t* __restrict__ a_starts, int K, int r0, int Ta,
+                                                                    int64_t cols, float* __restrict__ out) {
+  const int j = blockIdx.x, r = r0 + j;
+  const int wi = r / K;
+  const float* mel = mels + (int64_t)(r - wi * K) * F * Ta_full;
+  const int a = a_starts[wi - r0 / K];
+  float* dst = out + (int64_t)j * Ta;
+  const int n = F * Ta;
+  for (int e = threadIdx.x; e < n; e += blockDim.x) {
+    const int f = e / Ta, c = e - f * Ta;
+    int col = a + c;
+    col = col >= Ta_full ? Ta_full - 1 : col;
+    col = col < 0 ? 0 : col;
+    dst[(int64_t)f * cols + c] = mel[(int64_t)f * Ta_full + col];
+  }
+}
+
 }  // namespace
+
+void launch_gather_audio_variants(const float* mels, int F, int Ta_full, const int32_t* a_starts, int K, int r0, int nb, int Ta,
+                                  float* out, cudaStream_t s) {
+  if (nb < 1) return;
+  gather_audio_variants_kernel<<<(unsigned)nb, 256, 0, s>>>(mels, F, Ta_full, a_starts, K, r0, Ta, (int64_t)nb * Ta, out);
+  count_launch();
+}
 
 void launch_mask_audio_windows(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, const int32_t* boxes, int K,
                                int r0, int nb, int Ta, float fill, float* out, cudaStream_t s) {

@@ -1138,6 +1138,160 @@ class Predictor:
         res["window_starts"] = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
         return res
 
+    # ------------------------------------------------------------------ audio robustness (lsd_degrade_audio, lsd_score_audio_clips)
+    _AD_KEYS = (("rt60", _cabi.LSD_AD_REVERB, 0.05, 2.0), ("snr_db", _cabi.LSD_AD_NOISE, -20.0, 60.0),
+                ("gain_db", _cabi.LSD_AD_CLIP, 0.0, 40.0))
+
+    @classmethod
+    def _degradation(cls, k: int, v) -> "_cabi.LsdAudioDegradation":
+        """One variant as lsd_audio_degradation, checked as lsd_degrade_audio checks it (ValueError).  A dict enables the stages whose
+        keys it has: `rt60`, `snr_db`, `gain_db`, `band_rate`, `mulaw` (True); `seed` (default 0) keys the generator.  A tuple is
+        `(stages, rt60, snr_db, gain_db, band_rate, seed)` with the LSD_AD_* bits."""
+        if isinstance(v, dict):
+            unknown = set(v) - {"rt60", "snr_db", "gain_db", "band_rate", "mulaw", "seed"}
+            if unknown:
+                raise ValueError(f"audio degradation {k}: unknown keys {sorted(unknown)}")
+            stages = sum(bit for key, bit, _, _ in cls._AD_KEYS if key in v)
+            stages |= _cabi.LSD_AD_BAND if "band_rate" in v else 0
+            stages |= _cabi.LSD_AD_MULAW if v.get("mulaw", False) else 0
+            t = (stages, v.get("rt60", 0.0), v.get("snr_db", 0.0), v.get("gain_db", 0.0), v.get("band_rate", 0), v.get("seed", 0))
+        else:
+            t = tuple(v)
+            if len(t) != 6:
+                raise ValueError(f"audio degradation {k}: expected (stages, rt60, snr_db, gain_db, band_rate, seed), got {v!r}")
+        stages, rt60, snr, gain, rate, seed = t
+        all_bits = _cabi.LSD_AD_REVERB | _cabi.LSD_AD_NOISE | _cabi.LSD_AD_CLIP | _cabi.LSD_AD_BAND | _cabi.LSD_AD_MULAW
+        if not isinstance(stages, (int, np.integer)) or int(stages) & ~all_bits or int(stages) < 0:
+            raise ValueError(f"audio degradation {k}: bad stage bits {stages!r}")
+        stages = int(stages)
+        for (key, bit, lo, hi), val in zip(cls._AD_KEYS, (rt60, snr, gain)):
+            if stages & bit and not (np.isfinite(float(val)) and lo <= float(np.float32(val)) <= hi):
+                raise ValueError(f"audio degradation {k}: {key} {val!r} is outside [{lo:g}, {hi:g}]")
+        if stages & _cabi.LSD_AD_BAND and rate not in (8000, 4000):
+            raise ValueError(f"audio degradation {k}: band_rate must be 8000 or 4000, got {rate!r}")
+        if not (isinstance(seed, (int, np.integer)) and 0 <= int(seed) < 2 ** 32):
+            raise ValueError(f"audio degradation {k}: seed must be an integer in [0, 2^32), got {seed!r}")
+        return _cabi.LsdAudioDegradation(stages, float(rt60), float(snr), float(gain), int(rate) if stages & _cabi.LSD_AD_BAND else 0,
+                                         int(seed))
+
+    def degrade_audio(self, pcm, variants) -> torch.Tensor:
+        """K degraded copies of one 16 kHz mono clip (`lsd_degrade_audio`): fp32 `(K, n)` on the device, variant k at row k.  `pcm`: a
+        1-D float tensor or array.  `variants`: dicts or `lsd_audio_degradation`-shaped tuples (`_degradation`); the stages run in the
+        order reverb, noise, clip, band, mu-law, and a variant with none copies the clip."""
+        vs = [self._degradation(k, v) for k, v in enumerate(variants)]
+        K = len(vs)
+        if not 1 <= K <= _cabi.LSD_MAX_AUDIO_DEGRADATIONS:
+            raise ValueError(f"{K} audio degradations: expected 1 to {_cabi.LSD_MAX_AUDIO_DEGRADATIONS}")
+        x = (pcm if isinstance(pcm, torch.Tensor) else torch.from_numpy(np.asarray(pcm)))
+        if x.dim() != 1 or x.numel() < 1:
+            raise ValueError(f"pcm must be a non-empty 1-D clip, got shape {tuple(x.shape)}")
+        m = self.model
+        dev = m._device()
+        x = x.to(device=dev, dtype=torch.float32).contiguous()
+        n = int(x.numel())
+        out = torch.empty((K, n), dtype=torch.float32, device=dev)
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            ws = torch.empty(int(L.lsd_degrade_audio_workspace_bytes(n, K)), dtype=torch.uint8, device=dev)
+            rc = L.lsd_degrade_audio(h.ptr, x.data_ptr(), n, (_cabi.LsdAudioDegradation * K)(*vs), K, out.data_ptr(), ws.data_ptr(),
+                                     ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return out
+
+    def score_track_audio_clips(self, track_u8: torch.Tensor, starts: Sequence[int], mels: torch.Tensor, total_v_frames: int,
+                                chunk_a_size: int = 128, audio_starts_from: Optional[Sequence[int]] = None) -> torch.Tensor:
+        """`score_track_logits` against K clip log-mels at once (`lsd_score_audio_clips`).  `mels`: `(K, F, T_full)` on the device,
+        e.g. the log-mels of `degrade_audio`'s clips, or of the clip run through a lossy codec on the host.  The video side of a window
+        runs once for all K.  Returns fp32 logits `(n, K)` on the device; column k is bit for bit `score_track_logits(track, starts,
+        mels[k:k+1], ...)`."""
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        if mels.dim() != 3 or mels.shape[2] < 1:
+            raise ValueError(f"mels must be (K, F, T_full), got {tuple(mels.shape)}")
+        K = int(mels.shape[0])
+        if not 1 <= K <= _cabi.LSD_MAX_AUDIO_DEGRADATIONS:
+            raise ValueError(f"{K} clips: expected 1 to {_cabi.LSD_MAX_AUDIO_DEGRADATIONS}")
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        F_, Ta_full = int(mels.shape[1]), int(mels.shape[2])
+        T, Ta = self.chunk_size, int(chunk_a_size)
+        n = len(starts)
+        if audio_starts_from is not None and len(audio_starts_from) != n:
+            raise ValueError("audio_starts_from must have one entry per window")
+        for i, s in enumerate(starts):
+            if not 0 <= int(s) <= n_frames - T:
+                raise ValueError(f"window {i} [{int(s)},{int(s) + T}) is outside the {n_frames}-frame track")
+        m = self.model
+        dev = m._device()
+        logits = torch.empty(n, K, dtype=torch.float32, device=dev)
+        if n == 0:
+            return logits
+        track_u8 = track_u8.contiguous()
+        mels = mels.to(torch.float32).contiguous()
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = m._precision()
+            batch = min(self.batch_size, n)
+            need = L.lsd_score_audio_clips_workspace_bytes(h.ptr, batch, K, T, H, W, F_, Ta, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            ws = m._workspace(need, dev)
+            st = (C.c_int32 * n)(*[int(s) for s in starts])
+            ast = None
+            if audio_starts_from is not None:
+                ast = (C.c_int32 * n)(*[self._audio_start(int(v), Ta_full, int(total_v_frames), Ta) for v in audio_starts_from])
+            rc = L.lsd_score_audio_clips(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, T, mels.data_ptr(), F_, Ta_full,
+                                         int(total_v_frames), Ta, K, prec, batch, logits.data_ptr(), ws.data_ptr(), ws.numel(),
+                                         torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return logits
+
+    @staticmethod
+    def audio_degradation_variants() -> Tuple[List[str], List[Dict[str, Any]]]:
+        """The K = 10 degradations of `audio_robustness_track`: names and variant dicts.  The clean clip, white noise at 30, 20, 10, 5
+        and 0 dB SNR, a phone line (8 kHz band + mu-law), a phone line in a noisy room (10 dB, then the phone line), a reverberant
+        room (rt60 0.5 s) and a microphone overdriven by 12 dB."""
+        ladder = (30, 20, 10, 5, 0)
+        names = ["none"] + [f"snr{s}" for s in ladder] + ["phone", "noisy_phone", "reverb", "clipped"]
+        variants = [{}] + [{"snr_db": float(s)} for s in ladder] + [
+            {"band_rate": 8000, "mulaw": True}, {"snr_db": 10.0, "band_rate": 8000, "mulaw": True}, {"rt60": 0.5}, {"gain_db": 12.0}]
+        return names, variants
+
+    def audio_robustness_track(self, track_u8: torch.Tensor, starts: Sequence[int], pcm, total_v_frames: int,
+                               confidence_threshold: float = 0.5, variants=None,
+                               audio_starts_from: Optional[Sequence[int]] = None) -> Dict[str, Any]:
+        """Audio robustness of a track's verdict: `degrade_audio` on the clip's PCM, the log-mel of the K copies in one call
+        (`audio.logmel_db`), one `score_track_audio_clips` call, and the calibrated P(real) summarised by
+        `aggregate.augmentation_stability` (column 0 is the identity).  `variants`: `(names, variants)` as `audio_degradation_variants`
+        returns them (the default), column 0 the clean clip.  Returns:
+          `variants`: the variant names (column order); `snr_db`: the SNR of the variants on the noise ladder (noise only), None for
+          the others;
+          `confidence`, `variant_confidence`, `tta_confidence`, `window_spread`, `decision_flip_rate`, `verdict_stable`: as in
+          `robustness_track`;
+          `lowest_stable_snr`: `aggregate.lowest_stable_quality` on the SNR ladder (a higher SNR is milder noise, the ordering of JPEG
+          quality): the lowest SNR down to which every noise variant keeps the clean confidence's side of `confidence_threshold`,
+          None when the mildest already flips it;
+          `window_starts`: the windows' first frames (those of `audio_starts_from` when given: absolute video frames).
+        It reports only: nothing here enters a verdict."""
+        from .audio import logmel_db
+        names, vs = variants if variants is not None else self.audio_degradation_variants()
+        names = list(names)
+        if len(names) != len(vs):
+            raise ValueError(f"{len(names)} names for {len(vs)} audio degradations")
+        clips = self.degrade_audio(pcm, vs)
+        mels = logmel_db(clips)
+        logits = self.score_track_audio_clips(track_u8, starts, mels, total_v_frames, audio_starts_from=audio_starts_from)
+        probs = np.array([self._calibrate(float(x)) for x in logits.cpu().flatten().tolist()], dtype=np.float64).reshape(len(starts), len(names))
+        res = _agg.augmentation_stability(probs, confidence_threshold, self.confidence_smoothing, self.trim_ratio)
+        degr = [self._degradation(k, v) for k, v in enumerate(vs)]
+        snr = [float(d.snr_db) if d.stages == _cabi.LSD_AD_NOISE else None for d in degr]
+        res["variants"] = names
+        res["snr_db"] = snr
+        res["lowest_stable_snr"] = _agg.lowest_stable_quality(snr, res["variant_confidence"], res["confidence"], confidence_threshold)
+        res["window_starts"] = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
+        return res
+
     def score_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int):
         logits = self.score_track_logits(track_u8, starts, mel_full, total_v_frames)
         confs = [self._calibrate(float(x)) for x in logits.cpu().tolist()]
