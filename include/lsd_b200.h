@@ -419,9 +419,18 @@ int lsd_expand_u8(const uint8_t* src, float* dst, int64_t n, void* stream);
 int64_t lsd_state_generation(lsd_handle* h);
 
 /* Activation tensor of the last tensor-core (BF16) lsd_forward, kept in the workspace in the padded planar bf16 layout
- * (DESIGN.md §4), converted to fp32 channels-last (N, T, H_full, W_full, C) for per-stage parity tests.  Names: "x1" (stem +
- * pool), "y1".."y4" (visual_encoder.layer1..4; y1..y3 are parity-split: pass the full-resolution extent), "ya4" (+ "ya4_lo":
- * audio_encoder.layer4), "hf_f" / "hf_b" (high-frequency branch), "art_b", "artd_b" (artifact branch). */
+ * (DESIGN.md §4), converted to fp32 channels-last (N, T, H_full, W_full, C) for per-stage parity tests.  Names:
+ *   visual encoder: "s_out" (stem conv), "x1" (after the max-pool), "l1a" / "y1" .. "l4a" / "y4" (visual_encoder.layer1..4:
+ *   conv1 output / block output);
+ *   artifact branch: "art_a" / "art_b" (temporal-inconsistency convs on y4), "delta" (y4[t+1] - y4[t], T-1 frames, or one zero
+ *   frame when T == 1), "artd_a" / "artd_b" (the same convs on delta), "hf_f" / "hf_b" (high-frequency branch);
+ *   audio encoder, (hi, lo) pairs with the low part named "<name>_lo": "sa_out", "a1" (after the max-pool), "a1a" / "ya1" ..
+ *   "a4a" / "ya4" (T = 1, H = mel bins, W = time);
+ *   token path: "<name>_p" GEMM operands.
+ * Parity-split buffers (y1, y2 / y3 on the padded route, ya1 .. ya3, hf_f) are re-interleaved, and folded buffers (y2 / l3a / y3 /
+ * l4a when layer3 / layer4 run on the folded small-map route) are read back as the map.  (H_full, W_full) must be the map's true
+ * full-resolution extent, which depends on the input geometry only: any other extent, an out_elems that does not match, or a
+ * low part whose layout differs from the high part's returns LSD_ERR_SHAPE before anything is launched. */
 int lsd_planar_stage_read(lsd_handle* h, const char* name, const char* name_lo_or_null, const void* workspace, float* out,
                           int64_t out_elems, int H_full, int W_full, void* stream);
 /* Number of kernels this library launched on behalf of the handle since creation. */

@@ -252,6 +252,8 @@ struct Packer {
 struct PBuf {
   size_t off = 0;          // byte offset into the workspace
   int C = 0, sets = 1;
+  int kind = PK_PLAIN;     // layout (PlanarKind) and full-resolution map extent: what lsd_planar_stage_read accepts
+  int map_h = 0, map_w = 0;
   UcGeom g;                // geometry of each plane set
   int64_t plane_stride = 0, set_stride = 0, origin = 0;  // elements
   size_t bytes() const { return (size_t)sets * set_stride * 2; }
@@ -286,8 +288,12 @@ struct BPlan {
   std::map<std::string, PBuf> pb;
   size_t planar_begin = 0, planar_end = 0;
   UcGeom gt, g33, gta;                    // token geometries: T tokens (+3 pad), T+1 tokens (rows), audio tokens (rows)
-  void addp(const char* name, int C, int sets, UcGeom g) {
+  // kind PK_PLAIN: the map is the plane geometry itself; the other kinds name the map extent (mh, mw) they hold
+  void addp(const char* name, int C, int sets, UcGeom g, int kind = PK_PLAIN, int mh = 0, int mw = 0) {
     PBuf b = make_pbuf(C, sets, g);
+    b.kind = kind;
+    b.map_h = kind == PK_PLAIN ? g.H : mh;
+    b.map_w = kind == PK_PLAIN ? g.W : mw;
     f32.cursor = (f32.cursor + 255) & ~size_t(255);
     b.off = f32.cursor;
     f32.cursor += b.bytes();
@@ -333,44 +339,44 @@ void build_plan(const Shapes& s, BPlan& P, bool video = true) {
   //  last output reaches one unit past the data — so the row pitch is W/2 + 2, not W/2 + 4: 4 % fewer positions for the stem and hf0)
   const UcGeom gs = make_geom_ex(Bn, Tn, s.Hs, s.Ws, 1, 2, 0, 0, 2);
   if (video) {
-  P.addp("xs", 8, 2, gs);
-  P.addp("xl", 8, 2, gs);
+  P.addp("xs", 8, 2, gs, PK_ROWS, s.H, s.W);
+  P.addp("xl", 8, 2, gs, PK_ROWS, s.H, s.W);
   P.addp("s_out", 64, 1, gs);    // stem conv output (stem geometry), before the max-pool
   P.addp("x1", 64, 1, g1);
   P.addp("l1a", 64, 1, g1);
-  P.addp("y1", 64, 4, g2);       // parity-split: four half-resolution plane sets
+  P.addp("y1", 64, 4, g2, PK_PARITY_HW, s.H1, s.W1);   // parity-split: four half-resolution plane sets
   P.addp("l2a", 128, 1, g2);
   // folded route (small maps): y2 / l3a / y3 / l4a hold one plane set per map position in the row geometry gr
   P.fold3 = fold_route(s.H3, s.W3);
   P.fold4 = fold_route(s.H4, s.W4);
   const UcGeom gr = make_geom_ex(Bn, Tn, 1, 1, 1, 0, 0, 0, 0);
-  if (P.fold3) P.addp("y2", 128, s.H2 * s.W2, gr); else P.addp("y2", 128, 4, g3);
-  if (P.fold3) P.addp("l3a", 256, s.H3 * s.W3, gr); else P.addp("l3a", 256, 1, g3);
-  if (P.fold4) P.addp("y3", 256, s.H3 * s.W3, gr); else P.addp("y3", 256, 4, g4);
-  if (P.fold4) P.addp("l4a", 256, s.H4 * s.W4, gr); else P.addp("l4a", 256, 1, g4);
+  if (P.fold3) P.addp("y2", 128, s.H2 * s.W2, gr, PK_FOLD, s.H2, s.W2); else P.addp("y2", 128, 4, g3, PK_PARITY_HW, s.H2, s.W2);
+  if (P.fold3) P.addp("l3a", 256, s.H3 * s.W3, gr, PK_FOLD, s.H3, s.W3); else P.addp("l3a", 256, 1, g3);
+  if (P.fold4) P.addp("y3", 256, s.H3 * s.W3, gr, PK_FOLD, s.H3, s.W3); else P.addp("y3", 256, 4, g4, PK_PARITY_HW, s.H3, s.W3);
+  if (P.fold4) P.addp("l4a", 256, s.H4 * s.W4, gr, PK_FOLD, s.H4, s.W4); else P.addp("l4a", 256, 1, g4);
   P.addp("y4", 256, 1, g4);
   P.addp("art_a", 128, 1, g4);
   P.addp("art_b", 64, 1, g4);
   P.addp("delta", 256, 1, gd);
   P.addp("artd_a", 128, 1, gd);
   P.addp("artd_b", 64, 1, gd);
-  P.addp("hf_f", 32, 4, gh);
+  P.addp("hf_f", 32, 4, gh, PK_PARITY_HW, s.Hh, s.Wh);
   P.addp("hf_b", 64, 1, gh);
   }
   // audio encoder: 2-D geometries (one slab per window, no temporal padding)
   const UcGeom as = make_geom_ex(Bn, 1, s.Fs, s.As, 0, 2, 0, 0, 4);
   auto g2d = [&](int H, int W) { return make_geom_ex(Bn, 1, H, W, 0, 1, 0, 1, 0); };
-  P.addp("xa", 8, 2, as);
+  P.addp("xa", 8, 2, as, PK_ROWS, s.F, s.Ta);
   for (const char* sfx : {"", "_lo"}) {      // audio activations are (hi, lo) bf16 pairs (split-bf16 convolutions)
     auto nm = [&](const char* n) { return std::string(n) + sfx; };
     P.addp(nm("sa_out").c_str(), 64, 1, as);
     P.addp(nm("a1").c_str(), 64, 1, g2d(s.F1, s.A1));
     P.addp(nm("a1a").c_str(), 64, 1, g2d(s.F1, s.A1));
-    P.addp(nm("ya1").c_str(), 64, 4, g2d(s.F2, s.A2));
+    P.addp(nm("ya1").c_str(), 64, 4, g2d(s.F2, s.A2), PK_PARITY_HW, s.F1, s.A1);
     P.addp(nm("a2a").c_str(), 128, 1, g2d(s.F2, s.A2));
-    P.addp(nm("ya2").c_str(), 128, 4, g2d(s.F3, s.A3));   // h-parity only (stride (2,1)): sets 0 and 2 are used
+    P.addp(nm("ya2").c_str(), 128, 4, g2d(s.F3, s.A3), PK_PARITY_H, s.F2, s.A2);   // h-parity only (stride (2,1)): sets 0 and 2 are used
     P.addp(nm("a3a").c_str(), 256, 1, g2d(s.F3, s.A3));
-    P.addp(nm("ya3").c_str(), 256, 4, g2d(s.F4, s.A4));
+    P.addp(nm("ya3").c_str(), 256, 4, g2d(s.F4, s.A4), PK_PARITY_H, s.F3, s.A3);
     P.addp(nm("a4a").c_str(), 256, 1, g2d(s.F4, s.A4));
     P.addp(nm("ya4").c_str(), 256, 1, g2d(s.F4, s.A4));
   }
@@ -1407,7 +1413,7 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   for (const auto& kv : P.pb) {
     const PBuf& b = kv.second;
     PlanarStage ps;
-    ps.off = b.off; ps.C = b.C; ps.sets = b.sets; ps.plane_stride = b.plane_stride; ps.set_stride = b.set_stride; ps.origin = b.origin;
+    ps.off = b.off; ps.C = b.C; ps.sets = b.sets; ps.kind = b.kind; ps.map_h = b.map_h; ps.map_w = b.map_w; ps.plane_stride = b.plane_stride; ps.set_stride = b.set_stride; ps.origin = b.origin;
     ps.N = b.g.N; ps.T = b.g.T; ps.H = b.g.H; ps.W = b.g.W; ps.ot = b.g.ot; ps.oh = b.g.oh; ps.hp_extra = b.g.HP - b.g.H - b.g.oh;
     ps.ow = b.g.ow; ps.wp_extra = b.g.RW - b.g.W - b.g.ow;
     h->planar_stages[kv.first] = ps;
@@ -1647,8 +1653,9 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
 }
 
 // Introspection (tests): a planar bf16 buffer of the last tensor-core forward -> fp32 channels-last (N, T, Hf, Wf, C).
-// Parity-split buffers (4 plane sets) are re-interleaved: (Hf, Wf) is the full-resolution extent; h-parity-only splits (the
-// stride-(2,1) audio layers) have Wf equal to the plane width.  name_lo: optional low part of a (hi, lo) pair, added in.
+// (Hf, Wf) must be the full-resolution extent of the map the buffer holds (recorded by build_plan), whatever its layout: the unpack
+// kernel derives its addressing from (sets, Hf, Wf), so any other extent would read outside the buffer.  name_lo: optional low
+// part of a (hi, lo) pair, added in; it must have the layout of the high part.
 int planar_stage_read(lsd_handle* h, const char* name, const char* name_lo, const char* ws, float* out, int64_t out_elems, int Hf, int Wf,
                       cudaStream_t st) {
   auto it = h->planar_stages.find(name);
@@ -1660,8 +1667,20 @@ int planar_stage_read(lsd_handle* h, const char* name, const char* name_lo, cons
     if (il == h->planar_stages.end()) return lsd_fail(h, LSD_ERR_ARG, "unknown planar stage %s", name_lo);
     pl = &il->second;
   }
+  if (ps.kind == PK_ROWS) return lsd_fail(h, LSD_ERR_ARG, "stage %s holds pixel rows, not a channel map", name);
+  if (Hf != ps.map_h || Wf != ps.map_w)
+    return lsd_fail(h, LSD_ERR_SHAPE, "stage %s holds a %d x %d map, got %d x %d", name, ps.map_h, ps.map_w, Hf, Wf);
+  if (pl && (pl->kind != ps.kind || pl->C != ps.C || pl->sets != ps.sets || pl->map_h != ps.map_h || pl->map_w != ps.map_w ||
+             pl->plane_stride != ps.plane_stride || pl->set_stride != ps.set_stride || pl->origin != ps.origin || pl->N != ps.N ||
+             pl->T != ps.T || pl->H != ps.H || pl->W != ps.W || pl->ot != ps.ot || pl->oh != ps.oh || pl->hp_extra != ps.hp_extra ||
+             pl->ow != ps.ow || pl->wp_extra != ps.wp_extra))
+    return lsd_fail(h, LSD_ERR_SHAPE, "stage %s does not have the layout of %s", name_lo, name);
   const UcGeom g = make_geom_ex(ps.N, ps.T, ps.H, ps.W, ps.ot, ps.oh, ps.hp_extra, ps.ow, ps.wp_extra);
-  if (ps.sets == 1) { Hf = ps.H; Wf = ps.W; }
+  // the layout unpack_planar_any_kernel selects for the true extent must be the recorded one (a folded 1 x 1 map is plain, and the
+  // two parity splits address a 1-wide map alike)
+  const int sel = ps.sets == 1 ? PK_PLAIN : (g.SL == 1 && ps.sets == Hf * Wf) ? PK_FOLD : Wf == g.W ? PK_PARITY_H : PK_PARITY_HW;
+  const int want = (ps.kind == PK_FOLD && ps.sets == 1) ? PK_PLAIN : (ps.kind == PK_PARITY_HW && Wf == 1) ? PK_PARITY_H : ps.kind;
+  if (sel != want) return lsd_fail(h, LSD_ERR_SHAPE, "stage %s: layout %d cannot be unpacked (reads as %d)", name, ps.kind, sel);
   if ((int64_t)ps.N * ps.T * Hf * Wf * ps.C != out_elems) return lsd_fail(h, LSD_ERR_SHAPE, "stage %s holds %lld elements", name, (long long)ps.N * ps.T * Hf * Wf * ps.C);
   const __nv_bfloat16* x = reinterpret_cast<const __nv_bfloat16*>(ws + ps.off) + ps.origin;
   const __nv_bfloat16* xlo = pl ? reinterpret_cast<const __nv_bfloat16*>(ws + pl->off) + pl->origin : nullptr;

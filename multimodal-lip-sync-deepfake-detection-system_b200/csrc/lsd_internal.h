@@ -47,9 +47,16 @@ struct Prof {             // CUDA-event brackets around the dominant kernel clas
   }
 };
 
+// Layout of a planar bf16 buffer: plain (one plane set, the map itself), parity-split (4 half-resolution plane sets by (h&1, w&1),
+// or by h&1 only for the stride-(2,1) audio layers: sets 0 and 2), folded (one plane set per map position, frame-row geometry),
+// or bf16 pixel rows (stem / laplacian / audio stem inputs: 2 h-parity sets of 2-pixel units, not a channel map).
+enum PlanarKind { PK_PLAIN = 0, PK_PARITY_H = 1, PK_PARITY_HW = 2, PK_FOLD = 3, PK_ROWS = 4 };
+
 struct PlanarStage {      // planar bf16 buffer of the last tensor-core forward (introspection: lsd_planar_stage_read)
   size_t off = 0;
   int C = 0, sets = 1;
+  int kind = PK_PLAIN;
+  int map_h = 0, map_w = 0;   // full-resolution extent of the map the buffer holds
   int64_t plane_stride = 0, set_stride = 0, origin = 0;
   int N = 0, T = 0, H = 0, W = 0, ot = 0, oh = 0, hp_extra = 0, ow = 0, wp_extra = 0;
 };

@@ -376,7 +376,8 @@ class LipSyncModel(nn.Module):
 
     def planar_stage(self, name: str, shape, lo: Optional[str] = None) -> Tensor:
         """fp32 channels-last copy `(N, T, H, W, C)` of a planar bf16 activation buffer of the last tensor-core forward
-        (`lsd_planar_stage_read`); `lo`: name of the low part of a (hi, lo) pair."""
+        (`lsd_planar_stage_read`); H, W: the map's true full-resolution extent, whatever the buffer's layout (plain, parity-split
+        or folded); `lo`: name of the low part of a (hi, lo) pair."""
         h = self._lsd_handle
         out = torch.empty(tuple(int(x) for x in shape), dtype=torch.float32, device=self._lsd_ws.device)
         rc = _cabi.lib().lsd_planar_stage_read(h.ptr, name.encode(), lo.encode() if lo else None, self._lsd_ws.data_ptr(), out.data_ptr(),
