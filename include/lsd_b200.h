@@ -280,6 +280,47 @@ int lsd_jpeg_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, i
                      const int32_t* starts_host, int n_windows, int T, const lsd_jpeg* variants, int K, int channel_order,
                      uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- resolution robustness: window scores of down- and re-upscaled windows -------------------------------- */
+/* This entry has no reference counterpart.  A face that covers 40 px of a 360p video reaches the model as a 96x96 crop upscaled
+ * from that size, without the fine detail a 96 px face has, and the artifact branch's Laplacian measures exactly that detail; it
+ * asks whether a window's score would hold had the face been smaller in the source video.  Every window is scored K times, once
+ * per variant.  Variant k is a face size (h, w), 1 <= h <= H, 1 <= w <= W; every frame of the window becomes
+ *   out[t] = cv2.resize(cv2.resize(win[t], (w, h), interpolation=cv2.INTER_AREA), (W, H), interpolation=cv2.INTER_LINEAR)
+ * bit for bit (OpenCV 4.13's 8-bit paths: INTER_AREA's 2x2, integer-ratio and float32 weighted-tap paths, INTER_LINEAR's 11-bit
+ * fixed point), on tables built on the host as cv::resize builds them.  The channels are independent, so the channel order does
+ * not matter.  (h, w) == (H, W) copies the frame: the plain column. */
+typedef struct { int32_t h, w; } lsd_resize;
+#define LSD_MAX_RESIZE_VARIANTS 64
+/* variants: host, K entries.  Rows are (window, variant) pairs in window-major order, row r = i*K + k; `batch` counts rows.  A
+ * row's audio slice is its window's slice, with the base-start rule of lsd_score_windows (computed, or audio_starts_host_or_null[i],
+ * clamped).  The resized windows of a batch are built on the device and scored by the plain batch path of lsd_score_windows, so
+ * logits_out (device, (n_windows, K) fp32) entry (i, k) is bit for bit lsd_score_windows on window i resized on the host, with the
+ * same audio start.  A workspace of at least twice lsd_score_resizes_workspace_bytes enables the cross-batch pipelining of
+ * lsd_score_windows; a short last batch runs in exactly the queried size.  Everything is checked before any GPU work:
+ * LSD_ERR_SHAPE for K outside 1..LSD_MAX_RESIZE_VARIANTS, a window outside the track, a face size outside 1..H x 1..W, or a crop
+ * whose frame, face-size frame and tables do not fit in 227 KB of shared memory (6*H*W + 36*(H+W) bytes, about 190x190);
+ * LSD_ERR_ARG for variants == NULL or another null pointer. */
+size_t lsd_score_resizes_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision);
+int lsd_score_resizes(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                      const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                      const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                      const lsd_resize* variants, int K, int precision, int batch,
+                      float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
+/* The tables the resize kernel reads for K face sizes of an H x W crop, built on the host without a device (to inspect or test
+ * them).  Returns their int32 count, or LSD_ERR_ARG / LSD_ERR_SHAPE as lsd_score_resizes would; writes them when out_or_null is
+ * not NULL.  Per variant, 10 + 9*(H+W) int32: [mode (0 copy, 1 INTER_AREA ratio 2, 2 other integer ratios, 3 weighted taps),
+ * h, w, kx, ky, float32 1/(kx*ky), 0, 0]; INTER_AREA x taps: first tap of output column d at [d] (W+1 entries), source columns
+ * (2W), float32 weights (2W); the same along y (H+1, 2H, 2H); INTER_LINEAR x: source columns s0, s1 and coefficients a0, a1
+ * (W each); y: the same (H each). */
+int64_t lsd_resize_tables(const lsd_resize* variants, int K, int H, int W, int32_t* out_or_null);
+/* The resized windows themselves, built by the same kernel lsd_score_resizes scores: out (device uint8, (n_windows, K, T, H, W, 3))
+ * holds window i under variant k at [i][k].  Same checks as lsd_score_resizes; workspace: lsd_resize_windows_workspace_bytes (the
+ * tap tables and the window starts). */
+size_t lsd_resize_windows_workspace_bytes(int n_windows, int K, int T, int H, int W);
+int lsd_resize_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                       const int32_t* starts_host, int n_windows, int T, const lsd_resize* variants, int K,
+                       uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- audio occlusion evidence: window scores with a region of the window's log-mel masked ------------------ */
 /* This entry has no reference counterpart.  Window i's audio slice is the (F, Ta) log-mel window of Predictor._align_audio_chunk
  * (predictor.py:525-552) that lsd_score_windows gives it: first column the base start a_i (computed, or

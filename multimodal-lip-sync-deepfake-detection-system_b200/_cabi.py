@@ -25,6 +25,7 @@ LSD_MAX_WARPS = 64
 LSD_JPEG_NONE, LSD_JPEG_444, LSD_JPEG_420 = 0, 1, 2
 LSD_MAX_JPEG_VARIANTS = 64
 LSD_RGB, LSD_BGR = 0, 1
+LSD_MAX_RESIZE_VARIANTS = 64
 LSD_AD_REVERB, LSD_AD_NOISE, LSD_AD_CLIP, LSD_AD_BAND, LSD_AD_MULAW = 1, 2, 4, 8, 16
 LSD_MAX_AUDIO_DEGRADATIONS = LSD_MAX_AUDIO_VARIANTS
 
@@ -42,6 +43,7 @@ EXPORTS = [
     "lsd_score_audio_occlusions_workspace_bytes", "lsd_score_audio_occlusions",
     "lsd_score_warps_workspace_bytes", "lsd_score_warps", "lsd_warp_windows_workspace_bytes", "lsd_warp_windows",
     "lsd_score_jpeg_workspace_bytes", "lsd_score_jpeg", "lsd_jpeg_windows_workspace_bytes", "lsd_jpeg_windows",
+    "lsd_score_resizes_workspace_bytes", "lsd_score_resizes", "lsd_resize_tables", "lsd_resize_windows_workspace_bytes", "lsd_resize_windows",
     "lsd_degrade_audio_workspace_bytes", "lsd_degrade_audio", "lsd_score_audio_clips_workspace_bytes", "lsd_score_audio_clips",
 ]
 
@@ -71,6 +73,12 @@ class LsdWarp(C.Structure):
 class LsdJpeg(C.Structure):
     """One recompression: baseline JPEG quality 1..100 and chroma sampling (LSD_JPEG_420 / LSD_JPEG_444; LSD_JPEG_NONE copies)."""
     _fields_ = [("quality", C.c_int32), ("sampling", C.c_int32)]
+
+
+class LsdResize(C.Structure):
+    """One face size (h, w): every frame down to it with cv2's INTER_AREA and back to the crop size with INTER_LINEAR; the crop
+    size itself copies the frame."""
+    _fields_ = [("h", C.c_int32), ("w", C.c_int32)]
 
 
 class LsdAudioDegradation(C.Structure):
@@ -168,6 +176,14 @@ def lib() -> C.CDLL:
         L.lsd_jpeg_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_jpeg_windows_workspace_bytes.restype = sz
         L.lsd_jpeg_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdJpeg), i, i, vp, vp, sz, vp]
         L.lsd_jpeg_windows.restype = i
+        L.lsd_score_resizes_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_resizes_workspace_bytes.restype = sz
+        L.lsd_score_resizes.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
+                                        C.POINTER(LsdResize), i, i, i, vp, vp, sz, vp]
+        L.lsd_score_resizes.restype = i
+        L.lsd_resize_tables.argtypes = [C.POINTER(LsdResize), i, i, i, vp]; L.lsd_resize_tables.restype = i64
+        L.lsd_resize_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_resize_windows_workspace_bytes.restype = sz
+        L.lsd_resize_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdResize), i, vp, vp, sz, vp]
+        L.lsd_resize_windows.restype = i
         L.lsd_degrade_audio_workspace_bytes.argtypes = [i64, i]; L.lsd_degrade_audio_workspace_bytes.restype = sz
         L.lsd_degrade_audio.argtypes = [vp, vp, i64, C.POINTER(LsdAudioDegradation), i, vp, vp, sz, vp]; L.lsd_degrade_audio.restype = i
         L.lsd_score_audio_clips_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_audio_clips_workspace_bytes.restype = sz

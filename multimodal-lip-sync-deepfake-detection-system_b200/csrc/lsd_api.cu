@@ -89,6 +89,7 @@ extern "C" int lsd_create(lsd_handle** out, int device) {
     if (ce == cudaSuccess) ce = lsd::tok_front_device_init();
     if (ce == cudaSuccess) ce = lsd::warp_windows_device_init();
     if (ce == cudaSuccess) ce = lsd::jpeg_windows_device_init();
+    if (ce == cudaSuccess) ce = lsd::resize_windows_device_init();
     if (ce != cudaSuccess) rc = lsd_fail(h, LSD_ERR_CUDA, "lsd_create: kernel attribute setup: %s", cudaGetErrorString(ce));
   }
   if (rc != 0) { g_create_error = h->err; delete h; return rc; }
@@ -569,7 +570,7 @@ extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_fram
 }
 
 // ================================================================================================
-// Window variants: K device-built copies of every window (occlusion.cu, warp.cu, jpeg.cu), scored by the batch loop of
+// Window variants: K device-built copies of every window (occlusion.cu, warp.cu, jpeg.cu, resize.cu), scored by the batch loop of
 // lsd_score_windows
 // ================================================================================================
 // Workspace: [variant tables | track starts of one batch's windows | pseudo-track of `batch` built windows | lsd_score_windows
@@ -590,7 +591,7 @@ size_t variant_workspace_bytes(lsd_handle* h, size_t table_bytes, int batch, int
 // tables, d_wins: the track starts of windows r0 / K, r0 / K + 1, ...
 using VariantBuilder = std::function<void(const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* pseudo, cudaStream_t st)>;
 
-// The common part of lsd_score_occlusions / lsd_score_warps / lsd_score_jpeg, after each has checked its variants: the remaining
+// The common part of lsd_score_occlusions / lsd_score_warps / lsd_score_jpeg / lsd_score_resizes, after each has checked its variants: the remaining
 // argument checks, the row table (row r reads frames (r % batch) * T .. of the batch's pseudo-track and the audio slice of window
 // r / K), one copy of the K variants' tables (`table_bytes` of them, from tables_host; their region is table_region bytes) and the
 // per-batch hook that copies the batch's window starts and runs `build`.  `what` names the variants in messages.
@@ -641,7 +642,7 @@ int score_window_variants(lsd_handle* h, const char* fn, const char* what, const
 }
 
 // The variant tables and the window starts of the entries that return the built windows themselves (lsd_warp_windows,
-// lsd_jpeg_windows): one launch over all n_windows x K rows into the caller's buffer.
+// lsd_jpeg_windows, lsd_resize_windows): one launch over all n_windows x K rows into the caller's buffer.
 int build_window_variants(lsd_handle* h, const int32_t* starts_host, int n_windows, int K, void* workspace, void* stream,
                           const void* tables_host, size_t table_bytes, uint8_t* out, const VariantBuilder& build) {
   ENTER_DEVICE(h);
@@ -844,6 +845,87 @@ extern "C" int lsd_jpeg_windows(lsd_handle* h, const uint8_t* track, int n_frame
   };
   return build_window_variants(h, starts_host, n_windows, K, workspace, stream, h->variant_tab_host.data(),
                                h->variant_tab_host.size() * sizeof(int32_t), out, jpeg);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Resolution robustness: K down- and re-upscaled copies of every window (resize.cu); tables resize_tables_ints int32
+// ------------------------------------------------------------------------------------------------
+namespace {
+// The checks every resize entry makes before any GPU work; on success h->variant_tab_host holds the K variants' tables.
+int resize_tables_checked(lsd_handle* h, const char* fn, const lsd_resize* v, int K, int T, int H, int W) {
+  if (!v) return lsd_fail(h, LSD_ERR_ARG, "%s: variants is NULL", fn);
+  if (K < 1 || K > LSD_MAX_RESIZE_VARIANTS)
+    return lsd_fail(h, LSD_ERR_SHAPE, "K = %d resize variants: expected 1 <= K <= %d", K, LSD_MAX_RESIZE_VARIANTS);
+  if (T < 1 || !resize_extents_ok(H, W))
+    return lsd_fail(h, LSD_ERR_SHAPE, "%s: bad window extents T=%d H=%d W=%d (frame, face-size frame and tables within shared memory)",
+                    fn, T, H, W);
+  for (int k = 0; k < K; ++k)
+    if (v[k].h < 1 || v[k].h > H || v[k].w < 1 || v[k].w > W)
+      return lsd_fail(h, LSD_ERR_SHAPE, "resize variant %d: face size %dx%d is outside 1..%d x 1..%d", k, v[k].h, v[k].w, H, W);
+  static_assert(sizeof(lsd_resize) == 2 * sizeof(int32_t), "lsd_resize is two packed int32");
+  h->variant_tab_host.resize(resize_tables_ints(K, H, W));
+  resize_tables(reinterpret_cast<const int32_t*>(v), K, H, W, h->variant_tab_host.data());
+  return 0;
+}
+}  // namespace
+
+extern "C" size_t lsd_score_resizes_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  if (batch < 1 || K < 1 || K > LSD_MAX_RESIZE_VARIANTS || !resize_extents_ok(H, W)) return 0;
+  return variant_workspace_bytes(h, resize_tables_ints(K, H, W) * sizeof(int32_t), batch, T, H, W, F, Ta, precision);
+}
+
+extern "C" int lsd_score_resizes(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                 const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full,
+                                 int total_v_frames, int Ta, const lsd_resize* variants, int K, int precision, int batch,
+                                 float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_resizes: no weights loaded");
+  const int rc = resize_tables_checked(h, "lsd_score_resizes", variants, K, T, H, W);
+  if (rc) return rc;
+  const size_t tab_bytes = h->variant_tab_host.size() * sizeof(int32_t);
+  const VariantBuilder resize = [&](const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* pseudo, cudaStream_t st) {
+    launch_resize_windows(track, d_wins, d_tabs, K, r0, nb, T, H, W, pseudo, st);
+  };
+  return score_window_variants(h, "lsd_score_resizes", "resize variants", track, n_frames, H, W, starts_host, audio_starts_host, n_windows,
+                               T, mel_full, F, Ta_full, total_v_frames, Ta, K, precision, batch, logits_out, workspace, workspace_bytes,
+                               stream, h->variant_tab_host.data(), tab_bytes, tab_bytes, resize);
+}
+
+// The tap tables of K face sizes, as the kernel reads them: no handle and no device needed.
+extern "C" int64_t lsd_resize_tables(const lsd_resize* variants, int K, int H, int W, int32_t* out_or_null) {
+  if (!variants) return LSD_ERR_ARG;
+  if (K < 1 || K > LSD_MAX_RESIZE_VARIANTS || !resize_extents_ok(H, W)) return LSD_ERR_SHAPE;
+  for (int k = 0; k < K; ++k)
+    if (variants[k].h < 1 || variants[k].h > H || variants[k].w < 1 || variants[k].w > W) return LSD_ERR_SHAPE;
+  if (out_or_null) resize_tables(reinterpret_cast<const int32_t*>(variants), K, H, W, out_or_null);
+  return (int64_t)resize_tables_ints(K, H, W);
+}
+
+// The resized windows themselves, written to a caller buffer by the builder lsd_score_resizes uses.
+extern "C" size_t lsd_resize_windows_workspace_bytes(int n_windows, int K, int T, int H, int W) {
+  if (n_windows < 1 || K < 1 || K > LSD_MAX_RESIZE_VARIANTS || T < 1 || !resize_extents_ok(H, W)) return 0;
+  return built_windows_workspace_bytes(resize_tables_ints(K, H, W) * sizeof(int32_t), n_windows);
+}
+
+extern "C" int lsd_resize_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host, int n_windows,
+                                  int T, const lsd_resize* variants, int K, uint8_t* out, void* workspace, size_t workspace_bytes,
+                                  void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  int rc = resize_tables_checked(h, "lsd_resize_windows", variants, K, T, H, W);
+  if (rc) return rc;
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_resize_windows: null pointer argument");
+  if (n_windows < 0 || n_frames < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_resize_windows: bad extents");
+  if ((int64_t)n_windows * K * T > INT32_MAX)
+    return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d resize variants: too many frames for one call", n_windows, K);
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = lsd_resize_windows_workspace_bytes(n_windows, K, T, H, W);
+  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  const VariantBuilder resize = [&](const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* o, cudaStream_t st) {
+    launch_resize_windows(track, d_wins, d_tabs, K, r0, nb, T, H, W, o, st);
+  };
+  return build_window_variants(h, starts_host, n_windows, K, workspace, stream, h->variant_tab_host.data(),
+                               h->variant_tab_host.size() * sizeof(int32_t), out, resize);
 }
 
 // ================================================================================================

@@ -76,6 +76,15 @@ void launch_jpeg_windows(const uint8_t* track, const int32_t* win_starts, const 
 void jpeg_tables(const int32_t* qs, int K, int32_t* out);
 cudaError_t jpeg_windows_device_init();
 bool jpeg_extents_ok(int H, int W, bool any444);
+// down- and re-upscaled windows (resize.cu): rows r0 .. r0+nb-1 = (window r / K, variant r % K) -> uint8 pseudo-track out (nb*T, H, W, 3),
+// every frame of row r as cv2.resize(cv2.resize(frame, (w, h), INTER_AREA), (W, H), INTER_LINEAR) with the face size (h, w) of
+// variant k; win_starts: track start of windows r0 / K, r0 / K + 1, ...; tabs: resize_tables of the K sizes
+void launch_resize_windows(const uint8_t* track, const int32_t* win_starts, const int32_t* tabs, int K, int r0, int nb, int T, int H, int W,
+                           uint8_t* out, cudaStream_t s);
+size_t resize_tables_ints(int K, int H, int W);
+void resize_tables(const int32_t* hw, int K, int H, int W, int32_t* out);
+cudaError_t resize_windows_device_init();
+bool resize_extents_ok(int H, int W);
 // mel_full (F, Ta_full) + per-window a_start -> (n, F, Ta) with repeat-last-column padding (predictor.py:525-552)
 void launch_gather_audio(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, float* dst,
                          int n, int Ta, cudaStream_t s);

@@ -1138,6 +1138,125 @@ class Predictor:
         res["window_starts"] = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
         return res
 
+    # ------------------------------------------------------------------ resolution robustness (lsd_score_resizes)
+    def _resize_args(self, track_u8: torch.Tensor, starts: Sequence[int], variants):
+        """Checks what `lsd_score_resizes` / `lsd_resize_windows` would reject, as ValueError (all but the shared-memory limit of the
+        crop size, which the library reports as ValueError before any launch); returns (K, variants as lsd_resize)."""
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        vs = [tuple(v) for v in variants]
+        if not 1 <= len(vs) <= _cabi.LSD_MAX_RESIZE_VARIANTS:
+            raise ValueError(f"{len(vs)} resize variants: expected 1 to {_cabi.LSD_MAX_RESIZE_VARIANTS}")
+        for k, v in enumerate(vs):
+            if len(v) != 2 or not all(isinstance(x, (int, np.integer)) for x in v) or not (1 <= v[0] <= H and 1 <= v[1] <= W):
+                raise ValueError(f"resize variant {k}: face size must be integers (h, w) in 1..{H} x 1..{W}, got {v!r}")
+        T = self.chunk_size
+        for i, s in enumerate(starts):
+            if not 0 <= int(s) <= n_frames - T:
+                raise ValueError(f"window {i} [{int(s)},{int(s) + T}) is outside the {n_frames}-frame track")
+        return len(vs), (_cabi.LsdResize * len(vs))(*[_cabi.LsdResize(int(h), int(w)) for h, w in vs])
+
+    def score_track_resizes(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int, variants,
+                            chunk_a_size: int = 128, audio_starts_from: Optional[Sequence[int]] = None) -> torch.Tensor:
+        """`score_track_logits` with K face sizes per window (`lsd_score_resizes`).  `variants`: a sequence of `(h, w)`, 1 <= h <= H,
+        1 <= w <= W; `(H, W)` is the plain window.  Every frame of variant k is `cv2.resize(cv2.resize(frame, (w, h), INTER_AREA),
+        (W, H), INTER_LINEAR)`, bit for bit, built on the device: the crop as a face of h x w pixels in the source video would give
+        it.  Returns fp32 logits `(n, K)` on the device; entry (i, k) is bit for bit the logit of window i resized by variant k, with
+        window i's audio slice."""
+        if mel_full.dim() != 3 or mel_full.shape[0] != 1:
+            raise ValueError(f"mel_full must be (1, F, T_full), got {tuple(mel_full.shape)}")
+        K, vc = self._resize_args(track_u8, starts, variants)
+        n = len(starts)
+        if audio_starts_from is not None and len(audio_starts_from) != n:
+            raise ValueError("audio_starts_from must have one entry per window")
+        m = self.model
+        dev = m._device()
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T = self.chunk_size
+        logits = torch.empty(n, K, dtype=torch.float32, device=dev)
+        if n == 0:
+            return logits
+        track_u8 = track_u8.contiguous()
+        mel_full = mel_full.to(torch.float32).contiguous()
+        F_, Ta_full = int(mel_full.shape[1]), int(mel_full.shape[2])
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = m._precision()
+            batch = min(self.batch_size, n * K)
+            need = L.lsd_score_resizes_workspace_bytes(h.ptr, batch, K, T, H, W, F_, chunk_a_size, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            if n * K > batch and prec == _cabi.LSD_PREC_BF16:
+                need = 2 * need      # a double workspace lets the batches overlap as in score_track_logits
+            ws = m._workspace(need, dev)
+            st = (C.c_int32 * n)(*[int(s) for s in starts])
+            ast = None
+            if audio_starts_from is not None:
+                ast = (C.c_int32 * n)(*[self._audio_start(int(v), Ta_full, int(total_v_frames), chunk_a_size) for v in audio_starts_from])
+            rc = L.lsd_score_resizes(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, T, mel_full.data_ptr(), F_, Ta_full,
+                                     int(total_v_frames), chunk_a_size, vc, K, prec, batch, logits.data_ptr(), ws.data_ptr(),
+                                     ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return logits
+
+    def resize_track_windows(self, track_u8: torch.Tensor, starts: Sequence[int], variants) -> torch.Tensor:
+        """The resized windows `score_track_resizes` scores, built by the same kernel (`lsd_resize_windows`): uint8
+        `(n, K, T, H, W, 3)` on the device, window i under variant k at [i, k].  To look at what a face size does to the crop."""
+        K, vc = self._resize_args(track_u8, starts, variants)
+        m = self.model
+        dev = m._device()
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T, n = self.chunk_size, len(starts)
+        out = torch.empty((n, K, T, H, W, 3), dtype=torch.uint8, device=dev)
+        if n == 0:
+            return out
+        track_u8 = track_u8.contiguous()
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            need = L.lsd_resize_windows_workspace_bytes(n, K, T, H, W)
+            ws = torch.empty(max(int(need), 1), dtype=torch.uint8, device=dev)
+            rc = L.lsd_resize_windows(h.ptr, track_u8.data_ptr(), n_frames, H, W, (C.c_int32 * n)(*[int(s) for s in starts]), n, T, vc,
+                                      K, out.data_ptr(), ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return out
+
+    @staticmethod
+    def resolution_variants(H: int, W: int) -> Tuple[List[str], List[Tuple[int, int]]]:
+        """The K = 8 face sizes of `resolution_track`: names and `(h, w)`.  The plain window, then both sides scaled by 80, 64, 56,
+        48, 40, 32 and 24 over 96 and rounded (half up, at least 1): for a 96x96 crop exactly those sides, a 96 px face seen as an
+        80 ... 24 px one.  With 96x96 crops the ladder takes all three INTER_AREA paths: ratio 2 (48), other integer ratios (32, 24)
+        and weighted taps (the rest)."""
+        sides = (80, 64, 56, 48, 40, 32, 24)
+        sizes = [(int(H), int(W))] + [(max(1, (int(H) * s + 48) // 96), max(1, (int(W) * s + 48) // 96)) for s in sides]
+        return ["none"] + [f"{h}x{w}" for h, w in sizes[1:]], sizes
+
+    def resolution_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                         confidence_threshold: float = 0.5, audio_starts_from: Optional[Sequence[int]] = None) -> Dict[str, Any]:
+        """Resolution robustness of a track's verdict: one `score_track_resizes` call with the K = 8 `resolution_variants`, the
+        calibrated P(real) summarised by `aggregate.augmentation_stability` (column 0, the plain window, is the identity):
+          `variants`: the variant names (column order); `sizes`: their face sizes `(h, w)` (the crop size for the plain window);
+          `confidence`, `variant_confidence`, `tta_confidence`, `window_spread`, `decision_flip_rate`, `verdict_stable`: as in
+          `robustness_track`;
+          `lowest_stable_side`: the lowest face height h such that every variant of height >= h keeps the plain confidence's side
+          of `confidence_threshold` (`aggregate.lowest_stable_quality` on the heights, the plain window left out), None when the
+          largest face size already flips it;
+          `window_starts`: the windows' first frames (those of `audio_starts_from` when given: absolute video frames).
+        It reports only: nothing here enters a verdict."""
+        H, W = int(track_u8.shape[1]), int(track_u8.shape[2])
+        names, sizes = self.resolution_variants(H, W)
+        logits = self.score_track_resizes(track_u8, starts, mel_full, total_v_frames, sizes, audio_starts_from=audio_starts_from)
+        probs = np.array([self._calibrate(float(x)) for x in logits.cpu().flatten().tolist()], dtype=np.float64).reshape(len(starts), len(names))
+        res = _agg.augmentation_stability(probs, confidence_threshold, self.confidence_smoothing, self.trim_ratio)
+        heights = [None] + [h for h, _ in sizes[1:]]
+        res["variants"] = names
+        res["sizes"] = sizes
+        res["lowest_stable_side"] = _agg.lowest_stable_quality(heights, res["variant_confidence"], res["confidence"], confidence_threshold)
+        res["window_starts"] = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
+        return res
+
     # ------------------------------------------------------------------ audio robustness (lsd_degrade_audio, lsd_score_audio_clips)
     _AD_KEYS = (("rt60", _cabi.LSD_AD_REVERB, 0.05, 2.0), ("snr_db", _cabi.LSD_AD_NOISE, -20.0, 60.0),
                 ("gain_db", _cabi.LSD_AD_CLIP, 0.0, 40.0))
