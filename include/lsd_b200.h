@@ -321,6 +321,42 @@ int lsd_resize_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H,
                        const int32_t* starts_host, int n_windows, int T, const lsd_resize* variants, int K,
                        uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- temporal robustness: window scores of retimed windows ------------------------------------------------- */
+/* This entry has no reference counterpart.  Call and stream video is held from a lower capture rate, stalls, drops frames and is
+ * converted between frame rates by blending neighbours; the delta branch works on frame differences and the token path attends
+ * over 32 frame tokens, so these faults reach the model directly.  It asks whether a window's score would hold had its frames
+ * been retimed so.  Every window is scored K times, once per variant.  A variant is one lsd_retime per output frame t: up to four
+ * taps (src[i], weight[i]).  src[i] is a frame offset from the window's first track frame, -T <= src[i] <= 2T-1, and names the track
+ * frame clamp(window_start + src[i], 0, n_frames - 1): a replicate border in time, and frames outside the window but inside the
+ * track are the track's own.  The weights are Q15 integers >= 0 summing to LSD_RETIME_ONE; every byte of output frame t is
+ *   out = (sum_i weight[i] * p_i + 16384) >> 15
+ * so a single tap of weight LSD_RETIME_ONE copies its frame, and src[t] = t with one such tap is the plain window. */
+typedef struct { int32_t src[4]; int32_t weight[4]; } lsd_retime;
+#define LSD_RETIME_ONE 32768
+#define LSD_MAX_RETIMES 64
+/* variants: host, K*T entries, variant k frame t at [k*T + t].  Rows are (window, variant) pairs in window-major order, row
+ * r = i*K + k; `batch` counts rows.  A row's audio slice is its window's slice, with the base-start rule of lsd_score_windows
+ * (computed, or audio_starts_host_or_null[i], clamped).  The retimed windows of a batch are built on the device and scored by the
+ * plain batch path of lsd_score_windows, so logits_out (device, (n_windows, K) fp32) entry (i, k) is bit for bit
+ * lsd_score_windows on window i retimed by variant k on the host, with the same audio start.  A workspace of at least twice
+ * lsd_score_retimes_workspace_bytes enables the cross-batch pipelining of lsd_score_windows; a short last batch runs in exactly
+ * the queried size.  Everything is checked before any GPU work: LSD_ERR_SHAPE for K outside 1..LSD_MAX_RETIMES, a window outside
+ * the track, a src outside -T..2T-1 (taps of weight 0 included) or n_windows*K*T above INT32_MAX; LSD_ERR_ARG for variants == NULL
+ * or another null pointer, a negative weight, or a frame whose weights do not sum to LSD_RETIME_ONE. */
+size_t lsd_score_retimes_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision);
+int lsd_score_retimes(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                      const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                      const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                      const lsd_retime* variants, int K, int precision, int batch,
+                      float* logits_out, void* workspace, size_t workspace_bytes, void* stream);
+/* The retimed windows themselves, built by the same kernel lsd_score_retimes scores: out (device uint8, (n_windows, K, T, H, W, 3))
+ * holds window i under variant k at [i][k].  Same checks as lsd_score_retimes; workspace: lsd_retime_windows_workspace_bytes (the
+ * variant tables and the window starts). */
+size_t lsd_retime_windows_workspace_bytes(int n_windows, int K, int T, int H, int W);
+int lsd_retime_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                       const int32_t* starts_host, int n_windows, int T, const lsd_retime* variants, int K,
+                       uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- audio occlusion evidence: window scores with a region of the window's log-mel masked ------------------ */
 /* This entry has no reference counterpart.  Window i's audio slice is the (F, Ta) log-mel window of Predictor._align_audio_chunk
  * (predictor.py:525-552) that lsd_score_windows gives it: first column the base start a_i (computed, or

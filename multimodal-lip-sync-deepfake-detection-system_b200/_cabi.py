@@ -26,6 +26,8 @@ LSD_JPEG_NONE, LSD_JPEG_444, LSD_JPEG_420 = 0, 1, 2
 LSD_MAX_JPEG_VARIANTS = 64
 LSD_RGB, LSD_BGR = 0, 1
 LSD_MAX_RESIZE_VARIANTS = 64
+LSD_RETIME_ONE = 32768
+LSD_MAX_RETIMES = 64
 LSD_AD_REVERB, LSD_AD_NOISE, LSD_AD_CLIP, LSD_AD_BAND, LSD_AD_MULAW = 1, 2, 4, 8, 16
 LSD_MAX_AUDIO_DEGRADATIONS = LSD_MAX_AUDIO_VARIANTS
 
@@ -44,6 +46,7 @@ EXPORTS = [
     "lsd_score_warps_workspace_bytes", "lsd_score_warps", "lsd_warp_windows_workspace_bytes", "lsd_warp_windows",
     "lsd_score_jpeg_workspace_bytes", "lsd_score_jpeg", "lsd_jpeg_windows_workspace_bytes", "lsd_jpeg_windows",
     "lsd_score_resizes_workspace_bytes", "lsd_score_resizes", "lsd_resize_tables", "lsd_resize_windows_workspace_bytes", "lsd_resize_windows",
+    "lsd_score_retimes_workspace_bytes", "lsd_score_retimes", "lsd_retime_windows_workspace_bytes", "lsd_retime_windows",
     "lsd_degrade_audio_workspace_bytes", "lsd_degrade_audio", "lsd_score_audio_clips_workspace_bytes", "lsd_score_audio_clips",
 ]
 
@@ -79,6 +82,12 @@ class LsdResize(C.Structure):
     """One face size (h, w): every frame down to it with cv2's INTER_AREA and back to the crop size with INTER_LINEAR; the crop
     size itself copies the frame."""
     _fields_ = [("h", C.c_int32), ("w", C.c_int32)]
+
+
+class LsdRetime(C.Structure):
+    """One output frame of a retimed window: up to four taps, frame offsets `src` from the window's first track frame (clamped to the
+    track) and Q15 weights >= 0 summing to LSD_RETIME_ONE."""
+    _fields_ = [("src", C.c_int32 * 4), ("weight", C.c_int32 * 4)]
 
 
 class LsdAudioDegradation(C.Structure):
@@ -184,6 +193,13 @@ def lib() -> C.CDLL:
         L.lsd_resize_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_resize_windows_workspace_bytes.restype = sz
         L.lsd_resize_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdResize), i, vp, vp, sz, vp]
         L.lsd_resize_windows.restype = i
+        L.lsd_score_retimes_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_retimes_workspace_bytes.restype = sz
+        L.lsd_score_retimes.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i,
+                                        C.POINTER(LsdRetime), i, i, i, vp, vp, sz, vp]
+        L.lsd_score_retimes.restype = i
+        L.lsd_retime_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_retime_windows_workspace_bytes.restype = sz
+        L.lsd_retime_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdRetime), i, vp, vp, sz, vp]
+        L.lsd_retime_windows.restype = i
         L.lsd_degrade_audio_workspace_bytes.argtypes = [i64, i]; L.lsd_degrade_audio_workspace_bytes.restype = sz
         L.lsd_degrade_audio.argtypes = [vp, vp, i64, C.POINTER(LsdAudioDegradation), i, vp, vp, sz, vp]; L.lsd_degrade_audio.restype = i
         L.lsd_score_audio_clips_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_audio_clips_workspace_bytes.restype = sz

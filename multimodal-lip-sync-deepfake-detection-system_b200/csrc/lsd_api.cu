@@ -570,8 +570,8 @@ extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_fram
 }
 
 // ================================================================================================
-// Window variants: K device-built copies of every window (occlusion.cu, warp.cu, jpeg.cu, resize.cu), scored by the batch loop of
-// lsd_score_windows
+// Window variants: K device-built copies of every window (occlusion.cu, warp.cu, jpeg.cu, resize.cu, retime.cu), scored by the batch
+// loop of lsd_score_windows
 // ================================================================================================
 // Workspace: [variant tables | track starts of one batch's windows | pseudo-track of `batch` built windows | lsd_score_windows
 // workspace].  The pseudo-track is read only by the batch's first kernel on the caller's stream (the tensor-core pixel rows or the
@@ -591,7 +591,7 @@ size_t variant_workspace_bytes(lsd_handle* h, size_t table_bytes, int batch, int
 // tables, d_wins: the track starts of windows r0 / K, r0 / K + 1, ...
 using VariantBuilder = std::function<void(const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* pseudo, cudaStream_t st)>;
 
-// The common part of lsd_score_occlusions / lsd_score_warps / lsd_score_jpeg / lsd_score_resizes, after each has checked its variants: the remaining
+// The common part of lsd_score_occlusions / lsd_score_warps / lsd_score_jpeg / lsd_score_resizes / lsd_score_retimes, after each has checked its variants: the remaining
 // argument checks, the row table (row r reads frames (r % batch) * T .. of the batch's pseudo-track and the audio slice of window
 // r / K), one copy of the K variants' tables (`table_bytes` of them, from tables_host; their region is table_region bytes) and the
 // per-batch hook that copies the batch's window starts and runs `build`.  `what` names the variants in messages.
@@ -642,7 +642,7 @@ int score_window_variants(lsd_handle* h, const char* fn, const char* what, const
 }
 
 // The variant tables and the window starts of the entries that return the built windows themselves (lsd_warp_windows,
-// lsd_jpeg_windows, lsd_resize_windows): one launch over all n_windows x K rows into the caller's buffer.
+// lsd_jpeg_windows, lsd_resize_windows, lsd_retime_windows): one launch over all n_windows x K rows into the caller's buffer.
 int build_window_variants(lsd_handle* h, const int32_t* starts_host, int n_windows, int K, void* workspace, void* stream,
                           const void* tables_host, size_t table_bytes, uint8_t* out, const VariantBuilder& build) {
   ENTER_DEVICE(h);
@@ -926,6 +926,87 @@ extern "C" int lsd_resize_windows(lsd_handle* h, const uint8_t* track, int n_fra
   };
   return build_window_variants(h, starts_host, n_windows, K, workspace, stream, h->variant_tab_host.data(),
                                h->variant_tab_host.size() * sizeof(int32_t), out, resize);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Temporal robustness: K retimed copies of every window (retime.cu); tables K*T lsd_retime entries
+// ------------------------------------------------------------------------------------------------
+namespace {
+// The checks every retime entry makes before any GPU work; on success h->variant_tab_host holds the K*T entries.
+int retime_tables_checked(lsd_handle* h, const char* fn, const lsd_retime* v, int K, int T, int H, int W) {
+  if (!v) return lsd_fail(h, LSD_ERR_ARG, "%s: variants is NULL", fn);
+  if (K < 1 || K > LSD_MAX_RETIMES) return lsd_fail(h, LSD_ERR_SHAPE, "K = %d retime variants: expected 1 <= K <= %d", K, LSD_MAX_RETIMES);
+  if (T < 1 || H < 1 || W < 1 || (int64_t)H * W * 3 > INT32_MAX)
+    return lsd_fail(h, LSD_ERR_SHAPE, "%s: bad window extents T=%d H=%d W=%d", fn, T, H, W);
+  for (int64_t e = 0; e < (int64_t)K * T; ++e) {
+    const int k = (int)(e / T), t = (int)(e % T);
+    int64_t sum = 0;
+    for (int i = 0; i < 4; ++i) {
+      if (v[e].src[i] < -T || v[e].src[i] > 2 * T - 1)
+        return lsd_fail(h, LSD_ERR_SHAPE, "retime variant %d, frame %d: tap %d src %d is outside %d..%d", k, t, i, v[e].src[i], -T, 2 * T - 1);
+      if (v[e].weight[i] < 0)
+        return lsd_fail(h, LSD_ERR_ARG, "retime variant %d, frame %d: tap %d has a negative weight %d", k, t, i, v[e].weight[i]);
+      sum += v[e].weight[i];
+    }
+    if (sum != LSD_RETIME_ONE)
+      return lsd_fail(h, LSD_ERR_ARG, "retime variant %d, frame %d: weights sum to %lld, not %d", k, t, (long long)sum, LSD_RETIME_ONE);
+  }
+  static_assert(sizeof(lsd_retime) == 8 * sizeof(int32_t), "lsd_retime is eight packed int32");
+  const int32_t* p = reinterpret_cast<const int32_t*>(v);
+  h->variant_tab_host.assign(p, p + retime_tables_ints(K, T));
+  return 0;
+}
+}  // namespace
+
+extern "C" size_t lsd_score_retimes_workspace_bytes(lsd_handle* h, int batch, int K, int T, int H, int W, int F, int Ta, int precision) {
+  if (batch < 1 || K < 1 || K > LSD_MAX_RETIMES || T < 1) return 0;
+  return variant_workspace_bytes(h, retime_tables_ints(K, T) * sizeof(int32_t), batch, T, H, W, F, Ta, precision);
+}
+
+extern "C" int lsd_score_retimes(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                 const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full,
+                                 int total_v_frames, int Ta, const lsd_retime* variants, int K, int precision, int batch,
+                                 float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_retimes: no weights loaded");
+  const int rc = retime_tables_checked(h, "lsd_score_retimes", variants, K, T, H, W);
+  if (rc) return rc;
+  if ((int64_t)n_windows * K * T > INT32_MAX)
+    return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d retime variants: too many frames for one call", n_windows, K);
+  const size_t tab_bytes = h->variant_tab_host.size() * sizeof(int32_t);
+  const VariantBuilder retime = [&](const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* pseudo, cudaStream_t st) {
+    launch_retime_windows(track, n_frames, d_wins, d_tabs, K, r0, nb, T, H, W, pseudo, st);
+  };
+  return score_window_variants(h, "lsd_score_retimes", "retime variants", track, n_frames, H, W, starts_host, audio_starts_host, n_windows,
+                               T, mel_full, F, Ta_full, total_v_frames, Ta, K, precision, batch, logits_out, workspace, workspace_bytes,
+                               stream, h->variant_tab_host.data(), tab_bytes, tab_bytes, retime);
+}
+
+// The retimed windows themselves, written to a caller buffer by the builder lsd_score_retimes uses.
+extern "C" size_t lsd_retime_windows_workspace_bytes(int n_windows, int K, int T, int H, int W) {
+  if (n_windows < 1 || K < 1 || K > LSD_MAX_RETIMES || T < 1 || H < 1 || W < 1) return 0;
+  return built_windows_workspace_bytes(retime_tables_ints(K, T) * sizeof(int32_t), n_windows);
+}
+
+extern "C" int lsd_retime_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host, int n_windows,
+                                  int T, const lsd_retime* variants, int K, uint8_t* out, void* workspace, size_t workspace_bytes,
+                                  void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  int rc = retime_tables_checked(h, "lsd_retime_windows", variants, K, T, H, W);
+  if (rc) return rc;
+  if (n_windows == 0) return LSD_OK;
+  if (!track || !starts_host || !out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_retime_windows: null pointer argument");
+  if (n_windows < 0 || n_frames < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_retime_windows: bad extents");
+  if ((int64_t)n_windows * K * T > INT32_MAX)
+    return lsd_fail(h, LSD_ERR_SHAPE, "%d windows x %d retime variants: too many frames for one call", n_windows, K);
+  if ((rc = check_windows(h, starts_host, n_windows, T, n_frames))) return rc;
+  const size_t need = lsd_retime_windows_workspace_bytes(n_windows, K, T, H, W);
+  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  const VariantBuilder retime = [&](const int32_t* d_tabs, const int32_t* d_wins, int r0, int nb, uint8_t* o, cudaStream_t st) {
+    launch_retime_windows(track, n_frames, d_wins, d_tabs, K, r0, nb, T, H, W, o, st);
+  };
+  return build_window_variants(h, starts_host, n_windows, K, workspace, stream, h->variant_tab_host.data(),
+                               h->variant_tab_host.size() * sizeof(int32_t), out, retime);
 }
 
 // ================================================================================================

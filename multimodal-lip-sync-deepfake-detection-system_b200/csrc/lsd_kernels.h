@@ -85,6 +85,12 @@ size_t resize_tables_ints(int K, int H, int W);
 void resize_tables(const int32_t* hw, int K, int H, int W, int32_t* out);
 cudaError_t resize_windows_device_init();
 bool resize_extents_ok(int H, int W);
+// retimed windows (retime.cu): rows r0 .. r0+nb-1 = (window r / K, variant r % K) -> uint8 pseudo-track out (nb*T, H, W, 3), frame t
+// of row r the Q15 blend of the taps of (variant k, frame t), tap frames clamp(window start + src, 0, n_frames - 1); win_starts:
+// track start of windows r0 / K, r0 / K + 1, ...; tabs: the K*T lsd_retime entries (retime_tables_ints int32), variant-major
+void launch_retime_windows(const uint8_t* track, int n_frames, const int32_t* win_starts, const int32_t* tabs, int K, int r0, int nb,
+                           int T, int H, int W, uint8_t* out, cudaStream_t s);
+size_t retime_tables_ints(int K, int T);
 // mel_full (F, Ta_full) + per-window a_start -> (n, F, Ta) with repeat-last-column padding (predictor.py:525-552)
 void launch_gather_audio(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, float* dst,
                          int n, int Ta, cudaStream_t s);

@@ -15,8 +15,10 @@ Video decode, face tracking, VAD and the gate/verdict block of `_predict_long_vi
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
 import time
+from fractions import Fraction
 from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -1255,6 +1257,287 @@ class Predictor:
         res["sizes"] = sizes
         res["lowest_stable_side"] = _agg.lowest_stable_quality(heights, res["variant_confidence"], res["confidence"], confidence_threshold)
         res["window_starts"] = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
+        return res
+
+    # ------------------------------------------------------------------ temporal robustness (lsd_score_retimes)
+    # A retime variant has one row per output frame t of the window: up to 4 taps (src, weight).  src is a frame offset from the
+    # window's first track frame in -T .. 2T-1 (the library clamps the frame to the track), weights are Q15 integers >= 0 summing to
+    # LSD_RETIME_ONE, and every byte is (sum w_i p_i + 16384) >> 15.  The builders below are pure, run on the CPU and return
+    # (src, weight) int32 arrays of shape (T, 4); rates are exact rationals and every rounding is half up.
+    @staticmethod
+    def _exact_rate(x, what: str) -> Fraction:
+        """`Fraction(x).limit_denominator(1001)`: 15 -> 15, 30000 / 1001 (NTSC, as a float) -> 30000/1001."""
+        q = Fraction(x).limit_denominator(1001)
+        if q <= 0:
+            raise ValueError(f"{what} must be positive, got {x!r}")
+        return q
+
+    @staticmethod
+    def _retime_table(T: int, rows) -> Tuple[np.ndarray, np.ndarray]:
+        """(src, weight) int32 (T, 4) from T lists of (src, weight) taps, unused taps (0, 0); ValueError for a src outside -T .. 2T-1."""
+        src = np.zeros((T, 4), np.int32)
+        wt = np.zeros((T, 4), np.int32)
+        for t, taps in enumerate(rows):
+            for i, (s, w) in enumerate(taps):
+                if not -T <= s <= 2 * T - 1:
+                    raise ValueError(f"frame {t} reads frame offset {s}, outside {-T}..{2 * T - 1}: a rate or length too far out")
+                src[t, i], wt[t, i] = s, w
+        return src, wt
+
+    @staticmethod
+    def _capture_frame(j: int, fps: Fraction, rate: Fraction) -> int:
+        """The window frame that holds capture j of a source capturing at `rate`: floor(j fps / rate + 1/2)."""
+        return math.floor(j * fps / rate + Fraction(1, 2))
+
+    @staticmethod
+    def hold_retime(T: int, fps: float, rate: float) -> Tuple[np.ndarray, np.ndarray]:
+        """A source that captures only at `rate` frames per second, shown at `fps`: frame t shows capture j = floor(t rate / fps),
+        which sits at frame floor(j fps / rate + 1/2), never later than t.  `hold_retime(32, 15, 5)` repeats every third frame
+        three times."""
+        T = int(T)
+        fq, rq = Predictor._exact_rate(fps, "fps"), Predictor._exact_rate(rate, "rate")
+        cap = Predictor._capture_frame
+        return Predictor._retime_table(T, [[(cap(math.floor(t * rq / fq), fq, rq), _cabi.LSD_RETIME_ONE)] for t in range(T)])
+
+    @staticmethod
+    def blend_retime(T: int, fps: float, rate: float) -> Tuple[np.ndarray, np.ndarray]:
+        """Blended frame-rate conversion from `rate` to `fps` (ghosting): frame t is the linear blend of captures j and j + 1 at the
+        fraction f = x - j, x = t rate / fps, j = floor(x); w1 = floor(f 32768 + 1/2), w0 = 32768 - w1, one tap when w1 == 0.  The
+        captures sit at the frames of `hold_retime`."""
+        T = int(T)
+        fq, rq = Predictor._exact_rate(fps, "fps"), Predictor._exact_rate(rate, "rate")
+        cap = Predictor._capture_frame
+        rows = []
+        for t in range(T):
+            x = t * rq / fq
+            j = math.floor(x)
+            w1 = math.floor((x - j) * _cabi.LSD_RETIME_ONE + Fraction(1, 2))
+            rows.append([(cap(j, fq, rq), _cabi.LSD_RETIME_ONE)] if w1 == 0 else
+                        [(cap(j, fq, rq), _cabi.LSD_RETIME_ONE - w1), (cap(j + 1, fq, rq), w1)])
+        return Predictor._retime_table(T, rows)
+
+    @staticmethod
+    def freeze_retime(T: int, at: int, length: int) -> Tuple[np.ndarray, np.ndarray]:
+        """A stall that resumes live: frames at .. at + length - 1 show frame at - 1, every other frame t shows itself."""
+        T, at, length = int(T), int(at), int(length)
+        if at < 0 or length < 0:
+            raise ValueError(f"freeze at {at} for {length} frames: both must be >= 0")
+        return Predictor._retime_table(T, [[(at - 1 if at <= t < at + length else t, _cabi.LSD_RETIME_ONE)] for t in range(T)])
+
+    @staticmethod
+    def drop_retime(T: int, every: int, repeat: bool = True) -> Tuple[np.ndarray, np.ndarray]:
+        """Every `every`-th source frame (s with (s + 1) % every == 0) is lost.  repeat=True: the previous frame is shown in its
+        place, which keeps time.  repeat=False: the next frames are shown early, frame t shows the t-th source frame that is not
+        lost, so the video drifts ahead of the audio by one frame per loss."""
+        T, every = int(T), int(every)
+        if every < 2:
+            raise ValueError(f"drop every {every}-th frame: expected >= 2")
+        if repeat:
+            src: List[int] = []
+            for t in range(T):
+                src.append(src[-1] if (t + 1) % every == 0 else t)
+        else:
+            src = [s for s in range(2 * T) if (s + 1) % every != 0][:T]
+        return Predictor._retime_table(T, [[(s, _cabi.LSD_RETIME_ONE)] for s in src])
+
+    @staticmethod
+    def exposure_retime(T: int, n: int) -> Tuple[np.ndarray, np.ndarray]:
+        """Motion smear of an n-frame exposure, 2 <= n <= 4: frame t is the mean of frames t - c .. t - c + n - 1, c = (n - 1) // 2,
+        each of weight 32768 // n, the remainder on tap c (frame t)."""
+        T, n = int(T), int(n)
+        if not 2 <= n <= 4:
+            raise ValueError(f"exposure over {n} frames: expected 2..4")
+        c, w = (n - 1) // 2, _cabi.LSD_RETIME_ONE // n
+        rem = _cabi.LSD_RETIME_ONE - n * w
+        return Predictor._retime_table(T, [[(t - c + i, w + (rem if i == c else 0)) for i in range(n)] for t in range(T)])
+
+    @staticmethod
+    def loss_retime(T: int, rate: float, burst: float, seed: int = 0) -> Tuple[np.ndarray, np.ndarray]:
+        """Bursty frame loss (Gilbert-Elliott): a good / bad channel, P(bad -> good) = 1 / burst and P(good -> bad) =
+        rate / (burst (1 - rate)), so `rate` of the frames are lost in bursts of `burst` frames on average.  Frame 0 is always
+        received; frame t >= 1 draws one `np.random.default_rng(seed).random()` for its transition, and a lost frame shows the last
+        received one.  Deterministic for a seed."""
+        T, rate, burst = int(T), float(rate), float(burst)
+        if not (0.0 <= rate < 1.0 and burst >= 1.0):
+            raise ValueError(f"loss rate {rate} with bursts of {burst}: expected 0 <= rate < 1, burst >= 1")
+        p_gb, p_bg = rate / (burst * (1.0 - rate)), 1.0 / burst
+        if p_gb > 1.0:
+            raise ValueError(f"loss rate {rate} with bursts of {burst}: P(good -> bad) = {p_gb:.3f} > 1")
+        g = np.random.default_rng(int(seed))
+        good, last, src = True, 0, [0]
+        for t in range(1, T):
+            u = g.random()
+            good = (u >= p_gb) if good else (u < p_bg)
+            if good:
+                last = t
+            src.append(last)
+        return Predictor._retime_table(T, [[(s, _cabi.LSD_RETIME_ONE)] for s in src])
+
+    @staticmethod
+    def temporal_variants(T: int, fps: float = 15.0) -> Tuple[List[str], List[Tuple[np.ndarray, np.ndarray]], List[Optional[int]]]:
+        """The default ladder of `temporal_track`: names, (src, weight) tables and the hold rate of each variant (None for the
+        others).  The plain window (`none`); captures held from 12, 10, 8, 6 and 5 fps (`hold12` .. `hold5`) and blended from 10 fps
+        (`blend10`), each only when its rate is below `fps`; stalls of 4 and 10 frames at T // 2 (`freeze4`, `freeze10`); 10 % bursty
+        loss with bursts of 3 frames, seed 0 (`loss10`); every 8th frame dropped without a repeat, so the video runs ahead of the
+        audio (`drift8`: 4 frames by the last frame of a 32-frame window); a 3-frame exposure (`exposure3`).  K = 12 at 15 fps."""
+        T = int(T)
+        P = Predictor
+        fq = P._exact_rate(fps, "fps")
+        names, tabs, rates = ["none"], [P._retime_table(T, [[(t, _cabi.LSD_RETIME_ONE)] for t in range(T)])], [None]
+        for r in (12, 10, 8, 6, 5):
+            if r < fq:
+                names.append(f"hold{r}")
+                tabs.append(P.hold_retime(T, fps, r))
+                rates.append(r)
+        if 10 < fq:
+            names.append("blend10")
+            tabs.append(P.blend_retime(T, fps, 10))
+            rates.append(None)
+        rest = [("freeze4", P.freeze_retime(T, T // 2, 4)), ("freeze10", P.freeze_retime(T, T // 2, 10)),
+                ("loss10", P.loss_retime(T, 0.10, 3, 0)), ("drift8", P.drop_retime(T, 8, repeat=False)),
+                ("exposure3", P.exposure_retime(T, 3))]
+        for name, tab in rest:
+            names.append(name)
+            tabs.append(tab)
+            rates.append(None)
+        return names, tabs, rates
+
+    def _retime_args(self, track_u8: torch.Tensor, starts: Sequence[int], variants):
+        """Checks what `lsd_score_retimes` / `lsd_retime_windows` would reject, as ValueError; returns (K, the K*T entries as
+        lsd_retime).  A variant is `(src, weight)` of shape (T, n), 1 <= n <= 4, or a bare (T,) src array: one full-weight tap."""
+        if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
+            raise ValueError(f"track must be uint8 (n_frames, H, W, 3), got {track_u8.dtype} {tuple(track_u8.shape)}")
+        n_frames = int(track_u8.shape[0])
+        T = self.chunk_size
+        vs = list(variants)
+        if not 1 <= len(vs) <= _cabi.LSD_MAX_RETIMES:
+            raise ValueError(f"{len(vs)} retime variants: expected 1 to {_cabi.LSD_MAX_RETIMES}")
+        tab = np.zeros((len(vs), T, 8), np.int32)
+        for k, v in enumerate(vs):
+            if isinstance(v, (tuple, list)) and len(v) == 2 and np.ndim(v[0]) == 2:
+                src, wt = np.asarray(v[0]), np.asarray(v[1])
+            else:
+                src = np.asarray(v)
+                if src.ndim != 1:
+                    raise ValueError(f"retime variant {k}: expected (src, weight) of shape (T, n) or a (T,) src array, got shape {src.shape}")
+                src = src[:, None]
+                wt = np.full(src.shape, _cabi.LSD_RETIME_ONE, np.int64)
+            if src.shape != wt.shape or src.shape[0] != T or not 1 <= src.shape[1] <= 4:
+                raise ValueError(f"retime variant {k}: src {src.shape} and weight {wt.shape} must both be ({T}, n), 1 <= n <= 4")
+            if src.dtype.kind not in "iu" or wt.dtype.kind not in "iu":
+                raise ValueError(f"retime variant {k}: src and weight must be integers, got {src.dtype} and {wt.dtype}")
+            src, wt = src.astype(np.int64), wt.astype(np.int64)
+            if src.min() < -T or src.max() > 2 * T - 1:
+                raise ValueError(f"retime variant {k}: src must lie in {-T}..{2 * T - 1}, got {src.min()}..{src.max()}")
+            if wt.min() < 0:
+                raise ValueError(f"retime variant {k}: negative weight {wt.min()}")
+            bad = np.nonzero(wt.sum(axis=1) != _cabi.LSD_RETIME_ONE)[0]
+            if len(bad):
+                raise ValueError(f"retime variant {k}, frame {bad[0]}: weights sum to {wt[bad[0]].sum()}, not {_cabi.LSD_RETIME_ONE}")
+            tab[k, :, : src.shape[1]] = src
+            tab[k, :, 4: 4 + src.shape[1]] = wt
+        for i, s in enumerate(starts):
+            if not 0 <= int(s) <= n_frames - T:
+                raise ValueError(f"window {i} [{int(s)},{int(s) + T}) is outside the {n_frames}-frame track")
+        if len(starts) * len(vs) * T > 2 ** 31 - 1:
+            raise ValueError(f"{len(starts)} windows x {len(vs)} retime variants: too many frames for one call")
+        return len(vs), (_cabi.LsdRetime * (len(vs) * T)).from_buffer_copy(tab.tobytes())
+
+    def score_track_retimes(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int, variants,
+                            chunk_a_size: int = 128, audio_starts_from: Optional[Sequence[int]] = None) -> torch.Tensor:
+        """`score_track_logits` with K retimed copies of every window (`lsd_score_retimes`).  `variants`: up to 64 retime tables,
+        each `(src, weight)` of shape (T, n), 1 <= n <= 4, or a bare (T,) src array (one full-weight tap per frame), as the
+        `*_retime` builders return them.  Frame t of variant k is the Q15 blend of its taps, tap frames clamp(start + src, 0,
+        n_frames - 1) of the track, built on the device.  Returns fp32 logits `(n, K)` on the device; entry (i, k) is bit for bit
+        the logit of window i retimed by variant k, with window i's audio slice: only the video is retimed."""
+        if mel_full.dim() != 3 or mel_full.shape[0] != 1:
+            raise ValueError(f"mel_full must be (1, F, T_full), got {tuple(mel_full.shape)}")
+        K, vc = self._retime_args(track_u8, starts, variants)
+        n = len(starts)
+        if audio_starts_from is not None and len(audio_starts_from) != n:
+            raise ValueError("audio_starts_from must have one entry per window")
+        m = self.model
+        dev = m._device()
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T = self.chunk_size
+        logits = torch.empty(n, K, dtype=torch.float32, device=dev)
+        if n == 0:
+            return logits
+        track_u8 = track_u8.contiguous()
+        mel_full = mel_full.to(torch.float32).contiguous()
+        F_, Ta_full = int(mel_full.shape[1]), int(mel_full.shape[2])
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            prec = m._precision()
+            batch = min(self.batch_size, n * K)
+            need = L.lsd_score_retimes_workspace_bytes(h.ptr, batch, K, T, H, W, F_, chunk_a_size, prec)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            if n * K > batch and prec == _cabi.LSD_PREC_BF16:
+                need = 2 * need      # a double workspace lets the batches overlap as in score_track_logits
+            ws = m._workspace(need, dev)
+            st = (C.c_int32 * n)(*[int(s) for s in starts])
+            ast = None
+            if audio_starts_from is not None:
+                ast = (C.c_int32 * n)(*[self._audio_start(int(v), Ta_full, int(total_v_frames), chunk_a_size) for v in audio_starts_from])
+            rc = L.lsd_score_retimes(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, T, mel_full.data_ptr(), F_, Ta_full,
+                                     int(total_v_frames), chunk_a_size, vc, K, prec, batch, logits.data_ptr(), ws.data_ptr(),
+                                     ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return logits
+
+    def retime_track_windows(self, track_u8: torch.Tensor, starts: Sequence[int], variants) -> torch.Tensor:
+        """The retimed windows `score_track_retimes` scores, built by the same kernel (`lsd_retime_windows`): uint8
+        `(n, K, T, H, W, 3)` on the device, window i under variant k at [i, k].  To look at what a retiming does to a window."""
+        K, vc = self._retime_args(track_u8, starts, variants)
+        m = self.model
+        dev = m._device()
+        n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
+        T, n = self.chunk_size, len(starts)
+        out = torch.empty((n, K, T, H, W, 3), dtype=torch.uint8, device=dev)
+        if n == 0:
+            return out
+        track_u8 = track_u8.contiguous()
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            need = L.lsd_retime_windows_workspace_bytes(n, K, T, H, W)
+            ws = torch.empty(max(int(need), 1), dtype=torch.uint8, device=dev)
+            rc = L.lsd_retime_windows(h.ptr, track_u8.data_ptr(), n_frames, H, W, (C.c_int32 * n)(*[int(s) for s in starts]), n, T, vc,
+                                      K, out.data_ptr(), ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return out
+
+    def temporal_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                       fps: float = 15.0, confidence_threshold: float = 0.5,
+                       audio_starts_from: Optional[Sequence[int]] = None) -> Dict[str, Any]:
+        """Temporal robustness of a track's verdict: one `score_track_retimes` call with the `temporal_variants` of the track's
+        `fps`, the calibrated P(real) summarised by `aggregate.augmentation_stability` (column 0, the plain window, is the identity):
+          `variants`: the variant names (column order); `rates`: the hold rate of each variant, None for the others;
+          `confidence`, `variant_confidence`, `tta_confidence`, `window_spread`, `decision_flip_rate`, `verdict_stable`: as in
+          `robustness_track`;
+          `lowest_stable_fps`: the lowest hold rate r such that every hold variant of rate >= r keeps the plain confidence's side of
+          `confidence_threshold` (`aggregate.lowest_stable_quality` on `rates`), None when the highest rate already flips it or no
+          rate is below `fps`;
+          `window_starts`: the windows' first frames (those of `audio_starts_from` when given: absolute video frames).
+        Frames just outside a window are read from the track, so give the whole track.  It reports only: nothing here enters a
+        verdict."""
+        names, tabs, rates = self.temporal_variants(self.chunk_size, fps)
+        logits = self.score_track_retimes(track_u8, starts, mel_full, total_v_frames, tabs, audio_starts_from=audio_starts_from)
+        return self._temporal_report(logits.cpu().numpy(), names, rates, confidence_threshold,
+                                     audio_starts_from if audio_starts_from is not None else starts)
+
+    def _temporal_report(self, logits: np.ndarray, names: List[str], rates: List[Optional[int]], confidence_threshold: float,
+                         window_starts: Sequence[int]) -> Dict[str, Any]:
+        """`temporal_track`'s dict from (n, K) logits of the `temporal_variants` columns `names` / `rates`."""
+        probs = np.array([self._calibrate(float(x)) for x in np.asarray(logits).flatten().tolist()],
+                         dtype=np.float64).reshape(len(window_starts), len(names))
+        res = _agg.augmentation_stability(probs, confidence_threshold, self.confidence_smoothing, self.trim_ratio)
+        res["variants"] = names
+        res["rates"] = rates
+        res["lowest_stable_fps"] = _agg.lowest_stable_quality(rates, res["variant_confidence"], res["confidence"], confidence_threshold)
+        res["window_starts"] = [int(s) for s in window_starts]
         return res
 
     # ------------------------------------------------------------------ audio robustness (lsd_degrade_audio, lsd_score_audio_clips)
