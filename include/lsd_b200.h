@@ -145,6 +145,34 @@ int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, 
  * only its own span of a sharded track passes span-relative `starts` and the audio starts computed from the absolute frame
  * indices (SURVEY.md §8e); NULL = computed here from `starts` as predictor.py:540-547 does. */
 
+/* ---- branch attribution: Shapley values of the head's four inputs ------------------------------------------------- */
+/* This entry has no reference counterpart.  The classifier head (artifact_detector.py:142-147, classifier.py:14-34) reads one
+ * 448-wide row per window, [cls 256 | raw 64 | delta 64 | hf 64]: the temporal transformer's CLS output (the only path of the
+ * audio), the temporal-inconsistency features of layer4's map and of its frame-to-frame difference, and the high-frequency
+ * features of the pixels.  The four slices are the players sync, raw, delta, hf = bits 0..3 of a coalition mask S.
+ * lsd_score_branch_features is lsd_score_windows (same arguments, same workspace: lsd_score_workspace_bytes) that also writes
+ * every window's head input row to feats_out (device fp32, (n_windows, LSD_BRANCH_FEATURES)); its logits are bit for bit those
+ * of lsd_score_windows. */
+#define LSD_BRANCHES 4
+#define LSD_BRANCH_FEATURES 448
+#define LSD_MAX_BACKGROUND 256
+int lsd_score_branch_features(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W,
+                              const int32_t* starts_host, const int32_t* audio_starts_host_or_null, int n_windows, int T,
+                              const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                              int precision, int batch, float* logits_out, float* feats_out,
+                              void* workspace, size_t workspace_bytes, void* stream);
+/* Hybrid row x^{S,j}: slice p from window row x_i when bit p of S is set, from background row b_j otherwise (the cls slice
+ * everywhere the head reads cls).  v_i(S) = (1/M) sum_j f(x^{S,j}), f the head in logit space; v_i(15) = f(x_i).
+ * phi_i,p = sum over S without p, in ascending mask order, of w_|S| (v_i(S | p) - v_i(S)), w = (1/4, 1/12, 1/12, 1/4), so
+ * sum_p phi_i,p = v_i(15) - v_i(0).  feats: device (n, 448); background: device (M, 448), 1 <= M <= LSD_MAX_BACKGROUND;
+ * values_out: device (n, 16), column S = v_i(S); phi_out: device (n, 4).  fp32 FFMA throughout; the bits depend neither on n nor
+ * on how the windows are split over calls.  Checked before any launch: LSD_ERR_ARG for a null pointer, LSD_ERR_WEIGHTS without
+ * weights, LSD_ERR_SHAPE for n < 0, M outside 1..LSD_MAX_BACKGROUND or n*(15M+1) rows above INT32_MAX, LSD_ERR_WORKSPACE for a
+ * workspace below lsd_branch_attribution_workspace_bytes(n, M) (0 for bad extents). */
+size_t lsd_branch_attribution_workspace_bytes(int n, int M);
+int lsd_branch_attribution(lsd_handle* h, const float* feats, int n, const float* background, int M, float* values_out, float* phi_out,
+                           void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- audio-offset sweep: one visual-encoder pass, K audio windows per video ------------------------------------ */
 /* The reference trains with torch.roll-shifted audio as sync negatives (train.py:169-182), so its logit as a function of the
  * audio offset is a sync profile: a real clip with a constant A/V delay peaks away from offset 0, a lip-sync fake has no clear

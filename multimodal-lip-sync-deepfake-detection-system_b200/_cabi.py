@@ -30,6 +30,9 @@ LSD_RETIME_ONE = 32768
 LSD_MAX_RETIMES = 64
 LSD_AD_REVERB, LSD_AD_NOISE, LSD_AD_CLIP, LSD_AD_BAND, LSD_AD_MULAW = 1, 2, 4, 8, 16
 LSD_MAX_AUDIO_DEGRADATIONS = LSD_MAX_AUDIO_VARIANTS
+LSD_BRANCHES = 4
+LSD_BRANCH_FEATURES = 448
+LSD_MAX_BACKGROUND = 256
 
 # every symbol include/lsd_b200.h declares (checked by tests/test_cabi.py)
 EXPORTS = [
@@ -48,6 +51,7 @@ EXPORTS = [
     "lsd_score_resizes_workspace_bytes", "lsd_score_resizes", "lsd_resize_tables", "lsd_resize_windows_workspace_bytes", "lsd_resize_windows",
     "lsd_score_retimes_workspace_bytes", "lsd_score_retimes", "lsd_retime_windows_workspace_bytes", "lsd_retime_windows",
     "lsd_degrade_audio_workspace_bytes", "lsd_degrade_audio", "lsd_score_audio_clips_workspace_bytes", "lsd_score_audio_clips",
+    "lsd_score_branch_features", "lsd_branch_attribution_workspace_bytes", "lsd_branch_attribution",
 ]
 
 
@@ -200,6 +204,11 @@ def lib() -> C.CDLL:
         L.lsd_retime_windows_workspace_bytes.argtypes = [i, i, i, i, i]; L.lsd_retime_windows_workspace_bytes.restype = sz
         L.lsd_retime_windows.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), i, i, C.POINTER(LsdRetime), i, vp, vp, sz, vp]
         L.lsd_retime_windows.restype = i
+        L.lsd_score_branch_features.argtypes = [vp, vp, i, i, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32), i, i, vp, i, i, i, i, i, i,
+                                                vp, vp, vp, sz, vp]
+        L.lsd_score_branch_features.restype = i
+        L.lsd_branch_attribution_workspace_bytes.argtypes = [i, i]; L.lsd_branch_attribution_workspace_bytes.restype = sz
+        L.lsd_branch_attribution.argtypes = [vp, vp, i, vp, i, vp, vp, vp, sz, vp]; L.lsd_branch_attribution.restype = i
         L.lsd_degrade_audio_workspace_bytes.argtypes = [i64, i]; L.lsd_degrade_audio_workspace_bytes.restype = sz
         L.lsd_degrade_audio.argtypes = [vp, vp, i64, C.POINTER(LsdAudioDegradation), i, vp, vp, sz, vp]; L.lsd_degrade_audio.restype = i
         L.lsd_score_audio_clips_workspace_bytes.argtypes = [vp, i, i, i, i, i, i, i, i]; L.lsd_score_audio_clips_workspace_bytes.restype = sz

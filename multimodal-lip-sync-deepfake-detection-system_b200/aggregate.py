@@ -96,6 +96,55 @@ def columns_to_frames(first_col: int, values: Sequence[Optional[float]], Ta_full
     return first, [float(t / c) if c else None for t, c in zip(total, count)]
 
 
+BRANCHES = ("sync", "raw", "delta", "hf")
+
+
+def branch_attribution_summary(phi, probs, confidence_threshold: float = 0.5, smoothing: str = "median", trim_ratio: float = 0.1,
+                               starts: Optional[Sequence[int]] = None, T: int = 32) -> Dict[str, Any]:
+    """Summary of branch attributions (`Predictor.attribution_track`).  `phi`: (n_windows, 4) Shapley values in logit space of the
+    branches `BRANCHES` (> 0 pushes a window toward real); `probs`: (n_windows,) calibrated P(real).  A window is decided real when
+    P(real) >= `confidence_threshold`.
+      `mean_phi`, `median_phi` (4,): per branch over the windows;
+      `share` (4,): each branch's mean |phi| over the sum of the four (zeros when every phi is 0);
+      `leading_branch` (n,): per window, the branch with the most positive phi when it is decided real, the most negative when
+        it is decided fake;
+      `confidence`, `verdict`: the robust aggregate of `probs` (`_robust`, predictor.py:246-260) and its side of the threshold;
+      `verdict_driver`: the branch whose mean phi pushes hardest toward that verdict (largest for "real", smallest for "fake");
+        None without windows;
+      `frame_first`, `frame_timeline`: with `starts` (first frame of every window, T frames each), per branch the per-frame mean
+        of phi over the windows covering the frame (`frame_evidence_timeline` with one segment per window)."""
+    p = np.asarray(phi, dtype=np.float64)
+    if p.ndim != 2 or p.shape[1] != len(BRANCHES):
+        raise ValueError(f"phi must be (n_windows, {len(BRANCHES)}), got shape {p.shape}")
+    pr = np.asarray(probs, dtype=np.float64).reshape(-1)
+    if pr.shape[0] != p.shape[0]:
+        raise ValueError(f"probs has {pr.shape[0]} entries for {p.shape[0]} windows")
+    thr = float(confidence_threshold)
+    n = p.shape[0]
+    mean_phi = p.mean(axis=0) if n else np.zeros(len(BRANCHES))
+    median_phi = np.median(p, axis=0) if n else np.zeros(len(BRANCHES))
+    mag = np.abs(p).mean(axis=0) if n else np.zeros(len(BRANCHES))
+    share = mag / mag.sum() if mag.sum() > 0 else np.zeros(len(BRANCHES))
+    real = pr >= thr
+    leading = [BRANCHES[int(np.argmax(p[i]) if real[i] else np.argmin(p[i]))] for i in range(n)]
+    conf = _robust(pr.tolist(), smoothing, trim_ratio)
+    verdict = "real" if conf >= thr else "fake"
+    driver = None
+    if n:
+        driver = BRANCHES[int(np.argmax(mean_phi) if verdict == "real" else np.argmin(mean_phi))]
+    res = {"mean_phi": mean_phi, "median_phi": median_phi, "share": share, "leading_branch": leading, "confidence": conf,
+           "verdict": verdict, "verdict_driver": driver}
+    if starts is not None:
+        if len(starts) != n:
+            raise ValueError(f"starts has {len(starts)} entries for {n} windows")
+        timeline = {}
+        first = 0
+        for b, name in enumerate(BRANCHES):
+            first, timeline[name] = frame_evidence_timeline(starts, p[:, b:b + 1], int(T), int(T))
+        res["frame_first"], res["frame_timeline"] = first, timeline
+    return res
+
+
 def augmentation_stability(probs, confidence_threshold: float = 0.5, smoothing: str = "median", trim_ratio: float = 0.1,
                            identity: int = 0) -> Dict[str, Any]:
     """Stability of a verdict under K variants of every window (`Predictor.robustness_track`).  `probs`: (n_windows, K) P(real);

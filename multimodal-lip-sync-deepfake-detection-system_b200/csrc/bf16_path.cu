@@ -1402,9 +1402,11 @@ static size_t dtype_bytes(int dt) { return dt == LSD_F32 ? 4 : (dt == LSD_U8 ? 1
 // pipe_parity >= 0 (lsd_score_windows with a double workspace): everything after the visual encoder is enqueued on
 // h->tail_stream, ordered after the encoder by ev_front[parity]; ev_tail_done[parity] marks the batch's logits complete.
 // vt != nullptr: shared-visual forward (see VarTail); requires the fused token path (variants_shared_route) and no aux.
+// feats_out (not with vt): row n receives the head's input row of window n, [cls | comb[:, 256:448]].
 static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, const lsd_aux* aux, char* ws, size_t ws_bytes,
                              cudaStream_t st, bool inputs_ready, const void* video, int vdt, int vlayout, const void* audio, int adt,
-                             const int32_t* vstarts = nullptr, int n_frames = 0, int pipe_parity = -1, const VarTail* vt = nullptr) {
+                             const int32_t* vstarts = nullptr, int n_frames = 0, int pipe_parity = -1, const VarTail* vt = nullptr,
+                             float* feats_out = nullptr) {
   BPlan P;
   build_plan(s, P);
   if (P.f32.cursor > ws_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", P.f32.cursor, ws_bytes);
@@ -1635,6 +1637,10 @@ static int forward_bf16_impl(lsd_handle* h, const Shapes& s, float* logits, cons
   cudaStreamWaitEvent(st, h->ev_join, 0);   // artifact features (comb[:, 256:448]) are complete
   // ---- artifact fusion MLP + classification head, fused, fp32 (artifact_detector.py:142-147,180-181; classifier.py:14-34)
   launch_head(tok, (int64_t)NT * 256, comb, hw, logits, B, st);
+  if (feats_out) {   // on the head's stream, before ev_tail_done: the pipelined tails reuse this workspace half afterwards
+    launch_copy_rows(tok, (int64_t)NT * 256, feats_out, LSD_BRANCH_FEATURES, B, 256, st);
+    launch_copy_rows(comb + 256, 448, feats_out + 256, LSD_BRANCH_FEATURES, B, 192, st);
+  }
   g_tl.mark(st, "T:head");
   g_tl.dump();
   if (aux) {
@@ -1766,7 +1772,7 @@ int forward_bf16(lsd_handle* h, int B, int T, int H, int W, int F, int Ta, const
 
 int score_batch_bf16(lsd_handle* h, const uint8_t* track, int n_frames, const int32_t* d_vstarts, const int32_t* d_astarts,
                      const float* mel_full, int Ta_full, int nb, int T, int H, int W, int F, int Ta, float* logits, char* ws,
-                     size_t ws_bytes, cudaStream_t st, int pipe_parity) {
+                     size_t ws_bytes, cudaStream_t st, int pipe_parity, float* feats_out) {
   Shapes s;
   int rc = make_shapes(h, nb, T, H, W, F, Ta, s);
   if (rc) return rc;
@@ -1776,9 +1782,10 @@ int score_batch_bf16(lsd_handle* h, const uint8_t* track, int n_frames, const in
   BCtx b{h, ws, &P, st};
   launch_gather_audio(mel_full, F, Ta_full, d_astarts, b.f("aud"), nb, Ta, st);
   if (video_rows_bulk_ok(track, LSD_U8, LSD_NDHWC, W))
-    return forward_bf16_impl(h, s, logits, nullptr, ws, ws_bytes, st, true, track, LSD_U8, LSD_NDHWC, nullptr, 0, d_vstarts, n_frames, pipe_parity);
+    return forward_bf16_impl(h, s, logits, nullptr, ws, ws_bytes, st, true, track, LSD_U8, LSD_NDHWC, nullptr, 0, d_vstarts, n_frames, pipe_parity,
+                             nullptr, feats_out);
   launch_gather_windows_u8(track, n_frames, d_vstarts, b.f("vid"), nb, T, H * W * 3, st);
-  return forward_bf16_impl(h, s, logits, nullptr, ws, ws_bytes, st, true, nullptr, 0, 0, nullptr, 0, nullptr, 0, pipe_parity);
+  return forward_bf16_impl(h, s, logits, nullptr, ws, ws_bytes, st, true, nullptr, 0, 0, nullptr, 0, nullptr, 0, pipe_parity, nullptr, feats_out);
 }
 
 // ---- shared-visual forward (lsd_forward_audio_variants / lsd_score_offsets)

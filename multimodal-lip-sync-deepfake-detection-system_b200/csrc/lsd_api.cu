@@ -17,6 +17,7 @@
 #include "tok_fused.cuh"
 #include "stem_ring.cuh"
 #include "umma_conv.cuh"
+#include "token_kernels.cuh"
 using namespace lsd;
 
 static thread_local std::string g_create_error;
@@ -90,6 +91,7 @@ extern "C" int lsd_create(lsd_handle** out, int device) {
     if (ce == cudaSuccess) ce = lsd::warp_windows_device_init();
     if (ce == cudaSuccess) ce = lsd::jpeg_windows_device_init();
     if (ce == cudaSuccess) ce = lsd::resize_windows_device_init();
+    if (ce == cudaSuccess) ce = lsd::attribution_device_init();
     if (ce != cudaSuccess) rc = lsd_fail(h, LSD_ERR_CUDA, "lsd_create: kernel attribute setup: %s", cudaGetErrorString(ce));
   }
   if (rc != 0) { g_create_error = h->err; delete h; return rc; }
@@ -482,10 +484,11 @@ namespace {
 using BatchTrack = std::function<int(int r0, int nb, const uint8_t*& track, int& n_frames)>;
 
 // The batch loop of lsd_score_windows, shared with score_window_variants.  h->idx_host holds the first track frame of row r at [r]
-// and its first mel column at [n_rows + r]; the caller has checked every argument and the workspace size.
+// and its first mel column at [n_rows + r]; the caller has checked every argument and the workspace size.  feats_out (optional):
+// row r receives the head's input row of row r, [cls | comb[:, 256:448]] (LSD_BRANCH_FEATURES floats).
 int score_rows(lsd_handle* h, const uint8_t* track, int n_frames, int n_rows, int T, int H, int W, const float* mel_full, int F,
                int Ta_full, int Ta, int precision, int batch, float* logits_out, void* workspace, size_t workspace_bytes,
-               cudaStream_t st, const BatchTrack& batch_track) {
+               cudaStream_t st, const BatchTrack& batch_track, float* feats_out = nullptr) {
   int rc = 0;
   const size_t idx_bytes = ((size_t)batch * sizeof(int32_t) + 255) & ~size_t(255);
   char* ws = reinterpret_cast<char*>(workspace);
@@ -507,11 +510,12 @@ int score_rows(lsd_handle* h, const uint8_t* track, int n_frames, int n_rows, in
     CUDA_OK(h, cudaMemcpyAsync(d_vs, &h->idx_host[w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     CUDA_OK(h, cudaMemcpyAsync(d_as, &h->idx_host[n_rows + w0], nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     if (batch_track && (rc = batch_track(w0, nb, track, n_frames))) return rc;
+    float* feats_b = feats_out ? feats_out + (size_t)w0 * LSD_BRANCH_FEATURES : nullptr;
     if (precision == LSD_PREC_BF16) {
       if (pipelined) rc = score_batch_bf16(h, track, n_frames, d_vs, d_as, mel_full, Ta_full, nb, T, H, W, F, Ta, logits_out + w0,
-                                           fws + (size_t)parity * fw_bytes, fw_bytes, st, parity);
+                                           fws + (size_t)parity * fw_bytes, fw_bytes, st, parity, feats_b);
       else rc = score_batch_bf16(h, track, n_frames, d_vs, d_as, mel_full, Ta_full, nb, T, H, W, F, Ta, logits_out + w0, fws,
-                                 workspace_bytes - 2 * idx_bytes, st);
+                                 workspace_bytes - 2 * idx_bytes, st, -1, feats_b);
       if (rc) return rc;
     } else {
       Shapes sb;
@@ -525,6 +529,8 @@ int score_rows(lsd_handle* h, const uint8_t* track, int n_frames, int n_rows, in
       launch_gather_audio(mel_full, F, Ta_full, d_as, c.buf("aud"), nb, Ta, st);
       rc = forward_f32(h, sb, pb, fws, nullptr, logits_out + w0, st, true, nullptr, 0, 0, nullptr, 0);
       if (rc) return rc;
+      // comb holds the whole head input row here: [cls (a copy of the token rows) | raw | delta | hf]
+      if (feats_b) CUDA_OK(h, cudaMemcpyAsync(feats_b, c.buf("comb"), (size_t)nb * LSD_BRANCH_FEATURES * sizeof(float), cudaMemcpyDeviceToDevice, st));
     }
   }
   if (pipelined) {   // the caller's stream sees every batch's logits
@@ -543,14 +549,16 @@ int check_windows(lsd_handle* h, const int32_t* starts_host, int n_windows, int 
 }
 }  // namespace
 
-extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
-                                 const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
-                                 int precision, int batch, float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
+namespace {
+// lsd_score_windows and lsd_score_branch_features (feats_out != nullptr)
+int score_windows(lsd_handle* h, const char* fn, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                  const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                  int precision, int batch, float* logits_out, float* feats_out, void* workspace, size_t workspace_bytes, void* stream) {
   if (!h) return LSD_ERR_ARG;
-  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_score_windows: no weights loaded");
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "%s: no weights loaded", fn);
   if (n_windows == 0) return LSD_OK;
-  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_windows: null pointer argument");
-  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "lsd_score_windows: bad extents");
+  if (!track || !starts_host || !mel_full || !logits_out || !workspace) return lsd_fail(h, LSD_ERR_ARG, "%s: null pointer argument", fn);
+  if (batch < 1 || n_windows < 0 || n_frames < 1 || Ta_full < 1) return lsd_fail(h, LSD_ERR_SHAPE, "%s: bad extents", fn);
   if (precision != LSD_PREC_FP32 && precision != LSD_PREC_BF16) return lsd_fail(h, LSD_ERR_ARG, "bad precision %d", precision);
   Shapes s;
   int rc = make_shapes(h, batch, T, H, W, F, Ta, s);
@@ -566,7 +574,72 @@ extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_fram
     h->idx_host[n_windows + i] = (int32_t)base_audio_start(starts_host, audio_starts_host, i, Ta, Ta_full, total_v_frames);
   }
   return score_rows(h, track, n_frames, n_windows, T, H, W, mel_full, F, Ta_full, Ta, precision, batch, logits_out, workspace,
-                    workspace_bytes, reinterpret_cast<cudaStream_t>(stream), BatchTrack());
+                    workspace_bytes, reinterpret_cast<cudaStream_t>(stream), BatchTrack(), feats_out);
+}
+}  // namespace
+
+extern "C" int lsd_score_windows(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                 const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full, int total_v_frames, int Ta,
+                                 int precision, int batch, float* logits_out, void* workspace, size_t workspace_bytes, void* stream) {
+  return score_windows(h, "lsd_score_windows", track, n_frames, H, W, starts_host, audio_starts_host, n_windows, T, mel_full, F, Ta_full,
+                       total_v_frames, Ta, precision, batch, logits_out, nullptr, workspace, workspace_bytes, stream);
+}
+
+// ================================================================================================
+// Branch attribution (attribution.cu): the head's input rows out of the plain scoring loop, then exact Shapley values of its
+// four inputs against a background set
+// ================================================================================================
+extern "C" int lsd_score_branch_features(lsd_handle* h, const uint8_t* track, int n_frames, int H, int W, const int32_t* starts_host,
+                                         const int32_t* audio_starts_host, int n_windows, int T, const float* mel_full, int F, int Ta_full,
+                                         int total_v_frames, int Ta, int precision, int batch, float* logits_out, float* feats_out,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+  if (h && h->loaded && n_windows > 0 && !feats_out) return lsd_fail(h, LSD_ERR_ARG, "lsd_score_branch_features: feats_out is NULL");
+  return score_windows(h, "lsd_score_branch_features", track, n_frames, H, W, starts_host, audio_starts_host, n_windows, T, mel_full, F,
+                       Ta_full, total_v_frames, Ta, precision, batch, logits_out, feats_out, workspace, workspace_bytes, stream);
+}
+
+namespace {
+// Workspace: [projections of the n window rows and M background rows | per-(window, mask, chunk) logit sums | v(15) per window]
+bool attribution_extents_ok(int n, int M) {
+  return n >= 0 && M >= 1 && M <= LSD_MAX_BACKGROUND && (int64_t)n * (15 * (int64_t)M + 1) <= INT32_MAX;
+}
+size_t attribution_partial_floats(int n, int M) { return (size_t)n * 15 * ((M + ATTR_CHUNK - 1) / ATTR_CHUNK); }
+}  // namespace
+
+extern "C" size_t lsd_branch_attribution_workspace_bytes(int n, int M) {
+  if (!attribution_extents_ok(n, M)) return 0;
+  return align256(((size_t)n + M) * ATTR_PROJ * sizeof(float)) + align256(attribution_partial_floats(n, M) * sizeof(float)) +
+         align256((size_t)n * sizeof(float)) + 256;
+}
+
+extern "C" int lsd_branch_attribution(lsd_handle* h, const float* feats, int n, const float* background, int M, float* values_out,
+                                      float* phi_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return LSD_ERR_ARG;
+  if (!feats || !background || !values_out || !phi_out || !workspace)
+    return lsd_fail(h, LSD_ERR_ARG, "lsd_branch_attribution: null pointer argument");
+  if (!h->loaded) return lsd_fail(h, LSD_ERR_WEIGHTS, "lsd_branch_attribution: no weights loaded");
+  if (!attribution_extents_ok(n, M))
+    return lsd_fail(h, LSD_ERR_SHAPE, "lsd_branch_attribution: n = %d windows, M = %d background rows: expected n >= 0, 1 <= M <= %d and "
+                    "n*(15M+1) <= INT32_MAX", n, M, LSD_MAX_BACKGROUND);
+  const size_t need = lsd_branch_attribution_workspace_bytes(n, M);
+  if (need > workspace_bytes) return lsd_fail(h, LSD_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  if (n == 0) return LSD_OK;
+  ENTER_DEVICE(h);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  char* ws = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+  float* proj = reinterpret_cast<float*>(ws);
+  float* partial = reinterpret_cast<float*>(ws + align256(((size_t)n + M) * ATTR_PROJ * sizeof(float)));
+  float* v15 = partial + align256(attribution_partial_floats(n, M) * sizeof(float)) / sizeof(float);
+  lsd::HeadW hw;
+  auto cw = [&](const char* key) { return h->warena + h->convs.at(key).w_off; };
+  auto cb = [&](const char* key) { return h->warena + h->convs.at(key).shift_off; };
+  hw.w0 = cw("art.fuse0"); hw.b0 = cb("art.fuse0"); hw.w2 = cw("art.fuse2"); hw.b2 = cb("art.fuse2");
+  hw.wc = cw("head.fc0"); hw.bc = cb("head.fc0");
+  hw.lng = h->warena + h->vecs.at("head.ln.w"); hw.lnb = h->warena + h->vecs.at("head.ln.b");
+  hw.wo = h->warena + h->vecs.at("head.out.w"); hw.bo = h->warena + h->vecs.at("head.out.b");
+  launch_branch_attribution(feats, n, background, M, hw, proj, partial, v15, values_out, phi_out, h->num_sms, st);
+  CUDA_OK(h, cudaGetLastError());
+  return LSD_OK;
 }
 
 // ================================================================================================

@@ -140,7 +140,7 @@ int token_path_bf16_run(lsd_handle* h, int B, int T, int TA, const float* v_emb,
                         char* ws, size_t ws_bytes, cudaStream_t st);
 int score_batch_bf16(lsd_handle* h, const uint8_t* track, int n_frames, const int32_t* d_vstarts, const int32_t* d_astarts,
                      const float* mel_full, int Ta_full, int nb, int T, int H, int W, int F, int Ta, float* logits,
-                     char* ws, size_t ws_bytes, cudaStream_t st, int pipe_parity = -1);
+                     char* ws, size_t ws_bytes, cudaStream_t st, int pipe_parity = -1, float* feats_out = nullptr);
 int ensure_pipeline(lsd_handle* h);
 // shared-visual forward: K audio windows per video, visual front once (bf16_path.cu, VarTail)
 bool variants_shared_route(int T);

@@ -91,6 +91,16 @@ bool resize_extents_ok(int H, int W);
 void launch_retime_windows(const uint8_t* track, int n_frames, const int32_t* win_starts, const int32_t* tabs, int K, int r0, int nb,
                            int T, int H, int W, uint8_t* out, cudaStream_t s);
 size_t retime_tables_ints(int K, int T);
+// branch attribution (attribution.cu): feats (n, 448) window rows, bg (M, 448) background rows -> values (n, 16), phi (n, 4).
+// proj: (n + M) * ATTR_PROJ floats, P_sync | P_raw | P_delta | P_hf (256 each) | C (128) per row, window rows first; partial:
+// n * 15 * ceil(M / ATTR_CHUNK) floats; v15: n floats.  The weights are the fp32 arena pointers of launch_head.
+constexpr int ATTR_PROJ = 4 * 256 + 128;
+constexpr int ATTR_CHUNK = 2;                      // background rows per coalition tile (the chunking depends on M only)
+struct HeadW;
+void launch_branch_attribution(const float* feats, int n, const float* bg, int M, const HeadW& w, float* proj, float* partial,
+                               float* v15, float* values, float* phi, int num_sms, cudaStream_t s);
+size_t attribution_tail_smem_bytes();
+cudaError_t attribution_device_init();
 // mel_full (F, Ta_full) + per-window a_start -> (n, F, Ta) with repeat-last-column padding (predictor.py:525-552)
 void launch_gather_audio(const float* mel_full, int F, int Ta_full, const int32_t* a_starts, float* dst,
                          int n, int Ta, cudaStream_t s);

@@ -500,6 +500,11 @@ class Predictor:
         -> fp32 logits `(n_windows,)` on the device.  Windows are built on the GPU (`/255`, audio alignment).
         `audio_starts_from`: absolute start frames used for the audio alignment when `track_u8` is only a rank-local span
         of the full track and `starts` are relative to that span (sharded long videos)."""
+        return self._score_windows(track_u8, starts, mel_full, total_v_frames, chunk_a_size, audio_starts_from, False)[0]
+
+    def _score_windows(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                       chunk_a_size: int, audio_starts_from: Optional[Sequence[int]], with_feats: bool):
+        """`score_track_logits`, and with `with_feats` also the head's input rows (`lsd_score_branch_features`): (logits, feats)."""
         m = self.model
         dev = m._device()
         if track_u8.dtype != torch.uint8 or track_u8.dim() != 4 or track_u8.shape[3] != 3:
@@ -508,8 +513,9 @@ class Predictor:
             raise ValueError(f"mel_full must be (1, F, T_full), got {tuple(mel_full.shape)}")
         n = len(starts)
         logits = torch.empty(n, dtype=torch.float32, device=dev)
+        feats = torch.empty((n, _cabi.LSD_BRANCH_FEATURES), dtype=torch.float32, device=dev) if with_feats else None
         if n == 0:
-            return logits
+            return logits, feats
         track_u8 = track_u8.contiguous()
         mel_full = mel_full.to(torch.float32).contiguous()
         n_frames, H, W = int(track_u8.shape[0]), int(track_u8.shape[1]), int(track_u8.shape[2])
@@ -531,11 +537,117 @@ class Predictor:
                 if len(audio_starts_from) != n:
                     raise ValueError("audio_starts_from must have one entry per window")
                 ast = (C.c_int32 * n)(*[self._audio_start(int(v), Ta_full, int(total_v_frames), chunk_a_size) for v in audio_starts_from])
-            rc = L.lsd_score_windows(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, self.chunk_size, mel_full.data_ptr(),
-                                     F_, Ta_full, int(total_v_frames), chunk_a_size, prec, batch, logits.data_ptr(),
-                                     ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            if with_feats:
+                rc = L.lsd_score_branch_features(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, self.chunk_size,
+                                                 mel_full.data_ptr(), F_, Ta_full, int(total_v_frames), chunk_a_size, prec, batch,
+                                                 logits.data_ptr(), feats.data_ptr(), ws.data_ptr(), ws.numel(), stream)
+            else:
+                rc = L.lsd_score_windows(h.ptr, track_u8.data_ptr(), n_frames, H, W, st, ast, n, self.chunk_size, mel_full.data_ptr(),
+                                         F_, Ta_full, int(total_v_frames), chunk_a_size, prec, batch, logits.data_ptr(),
+                                         ws.data_ptr(), ws.numel(), stream)
             _cabi.check(h.ptr, rc)
-        return logits
+        return logits, feats
+
+    # ------------------------------------------------------------------ branch attribution (lsd_score_branch_features, lsd_branch_attribution)
+    BRANCHES = _agg.BRANCHES
+    #: windows of the track background: at most this many, spread evenly over the track
+    TRACK_BACKGROUND_MAX = 64
+
+    def score_track_branch_features(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                                    audio_starts_from: Optional[Sequence[int]] = None, chunk_a_size: int = 128):
+        """`score_track_logits` that also returns every window's head input row: `(logits (n,), feats (n, 448))` fp32 on the
+        device.  feats row i is [cls 256 | raw 64 | delta 64 | hf 64], what the artifact fusion MLP and the head read for window i;
+        the logits are bit for bit those of `score_track_logits`.  Both precisions."""
+        return self._score_windows(track_u8, starts, mel_full, total_v_frames, chunk_a_size, audio_starts_from, True)
+
+    @staticmethod
+    def track_background_index(n: int, max_rows: int = 64) -> List[int]:
+        """Windows of the track background of an n-window track: M = min(n, max_rows) of them, (arange(M) * n) // M."""
+        M = min(int(n), int(max_rows))
+        return [(k * int(n)) // M for k in range(M)]
+
+    def branch_attribution(self, feats: torch.Tensor, background: torch.Tensor):
+        """Exact Shapley values of the head's four inputs (`lsd_branch_attribution`).  `feats`: (n, 448) head input rows
+        (`score_track_branch_features`); `background`: (M, 448) rows, 1 <= M <= 256, on the same device, fp32.  Returns
+        `(values (n, 16), phi (n, 4))` fp32 on the device: values[i, S] = v_i(S), the mean over the background rows j of the head's
+        logit on the row that takes branch p (sync, raw, delta, hf = bit p of S) from window i when bit p is set and from row j
+        otherwise; values[i, 15] is window i's own logit.  phi[i, p] is branch p's Shapley value; the four sum to
+        values[i, 15] - values[i, 0]."""
+        want = self.model._device() if self.model is not None else self.device
+        for name, t in (("feats", feats), ("background", background)):
+            if not isinstance(t, torch.Tensor) or t.dim() != 2 or t.shape[1] != _cabi.LSD_BRANCH_FEATURES:
+                raise ValueError(f"{name} must be a ({'n' if name == 'feats' else 'M'}, {_cabi.LSD_BRANCH_FEATURES}) tensor, got "
+                                 f"{tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__}")
+            if t.dtype != torch.float32:
+                raise ValueError(f"{name} must be float32, got {t.dtype}")
+            if t.device != want:
+                raise ValueError(f"{name} is on {t.device}, the model on {want}")
+        M = int(background.shape[0])
+        if not 1 <= M <= _cabi.LSD_MAX_BACKGROUND:
+            raise ValueError(f"{M} background rows: expected 1 to {_cabi.LSD_MAX_BACKGROUND}")
+        n = int(feats.shape[0])
+        if n * (15 * M + 1) > 2 ** 31 - 1:
+            raise ValueError(f"{n} windows x {M} background rows: too many coalition rows for one call")
+        if want.type != "cuda" or self.model is None:
+            raise ValueError(f"branch attribution runs on a CUDA model, the predictor is on {want}")
+        m = self.model
+        dev = m._device()
+        values = torch.empty((n, 16), dtype=torch.float32, device=dev)
+        phi = torch.empty((n, _cabi.LSD_BRANCHES), dtype=torch.float32, device=dev)
+        if n == 0:
+            return values, phi
+        feats = feats.contiguous()
+        background = background.contiguous()
+        with m._lsd_lock:
+            h = m._ensure_handle(dev)
+            L = _cabi.lib()
+            need = L.lsd_branch_attribution_workspace_bytes(n, M)
+            if need == 0:
+                _cabi.check(h.ptr, _cabi.LSD_ERR_SHAPE)
+            ws = torch.empty(int(need), dtype=torch.uint8, device=dev)
+            rc = L.lsd_branch_attribution(h.ptr, feats.data_ptr(), n, background.data_ptr(), M, values.data_ptr(), phi.data_ptr(),
+                                          ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(h.ptr, rc)
+        return values, phi
+
+    def attribution_track(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
+                          background="track", confidence_threshold: float = 0.5,
+                          audio_starts_from: Optional[Sequence[int]] = None) -> Dict[str, Any]:
+        """Branch attribution of a track's windows: was a window called fake because lips and speech disagree (sync) or because
+        the pixels carry generator artifacts (raw, delta: the temporal-inconsistency detector; hf: the high-frequency detector)?
+        One `score_track_branch_features` call, then `branch_attribution` against `background`: "track" (the track's own windows,
+        `track_background_index`: what sets a window apart from the rest of the clip) or an (M, 448) tensor of feature rows, e.g.
+        those of windows known to be real ("reference").  Returns host arrays:
+          `branches`; `logits` (n,); `values` (n, 16); `phi` (n, 4); `base_logit` (n,) = values[:, 0], the background's expected
+          logit; `background` ("track" or "reference") and `background_size` (M);
+          the `aggregate.branch_attribution_summary` of phi and the calibrated P(real) at `confidence_threshold`, its timeline in
+          the frames of `window_starts`;
+          `window_starts`: the windows' first frames (those of `audio_starts_from` when given: absolute video frames).
+        It reports only: nothing here enters a verdict."""
+        n = len(starts)
+        if isinstance(background, str) and background != "track":
+            raise ValueError(f"background must be 'track' or an (M, {_cabi.LSD_BRANCH_FEATURES}) tensor, got {background!r}")
+        if isinstance(background, str) and n == 0:
+            raise ValueError("a track background needs at least one window")
+        logits, feats = self.score_track_branch_features(track_u8, starts, mel_full, total_v_frames, audio_starts_from=audio_starts_from)
+        if isinstance(background, str):
+            idx = torch.tensor(self.track_background_index(n, self.TRACK_BACKGROUND_MAX), dtype=torch.long, device=feats.device)
+            bg, kind = feats.index_select(0, idx), "track"
+        else:
+            bg, kind = background, "reference"
+        values, phi = self.branch_attribution(feats, bg)
+        lg = logits.cpu().numpy()
+        vals = values.cpu().numpy()
+        ph = phi.cpu().numpy()
+        probs = np.array([self._calibrate(float(x)) for x in lg.tolist()], dtype=np.float64)
+        window_starts = [int(s) for s in (audio_starts_from if audio_starts_from is not None else starts)]
+        res = {"branches": list(self.BRANCHES), "logits": lg, "values": vals, "phi": ph, "base_logit": vals[:, 0],
+               "background": kind, "background_size": int(bg.shape[0])}
+        res.update(_agg.branch_attribution_summary(ph, probs, confidence_threshold, self.confidence_smoothing, self.trim_ratio,
+                                                   starts=window_starts, T=self.chunk_size))
+        res["window_starts"] = window_starts
+        return res
 
     def score_track_offsets(self, track_u8: torch.Tensor, starts: Sequence[int], mel_full: torch.Tensor, total_v_frames: int,
                             offsets: Sequence[int], chunk_a_size: int = 128, audio_starts_from: Optional[Sequence[int]] = None):
